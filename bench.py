@@ -287,6 +287,8 @@ def run_cuda_arm(a):
     wall = time.perf_counter() - t0
     t_end = time.time()
     clocks = sampler.stop(t_end - wall, t_end) if rank == 0 else None
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(res, a.dump_outputs)
     # Per-kernel-class CUDA-event timing (the roofline's kernel time): the production path replays the SCF loop from ONE CUDA-graph launch
     # (while node, device-side condition), where host-side events cannot be recorded between the kernels; so the same sweep is run
     # `steps` more times, back to back with the timed ones, with set_option("profile", 1) - the host-driven loop with an event pair around
@@ -508,6 +510,34 @@ def run_cuda_arm(a):
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(res, out_dir):
+    """What the last timed sweep returned to its caller, atoms in input order (Z = 1..92), one float64 array per DIR/<name>.npy:
+    energies [atom][Etotal, Ekin, Ecoul, Eenuc, Exc]; n_steps [atom]; status [atom] (0 = converged); n_levels [atom][spin] (0 for the
+    second spin of an unpolarised atom).  The levels of all atoms are concatenated in (atom, spin) order, n_levels of them per block:
+    eigenvalues [level] and levels [level][n, l, occ, nodes] in (n, l) order, sorted_levels [level][n, l, occ, nodes, E] in eigenvalue
+    order.  A result with a non-finite value is an error: nothing is written and ValueError names the atoms."""
+    import numpy as np
+    n_levels = np.zeros((len(res), 2), np.float64)
+    eig, levels, sorted_levels = [], [], []
+    for i, r in enumerate(res):
+        for s, (chan, schan) in enumerate(zip(r.levels, r.sorted_levels)):
+            n_levels[i, s] = len(chan)
+            eig += [L.E for L in chan]
+            levels += [(L.n, L.l, L.occ, L.nodes) for L in chan]
+            sorted_levels += [(L.n, L.l, L.occ, L.nodes, L.E) for L in schan]
+    arrays = dict(energies=np.array([[r.Etotal, r.Ekin, r.Ecoul, r.Eenuc, r.Exc] for r in res], np.float64),
+                  n_steps=np.array([r.n_steps for r in res], np.float64), status=np.array([r.status for r in res], np.float64),
+                  n_levels=n_levels, eigenvalues=np.array(eig, np.float64), levels=np.array(levels, np.float64).reshape(-1, 4),
+                  sorted_levels=np.array(sorted_levels, np.float64).reshape(-1, 5))
+    bad = sorted({r.options.Z for r in res if not np.isfinite([r.Etotal, r.Ekin, r.Ecoul, r.Eenuc, r.Exc]
+                                                             + [L.E for ch in r.levels + r.sorted_levels for L in ch]).all()})
+    if bad:
+        raise ValueError(f"--dump-outputs: non-finite energies or eigenvalues in the results of Z = {bad}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), x)
 
 
 def poisson_record(prof, n_atoms, steps):
@@ -772,7 +802,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the parity block (worst deviation from the committed reference goldens per config)")
     ap.add_argument("--no-micro", action="store_true", help="skip the kernel micro-benchmarks (C5a Poisson V-cycle, C5b Numerov lanes)")
     ap.add_argument("--micro-densities", type=int, default=1024, help="densities of the C5a micro-benchmark (1024 = BASELINE.json; ~34 GiB)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one returned (per-atom energies, eigenvalues, level tables) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs records the CUDA arm's results; the reference arm has none to write")
     if a.impl == "reference":
         run_reference_arm(a)
     else:

@@ -52,6 +52,32 @@ def test_clock_sampler_selects_the_timed_region():
     assert c["samples"] == 2 and c["window"] == "warm-up + timed region"
 
 
+def test_dump_outputs_writes_what_the_caller_received(tmp_path):
+    """`bench.py --dump-outputs DIR`: the results of a solve_batch call as float64 .npy files of finite values, atoms in input order, the
+    levels of all atoms concatenated with their counts per (atom, spin)."""
+    import dftatom_b200 as D
+    li = D.Result(D.Options(3, 10, 10.0, 0.01, 0.5, 1), 0, 31, [[(1, 0, 1, 0, -1.8), (2, 0, 1, 1, -0.1)], [(1, 0, 1, 0, -1.7)]],
+                  [[(2, 0, 1, 1, -0.1), (1, 0, 1, 0, -1.8)], [(1, 0, 1, 0, -1.7)]], -7.3, 7.2, 4.0, -17.0, -1.5)
+    he = D.Result(D.Options(2, 10, 10.0, 0.01, 0.5, 0), 1, 100, [[(1, 0, 2, 0, -0.57)]], [[(1, 0, 2, 0, -0.57)]], -2.8, 2.7, 2.0, -6.6, -0.9)
+    bench.dump_outputs([li, he], str(tmp_path))
+    out = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert sorted(out) == ["eigenvalues", "energies", "levels", "n_levels", "n_steps", "sorted_levels", "status"]
+    assert all(x.dtype == np.float64 and np.isfinite(x).all() for x in out.values())
+    assert out["energies"].tolist() == [[-7.3, 7.2, 4.0, -17.0, -1.5], [-2.8, 2.7, 2.0, -6.6, -0.9]]
+    assert out["n_steps"].tolist() == [31, 100] and out["status"].tolist() == [0, 1]
+    assert out["n_levels"].tolist() == [[2, 1], [1, 0]]
+    assert out["eigenvalues"].tolist() == [-1.8, -0.1, -1.7, -0.57]
+    assert out["levels"].tolist() == [[1, 0, 1, 0], [2, 0, 1, 1], [1, 0, 1, 0], [1, 0, 2, 0]]
+    assert out["sorted_levels"][:2].tolist() == [[2, 0, 1, 1, -0.1], [1, 0, 1, 0, -1.8]] and out["sorted_levels"].shape == (4, 5)
+    assert sum(x.nbytes for x in out.values()) < 64 << 20
+    # a non-finite result is refused, and nothing is written
+    broken = D.Result(D.Options(5, 10, 10.0, 0.01, 0.5, 0), 1, 100, [[(1, 0, 2, 0, float("nan"))]], [[(1, 0, 2, 0, float("nan"))]],
+                      -24.0, 24.0, 10.0, -60.0, -3.0)
+    with pytest.raises(ValueError, match=r"Z = \[5\]"):
+        bench.dump_outputs([li, broken], str(tmp_path / "broken"))
+    assert not (tmp_path / "broken").exists()
+
+
 def test_reference_arm_prints_one_json_line():
     """`bench.py --impl reference`: the unmodified reference's CPU solver on the host cores, one JSON line with the arm's keys.
     (One bounded sample; skipped when neither oracle/_ref nor the oracle binary can be run.)"""
