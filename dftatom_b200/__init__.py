@@ -12,6 +12,7 @@ from .api import (  # noqa: F401
     DFTAtomError,
     Level,
     Options,
+    Radial,
     Result,
     Step,
     aufbau,
@@ -19,12 +20,13 @@ from .api import (  # noqa: F401
     lib_path,
     load_library,
     n_nodes,
+    orbital_count,
     partition,
     split_spin,
 )
 from .report import format_report, parse_report  # noqa: F401
 
 __all__ = [
-    "Context", "DFTAtom", "DFTAtomError", "Level", "Options", "Result", "Step", "aufbau", "split_spin", "n_nodes",
-    "lib_path", "load_library", "format_report", "parse_report", "estimate_cost", "partition",
+    "Context", "DFTAtom", "DFTAtomError", "Level", "Options", "Radial", "Result", "Step", "aufbau", "split_spin", "n_nodes",
+    "lib_path", "load_library", "format_report", "parse_report", "estimate_cost", "partition", "orbital_count",
 ]

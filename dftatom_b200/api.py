@@ -12,6 +12,7 @@ from .report import format_report
 MAX_LEVELS = 24
 MAX_STEPS_LDA = 100
 MAX_STEPS_LSDA = 150
+N_MOMENTS = 3            # <1/r>, <r>, <r^2> of every exported orbital (DFTATOM_N_MOMENTS)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -42,6 +43,12 @@ class _CResult(C.Structure):
     _fields_ = [("status", C.c_int), ("n_steps", C.c_int), ("n_spin", C.c_int), ("n_levels", C.c_int * 2),
                 ("levels", (_CLevel * MAX_LEVELS) * 2), ("sorted", (_CLevel * MAX_LEVELS) * 2),
                 ("Etotal", C.c_double), ("Ekin", C.c_double), ("Ecoul", C.c_double), ("Eenuc", C.c_double), ("Exc", C.c_double)]
+
+
+class _CRadial(C.Structure):
+    _fields_ = [("r", C.POINTER(C.c_double)), ("rho", C.POINTER(C.c_double)), ("v", C.POINTER(C.c_double)), ("v_hartree", C.POINTER(C.c_double)),
+                ("orbitals", C.POINTER(C.c_double)), ("orbital_rows", C.c_longlong), ("moments", C.POINTER(C.c_double)),
+                ("atom_moments", C.POINTER(C.c_double))]
 
 
 _RESULT_DTYPE = np.dtype(_CResult)      # numpy views of the C structs (same layout: built from the ctypes definitions)
@@ -85,6 +92,9 @@ def load_library():
     lib.dftatom_estimate_cost.restype = C.c_double
     lib.dftatom_partition.argtypes = [_ip, _ip, C.c_int, C.c_int, _ip]
     lib.dftatom_solve_batch.argtypes = [C.c_void_p, C.POINTER(_COptions), C.c_int, C.POINTER(_CResult), C.POINTER(_CStep), C.c_int]
+    lib.dftatom_solve_batch_radial.argtypes = [C.c_void_p, C.POINTER(_COptions), C.c_int, C.POINTER(_CResult), C.POINTER(_CStep), C.c_int,
+                                               C.POINTER(_CRadial)]
+    lib.dftatom_radial_moments.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp]
     lib.dftatom_last_timing.argtypes = [C.c_void_p, _dp, C.POINTER(C.c_longlong)]
     lib.dftatom_last_graph_iterations.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
     lib.dftatom_last_transfer.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
@@ -172,13 +182,14 @@ class Result:
     """One atom of a solve_batch call.  `levels` ([spin][level] in (n, l) order, eigenvalues of the last step) and `sorted_levels` (sorted by
     eigenvalue: the reference's last line) are lists of Level objects, built on first use from the (n, l, occ, nodes, E) records the library
     returned (a sweep that only reads the energies does not pay for 2000 Python objects)."""
-    __slots__ = ("options", "status", "n_steps", "Etotal", "Ekin", "Ecoul", "Eenuc", "Exc", "steps", "_lv", "_sl")
+    __slots__ = ("options", "status", "n_steps", "Etotal", "Ekin", "Ecoul", "Eenuc", "Exc", "steps", "_lv", "_sl", "radial")
 
     def __init__(self, options, status, n_steps, levels, sorted_levels, Etotal, Ekin, Ecoul, Eenuc, Exc, steps=None):
         self.options, self.status, self.n_steps = options, status, n_steps
         self._lv, self._sl = levels, sorted_levels            # [spin][k]: Level objects or raw tuples
         self.Etotal, self.Ekin, self.Ecoul, self.Eenuc, self.Exc = Etotal, Ekin, Ecoul, Eenuc, Exc
         self.steps = steps if steps is not None else []
+        self.radial = None                 # a Radial when solve_batch(..., radial=True)
 
     @staticmethod
     def _as_levels(chans):
@@ -214,6 +225,34 @@ class Result:
         conf = [[(L.n, L.l, L.occ) for L in chan] for chan in self.sorted_levels]
         return format_report(self.options.Z, self.options.method, st, self.finished, conf[0], conf[1] if len(conf) > 1 else None,
                              precision, n_alpha=len(self.levels[0]))
+
+
+@dataclass
+class Radial:
+    """The converged radial state of one atom (Context.solve_batch(..., radial=True); conventions: dftatom_solve_batch_radial in
+    include/dftatom_b200.h).  Arrays are views of one allocation per batch.
+
+    r: [N] grid nodes.  rho, V: [n_spin][N] density and Kohn-Sham potential per spin (LDA: one row, the total density).  V_H: [N]
+    Hartree potential U / r.  orbitals: one [n_levels][N] array of u_nl(r) = r R_nl(r) per spin, rows aligned with Result.levels.
+    moments: the same shape with N_MOMENTS columns: <1/r>, <r>, <r^2>.  n_electrons: integral of 4 pi r^2 rho.  r2: <r^2> of the
+    total density summed over the electrons."""
+    r: np.ndarray
+    rho: np.ndarray
+    V: np.ndarray
+    V_H: np.ndarray
+    orbitals: List[np.ndarray]
+    moments: List[np.ndarray]
+    n_electrons: float
+    r2: float
+
+
+def orbital_count(Z: int, method: int = 0) -> int:
+    """Orbital rows of one atom in the radial export: its levels (dftatom_aufbau), or alpha plus beta levels (dftatom_split_spin) for
+    LSDA (method 1 / 3)."""
+    if int(method) & 1:
+        a, b, _, _ = split_spin(Z)
+        return len(a) + len(b)
+    return len(aufbau(Z))
 
 
 def _levels_from_c(arr, n):
@@ -283,13 +322,30 @@ class Context:
         _check(self._lib.dftatom_set_option(self._h, key.encode(), float(value)))
 
     # ---- L2 ----
-    def solve_batch(self, options: Sequence[Options], keep_steps: bool = True) -> List[Result]:
+    def solve_batch(self, options: Sequence[Options], keep_steps: bool = True, radial: bool = False) -> List[Result]:
+        """One batch of independent atoms (dftatom_solve_batch).  radial=True: every Result also gets `radial` (a Radial: converged
+        density, potentials, orbitals and their moments, dftatom_solve_batch_radial)."""
         n = len(options)
         copts = (_COptions * n)(*[o._c() for o in options])
         cres = (_CResult * n)()
         stride = MAX_STEPS_LSDA if any(o.method for o in options) else MAX_STEPS_LDA
         csteps = (_CStep * (n * stride))() if keep_steps else None
-        _check(self._lib.dftatom_solve_batch(self._h, copts, n, cres, csteps, stride if keep_steps else 0))
+        if radial and n:
+            N = n_nodes(options[0].MultigridLevels)
+            rows = sum(orbital_count(o.Z, o.method) for o in options)
+            buf = np.zeros(N + n * 5 * N + n * 2 + rows * (N + N_MOMENTS))      # r | rho | V | V_H | atom moments | orbitals | moments
+            r = buf[:N]
+            rho = buf[N:N + 2 * n * N].reshape(n, 2, N)
+            V = buf[N + 2 * n * N:N + 4 * n * N].reshape(n, 2, N)
+            VH = buf[N + 4 * n * N:N + 5 * n * N].reshape(n, N)
+            am = buf[N + 5 * n * N:N + 5 * n * N + 2 * n].reshape(n, 2)
+            q = N + 5 * n * N + 2 * n
+            orb = buf[q:q + rows * N].reshape(rows, N)
+            mom = buf[q + rows * N:].reshape(rows, N_MOMENTS)
+            crad = _CRadial(_d(r), _d(rho), _d(V), _d(VH), _d(orb), rows, _d(mom), _d(am))
+            _check(self._lib.dftatom_solve_batch_radial(self._h, copts, n, cres, csteps, stride if keep_steps else 0, C.byref(crad)))
+        else:
+            _check(self._lib.dftatom_solve_batch(self._h, copts, n, cres, csteps, stride if keep_steps else 0))
         # host structs -> Python objects in bulk (numpy structured views of the ctypes arrays: one pass in C instead of a ctypes
         # attribute access per field)
         ra = np.frombuffer(cres, dtype=_RESULT_DTYPE, count=n)
@@ -318,6 +374,16 @@ class Context:
                     r_ = rest[k]
                     steps.append(Step([E[k][s][:nl[s]] for s in range(n_spin)], r_[0], r_[1], r_[2], r_[3], r_[4], bool(r_[5]), bool(r_[6])))
             out.append(Result(options[a], status, n_steps, lv, sl, etot, ekin, ecoul, eenuc, exc, steps))
+        if radial and n:
+            row = 0
+            for a, res in enumerate(out):
+                ns = 2 if options[a].method & 1 else 1
+                orbs, moms = [], []
+                for s in range(ns):
+                    k = n_levels[a][s]
+                    orbs.append(orb[row:row + k]); moms.append(mom[row:row + k])
+                    row += k
+                res.radial = Radial(r, rho[a, :ns], V[a, :ns], VH[a], orbs, moms, float(am[a, 0]), float(am[a, 1]))
         return out
 
     def last_timing(self):
@@ -420,6 +486,14 @@ class Context:
         vexc = np.zeros(n); edif = np.zeros(n)
         _check(self._lib.dftatom_xc_lda(self._h, int(functional), n, _d(r), _d(vexc), _d(edif)))
         return vexc, edif
+
+    def radial_moments(self, levels, delta, max_r, u):
+        """[n_rows][N_MOMENTS] moments <1/r>, <r>, <r^2> of the rows of u (used as given) on the grid (levels, delta, max_r; delta 0:
+        uniform), with the quadrature of the radial export (dftatom_radial_moments)."""
+        u = _f64(np.atleast_2d(u))
+        out = np.zeros((u.shape[0], N_MOMENTS))
+        _check(self._lib.dftatom_radial_moments(self._h, int(levels), float(delta), float(max_r), _d(u), u.shape[0], _d(out)))
+        return out
 
     def integrate(self, rule, step, v):
         """Integral.h quadratures by rule: 0 Trapezoid, 1 SimpsonOneThird, 2 Simpson38, 3 Boole, 4 Romberg; one result per row of v."""

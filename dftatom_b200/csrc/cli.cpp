@@ -4,17 +4,23 @@
 // -> DFTAtom.cpp:358-490 / :857-1021).  All computation goes through the C ABI of include/dftatom_b200.h.
 //
 //   dftatom [--Z 18 | --Z 1-92 | --Z 21,22,57] [--levels 14] [--delta 0.0005] [--mixing 0.5] [--rmax 25]
-//           [--method 0|1|lda|lsda] [--precision 6] [--json] [--quiet-steps] [--device 0] [--gpus N] [--ini DFTAtom.ini]
+//           [--method 0|1|lda|lsda] [--precision 6] [--json] [--quiet-steps] [--device 0] [--gpus N] [--ini DFTAtom.ini] [--radial DIR]
 // --json: one record per atom (final energies, levels, and - unless --quiet-steps - every step at 17 digits)
 // --gpus N: the batch is sharded over N GPUs, ONE PROCESS PER GPU (fork + exec of this binary with --device r and its share of the
 //           atoms, longest-processing-time-first on dftatom_estimate_cost), no collective; the parent gathers the children's output
 //           through pipes and prints it in the order of --Z, so the result is byte-identical to the 1-GPU run.
+// --radial DIR: the converged radial state of every atom as a text table DIR/<index>_Z<Z>.tsv (index = position in --Z), one row per
+//           grid node at 17 digits: r, rho per spin, V per spin, V_H, u(r) of every orbital (dftatom_solve_batch_radial).  With --gpus
+//           every shard writes the files of its own atoms, named by their position in the whole --Z list.
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
 #include <string>
 #include <vector>
+#include <cerrno>
+#include <sys/stat.h>
 #include <sys/types.h>
 #include <sys/wait.h>
 #include <unistd.h>
@@ -90,7 +96,9 @@ static int run_sharded(const char* self, const std::vector<int>& zs, int method,
             // shards on one GPU
             int dev = r;
             if (const char* map = std::getenv("DFTATOM_SHARD_DEVICES")) { const std::vector<int> ids = parse_z(map); if (!ids.empty()) dev = ids[r % ids.size()]; }
-            std::vector<std::string> args = { self, "--framed", "--device", std::to_string(dev), "--Z", zlist };
+            std::string ilist;
+            for (size_t q = 0; q < c.atoms.size(); ++q) ilist += (q ? "," : "") + std::to_string(c.atoms[q]);
+            std::vector<std::string> args = { self, "--framed", "--device", std::to_string(dev), "--Z", zlist, "--atom-index", ilist };
             args.insert(args.end(), pass.begin(), pass.end());
             std::vector<char*> av;
             for (auto& a : args) av.push_back(const_cast<char*>(a.c_str()));
@@ -133,10 +141,44 @@ static int run_sharded(const char* self, const std::vector<int>& zs, int method,
     return 0;
 }
 
+// --radial: one table per atom, columns r | rho per spin | V per spin | V_H | u of every orbital (headed like the report: "2p"; LSDA "alpha 2p")
+static int write_radial(const std::string& dir, int index, const dftatom_options& o, const dftatom_result& R, int N, const double* r,
+                        const double* rho, const double* v, const double* vh, const double* orb)
+{
+    const std::string path = dir + "/" + std::to_string(index) + "_Z" + std::to_string(o.Z) + ".tsv";
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) { std::perror(path.c_str()); return 1; }
+    const int ns = R.n_spin;
+    static const char* const kSpin[2] = { "alpha", "beta" };
+    std::fprintf(f, "# r");
+    for (const char* q : { "rho", "V" })
+        for (int s = 0; s < ns; ++s) std::fprintf(f, ns == 2 ? "\t%s %s" : "\t%s", q, kSpin[s]);
+    std::fprintf(f, "\tV_H");
+    int n_orb = 0;
+    for (int s = 0; s < ns; ++s)
+        for (int k = 0; k < R.n_levels[s]; ++k, ++n_orb) {
+            if (ns == 2) std::fprintf(f, "\t%s %d%c", kSpin[s], R.levels[s][k].n, kOrb[R.levels[s][k].l]);
+            else std::fprintf(f, "\t%d%c", R.levels[s][k].n, kOrb[R.levels[s][k].l]);
+        }
+    std::fprintf(f, "\n");
+    for (int i = 0; i < N; ++i) {
+        std::fprintf(f, "%.17g", r[i]);
+        for (int s = 0; s < ns; ++s) std::fprintf(f, "\t%.17g", rho[(size_t)s * N + i]);
+        for (int s = 0; s < ns; ++s) std::fprintf(f, "\t%.17g", v[(size_t)s * N + i]);
+        std::fprintf(f, "\t%.17g", vh[i]);
+        for (int k = 0; k < n_orb; ++k) std::fprintf(f, "\t%.17g", orb[(size_t)k * N + i]);
+        std::fprintf(f, "\n");
+    }
+    const bool bad = std::ferror(f) != 0;
+    if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
+    return 0;
+}
+
 int main(int argc, char** argv)
 {
     dftatom_options base = { 36, 12, 10.0, 0.001, 0.5, 0 };     // Options.cpp:6
-    std::vector<int> zs;
+    std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
+    std::string radial_dir;
     int precision = 6, device = 0, gpus = 1;
     bool json = false, quiet = false, framed = false;      // framed: child of --gpus (one frame per atom on stdout)
     std::vector<std::string> passthrough;                   // flags a --gpus parent hands to its children unchanged
@@ -147,6 +189,8 @@ int main(int argc, char** argv)
         if (a == "--Z") zs = parse_z(next());
         else if (a == "--gpus") gpus = std::atoi(next());
         else if (a == "--framed") framed = true;
+        else if (a == "--atom-index") atom_index = parse_z(next());
+        else if (a == "--radial") radial_dir = next();
         else if (a == "--levels") base.levels = std::atoi(next());
         else if (a == "--delta") base.delta = std::atof(next());
         else if (a == "--mixing" || a == "--alpha") base.mixing = std::atof(next());
@@ -163,12 +207,15 @@ int main(int argc, char** argv)
         else if (a == "--quiet-steps") quiet = true;
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
-                        "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file]\n");
+                        "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR]\n"
+                        "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
-        if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
+        if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
     }
     if (zs.empty()) zs.push_back(base.Z);
+    if (!atom_index.empty() && atom_index.size() != zs.size()) { std::fprintf(stderr, "dftatom: --atom-index needs one index per --Z entry\n"); return 2; }
+    if (!radial_dir.empty() && mkdir(radial_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(radial_dir.c_str()); return 1; }
     if (gpus > 1) {
         char self[4096];
         const ssize_t len = readlink("/proc/self/exe", self, sizeof self - 1);
@@ -185,13 +232,32 @@ int main(int argc, char** argv)
     const int stride = DFTATOM_MAX_STEPS_LSDA;
     std::vector<dftatom_result> res(n);
     std::vector<dftatom_step> steps((size_t)n * stride);
-    if (dftatom_solve_batch(ctx, opts.data(), n, res.data(), steps.data(), stride) != DFTATOM_OK) {
+    // --radial: arrays of the whole batch, rows of the orbitals in call order (dftatom_radial)
+    const int N = dftatom_n_nodes(base.levels);
+    std::vector<long long> row0(n + 1, 0);
+    for (int k = 0; k < n && !radial_dir.empty(); ++k) {
+        dftatom_level la[DFTATOM_MAX_LEVELS], lb[DFTATOM_MAX_LEVELS];
+        int na = 0, nb = 0, ea = 0, eb = 0;
+        if (opts[k].method & 1) dftatom_split_spin(opts[k].Z, la, &na, lb, &nb, &ea, &eb);
+        else na = std::max(0, dftatom_aufbau(opts[k].Z, la, DFTATOM_MAX_LEVELS));
+        row0[k + 1] = row0[k] + na + nb;
+    }
+    std::vector<double> r_grid, rho, vks, vh, orb;
+    dftatom_radial rad = {};
+    if (!radial_dir.empty()) {
+        r_grid.resize(N); rho.resize((size_t)n * 2 * N); vks.resize((size_t)n * 2 * N); vh.resize((size_t)n * N); orb.resize((size_t)row0[n] * N);
+        rad.r = r_grid.data(); rad.rho = rho.data(); rad.v = vks.data(); rad.v_hartree = vh.data(); rad.orbitals = orb.data(); rad.orbital_rows = row0[n];
+    }
+    if (dftatom_solve_batch_radial(ctx, opts.data(), n, res.data(), steps.data(), stride, radial_dir.empty() ? nullptr : &rad) != DFTATOM_OK) {
         std::fprintf(stderr, "dftatom: %s\n", dftatom_last_error());
         dftatom_destroy(ctx);
         return 1;
     }
     double ms = 0; long long launches = 0;
     dftatom_last_timing(ctx, &ms, &launches);
+    for (int a = 0; a < n && !radial_dir.empty(); ++a)
+        if (write_radial(radial_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a], N, r_grid.data(), &rho[(size_t)a * 2 * N], &vks[(size_t)a * 2 * N],
+                         &vh[(size_t)a * N], &orb[(size_t)row0[a] * N])) { dftatom_destroy(ctx); return 1; }
 
     if (json && !framed) std::printf("[");
     for (int a = 0; a < n; ++a) {

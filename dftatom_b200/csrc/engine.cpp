@@ -140,6 +140,7 @@ struct dftatom_ctx {
     // reusable buffers
     DevBuf atoms, astate, orbs, ss, rho, rhot, vpot, atab, psi, match_pt, inv_norm, epart, eticket, team_bar, phi, src, u0, ubuf, zbc, tab_of, steps, n_active;
     DevBuf scratch[8];
+    DevBuf radial, radial_part, radial_ticket;     // export of the radial state (dftatom_solve_batch_radial): staging, partial sums, tickets
     int* h_active = nullptr;       // pinned
     char* h_up = nullptr; size_t h_up_cap = 0, h_up_used = 0;      // pinned staging of the descriptor uploads of one solve (reset at its start)
     // timing of the last solve
@@ -335,6 +336,7 @@ void dftatom_destroy(dftatom_ctx* c)
                       &c->phi, &c->src, &c->u0, &c->ubuf, &c->zbc, &c->tab_of, &c->steps, &c->n_active };
     for (DevBuf* b : all) b->release();
     for (DevBuf& b : c->scratch) b.release();
+    c->radial.release(); c->radial_part.release(); c->radial_ticket.release();
     c->stream_G.release(); c->stream_src0.release(); c->stream_scratch.release(); c->exact_work.release(); c->last_steps.release(); c->rho_prev.release(); c->d_src.release(); c->d_u.release();
     if (c->h_active) cudaFreeHost(c->h_active);
     if (c->h_up) cudaFreeHost(c->h_up);
@@ -461,9 +463,61 @@ int dftatom_measure_fp64_peak(dftatom_ctx* c, double* tflops)
     return 0;
 }
 
+// Where the radial arrays of the atoms of one group go in the caller's arrays: per local atom its index in the caller's batch and its
+// first orbital row (a group of a stream-group split holds a permuted subset of the batch)
+struct RadialDest {
+    const dftatom_radial* rad;
+    const int* atom;
+    const long long* row;
+    bool copy_r;               // this group copies the grid nodes (once per call)
+};
+
+// The radial state of the group's atoms: packed into the staging buffer by radial.cu, then one copy per contiguous block of the
+// caller's arrays (a run of atoms whose destinations are consecutive).  Runs after the SCF loop; neither timed nor counted as SCF launches.
+static int export_radial(dftatom_ctx* c, const GridDev& g, const ScfBuffers& b, const std::vector<AtomDev>& atoms, const RadialDest& rd)
+{
+    const dftatom_radial& R = *rd.rad;
+    const int n_atoms = b.n_atoms, n_orbs = b.n_orbs;
+    const size_t N = (size_t)g.N;
+    cudaStream_t st = c->stream;
+    const bool fields = R.rho || R.v || R.v_hartree || R.atom_moments, orbitals = R.orbitals || R.moments;
+    const size_t o_rho = 0, o_v = o_rho + (size_t)n_atoms * 2 * N, o_vh = o_v + (size_t)n_atoms * 2 * N, o_am = o_vh + (size_t)n_atoms * N;
+    const size_t o_u = o_am + (size_t)n_atoms * 2, o_mom = o_u + (size_t)n_orbs * N, total = o_mom + (size_t)n_orbs * DFTATOM_N_MOMENTS;
+    const int rows = std::max(n_atoms, n_orbs);
+    int rc;
+    if ((rc = c->radial.ensure(sizeof(double) * total)) || (rc = c->radial_part.ensure(sizeof(double) * (size_t)radial_part_doubles(g.N, rows)))
+        || (rc = c->radial_ticket.ensure(sizeof(int) * (size_t)rows))) return rc;
+    double* sb = c->radial.as<double>();
+    DFT_CHECK(cudaMemsetAsync(c->radial_ticket.p, 0, sizeof(int) * (size_t)rows, st));
+    if (fields) launch_radial_fields(g, b, sb + o_rho, sb + o_v, sb + o_vh, sb + o_am, c->radial_part.as<double>(), c->radial_ticket.as<int>(), st);
+    if (orbitals) launch_radial_orbitals(g, b.psi, b.inv_norm, 1, n_orbs, sb + o_u, sb + o_mom, c->radial_part.as<double>(), c->radial_ticket.as<int>(), st);
+    long long bytes = 0;
+    auto copy = [&](double* dst, const double* src, size_t n) -> int {
+        DFT_CHECK(cudaMemcpyAsync(dst, src, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+        bytes += (long long)(sizeof(double) * n);
+        return 0;
+    };
+    if (rd.copy_r && R.r && (rc = copy(R.r, g.r, N))) return rc;
+    for (int a0 = 0, a1; a0 < n_atoms; a0 = a1) {
+        int n_rows = atoms[a0].orb_count[0] + atoms[a0].orb_count[1];
+        for (a1 = a0 + 1; a1 < n_atoms && rd.atom[a1] == rd.atom[a1 - 1] + 1; ++a1) n_rows += atoms[a1].orb_count[0] + atoms[a1].orb_count[1];
+        const size_t na = (size_t)(a1 - a0), d = (size_t)rd.atom[a0], o0 = (size_t)atoms[a0].orb_begin[0], r0 = (size_t)rd.row[a0];
+        if (R.rho && (rc = copy(R.rho + d * 2 * N, sb + o_rho + a0 * 2 * N, na * 2 * N))) return rc;
+        if (R.v && (rc = copy(R.v + d * 2 * N, sb + o_v + a0 * 2 * N, na * 2 * N))) return rc;
+        if (R.v_hartree && (rc = copy(R.v_hartree + d * N, sb + o_vh + a0 * N, na * N))) return rc;
+        if (R.atom_moments && (rc = copy(R.atom_moments + d * 2, sb + o_am + a0 * 2, na * 2))) return rc;
+        if (R.orbitals && (rc = copy(R.orbitals + r0 * N, sb + o_u + o0 * N, (size_t)n_rows * N))) return rc;
+        if (R.moments && (rc = copy(R.moments + r0 * DFTATOM_N_MOMENTS, sb + o_mom + o0 * DFTATOM_N_MOMENTS, (size_t)n_rows * DFTATOM_N_MOMENTS))) return rc;
+    }
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
+    c->last_d2h_bytes += bytes;
+    return 0;
+}
+
 // one group of atoms: its whole SCF, enqueued on the context's stream
 static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
-                       int steps_stride)
+                       int steps_stride, const RadialDest* rd = nullptr)
 {
     if (!c || !opts || !out || n_atoms <= 0) { set_error("bad argument"); return DFTATOM_E_ARG; }
     const bool host_dbg = getenv("DFTATOM_DEBUG_HOST") != nullptr;      // development aid: wall-clock of the host-side stages
@@ -948,6 +1002,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
         }
     }
     (void)steps_enqueued;
+    if (rd && (rc = export_radial(c, g, b, atoms, *rd))) return rc;
     th4 = now();
     if (host_dbg) fprintf(stderr, "solve_group host stages: setup+uploads %.3f ms | cold steps + graph build %.3f ms | device loop %.3f ms | results %.3f ms | device time %.3f ms\n",
                           th1 - th0, (th2 > 0. ? th2 : th1) - th1, th3 - (th2 > 0. ? th2 : th1), th4 - th3, c->last_ms);
@@ -961,9 +1016,38 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
 int dftatom_solve_batch(dftatom_ctx* c, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
                         int steps_stride)
 {
+    return dftatom_solve_batch_radial(c, opts, n_atoms, out, steps, steps_stride, nullptr);
+}
+
+int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
+                               int steps_stride, const dftatom_radial* radial)
+{
     if (!c || !opts || !out || n_atoms <= 0) { set_error("bad argument"); return DFTATOM_E_ARG; }
-    if (c->stream_groups < 2 || n_atoms < 32) return solve_group(c, opts, n_atoms, out, steps, steps_stride);
-    if (opts[0].levels > 14) return solve_group(c, opts, n_atoms, out, steps, steps_stride);      // (large grids: one group - the stream-mode Poisson solver wants all densities in one launch)
+    // radial export: the first orbital row of every atom in the caller's arrays, and the capacity check before anything is solved
+    std::vector<int> dest_atom;
+    std::vector<long long> dest_row;
+    if (radial) {
+        long long rows = 0;
+        for (int a = 0; a < n_atoms; ++a) {
+            int rc = validate(opts[a]);
+            if (rc) return rc;
+            dftatom_level la[DFTATOM_MAX_LEVELS], lb[DFTATOM_MAX_LEVELS];
+            int na = 0, nb = 0, ea = 0, eb = 0;
+            if (opts[a].method & 1) { rc = split_spin(opts[a].Z, la, &na, lb, &nb, &ea, &eb); if (rc) return rc; }
+            else { na = aufbau(opts[a].Z, la, DFTATOM_MAX_LEVELS); if (na < 0) return na; }
+            dest_atom.push_back(a);
+            dest_row.push_back(rows);
+            rows += na + nb;
+        }
+        if ((radial->orbitals || radial->moments) && radial->orbital_rows < rows) {
+            set_error("dftatom_radial.orbital_rows is " + std::to_string(radial->orbital_rows) + ", the batch has " + std::to_string(rows) + " orbitals");
+            return DFTATOM_E_ARG;
+        }
+    }
+    const RadialDest rd_all{ radial, dest_atom.data(), dest_row.data(), true };
+    const RadialDest* rd = radial ? &rd_all : nullptr;
+    if (c->stream_groups < 2 || n_atoms < 32) return solve_group(c, opts, n_atoms, out, steps, steps_stride, rd);
+    if (opts[0].levels > 14) return solve_group(c, opts, n_atoms, out, steps, steps_stride, rd);      // (large grids: one group - the stream-mode Poisson solver wants all densities in one launch)
     for (int a = 0; a < n_atoms; ++a) {
         int rc = validate(opts[a]);
         if (rc) return rc;
@@ -995,15 +1079,24 @@ int dftatom_solve_batch(dftatom_ctx* c, const dftatom_options* opts, int n_atoms
         gout[gI].resize(idx[gI].size());
         if (steps) gsteps[gI].resize(idx[gI].size() * (size_t)steps_stride);
     }
+    // radial export: every group scatters its atoms' arrays straight into the caller's, at their indices in the batch
+    std::vector<std::vector<int>> gatom(G);
+    std::vector<std::vector<long long>> grow(G);
+    std::vector<RadialDest> grd(G);
+    for (int gI = 0; gI < G && radial; ++gI) {
+        for (int a : idx[gI]) { gatom[gI].push_back(a); grow[gI].push_back(dest_row[a]); }
+        grd[gI] = RadialDest{ radial, gatom[gI].data(), grow[gI].data(), gI == 0 };
+    }
     std::vector<int> rcs(G, 0);
     std::vector<std::string> errs(G);
     std::vector<std::thread> th;
     for (int gI = 1; gI < G; ++gI)
         th.emplace_back([&, gI]() {
-            rcs[gI] = solve_group(ctxs[gI], gopts[gI].data(), (int)gopts[gI].size(), gout[gI].data(), steps ? gsteps[gI].data() : nullptr, steps_stride);
+            rcs[gI] = solve_group(ctxs[gI], gopts[gI].data(), (int)gopts[gI].size(), gout[gI].data(), steps ? gsteps[gI].data() : nullptr, steps_stride,
+                                  radial ? &grd[gI] : nullptr);
             if (rcs[gI]) errs[gI] = g_err;
         });
-    rcs[0] = solve_group(c, gopts[0].data(), (int)gopts[0].size(), gout[0].data(), steps ? gsteps[0].data() : nullptr, steps_stride);
+    rcs[0] = solve_group(c, gopts[0].data(), (int)gopts[0].size(), gout[0].data(), steps ? gsteps[0].data() : nullptr, steps_stride, radial ? &grd[0] : nullptr);
     for (auto& t : th) t.join();
     if (rcs[0]) return rcs[0];
     for (int gI = 1; gI < G; ++gI) if (rcs[gI]) { set_error(errs[gI]); return rcs[gI]; }
@@ -1425,6 +1518,27 @@ int dftatom_integrate(dftatom_ctx* c, int rule, double step, const double* v, in
     DFT_CHECK(cudaMemcpyAsync(d.p, v, sizeof(double) * (size_t)n * n_rows, cudaMemcpyHostToDevice, st));
     launch_integrate(rule, step, d.as<double>(), n, n_rows, o.as<double>(), st);
     DFT_CHECK(cudaMemcpyAsync(out, o.p, sizeof(double) * n_rows, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int dftatom_radial_moments(dftatom_ctx* c, int levels, double delta, double max_r, const double* u, int n_rows, double* moments)
+{
+    if (!c || !u || !moments || n_rows <= 0) return DFTATOM_E_ARG;
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp = nullptr;
+    int rc = get_grid(c, levels, delta, max_r, &gp);
+    if (rc) return rc;
+    const GridDev g = *gp;
+    cudaStream_t st = c->stream;
+    DevBuf& d = c->scratch[0]; DevBuf& o = c->scratch[1]; DevBuf& p = c->scratch[2]; DevBuf& t = c->scratch[3];
+    if ((rc = d.ensure(sizeof(double) * (size_t)g.N * n_rows)) || (rc = o.ensure(sizeof(double) * DFTATOM_N_MOMENTS * (size_t)n_rows))
+        || (rc = p.ensure(sizeof(double) * (size_t)radial_part_doubles(g.N, n_rows))) || (rc = t.ensure(sizeof(int) * (size_t)n_rows))) return rc;
+    DFT_CHECK(cudaMemcpyAsync(d.p, u, sizeof(double) * (size_t)g.N * n_rows, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemsetAsync(t.p, 0, sizeof(int) * (size_t)n_rows, st));
+    launch_radial_orbitals(g, d.as<double>(), nullptr, 0, n_rows, nullptr, o.as<double>(), p.as<double>(), t.as<int>(), st);
+    DFT_CHECK(cudaMemcpyAsync(moments, o.p, sizeof(double) * DFTATOM_N_MOMENTS * (size_t)n_rows, cudaMemcpyDeviceToHost, st));
     DFT_CHECK(cudaStreamSynchronize(st));
     DFT_CHECK(cudaGetLastError());
     return 0;

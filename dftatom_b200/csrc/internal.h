@@ -338,6 +338,13 @@ void launch_orbital_norms(const GridDev& g, const ScfBuffers& b, cudaStream_t st
 void launch_density_update(const GridDev& g, const ScfBuffers& b, cudaStream_t st);
 void launch_potential_energy(const GridDev& g, const PoissonLevels& lv, const ScfBuffers& b, int first, cudaStream_t st);
 
+// export of the radial state (radial.cu): part / ticket: radial_part_doubles(N, rows) doubles / rows ints (tickets zero before the launch)
+long long radial_part_doubles(int N, int n_rows);
+void launch_radial_orbitals(const GridDev& g, const double* src, const double* inv_norm, int from_scf, int n_rows, double* u_out, double* moments,
+                            double* part, int* ticket, cudaStream_t st);
+void launch_radial_fields(const GridDev& g, const ScfBuffers& b, double* rho_out, double* v_out, double* vh_out, double* atom_moments,
+                          double* part, int* ticket, cudaStream_t st);
+
 // host rules (aufbau.cpp)
 int aufbau(int Z, dftatom_level* out, int max_out);
 int split_spin(int Z, dftatom_level* a, int* na, dftatom_level* b, int* nb, int* ea, int* eb);

@@ -196,6 +196,50 @@ int dftatom_partition(const int* Z, const int* method, int n_atoms, int n_ranks,
  * All atoms of one call must share (levels, delta, max_r); Z, mixing, method may differ. */
 int dftatom_solve_batch(dftatom_ctx* ctx, const dftatom_options* opts, int n_atoms, dftatom_result* out,
                         dftatom_step* steps, int steps_stride);
+
+/* ---- L2 with the converged radial state ----
+ * dftatom_solve_batch_radial = dftatom_solve_batch plus, when `radial` is not NULL, the radial arrays of every atom copied into the
+ * caller's HOST arrays below (dftatom_solve_batch is this call with radial == NULL).  Every pointer may be NULL: that array is not
+ * exported.  N = dftatom_n_nodes(levels); atoms are indexed in call order.
+ *
+ * What the arrays hold: the state of the atom's LAST SCF step, in the reference's loop order (DFTAtom.cpp:396-481 / :908-1006) - the
+ * orbitals were solved in the potential of the step before, `rho` is the mixed density of the last step, and `v` / `v_hartree` were
+ * computed from that rho.  These are the arrays the reference holds when its loop ends (the oracle's orc_scf_ex exports the same).  An
+ * atom that stopped keeps them frozen while the rest of the batch iterates (every SCF kernel returns at once for a finished atom), so
+ * they do not depend on what else is in the batch.
+ *
+ * Orbitals: u_nl(r) = r R_nl(r), the u whose square the density accumulates (u_i = y_i e^{i delta/2} / sqrt(integral of u^2 dr) on the
+ * logarithmic grid, DFTAtom.cpp:36-56; y_i / sqrt(...) on the uniform grid), normalised so that sum_i wjac_i u_i^2 = 1 with the Simpson38
+ * weights times the jacobian that the energies use (Integral.h:50-73 x DFTAtom.cpp:47,442).  The sign is fixed so that u > 0 at the
+ * first node away from the nucleus (u ~ r^{l+1}).  Node 0 (r = 0) holds 0 in every exported array (the SCF arrays hold 0 there).  The
+ * last node holds the orbital's value and is part of its normalisation; the density, like the reference's (DFTAtom.cpp:558-559), sums
+ * occ u^2 / (4 pi r^2) over nodes 1 .. N-2 only.
+ * Rows: atoms in call order, then spin (alpha, beta), then the (n, l) order of dftatom_result.levels; an atom has as many rows as
+ * dftatom_aufbau (LDA) or dftatom_split_spin (n_alpha + n_beta levels, LSDA) gives it.  An `orbital_rows` smaller than the batch needs
+ * (when `orbitals` or `moments` is given) returns DFTATOM_E_ARG before anything is solved.
+ * Moments: sum_i wjac_i u_i^2 f(r_i) for f = 1/r (node 0 left out), r, r^2 - <1/r>, <r>, <r^2> of the normalised orbital.
+ * atom_moments: sum_i wjac_i 4 pi r_i^2 rho_i (the electron count) and sum_i wjac_i 4 pi r_i^4 rho_i (<r^2> summed over the electrons),
+ * rho = the total density.
+ * The export runs after the SCF loop: its kernels and copies are not part of dftatom_last_timing; its bytes are part of the d2h count of
+ * dftatom_last_transfer. */
+#define DFTATOM_N_MOMENTS 3            /* <1/r>, <r>, <r^2> */
+typedef struct {                       /* HOST pointers; any may be NULL (not exported) */
+    double* r;                         /* [N] grid nodes r_i */
+    double* rho;                       /* [n_atoms][2][N] density per spin (LDA: row 0 = total density, row 1 = 0) */
+    double* v;                         /* [n_atoms][2][N] Kohn-Sham potential per spin (LDA: row 1 = 0) */
+    double* v_hartree;                 /* [n_atoms][N] V_H = U / r */
+    double* orbitals;                  /* [orbital_rows][N] u_nl(r), rows as described above */
+    long long orbital_rows;            /* capacity of `orbitals` / `moments` in rows */
+    double* moments;                   /* [orbital_rows][DFTATOM_N_MOMENTS] */
+    double* atom_moments;              /* [n_atoms][2]: electron count, <r^2> of the total density */
+} dftatom_radial;
+int dftatom_solve_batch_radial(dftatom_ctx* ctx, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
+                               int steps_stride, const dftatom_radial* radial);
+/* The moment reduction of the export on caller-supplied orbitals u[n_rows][N] (HOST) of the grid (levels, delta, max_r; delta = 0: the
+ * uniform grid): moments[n_rows][DFTATOM_N_MOMENTS] = sum_i wjac_i u_i^2 f(r_i), f = 1/r (node 0 left out), r, r^2.  The rows are used
+ * as given (no normalisation, no sign). */
+int dftatom_radial_moments(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* u, int n_rows, double* moments);
+
 /* device time (ms, CUDA events) of the last solve_batch's SCF loop, and number of kernel launches it issued */
 int dftatom_last_timing(dftatom_ctx* ctx, double* device_ms, long long* kernel_launches);
 /* bytes the last solve_batch copied host -> device (atom / orbital descriptors; grid tables are cached per context and not counted)
