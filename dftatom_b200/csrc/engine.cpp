@@ -72,9 +72,6 @@ struct Knobs {
     int refine_vcycles = 0;
     int warm_vcycles = 7;      // Poisson warm start from SCF step warm_after on: V-cycles per solve (0 = always the full cycle)
     int warm_after = 1;
-    int recold_at = -1;        // >= warm_after: this one SCF step solves the Poisson equation cold (full multigrid) again.  The increments never correct
-                               // U itself, so U keeps the rounding-floor bias of the last cold solve; the reference's bias follows its current density:
-                               // re-anchoring once the density has settled keeps the two closer (C3: worst deviation 7.6e-6 -> 2.7e-6 Ha)
     int team_poisson = 1;      // large grids, few atoms: several CTAs per density (poisson.cu, team mode)
     int r_segments = -1;       // radial segments per orbital of the parallel-in-r search; -1 = auto (16 up to 16385 nodes, 32 above), 0 / 1 = serial-in-r search only
     int seg_threshold = 2400;  // the parallel-in-r search runs once at most this many orbitals are still active; above it (>= 4 warps per
@@ -98,17 +95,9 @@ struct Knobs {
     int stream_min_levels = 15; // stream mode from this many levels on (at 14 levels one CTA per density is as fast: measured 57.6 against 58.5 ms on C3)
     int poisson_exact = 0;     // 1: bit-reproducible Poisson solve (poisson_exact.cu): the reference's FullCycle in its own operation order, 100 V-cycles
     int run_to_cap = 0;        // 1: the stop test (DFTAtom.cpp:474) is evaluated and recorded but never ends the SCF (trajectory parity beyond the stop step)
-    int warm_poisson = 1;      // warm-started solves in increment form on 2049 .. 16385 nodes: one CTA per density, visits in registers (poisson_warm.cu); 0 = cluster / one-CTA kernels below
-    int direct_after = 4;      // ... from this SCF step on (earlier warm steps: the V-cycle kernels)
     int direct_poisson = 1;    // warm solves in increment form on 2049 .. 16385 nodes: the level-0 system solved directly (Thomas algorithm as block scans,
-                               // poisson_direct.cu) instead of 7 V-cycles; 0 = the V-cycle kernels below
-    int coarse_exact = 1;      // warm solves: the levels below 2048 nodes are replaced by the exact solve of the 1024-node level (poisson_tri.cuh); 0 = visited
-                               // with 3 + 3 sweeps each like the reference does
-    int warm_until_step = 32;  // ... up to this SCF step; from it on the cluster kernel (0: the one-CTA kernel at every step)
-    int cluster_poisson = 1;   // warm-started solves on 2049 .. 16385 nodes: one cluster of 8 CTAs per density (poisson_cluster.cu); 0 = one CTA per density
-    int cluster_max_dens = 1 << 30; // ... while at most this many atoms are still iterating.  Default: always - which kernel solves a density must not depend on
-                               // what else is in the batch (an atom's records are bit-identical alone, in any batch and on any shard); a smaller
-                               // value trades that for throughput while many atoms are active (above ~37 densities the clusters need more than one wave)
+                               // poisson_direct.cu) instead of 7 V-cycles by one CTA per density (poisson_warm.cu)
+    int direct_after = 4;      // ... from this SCF step on (earlier warm steps: the V-cycle kernel)
     int delta_poisson = 1;     // warm-started Poisson solves in increment form (A dU = -dS, U += dU: scf.cu) - keeps consecutive SCF steps free of the
                                // rounding-floor noise of a plain FP64 multigrid solve; 0 = iterate on U itself
     int adaptive_mixing = 0;   // opt-in: per-atom damping raised when Etotal sloshes with period 2 (beyond the reference; default: its fixed linear mixing)
@@ -301,7 +290,7 @@ int dftatom_create(dftatom_ctx** out, int device)
     DFT_CHECK(cudaDeviceGetAttribute(&c->n_sm, cudaDevAttrMultiProcessorCount, device));
     // opt-in dynamic shared memory is per-device state: set it here, for this context's device (not cached process-wide)
     int rc_attr;
-    if ((rc_attr = poisson_init_device()) || (rc_attr = stream_init_device()) || (rc_attr = match_init_device()) || (rc_attr = rows_init_device()) || (rc_attr = poisson_warm_init_device()) || (rc_attr = poisson_direct_init_device()) || (rc_attr = poisson_cluster_init_device())) { delete c; return rc_attr; }
+    if ((rc_attr = poisson_init_device()) || (rc_attr = stream_init_device()) || (rc_attr = match_init_device()) || (rc_attr = rows_init_device()) || (rc_attr = poisson_warm_init_device()) || (rc_attr = poisson_direct_init_device())) { delete c; return rc_attr; }
     DFT_CHECK(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     DFT_CHECK(cudaMallocHost((void**)&c->h_active, sizeof(int) * 256));
     *out = c;
@@ -354,7 +343,6 @@ int dftatom_set_option(dftatom_ctx* c, const char* key, double value)
     else if (k == "refine_vcycles") c->k.refine_vcycles = std::max(0, (int)value);
     else if (k == "warm_vcycles") c->k.warm_vcycles = std::max(0, (int)value);
     else if (k == "warm_after") c->k.warm_after = std::max(0, (int)value);
-    else if (k == "recold_at") c->k.recold_at = std::max(-1, (int)value);
     else if (k == "team_poisson") c->k.team_poisson = value != 0.;
     else if (k == "r_segments") c->k.r_segments = (int)value;
     else if (k == "seg_threshold") c->k.seg_threshold = (int)value;
@@ -378,13 +366,8 @@ int dftatom_set_option(dftatom_ctx* c, const char* key, double value)
     else if (k == "stream_min_levels") c->k.stream_min_levels = std::min(23, std::max(13, (int)value));
     else if (k == "stream_variant") c->k.stream_variant = std::min(2, std::max(0, (int)value));
     else if (k == "poisson_exact") c->k.poisson_exact = value != 0.;
-    else if (k == "cluster_poisson") c->k.cluster_poisson = value != 0.;
-    else if (k == "warm_poisson") c->k.warm_poisson = value != 0.;
     else if (k == "direct_after") c->k.direct_after = std::max(0, (int)value);
     else if (k == "direct_poisson") c->k.direct_poisson = value != 0.;
-    else if (k == "coarse_exact") c->k.coarse_exact = value != 0.;
-    else if (k == "warm_until_step") c->k.warm_until_step = std::max(0, (int)value);
-    else if (k == "cluster_max_dens") c->k.cluster_max_dens = std::max(0, (int)value);
     else if (k == "delta_poisson") c->k.delta_poisson = value != 0.;
     else if (k == "adaptive_mixing") c->k.adaptive_mixing = value != 0.;
     else if (k == "step_cap") c->k.step_cap = std::max(0, (int)value);
@@ -646,22 +629,19 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
     xa.n_dens = n_atoms; xa.L = g.L; xa.delta = g.delta; xa.rho = b.rhot; xa.rho_stride = N; xa.r = g.r; xa.pex = g.pex; xa.Zbc = b.Zbc;
     xa.U = b.U; xa.ldU = ldU; xa.work = c->exact_work.as<double>(); xa.skip = &b.astate[0].done; xa.skip_stride_bytes = (int)sizeof(AtomState);
     xa.max_vcycles = 100;                                       // PoissonSolver.h:117
-    const bool cluster_ok = c->k.cluster_poisson && !exact && !stream && poisson_cluster_supported(g.L, g.delta) && g.coarse_op && c->k.refine_vcycles == 0 && !c->k.floor_stop;
-    ClusterPoissonArgs ca{};
-    ca.n_dens = n_atoms; ca.rho = b.rhot; ca.rho_stride = N; ca.U = b.U; ca.ldU = ldU; ca.Zbc = b.Zbc; ca.coarse_op = g.coarse_op;
-    ca.coarse_tri = c->k.coarse_exact ? g.coarse_tri : nullptr;
+    WarmPoissonArgs ca{};
+    ca.n_dens = n_atoms; ca.rho = b.rhot; ca.rho_stride = N; ca.U = b.U; ca.ldU = ldU; ca.Zbc = b.Zbc; ca.coarse_tri = g.coarse_tri;
     ca.skip = &b.astate[0].done; ca.skip_stride_bytes = (int)sizeof(AtomState);
     StreamSolveArgs sa{};
     sa.n_dens = n_atoms; sa.rho = b.rhot; sa.rho_stride = N; sa.psrc = g.psrc; sa.src0 = c->stream_src0.as<double>(); sa.U = b.U; sa.ld0 = ldU;
     sa.Zbc = b.Zbc; sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op; sa.variant = c->k.stream_variant;
     sa.skip = &b.astate[0].done; sa.skip_stride_bytes = (int)sizeof(AtomState);
     // the Poisson solve of one SCF step: FullCycle (ramp + max_vcycles V-cycles), or warm_vcycles V-cycles from the previous U
-    int act_est = n_atoms;          // atoms still iterating, as of `lag` steps ago (host-side estimate; only selects between two equivalent kernels)
     double* rho_prev = c->rho_prev.as<double>();
     double* d_src = c->d_src.as<double>();
     double* d_u = c->d_u.as<double>();
     const int* skip_p = &b.astate[0].done; const int skip_stride = (int)sizeof(AtomState);
-    const bool warm_ok = c->k.warm_poisson && delta && !stream && poisson_warm_supported(g.L, g.delta) && g.coarse_op && (long long)lv.total >= poisson_warm_scratch_doubles(g.L);
+    const bool warm_ok = delta && !stream && poisson_warm_supported(g.L, g.delta) && g.coarse_tri != nullptr && (long long)lv.total >= poisson_warm_scratch_doubles(g.L);
     const bool direct_ok = c->k.direct_poisson && delta && g.coarse_direct != nullptr;
     int cur_step = 0;               // SCF step being enqueued (the graph body is captured at the first steady-state step)
     auto poisson_solve = [&](int warm_vcycles, long long& n_launch) {
@@ -670,43 +650,12 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
             launch_poisson_exact(xa, st);
             ++n_launch;
         } else if (warm && direct_ok && cur_step >= c->k.direct_after) {
-            ca.work = pa.work; ca.rho_prev = rho_prev; ca.step = nullptr; ca.scratch = d_u; ca.scratch_stride = ldU;
+            ca.work = pa.work; ca.rho_prev = rho_prev; ca.scratch = d_u; ca.scratch_stride = ldU;
             launch_poisson_direct(g, ca, st);
             ++n_launch;
         } else if (warm && warm_ok) {
-            // one SM per density while most atoms are still iterating (throughput), the 8-SM cluster per density afterwards (latency): shared by
-            // SCF step index, both launched every step, the density's own step counter decides which one solves it
-            const bool both = cluster_ok && c->k.warm_until_step > 0;
             ca.n_vcycles = warm_vcycles; ca.work = pa.work; ca.rho_prev = rho_prev;
-            ca.step = both ? &b.astate[0].n_steps : nullptr; ca.step_min = 0; ca.step_max = c->k.warm_until_step;
             launch_poisson_warm(g, ca, pa.phi, pa.src, lv.total, st);
-            ++n_launch;
-            if (both) {
-                ca.step_min = c->k.warm_until_step; ca.step_max = 1 << 30;
-                { long long* keep = ca.dbg; ca.dbg = nullptr; launch_poisson_cluster(g, ca, st); ca.dbg = keep; }
-                ++n_launch;
-            }
-            ca.step = nullptr;
-        } else if (warm && cluster_ok && act_est <= c->k.cluster_max_dens) {
-            ca.n_vcycles = warm_vcycles; ca.work = pa.work; ca.rho_prev = delta ? rho_prev : nullptr;
-            if (getenv("DFTATOM_DEBUG_CLUSTER") && n_launch > 40 && !ca.dbg) {       // development aid: cycle counters of one solve
-                if (c->scratch[5].ensure(sizeof(long long) * 256)) return;
-                cudaMemsetAsync(c->scratch[5].p, 0, sizeof(long long) * 256, st);
-                ca.dbg = c->scratch[5].as<long long>();
-                launch_poisson_cluster(g, ca, st);
-                long long h[256];
-                cudaMemcpyAsync(h, ca.dbg, sizeof(h), cudaMemcpyDeviceToHost, st);
-                cudaStreamSynchronize(st);
-                for (int r = 0; r < 8; ++r) {
-                    fprintf(stderr, "cluster rank %d: total %lld local %lld wait1 %lld wait2 %lld waitL %lld load %lld sweeps %lld store %lld | levels", r, h[r * 32], h[r * 32 + 1], h[r * 32 + 2], h[r * 32 + 3], h[r * 32 + 7], h[r * 32 + 4], h[r * 32 + 5], h[r * 32 + 6]);
-                    for (int l = 0; l < 4; ++l) fprintf(stderr, " %lld", h[r * 32 + 8 + l]);
-                    fprintf(stderr, "\n");
-                }
-                ca.dbg = reinterpret_cast<long long*>(1);       // once
-                ++n_launch;
-                return;
-            }
-            { long long* keep = ca.dbg; ca.dbg = nullptr; launch_poisson_cluster(g, ca, st); ca.dbg = keep; }
             ++n_launch;
         } else if (warm && delta) {
             // increment form around the existing solvers: dS, dU = 0 -> V-cycles on (dS, dU) with zero boundary values -> U += dU
@@ -846,7 +795,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
         end_phase();
         begin_phase(DFTATOM_K_POISSON);
         cur_step = sp;
-        poisson_solve((sp >= c->k.warm_after && sp != c->k.recold_at) ? c->k.warm_vcycles : 0, nl);
+        poisson_solve(sp >= c->k.warm_after ? c->k.warm_vcycles : 0, nl);
         end_phase();
         begin_phase(DFTATOM_K_POTENTIAL);
         launch_potential_energy(g, lv, b, 0, st); ++nl;
@@ -858,10 +807,10 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
     // body (cudaGraphSetConditional): one graph launch runs the rest of the SCF of the whole batch with no host round trip at all.
     // Not used with per-class event timing (profile), the validation search / match modes, or the cooperative team-mode Poisson kernel.
     const bool team_possible = g.L >= 15 && !stream && !exact;
-    const bool graph_ok = c->k.use_graph && !prof && c->k.search_mode == 0 && c->k.match_mode == 0 && (!team_possible || direct_ok) && !getenv("DFTATOM_DEBUG_CLUSTER");
+    const bool graph_ok = c->k.use_graph && !prof && c->k.search_mode == 0 && c->k.match_mode == 0 && (!team_possible || direct_ok);
     bool graph_done = false;
     if (graph_ok) {
-        const int n_cold = std::min(max_steps, std::max(std::max(std::max(0, c->k.warm_after), c->k.recold_at + 1), direct_ok ? c->k.direct_after : 0));
+        const int n_cold = std::min(max_steps, std::max(std::max(0, c->k.warm_after), direct_ok ? c->k.direct_after : 0));
         for (int sp = 0; sp < n_cold; ++sp) { enqueue_step(sp, sp + 1, launches); ++steps_enqueued; }
         if (n_cold < max_steps) {
             // phases: the ranges of SCF steps between the step indices at which a kernel shape hands over to another one
@@ -928,7 +877,6 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
             // the host stays `lag` steps ahead of the device: it never idles the GPU, it only stops enqueueing
             DFT_CHECK(cudaEventSynchronize(step_ev[sp - lag]));
             if (c->h_active[sp - lag] == 0) break;
-            act_est = c->h_active[sp - lag];
         }
     }
     DFT_CHECK(cudaEventRecord(ev1, st));

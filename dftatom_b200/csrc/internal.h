@@ -40,7 +40,7 @@ struct GridDev {
     double* inv4pr2; // 1 / (4π r_i^2) (0 at i=0)                    (DFTAtom.cpp:340)
     double* pex;     // 4π Rp²δ² · e^{2δ i} in the reference's own product order (PoissonSolver.h:66-74; uniform grid: h² 4π, :26-40): poisson_exact.cu
     double* coarse_op; // [32*32] dense operator of the Poisson sub-cycle below the 32-node level (poisson.cu), NULL for L < 6
-    double* coarse_direct; // pivots of the direct solve of the level-0 system (poisson_direct.cu), NULL unless 11 <= L <= 14
+    double* coarse_direct; // pivots of the direct solve of the level-0 system (poisson_direct.cu), NULL unless 11 <= L <= 20
     double* coarse_tri; // table of the exact solve of the 1024-node level (poisson_tri.cuh), NULL unless 11 <= L <= 14
 };
 
@@ -232,43 +232,33 @@ struct ExactPoissonArgs {
 long long exact_poisson_work_doubles(int L);
 void launch_poisson_exact(const ExactPoissonArgs& a, cudaStream_t st);
 
-// Poisson, cluster mode (poisson_cluster.cu): warm-started V-cycles for 2049 .. 16385 nodes, one cluster of 8 CTAs per density, the
-// hierarchy resident in distributed shared memory
-struct ClusterPoissonArgs {
+// Poisson, warm solves in increment form (poisson_warm.cu, poisson_direct.cu): the densities' solutions U are updated in place
+struct WarmPoissonArgs {
     int n_dens;
     const double* rho; long long rho_stride;    // [n_dens][rho_stride] total densities, natural node order
-    double* rho_prev;                           // optional [n_dens][rho_stride], in / out: the density of the previous solve.  Given: increment form - the
-                                                // V-cycles solve A dU = -r 4 pi K (rho - rho_prev) from dU = 0 and U += dU (see scf.cu); NULL: they iterate on U
-    double* U; long long ldU;                   // [n_dens][ldU] in: previous solution (initial guess), out: U(r)
+    double* rho_prev;                           // [n_dens][rho_stride], in / out: the density of the previous solve.  Increment form: the solve is
+                                                // A dU = -r 4 pi K (rho - rho_prev) from dU = 0 and U += dU (see scf.cu)
+    double* U; long long ldU;                   // [n_dens][ldU] in: previous solution, out: U(r)
     const int* Zbc;                             // [n_dens] boundary value at Rmax
-    const double* coarse_op;                    // GridDev.coarse_op
-    const double* coarse_tri;                   // GridDev.coarse_tri or NULL.  Given: the levels below 2048 nodes are replaced by the exact solve of the
-                                                // 1024-node level (poisson_tri.cuh); NULL: they are visited like the reference does, down to the dense operator
+    const double* coarse_tri;                   // GridDev.coarse_tri (poisson_warm.cu): the levels below 2048 nodes are replaced by the exact solve of
+                                                // the 1024-node level (poisson_tri.cuh)
     const int* skip; int skip_stride_bytes;
-    const int* step; int step_min, step_max;    // optional: the density's SCF step counter (AtomState.n_steps, stride = skip_stride_bytes): it is solved by this launch
-                                                // only while step_min <= *step < step_max - two kernels that share the warm solves of one SCF by step index
-                                                // (a property of the atom alone: the records stay independent of what else is in the batch)
     int n_vcycles;
     double* scratch; long long scratch_stride;  // poisson_direct.cu above 16385 nodes: n_dens x scratch_stride doubles (>= N - 1 each)
     unsigned long long* work;                   // optional: += Gauss-Seidel node-updates
-    int smem_doubles;                           // set by the launcher
-    long long* dbg;                             // optional [8 * 32] cycle counters of the first density's CTAs (development aid)
 };
-bool poisson_cluster_supported(int L, double delta);
-void launch_poisson_cluster(const GridDev& g, const ClusterPoissonArgs& a, cudaStream_t st);
-int poisson_cluster_init_device();
 
-// Poisson, warm solves in increment form on one SM per density (poisson_warm.cu): the arguments of the cluster mode with rho_prev given;
+// Poisson, warm solves in increment form on one SM per density (poisson_warm.cu): V-cycles; a.coarse_tri must be set;
 // gphi / gsrc: scratch of n_dens x gstride doubles each (gstride >= poisson_warm_scratch_doubles(L)), contents irrelevant before and after
 bool poisson_warm_supported(int L, double delta);
 long long poisson_warm_scratch_doubles(int L);
-void launch_poisson_warm(const GridDev& g, const ClusterPoissonArgs& a, double* gphi, double* gsrc, long long gstride, cudaStream_t st);
+void launch_poisson_warm(const GridDev& g, const WarmPoissonArgs& a, double* gphi, double* gsrc, long long gstride, cudaStream_t st);
 int poisson_warm_init_device();
-// Poisson, warm solves in increment form as one direct (Thomas) solve per density (poisson_direct.cu): the arguments of the cluster mode with rho_prev given
+// Poisson, warm solves in increment form as one direct (Thomas) solve per density (poisson_direct.cu)
 bool poisson_direct_supported(int L);
 long long poisson_direct_table_doubles(int L);
 void coarse_direct_host(int L, double delta, double* W);      // host-side table builders (once per grid)
-void launch_poisson_direct(const GridDev& g, const ClusterPoissonArgs& a, cudaStream_t st);
+void launch_poisson_direct(const GridDev& g, const WarmPoissonArgs& a, cudaStream_t st);
 int poisson_direct_init_device();
 void coarse_tri_host(int L, double delta, double* T);
 

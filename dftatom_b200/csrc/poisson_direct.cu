@@ -13,7 +13,7 @@
 // Both passes are first-order recurrences with multipliers -> 1 (every node sees every source), i.e. scans of affine maps that cannot be
 // truncated: thread t owns NPT consecutive nodes (registers), runs its chunk with zero carry-in while accumulating the product of its
 // multipliers, the 512 maps are combined by a warp scan + one scan over the 16 warp totals, and the carry is patched in.  One CTA per
-// density; ~10 k cycles per solve against ~400 k (cluster of 8 CTAs) / ~700 k (one CTA) for the 7 V-cycles.
+// density; ~10 k cycles per solve against ~700 k for the 7 V-cycles of poisson_warm.cu.
 #include "internal.h"
 #include <algorithm>
 #include <cmath>
@@ -69,7 +69,7 @@ __device__ __forceinline__ double block_carry(double M, double C, double x_in)
 }
 
 template <int NPT>
-__device__ __forceinline__ void direct_solve(const GridDev& g, const ClusterPoissonArgs& a, int k)
+__device__ __forceinline__ void direct_solve(const GridDev& g, const WarmPoissonArgs& a, int k)
 {
     const int t = threadIdx.x;
     const int N = g.N, n = N - 1;                       // owned nodes 0 .. n-1 (node 0 and node n are the boundaries: dU = 0)
@@ -133,7 +133,7 @@ __device__ __forceinline__ void direct_solve(const GridDev& g, const ClusterPois
 
 // Grids above 16385 nodes: the same two passes chunk by chunk (16384 nodes = 512 threads x 32), the carry of one chunk entering the next;
 // delta of every chunk is parked in `scratch` (owner-major per chunk, coalesced) between the forward and the backward pass.
-__device__ __forceinline__ void direct_solve_chunked(const GridDev& g, const ClusterPoissonArgs& a, int k)
+__device__ __forceinline__ void direct_solve_chunked(const GridDev& g, const WarmPoissonArgs& a, int k)
 {
     constexpr int NPT = 32, CH = kDT * NPT;
     __shared__ double s_carry;
@@ -212,7 +212,7 @@ __device__ __forceinline__ void direct_solve_chunked(const GridDev& g, const Clu
 
 }  // namespace
 
-__global__ void __launch_bounds__(kDT, 1) poisson_direct_kernel(GridDev g, ClusterPoissonArgs a)
+__global__ void __launch_bounds__(kDT, 1) poisson_direct_kernel(GridDev g, WarmPoissonArgs a)
 {
     DFT_PDL_WAIT();
     const int k = blockIdx.x;
@@ -254,9 +254,9 @@ int poisson_direct_init_device()
     return 0;
 }
 
-// a: the arguments of poisson_cluster.cu (rho, rho_prev, U, skip; n_vcycles and the coarse tables are not used); g.coarse_direct must be set; above 14
+// a: rho, rho_prev, U, skip (n_vcycles and coarse_tri are not used); g.coarse_direct must be set; above 14
 // levels a.scratch (n_dens x scratch_stride doubles, scratch_stride >= N - 1) is required
-void launch_poisson_direct(const GridDev& g, const ClusterPoissonArgs& a, cudaStream_t st)
+void launch_poisson_direct(const GridDev& g, const WarmPoissonArgs& a, cudaStream_t st)
 {
     launch_step_kernel(poisson_direct_kernel, dim3(a.n_dens), dim3(kDT), direct_smem_bytes(g.L), st, g, a);
 }

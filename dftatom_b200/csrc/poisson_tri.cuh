@@ -1,4 +1,4 @@
-// Exact solve of the 1024-node correction level of the radial Poisson V-cycle by one warp (shared by poisson_warm.cu and poisson_cluster.cu).
+// Exact solve of the 1024-node correction level of the radial Poisson V-cycle by one warp (poisson_warm.cu).
 //
 // The reference's V-cycle (PoissonSolver.h:155-159, PoissonSolver.cpp:162-197) visits, below the 1024-node level, the levels of 512 .. 2
 // nodes with 3 + 3 Gauss-Seidel sweeps each: ~60 dependent sweeps of ~1100 cycles for a few hundred nodes - a quarter to a third of a

@@ -3,10 +3,8 @@
 // Replaces (reference DFTAtom/) PoissonSolver.h:155-159 VCycle, PoissonSolver.cpp:40-64 GaussSeidel, :110-123 Prolong, :126-157 Restrict,
 // :162-197 Ascend / Descend for the warm solves of the SCF: from SCF step `warm_after` on a solve is `warm_vcycles` V-cycles on
 //   A dU = -r 4 pi K (rho - rho_prev),  dU = 0 on both boundaries and as the initial guess,  U += dU        (scf.cu: increment form).
-// Same operators and the same order of sweeps / restriction / prolongation as poisson.cu and poisson_cluster.cu.  What this kernel is
-// built around: a solve is ~380 dependent Gauss-Seidel sweeps (7 V-cycles x 9 levels x 6) and ~130 level visits, each only a few hundred
-// cycles of work for one SM - poisson_cluster.cu spreads a density over 8 SMs and pays ~1350 cycles per sweep in window loads, cluster
-// barriers and the local sub-cycle on which 7 of its 8 CTAs wait (measured: 513 k cycles per solve; 5 waves for the 92 densities of C3).
+// Same operators and the same order of sweeps / restriction / prolongation as poisson.cu.  What this kernel is built around: a solve is a
+// chain of dependent Gauss-Seidel sweeps and level visits, each only a few hundred cycles of work for one SM.
 //  * Every level is visited by the whole CTA: thread t owns NPT = n / 512 consecutive nodes (one node per thread on the first n threads
 //    below 512 nodes).  A visit loads them into registers ONCE, (adds the prolongated correction,) runs its 3 or 6 sweeps on the
 //    registers, (forms the restricted residual of the next level,) and stores once.  Where a level lives is a template parameter: no
@@ -15,7 +13,7 @@
 //    (a ~ 1/2: a^64 < 1e-19) and the carry patch - with ONE block barrier: the right neighbour warp's old first node and the left
 //    neighbour warp's total are published before it (double buffered by sweep parity); what lane 31 could not know before the barrier
 //    (b x the neighbour's first node) is added to its last node and to the carry of the next warp after it.
-//  * The sub-cycle below the 32-node level is the grid's precomputed dense operator (coarse_op_kernel).
+//  * The levels below 2048 nodes are replaced by the exact solve of the 1024-node level (poisson_tri.cuh).
 //  * Source_0/2 and the levels of <= 2048 nodes live in shared memory (owner-major: thread t's k-th node at k x 513 + t, conflict-free both
 //    for the owner and for the coalesced import / export), Phi_0 and the two levels of 8192 / 4096 nodes in this density's block of the
 //    L2-resident hierarchy buffers (owner-major, coalesced): ~0.9 MB of L2 traffic per V-cycle and density.
@@ -48,8 +46,7 @@ struct WLevel {
 
 struct WShared {
     WLevel lv[12];
-    int m;                  // the dense level (32 owned nodes), or - exact coarse solve - the 1024-node level
-    int tri;                // 1: the levels below 2048 nodes are replaced by the exact solve of the 1024-node level (poisson_tri.cuh)
+    int m;                  // the exactly solved 1024-node level
     int offT;               // its table in w_dyn
     double* gphi; double* gsrc;     // this density's blocks of the global hierarchy buffers
     double* U;
@@ -57,7 +54,6 @@ struct WShared {
     double wtot[2][kWT / 32];       // scan total of every warp (without b x the right neighbour's first node)
     double last[kWT / 32];          // last node of every warp after the sweeps (restriction)
     unsigned long long updates;
-    double G[32 * 32];      // dense operator of the sub-cycle below the 32-node level, column-major G[j * 32 + i]
 #ifdef DFT_WARM_DEBUG
     long long clk[64];
 #endif
@@ -280,7 +276,7 @@ __device__ __forceinline__ void w_visit_level_impl(int l, int flags, int sweeps)
 {
     const WLevel& c = ws.lv[l];
     const bool cg = ws.lv[l + 1].gl != 0;
-    const bool ct = ws.tri && l + 1 == ws.m;      // the next level is the exactly solved one
+    const bool ct = l + 1 == ws.m;              // the next level is the exactly solved one
     if (l == 0) {               // Phi_0 in the global block, Source_0 / 2 in shared memory
         switch (c.npt) {
             case 32: w_visit<32, true, false, true>(l, flags, sweeps); break;
@@ -311,25 +307,6 @@ __device__ __forceinline__ void w_visit_level(int l, int flags, int sweeps)
 #endif
 }
 
-// Phi_m = G Source_m: the whole sub-cycle below the 32-node level (warp 0; natural order)
-__device__ __forceinline__ void w_dense()
-{
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        const WLevel& c = ws.lv[ws.m];
-        const int i = threadIdx.x;
-        double a0 = 0., a1 = 0., a2 = 0., a3 = 0.;
-#pragma unroll
-        for (int j = 0; j < 32; j += 4) {
-            a0 = fma(ws.G[(j + 0) * 32 + i], 2. * w_dyn[c.offS + j + 0], a0);
-            a1 = fma(ws.G[(j + 1) * 32 + i], 2. * w_dyn[c.offS + j + 1], a1);
-            a2 = fma(ws.G[(j + 2) * 32 + i], 2. * w_dyn[c.offS + j + 2], a2);
-            a3 = fma(ws.G[(j + 3) * 32 + i], 2. * w_dyn[c.offS + j + 3], a3);
-        }
-        w_dyn[c.offP + i] = (a0 + a1) + (a2 + a3);      // row 0 of G is zero: the left boundary stays 0
-    }
-}
-
 // exact solve of the 1024-node level (warp 0), in place of everything below the 2048-node level
 __device__ __forceinline__ void w_tri()
 {
@@ -342,15 +319,15 @@ __device__ __forceinline__ void w_tri()
     }
 }
 
-// placement of the levels 0 .. L-5.  Phi_0 and both arrays of the levels of >= 4096 nodes below it live in the global blocks (stride 512),
+// placement of the levels 0 .. L-10.  Phi_0 and both arrays of the levels of >= 4096 nodes below it live in the global blocks (stride 512),
 // everything else in shared memory (stride 513 with 512 owners; natural order below)
-__host__ __device__ inline void w_place_all(int L, bool tri, WLevel* out, int& dyn, int& gph, int& gsr, int& offT)
+__host__ __device__ inline void w_place_all(int L, WLevel* out, int& dyn, int& gph, int& gsr, int& offT)
 {
     dyn = 0; gph = 0; gsr = 0; offT = 0;
-    const int last = tri ? L - 10 : L - 5;
+    const int last = L - 10;
     for (int q = 0; q <= last; ++q) {
         const int n = 1 << (L - q);
-        if (tri && q == last) {         // the exactly solved level: lane-major rows of 33, and its table
+        if (q == last) {                // the exactly solved level: lane-major rows of 33, and its table
             const int offP = dyn, offS = dyn + 32 * 33 + 1;
             dyn += 2 * (32 * 33 + 1);
             offT = dyn; dyn += kTriTableDoubles;
@@ -372,22 +349,17 @@ __host__ __device__ inline void w_place_all(int L, bool tri, WLevel* out, int& d
 
 }  // namespace
 
-__global__ void __launch_bounds__(kWT, 1) poisson_warm_kernel(GridDev g, ClusterPoissonArgs a, double* gphi_all, double* gsrc_all, long long gstride)
+__global__ void __launch_bounds__(kWT, 1) poisson_warm_kernel(GridDev g, WarmPoissonArgs a, double* gphi_all, double* gsrc_all, long long gstride)
 {
     const int k = blockIdx.x;
     if (a.skip && *reinterpret_cast<const int*>(reinterpret_cast<const char*>(a.skip) + (size_t)k * a.skip_stride_bytes)) return;
-    if (a.step) {
-        const int sc = *reinterpret_cast<const int*>(reinterpret_cast<const char*>(a.step) + (size_t)k * a.skip_stride_bytes);
-        if (sc < a.step_min || sc >= a.step_max) return;
-    }
     const int L = g.L, N = g.N, t = threadIdx.x;
-    const bool tri = a.coarse_tri != nullptr;
-    const int m = tri ? L - 10 : L - 5;
+    const int m = L - 10;
     if (t == 0) {
         int dyn, gph, gsr, offT;
-        w_place_all(L, tri, ws.lv, dyn, gph, gsr, offT);
+        w_place_all(L, ws.lv, dyn, gph, gsr, offT);
         ws.lv[m + 1].gl = 0;
-        ws.m = m; ws.tri = tri; ws.offT = offT;
+        ws.m = m; ws.offT = offT;
         ws.gphi = gphi_all + (size_t)k * gstride; ws.gsrc = gsrc_all + (size_t)k * gstride;
         ws.U = a.U + (size_t)k * a.ldU;
         ws.updates = 0;
@@ -414,8 +386,7 @@ __global__ void __launch_bounds__(kWT, 1) poisson_warm_kernel(GridDev g, Cluster
             c.alane[ln] = al;
         }
     }
-    if (tri) { for (int i = t; i < kTriTableDoubles; i += kWT) w_dyn[ws.offT + i] = a.coarse_tri[i]; }
-    else { for (int i = t; i < 32 * 32; i += kWT) ws.G[i] = a.coarse_op[i]; }
+    for (int i = t; i < kTriTableDoubles; i += kWT) w_dyn[ws.offT + i] = a.coarse_tri[i];
     __syncthreads();
     // import: Source_0 / 2 = r 4 pi K (rho - rho_prev) / 2 into its owner-major rows; rho_prev = rho
     {
@@ -434,7 +405,7 @@ __global__ void __launch_bounds__(kWT, 1) poisson_warm_kernel(GridDev g, Cluster
     for (int cyc = 0; cyc < nv; ++cyc) {
         // down-leg (the level-0 down-visit of every cycle but the first was fused into the previous top); dU starts from 0
         for (int l = (cyc == 0 ? 0 : 1); l < m; ++l) w_visit_level(l, kWRestrict, 3);
-        if (tri) w_tri(); else w_dense();
+        w_tri();
         // up-leg
         for (int l = m - 1; l >= 1; --l) w_visit_level(l, kWLoad | kWProlong, 3);
         if (cyc == nv - 1) w_visit_level(0, kWLoad | kWProlong | kWExport, 3);
@@ -450,10 +421,10 @@ __global__ void __launch_bounds__(kWT, 1) poisson_warm_kernel(GridDev g, Cluster
 #endif
 }
 
-static int warm_smem_doubles(int L, bool tri)
+static int warm_smem_doubles(int L)
 {
     int dyn, gph, gsr, offT;
-    w_place_all(L, tri, nullptr, dyn, gph, gsr, offT);
+    w_place_all(L, nullptr, dyn, gph, gsr, offT);
     return dyn;
 }
 
@@ -465,20 +436,20 @@ bool poisson_warm_supported(int L, double delta) { return L >= 11 && L <= 14 && 
 long long poisson_warm_scratch_doubles(int L)
 {
     int dyn, gph, gsr, offT;
-    w_place_all(L, false, nullptr, dyn, gph, gsr, offT);
+    w_place_all(L, nullptr, dyn, gph, gsr, offT);
     return std::max(gph, gsr);
 }
 
 int poisson_warm_init_device()
 {
-    DFT_CHECK(cudaFuncSetAttribute(poisson_warm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, std::max(warm_smem_doubles(14, false), warm_smem_doubles(14, true)) * (int)sizeof(double)));
+    DFT_CHECK(cudaFuncSetAttribute(poisson_warm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, warm_smem_doubles(14) * (int)sizeof(double)));
     return 0;
 }
 
-// a: the arguments of poisson_cluster.cu (rho_prev required); gphi / gsrc: two scratch buffers of n_dens x gstride doubles, gstride >= poisson_warm_scratch_doubles(L)
-void launch_poisson_warm(const GridDev& g, const ClusterPoissonArgs& a, double* gphi, double* gsrc, long long gstride, cudaStream_t st)
+// a: a.coarse_tri required; gphi / gsrc: two scratch buffers of n_dens x gstride doubles, gstride >= poisson_warm_scratch_doubles(L)
+void launch_poisson_warm(const GridDev& g, const WarmPoissonArgs& a, double* gphi, double* gsrc, long long gstride, cudaStream_t st)
 {
-    poisson_warm_kernel<<<a.n_dens, kWT, (size_t)warm_smem_doubles(g.L, a.coarse_tri != nullptr) * sizeof(double), st>>>(g, a, gphi, gsrc, gstride);
+    poisson_warm_kernel<<<a.n_dens, kWT, (size_t)warm_smem_doubles(g.L) * sizeof(double), st>>>(g, a, gphi, gsrc, gstride);
 }
 
 }  // namespace dft

@@ -155,22 +155,15 @@ const char* dftatom_version(void);
  *   "step_cap"     (default 0 = the reference's caps, 100 LDA / 150 LSDA steps) a lower cap on the SCF steps of every atom of the batch
  *   "warm_vcycles" (default 7) / "warm_after" (default 1): from SCF step warm_after on the Poisson solve is warm_vcycles V-cycles in increment
  *                   form (A dU = -r 4 pi K (rho - rho_prev) from dU = 0, U += dU; "delta_poisson" 0 = iterate on U itself) instead of the full
- *                   multigrid cycle; warm_vcycles 0 = the full cycle at every step
- *   "warm_poisson" (default 1) those warm solves on grids of 2049 .. 16385 nodes by one CTA per density (poisson_warm.cu) while the atom's own
- *                   SCF step counter is below "warm_until_step" (default 32; 0 = always), by the cluster kernel below afterwards: both are
- *                   launched every step and the atom's step counter decides, so its records do not depend on what else is in the batch
- *   "coarse_exact" (default 1) warm solves: the levels below 2048 nodes (~60 latency-bound sweeps per V-cycle for a few hundred nodes) are
- *                   replaced by the exact solve of the 1024-node level's own equation (poisson_tri.cuh); 0 = swept like the reference does
+ *                   multigrid cycle; warm_vcycles 0 = the full cycle at every step.  On grids of 2049 .. 16385 nodes these V-cycles are run
+ *                   by one CTA per density (poisson_warm.cu), the levels below 2048 nodes (~60 latency-bound sweeps per V-cycle for a few
+ *                   hundred nodes) replaced by the exact solve of the 1024-node level's own equation (poisson_tri.cuh)
  *   "direct_poisson" (default 1) warm solves in increment form from SCF step "direct_after" (default 4) on: the level-0 system of the increment
  *                   is solved directly (Thomas algorithm as block scans of affine maps, poisson_direct.cu; every grid of >= 2049 nodes) instead
- *                   of by V-cycles; the warm steps before it (large increments) and "direct_poisson" 0 use the V-cycle kernels above
- *   "recold_at"    (default -1 = never) this one SCF step solves the Poisson equation cold (full multigrid) again
+ *                   of by V-cycles; the warm steps before it (large increments) and "direct_poisson" 0 use the V-cycles above
  *   "match_win_until_step" (default 32; 0 = always one window) / "match_win_nodes" (default 8192): grids that fit one window of the matched-solution
  *                   kernel: while the atom's step counter is below the former its orbitals are solved in windows of the latter (3 CTAs per SM),
  *                   afterwards in one window (one CTA per SM, lowest latency)
- *   "cluster_poisson" (default 1) warm-started Poisson solves on grids of 2049 .. 16385 nodes run as one thread-block cluster of 8 CTAs per
- *                   density with the whole multigrid hierarchy in distributed shared memory (poisson_cluster.cu); 0 = one CTA per density.
- *                   "cluster_max_dens" (default: unlimited) restricts it to steps with at most that many atoms still iterating.
  *   "stream_variant" (default 0) window shape of the stream-mode Poisson visits: 0 = 256 threads x 16 nodes, 1 = 256 x 8, 2 = 512 x 8
  */
 int dftatom_set_option(dftatom_ctx* ctx, const char* key, double value);

@@ -5,5 +5,4 @@ for m in g hg gg; do
   echo "== memcheck $m"; timeout 300 compute-sanitizer --tool memcheck --print-limit 3 python scripts/sanitize_r2d.py $m 2>&1 | grep -v "^=========     Host Frame" | tail -25
 done
 echo "== tail3 host loop (profile)"; python scripts/gpu_tail3.py
-echo "== tail3 host loop, cluster_poisson=0"; python scripts/gpu_tail3.py cluster_poisson=0
 echo "== C3 per-step"; DFTATOM_DEBUG_STEPS=1 python scripts/gpu_steps_c3.py 2> gpurun_out/steps_c3.txt; tail -3 gpurun_out/steps_c3.txt

@@ -1,6 +1,6 @@
 """Round-2 kernels under compute-sanitizer (memcheck / racecheck): the rows search (numerov_rows.cu: all three round shapes, lanes entry), the
-one-CTA warm Poisson kernel (poisson_warm.cu) with the exact coarse solve and with the swept coarse levels, the cluster kernel with the exact
-coarse solve, the step-window sharing between them.  Small grids and a low step cap: the tools slow the kernels down 20-100x."""
+one-CTA warm Poisson kernel (poisson_warm.cu) with the exact coarse solve, the direct warm Poisson solve (poisson_direct.cu).  Small grids and
+a low step cap: the tools slow the kernels down 20-100x."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -10,8 +10,7 @@ ctx = D.Context(0)
 ctx.set_option("use_graph", int(os.environ.get("SAN_GRAPH", "0")))
 ctx.set_option("step_cap", int(os.environ.get("SAN_STEPS", "8")))
 ctx.set_option("step_cap", int(os.environ.get("SAN_STEPS", "10")))
-ctx.set_option("warm_until_step", 3)            # steps 1, 2: poisson_warm_kernel; 3, 4: poisson_cluster_kernel; 5 .. 9: poisson_direct_kernel
-ctx.set_option("direct_after", 5)
+ctx.set_option("direct_after", 5)               # steps 1 .. 4: poisson_warm_kernel; 5 .. 9: poisson_direct_kernel
 ctx.set_option("rows_wide_from_step", 5)        # steps 0 .. 4: 4-warp search; 5 .. 9: 8-warp search
 ctx.set_option("match_win_until_step", 5)       # steps 0 .. 4: windowed matched solution (windows of 1024 nodes); 5 .. 9: one window
 ctx.set_option("match_win_nodes", 1024)
@@ -22,10 +21,6 @@ for cfg in (0x111, 0x412):
 ctx.set_option("rows_cfg", 0x111)
 r = ctx.solve_batch([D.Options(6, 12, 20.0, 0.001, 0.5, 0)], keep_steps=False)
 print("scf L12", [x.n_steps for x in r], r[0].Etotal, flush=True)
-ctx.set_option("coarse_exact", 0)
-r = ctx.solve_batch([D.Options(6, 12, 20.0, 0.001, 0.5, 0)], keep_steps=False)
-print("scf L12 swept coarse levels", [x.n_steps for x in r], r[0].Etotal, flush=True)
-ctx.set_option("coarse_exact", 1)
 ctx.set_option("direct_after", 2); ctx.set_option("step_cap", 5)
 r = ctx.solve_batch([D.Options(3, 15, 20.0, 0.0003, 0.5, 0)], keep_steps=False)
 print("scf L15 (chunked direct Poisson solve, windowed match)", [x.n_steps for x in r], r[0].Etotal, flush=True)

@@ -128,7 +128,7 @@ def test_argon_c1_every_step(ctx):
 def test_batch_independence_and_determinism(ctx):
     """Atoms never interact: an atom solved alone and inside a batch gives bit-identical records (what makes the
     multi-GPU sharding exact, SURVEY §8e); repeated runs are bit-identical."""
-    # (12 levels: the warm Poisson solves are shared between two kernels by the atom's own step index - still independent of the batch)
+    # (12 levels: the warm Poisson solves switch from the V-cycle kernel to the direct solve at a fixed SCF step - still independent of the batch)
     _check_batch_independence(ctx, [D.Options(Z, 10, 15.0, 0.004, 0.5, m) for Z, m in [(2, 0), (13, 0), (7, 1), (29, 0)]])
     _check_batch_independence(ctx, [D.Options(Z, 12, 20.0, 0.001, 0.5, m) for Z, m in [(3, 1), (30, 0), (10, 0)]])
 
@@ -150,15 +150,14 @@ def test_kernel_shapes_agree(ctx):
     opts = [D.Options(Z, 12, 20.0, 0.001, 0.5, m) for Z, m in [(4, 0), (18, 0), (26, 1), (47, 0)]]
     base = ctx.solve_batch(opts)
     # search: lanes across the radial grid (numerov_rows.cu, production; 4 / 8 / 16 trial energies per round) vs lanes across 32 trial
-    # energies (numerov_seg.cu / numerov_fast.cu); Poisson warm solves: one CTA per density / cluster per density / both shared by step index,
-    # exact solve of the 1024-node level vs its swept sub-cycle; host-driven SCF loop vs CUDA-graph while node
+    # energies (numerov_seg.cu / numerov_fast.cu); Poisson warm solves: V-cycles (poisson_warm.cu) at every warm step vs the direct solve
+    # (poisson_direct.cu) from step 1 on; host-driven SCF loop vs CUDA-graph while node
     variants = [{"search_kernel": 1}, {"search_kernel": 1, "r_segments": 0}, {"search_kernel": 1, "seg_threshold": 30}, {"search_kernel": 1, "r_segments": 32},
                 {"search_kernel": 1, "r_segments": 8}, {"rows_cfg": 0x412}, {"rows_cfg": 0x222}, {"warm_vcycles": 0}, {"match_mode": 2},
-                {"warm_poisson": 0}, {"coarse_exact": 0}, {"warm_poisson": 0, "coarse_exact": 0}, {"warm_until_step": 0}, {"warm_until_step": 12},
                 {"use_graph": 0}, {"match_win_until_step": 0}, {"match_win_until_step": 100, "match_win_nodes": 2048}, {"direct_poisson": 0}, {"direct_after": 1}, {"rows_wide_from_step": 0}, {"rows_wide_from_step": 1}, {"stream_groups": 1},
                 {"graph_phases": 0}, {"rows_wide_from_step": 10, "match_win_until_step": 20}, {"search_predict": 0}, {"use_pdl": 0}, {"unit_guess": 0}]
-    defaults = {"graph_phases": 1, "search_predict": 1, "use_pdl": 1, "unit_guess": 1, "r_segments": -1, "seg_threshold": 2400, "warm_vcycles": 7, "match_mode": 0, "search_kernel": 0, "rows_cfg": 0x111, "warm_poisson": 1,
-                "coarse_exact": 1, "warm_until_step": 32, "use_graph": 1, "match_win_until_step": 32, "match_win_nodes": 8192, "stream_groups": 4, "direct_poisson": 1, "direct_after": 4, "rows_wide_from_step": 32}
+    defaults = {"graph_phases": 1, "search_predict": 1, "use_pdl": 1, "unit_guess": 1, "r_segments": -1, "seg_threshold": 2400, "warm_vcycles": 7, "match_mode": 0, "search_kernel": 0, "rows_cfg": 0x111,
+                "use_graph": 1, "match_win_until_step": 32, "match_win_nodes": 8192, "stream_groups": 4, "direct_poisson": 1, "direct_after": 4, "rows_wide_from_step": 32}
     for v in variants:
         for k_, x in v.items():
             ctx.set_option(k_, x)
@@ -271,6 +270,14 @@ def test_options_validation(ctx):
             ctx.solve_batch([bad])
     with pytest.raises(D.DFTAtomError):
         ctx.solve_batch([D.Options(2, 10, 15.0, 0.004, 0.5, 0), D.Options(2, 11, 15.0, 0.004, 0.5, 0)])
+
+
+def test_removed_poisson_options_are_rejected(ctx):
+    """Options of the removed alternative warm Poisson paths are unknown keys: a script or DFTATOM_OPTIONS string that still sets one
+    stops with an error instead of silently running the default kernels."""
+    for key in ("cluster_poisson", "cluster_max_dens", "warm_until_step", "warm_poisson", "coarse_exact", "recold_at"):
+        with pytest.raises(D.DFTAtomError, match="unknown option"):
+            ctx.set_option(key, 1)
 
 
 def test_report_text_matches_reference_format(ctx):
