@@ -16,11 +16,14 @@ from .api import (  # noqa: F401
     Result,
     Step,
     aufbau,
+    config_aufbau,
     estimate_cost,
+    format_config,
     lib_path,
     load_library,
     n_nodes,
     orbital_count,
+    parse_config,
     partition,
     split_spin,
 )
@@ -29,4 +32,5 @@ from .report import format_report, parse_report  # noqa: F401
 __all__ = [
     "Context", "DFTAtom", "DFTAtomError", "Level", "Options", "Radial", "Result", "Step", "aufbau", "split_spin", "n_nodes",
     "lib_path", "load_library", "format_report", "parse_report", "estimate_cost", "partition", "orbital_count",
+    "config_aufbau", "parse_config", "format_config",
 ]

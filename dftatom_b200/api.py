@@ -1,6 +1,8 @@
 """ctypes binding of include/dftatom_b200.h and the Python mirror of the reference's solver surface."""
 import ctypes as C
+import math
 import os
+import re
 import sys
 from dataclasses import dataclass, field
 from typing import List, Optional, Sequence
@@ -51,6 +53,14 @@ class _CRadial(C.Structure):
                 ("atom_moments", C.POINTER(C.c_double))]
 
 
+class _COccupation(C.Structure):
+    _fields_ = [("n", C.c_int), ("l", C.c_int), ("spin", C.c_int), ("occ", C.c_double)]
+
+
+class _CConfig(C.Structure):
+    _fields_ = [("n_orbitals", C.c_int), ("orb", _COccupation * (2 * MAX_LEVELS))]
+
+
 _RESULT_DTYPE = np.dtype(_CResult)      # numpy views of the C structs (same layout: built from the ctypes definitions)
 _STEP_DTYPE = np.dtype(_CStep)
 _LEVEL_IDX = np.arange(MAX_LEVELS)[None, None, :]
@@ -94,6 +104,9 @@ def load_library():
     lib.dftatom_solve_batch.argtypes = [C.c_void_p, C.POINTER(_COptions), C.c_int, C.POINTER(_CResult), C.POINTER(_CStep), C.c_int]
     lib.dftatom_solve_batch_radial.argtypes = [C.c_void_p, C.POINTER(_COptions), C.c_int, C.POINTER(_CResult), C.POINTER(_CStep), C.c_int,
                                                C.POINTER(_CRadial)]
+    lib.dftatom_config_aufbau.argtypes = [C.c_int, C.c_int, C.c_double, C.POINTER(_CConfig)]
+    lib.dftatom_solve_batch_config.argtypes = [C.c_void_p, C.POINTER(_COptions), C.POINTER(_CConfig), C.c_int, C.POINTER(_CResult),
+                                               C.POINTER(_CStep), C.c_int, C.POINTER(_CRadial)]
     lib.dftatom_radial_moments.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp]
     lib.dftatom_last_timing.argtypes = [C.c_void_p, _dp, C.POINTER(C.c_longlong)]
     lib.dftatom_last_graph_iterations.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
@@ -152,16 +165,35 @@ class Options:
     deltaGrid: float = 0.001
     alpha: float = 0.5
     method: int = 0          # 0 = LDA ("LSD" in the banner), 1 = LSDA; 2 / 3 = the same on the uniform grid (CalculateUniformLDA / LSDA)
+    # beyond the reference: an ion of the reference's configuration (config_aufbau; fractional allowed, < 0 = anion), or an explicit
+    # configuration - a list of (n, l, occ) (LDA) / (n, l, spin, occ) (LSDA) entries or a string for parse_config.  At most one of the two.
+    charge: float = 0.0
+    config: object = None
 
     def _c(self):
         return _COptions(int(self.Z), int(self.MultigridLevels), float(self.MaxR), float(self.deltaGrid), float(self.alpha), int(self.method))
+
+    @property
+    def configured(self) -> bool:
+        return self.config is not None or float(self.charge) != 0.0
+
+    def entries(self):
+        """The configuration the atom is solved with as (n, l, spin, occ) entries, or None for the reference's Aufbau atom."""
+        if self.config is not None and float(self.charge) != 0.0:
+            raise DFTAtomError(f"Options(Z={self.Z}): set either `charge` or `config`, not both")
+        if self.config is not None:
+            cfg = parse_config(self.config, self.method) if isinstance(self.config, str) else self.config
+            return [_entry4(e, self.method) for e in cfg]
+        if float(self.charge) != 0.0:
+            return [_entry4(e, self.method) for e in config_aufbau(self.Z, self.method, self.charge)]
+        return None
 
 
 @dataclass
 class Level:
     n: int
     l: int
-    occ: int
+    occ: int                 # a float for an atom solved with a configuration (Options.charge / config)
     nodes: int
     E: float = 0.0
 
@@ -246,13 +278,93 @@ class Radial:
     r2: float
 
 
-def orbital_count(Z: int, method: int = 0) -> int:
+def orbital_count(Z: int, method: int = 0, config=None, charge: float = 0.0) -> int:
     """Orbital rows of one atom in the radial export: its levels (dftatom_aufbau), or alpha plus beta levels (dftatom_split_spin) for
-    LSDA (method 1 / 3)."""
+    LSDA (method 1 / 3); for a configured atom (`config` or `charge`, as in Options) its configuration's entries."""
+    if config is not None or float(charge) != 0.0:
+        return len(Options(int(Z), method=int(method), charge=charge, config=config).entries())
     if int(method) & 1:
         a, b, _, _ = split_spin(Z)
         return len(a) + len(b)
     return len(aufbau(Z))
+
+
+def _entry4(e, method):
+    """(n, l, occ) -> (n, l, 0, occ); (n, l, spin, occ) as given."""
+    if len(e) == 3:
+        if int(method) & 1:
+            raise DFTAtomError(f"configuration entry {tuple(e)}: LSDA entries are (n, l, spin, occ)")
+        return (int(e[0]), int(e[1]), 0, float(e[2]))
+    if len(e) == 4:
+        return (int(e[0]), int(e[1]), int(e[2]), float(e[3]))
+    raise DFTAtomError(f"configuration entry {tuple(e)}: expected (n, l, occ) or (n, l, spin, occ)")
+
+
+def _as_method_form(entries, method):
+    return [(n, l, occ) for n, l, _, occ in entries] if not int(method) & 1 else list(entries)
+
+
+def config_aufbau(Z: int, method: int = 0, charge: float = 0.0):
+    """The reference's configuration of atom Z ionised by `charge` electrons (fractional allowed, < 0 = anion; dftatom_config_aufbau):
+    (n, l, occ) entries for LDA, (n, l, spin, occ) for LSDA (alpha then beta, each in (n, l) order)."""
+    cfg = _CConfig()
+    _check(load_library().dftatom_config_aufbau(int(Z), int(method), float(charge), C.byref(cfg)))
+    return _as_method_form([(cfg.orb[k].n, cfg.orb[k].l, cfg.orb[k].spin, cfg.orb[k].occ) for k in range(cfg.n_orbitals)], method)
+
+
+_CORES = {"He": 2, "Ne": 10, "Ar": 18, "Kr": 36, "Xe": 54, "Rn": 86}
+_TOKEN = re.compile(r"^(\d)([spdf])((?:\d+(?:\.\d*)?|\.\d+)(?:[eE][-+]?\d+)?)(?:/((?:\d+(?:\.\d*)?|\.\d+)(?:[eE][-+]?\d+)?))?$")
+
+
+def parse_config(s: str, method: int = 0):
+    """A configuration string: whitespace-separated subshells "2p4.5" (n, letter, occupation), in LSDA also "2p3/1" (alpha / beta), and
+    the cores [He] [Ne] [Ar] [Kr] [Xe] [Rn] (that atom's reference Aufbau configuration).  A total in LSDA is split like split_spin
+    (alpha min(occ, 2l + 1), beta the rest, beta listed only when nonzero).  A subshell given again replaces the earlier one (all of
+    its spins): "[Ne] 2p5 3s1" is the excited neon.  Returns the entries in the form Options.config takes for `method`."""
+    lsda = bool(int(method) & 1)
+    out = []
+    for tok in s.split():
+        m = re.fullmatch(r"\[([A-Z][a-z])\]", tok)
+        if m:
+            if m.group(1) not in _CORES:
+                raise DFTAtomError(f"configuration {s!r}: unknown core {tok} (use one of {' '.join('[' + k + ']' for k in _CORES)})")
+            core = [_entry4(e, method) for e in config_aufbau(_CORES[m.group(1)], method, 0.0)]
+            out = [e for e in out if (e[0], e[1]) not in {(c[0], c[1]) for c in core}] + core
+            continue
+        m = _TOKEN.match(tok)
+        if not m:
+            raise DFTAtomError(f"configuration {s!r}: cannot read {tok!r} (expected e.g. 3d10, 2p4.5, [Ar]" + (", 2p3/1)" if lsda else ")"))
+        n, l = int(m.group(1)), "spdf".index(m.group(2))
+        a = float(m.group(3))
+        out = [e for e in out if (e[0], e[1]) != (n, l)]
+        if m.group(4) is not None:
+            if not lsda:
+                raise DFTAtomError(f"configuration {s!r}: the alpha/beta form {tok!r} needs LSDA (method 1 or 3)")
+            out += [(n, l, 0, a), (n, l, 1, float(m.group(4)))]
+        elif lsda:
+            up = min(a, float(2 * l + 1))
+            out.append((n, l, 0, up))
+            if a - up > 0:
+                out.append((n, l, 1, a - up))
+        else:
+            out.append((n, l, 0, a))
+    out.sort(key=lambda e: (e[2], e[0], e[1]))
+    return _as_method_form(out, method)
+
+
+def format_config(config, method: int = 0) -> str:
+    """The string form of a configuration (inverse of parse_config: parse_config(format_config(c, m), m) == c for entries in the order
+    parse_config returns)."""
+    e4 = [_entry4(e, method) for e in config]
+    beta = {(n, l): occ for n, l, spin, occ in e4 if spin == 1}
+    g = lambda x: f"{x:.17g}"
+    out = []
+    for n, l, spin, occ in e4:
+        if spin == 1:
+            continue
+        sub = f"{n}{'spdf'[l]}"
+        out.append(f"{sub}{g(occ)}/{g(beta[(n, l)])}" if (n, l) in beta else f"{sub}{g(occ)}")
+    return " ".join(out)
 
 
 def _levels_from_c(arr, n):
@@ -324,15 +436,28 @@ class Context:
     # ---- L2 ----
     def solve_batch(self, options: Sequence[Options], keep_steps: bool = True, radial: bool = False) -> List[Result]:
         """One batch of independent atoms (dftatom_solve_batch).  radial=True: every Result also gets `radial` (a Radial: converged
-        density, potentials, orbitals and their moments, dftatom_solve_batch_radial)."""
+        density, potentials, orbitals and their moments, dftatom_solve_batch_radial).  Atoms with a `charge` or a `config` are solved
+        with that configuration (dftatom_solve_batch_config); their Level.occ is the exact occupation."""
         n = len(options)
         copts = (_COptions * n)(*[o._c() for o in options])
+        entries = [o.entries() for o in options]
+        ccfg = None
+        if any(e is not None for e in entries):
+            ccfg = (_CConfig * n)()
+            for a, e in enumerate(entries):
+                if e is None:
+                    continue
+                if len(e) > 2 * MAX_LEVELS:
+                    raise DFTAtomError(f"atom {a} (Z = {options[a].Z}): {len(e)} configuration entries, at most {2 * MAX_LEVELS}")
+                ccfg[a].n_orbitals = len(e)
+                for k, x in enumerate(e):
+                    ccfg[a].orb[k] = _COccupation(*x)
         cres = (_CResult * n)()
         stride = MAX_STEPS_LSDA if any(o.method for o in options) else MAX_STEPS_LDA
         csteps = (_CStep * (n * stride))() if keep_steps else None
         if radial and n:
             N = n_nodes(options[0].MultigridLevels)
-            rows = sum(orbital_count(o.Z, o.method) for o in options)
+            rows = sum(len(e) if e is not None else orbital_count(o.Z, o.method) for o, e in zip(options, entries))
             buf = np.zeros(N + n * 5 * N + n * 2 + rows * (N + N_MOMENTS))      # r | rho | V | V_H | atom moments | orbitals | moments
             r = buf[:N]
             rho = buf[N:N + 2 * n * N].reshape(n, 2, N)
@@ -343,7 +468,9 @@ class Context:
             orb = buf[q:q + rows * N].reshape(rows, N)
             mom = buf[q + rows * N:].reshape(rows, N_MOMENTS)
             crad = _CRadial(_d(r), _d(rho), _d(V), _d(VH), _d(orb), rows, _d(mom), _d(am))
-            _check(self._lib.dftatom_solve_batch_radial(self._h, copts, n, cres, csteps, stride if keep_steps else 0, C.byref(crad)))
+            _check(self._lib.dftatom_solve_batch_config(self._h, copts, ccfg, n, cres, csteps, stride if keep_steps else 0, C.byref(crad)))
+        elif ccfg is not None:
+            _check(self._lib.dftatom_solve_batch_config(self._h, copts, ccfg, n, cres, csteps, stride if keep_steps else 0, None))
         else:
             _check(self._lib.dftatom_solve_batch(self._h, copts, n, cres, csteps, stride if keep_steps else 0))
         # host structs -> Python objects in bulk (numpy structured views of the ctypes arrays: one pass in C instead of a ctypes
@@ -365,6 +492,10 @@ class Context:
                 q = p + nl[s]
                 lv.append(lev[p:q]); sl.append(sor[p:q])
                 p = q
+            if entries[a] is not None:         # the exact occupations (the C records hold them rounded)
+                occ = {(x[0], x[1], x[2]): x[3] for x in entries[a]}
+                lv = [[(t[0], t[1], occ[(t[0], t[1], s)]) + tuple(t[3:]) for t in ch] for s, ch in enumerate(lv)]
+                sl = [[(t[0], t[1], occ[(t[0], t[1], s)]) + tuple(t[3:]) for t in ch] for s, ch in enumerate(sl)]
             steps = []
             if keep_steps and n_steps:
                 blk = sa[a * stride:a * stride + n_steps]

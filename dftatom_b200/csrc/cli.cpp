@@ -12,7 +12,12 @@
 // --radial DIR: the converged radial state of every atom as a text table DIR/<index>_Z<Z>.tsv (index = position in --Z), one row per
 //           grid node at 17 digits: r, rho per spin, V per spin, V_H, u(r) of every orbital (dftatom_solve_batch_radial).  With --gpus
 //           every shard writes the files of its own atoms, named by their position in the whole --Z list.
+// --charge Q: every atom of --Z is the reference's configuration ionised by Q electrons (dftatom_config_aufbau; fractional allowed,
+//           < 0 = anion), e.g. --Z 1-92 --charge 1 for all cations.  --config "[Ne] 3s1 3p0": one atom (a single --Z) in that configuration
+//           (subshells "2p4.5", LSDA also "2p3/1" = alpha / beta, cores [He] .. [Rn]; the same string form as dftatom_b200.parse_config).
+//           Both are passed on to the shards of --gpus and select the rows of --radial.
 #include <algorithm>
+#include <cctype>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -66,9 +71,63 @@ static void read_ini(const char* path, dftatom_options& o)
     }
 }
 
-static void print_conf(const dftatom_level* lv, int n)
+// the exact occupation of a level: a configured atom's entry with the same (n, l, spin) (dftatom_level.occ holds it rounded)
+static double exact_occ(const dftatom_level& L, int spin, const dftatom_config* cfg)
 {
-    for (int k = 0; k < n; ++k) std::printf("%d%c%d ", lv[k].n, kOrb[lv[k].l], lv[k].occ);
+    for (int q = 0; cfg && q < cfg->n_orbitals; ++q)
+        if (cfg->orb[q].n == L.n && cfg->orb[q].l == L.l && cfg->orb[q].spin == spin) return cfg->orb[q].occ;
+    return L.occ;
+}
+
+// occupations with %g: integers print as the reference prints them
+static void print_conf(const dftatom_level* lv, int n, int spin, const dftatom_config* cfg)
+{
+    for (int k = 0; k < n; ++k) std::printf("%d%c%g ", lv[k].n, kOrb[lv[k].l], exact_occ(lv[k], spin, cfg));
+}
+
+// the string form of a configuration (dftatom_b200.parse_config): returns false with a message on stderr
+static bool parse_config(const std::string& s, int method, dftatom_config* out)
+{
+    static const struct { const char* sym; int Z; } kCores[] = { { "[He]", 2 }, { "[Ne]", 10 }, { "[Ar]", 18 }, { "[Kr]", 36 }, { "[Xe]", 54 }, { "[Rn]", 86 } };
+    const bool lsda = method & 1;
+    std::vector<dftatom_occupation> v;
+    auto drop = [&](int n, int l) { v.erase(std::remove_if(v.begin(), v.end(), [&](const dftatom_occupation& e) { return e.n == n && e.l == l; }), v.end()); };
+    size_t pos = 0;
+    while (pos < s.size()) {
+        while (pos < s.size() && std::isspace((unsigned char)s[pos])) ++pos;
+        if (pos >= s.size()) break;
+        size_t end = pos;
+        while (end < s.size() && !std::isspace((unsigned char)s[end])) ++end;
+        const std::string tok = s.substr(pos, end - pos);
+        pos = end;
+        int coreZ = 0;
+        for (const auto& c : kCores) if (tok == c.sym) coreZ = c.Z;
+        if (coreZ) {
+            dftatom_config core;
+            if (dftatom_config_aufbau(coreZ, method, 0., &core) != DFTATOM_OK) return false;
+            for (int q = 0; q < core.n_orbitals; ++q) drop(core.orb[q].n, core.orb[q].l);
+            v.insert(v.end(), core.orb, core.orb + core.n_orbitals);
+            continue;
+        }
+        const char* p = tok.c_str();
+        const char* lp = tok.size() >= 3 && std::isdigit((unsigned char)p[0]) ? std::strchr(kOrb, p[1]) : nullptr;
+        char* e1 = nullptr;
+        const double a = lp && p[1] ? std::strtod(p + 2, &e1) : 0.;
+        double b = -1.;
+        bool ok = lp && e1 && e1 != p + 2;
+        if (ok && *e1 == '/') { char* e2 = nullptr; b = std::strtod(e1 + 1, &e2); ok = lsda && e2 != e1 + 1 && *e2 == 0; }
+        else ok = ok && *e1 == 0;
+        if (!ok) { std::fprintf(stderr, "dftatom: --config: cannot read '%s' (expected e.g. 3d10, 2p4.5, [Ar]%s)\n", tok.c_str(), lsda ? ", 2p3/1" : ""); return false; }
+        const int n = p[0] - '0', l = (int)(lp - kOrb);
+        drop(n, l);
+        if (b >= 0.) { v.push_back({ n, l, 0, a }); v.push_back({ n, l, 1, b }); }
+        else if (lsda) { const double up = std::min(a, 2. * l + 1.); v.push_back({ n, l, 0, up }); if (a - up > 0.) v.push_back({ n, l, 1, a - up }); }
+        else v.push_back({ n, l, 0, a });
+    }
+    if (v.size() > 2 * DFTATOM_MAX_LEVELS) { std::fprintf(stderr, "dftatom: --config: too many subshells\n"); return false; }
+    out->n_orbitals = (int)v.size();
+    std::copy(v.begin(), v.end(), out->orb);
+    return true;
 }
 
 // --gpus N: one child process per GPU (CUDA is only ever initialised in the children), each solving its shard as one batch.
@@ -178,7 +237,8 @@ int main(int argc, char** argv)
 {
     dftatom_options base = { 36, 12, 10.0, 0.001, 0.5, 0 };     // Options.cpp:6
     std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
-    std::string radial_dir;
+    std::string radial_dir, config_str;
+    double charge = 0.;
     int precision = 6, device = 0, gpus = 1;
     bool json = false, quiet = false, framed = false;      // framed: child of --gpus (one frame per atom on stdout)
     std::vector<std::string> passthrough;                   // flags a --gpus parent hands to its children unchanged
@@ -191,6 +251,8 @@ int main(int argc, char** argv)
         else if (a == "--framed") framed = true;
         else if (a == "--atom-index") atom_index = parse_z(next());
         else if (a == "--radial") radial_dir = next();
+        else if (a == "--charge") charge = std::atof(next());
+        else if (a == "--config") config_str = next();
         else if (a == "--levels") base.levels = std::atoi(next());
         else if (a == "--delta") base.delta = std::atof(next());
         else if (a == "--mixing" || a == "--alpha") base.mixing = std::atof(next());
@@ -207,13 +269,16 @@ int main(int argc, char** argv)
         else if (a == "--quiet-steps") quiet = true;
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
-                        "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR]\n"
-                        "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n");
+                        "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR] [--charge Q] [--config \"...\"]\n"
+                        "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n"
+                        "  --charge Q    solve every atom of --Z ionised by Q electrons (the reference's configuration; fractional allowed, < 0 = anion)\n"
+                        "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
         if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
     }
     if (zs.empty()) zs.push_back(base.Z);
+    if (!config_str.empty() && (zs.size() != 1 || charge != 0.)) { std::fprintf(stderr, "dftatom: --config needs a single --Z and no --charge\n"); return 2; }
     if (!atom_index.empty() && atom_index.size() != zs.size()) { std::fprintf(stderr, "dftatom: --atom-index needs one index per --Z entry\n"); return 2; }
     if (!radial_dir.empty() && mkdir(radial_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(radial_dir.c_str()); return 1; }
     if (gpus > 1) {
@@ -226,6 +291,15 @@ int main(int argc, char** argv)
     const int n = (int)zs.size();
     std::vector<dftatom_options> opts(n, base);
     for (int k = 0; k < n; ++k) opts[k].Z = zs[k];
+    // --charge / --config: every atom's configuration (none: the reference's Aufbau atom, dftatom_solve_batch_radial's arguments)
+    const bool configured = charge != 0. || !config_str.empty();
+    std::vector<dftatom_config> cfgs(configured ? n : 0);
+    for (int k = 0; k < n && configured; ++k) {
+        if (!config_str.empty() ? !parse_config(config_str, base.method, &cfgs[k]) : dftatom_config_aufbau(opts[k].Z, base.method, charge, &cfgs[k]) != DFTATOM_OK) {
+            if (config_str.empty()) std::fprintf(stderr, "dftatom: %s\n", dftatom_last_error());
+            return 2;
+        }
+    }
 
     dftatom_ctx* ctx = nullptr;
     if (dftatom_create(&ctx, device) != DFTATOM_OK) { std::fprintf(stderr, "dftatom: %s\n", dftatom_last_error()); return 1; }
@@ -238,7 +312,8 @@ int main(int argc, char** argv)
     for (int k = 0; k < n && !radial_dir.empty(); ++k) {
         dftatom_level la[DFTATOM_MAX_LEVELS], lb[DFTATOM_MAX_LEVELS];
         int na = 0, nb = 0, ea = 0, eb = 0;
-        if (opts[k].method & 1) dftatom_split_spin(opts[k].Z, la, &na, lb, &nb, &ea, &eb);
+        if (configured) na = cfgs[k].n_orbitals;
+        else if (opts[k].method & 1) dftatom_split_spin(opts[k].Z, la, &na, lb, &nb, &ea, &eb);
         else na = std::max(0, dftatom_aufbau(opts[k].Z, la, DFTATOM_MAX_LEVELS));
         row0[k + 1] = row0[k] + na + nb;
     }
@@ -248,7 +323,8 @@ int main(int argc, char** argv)
         r_grid.resize(N); rho.resize((size_t)n * 2 * N); vks.resize((size_t)n * 2 * N); vh.resize((size_t)n * N); orb.resize((size_t)row0[n] * N);
         rad.r = r_grid.data(); rad.rho = rho.data(); rad.v = vks.data(); rad.v_hartree = vh.data(); rad.orbitals = orb.data(); rad.orbital_rows = row0[n];
     }
-    if (dftatom_solve_batch_radial(ctx, opts.data(), n, res.data(), steps.data(), stride, radial_dir.empty() ? nullptr : &rad) != DFTATOM_OK) {
+    if (dftatom_solve_batch_config(ctx, opts.data(), configured ? cfgs.data() : nullptr, n, res.data(), steps.data(), stride,
+                                   radial_dir.empty() ? nullptr : &rad) != DFTATOM_OK) {
         std::fprintf(stderr, "dftatom: %s\n", dftatom_last_error());
         dftatom_destroy(ctx);
         return 1;
@@ -270,10 +346,18 @@ int main(int argc, char** argv)
             for (int s = 0; s < R.n_spin; ++s)
                 for (int k = 0; k < R.n_levels[s]; ++k) {
                     const dftatom_level& L = R.levels[s][k];
-                    std::printf("%s{\"spin\":%d,\"n\":%d,\"l\":%d,\"occ\":%d,\"nodes\":%d,\"E\":%.17g}", first ? "" : ",", s, L.n, L.l, L.occ, L.nodes, L.E);
+                    if (configured)
+                        std::printf("%s{\"spin\":%d,\"n\":%d,\"l\":%d,\"occ\":%.17g,\"nodes\":%d,\"E\":%.17g}", first ? "" : ",", s, L.n, L.l,
+                                    exact_occ(L, s, &cfgs[a]), L.nodes, L.E);
+                    else std::printf("%s{\"spin\":%d,\"n\":%d,\"l\":%d,\"occ\":%d,\"nodes\":%d,\"E\":%.17g}", first ? "" : ",", s, L.n, L.l, L.occ, L.nodes, L.E);
                     first = false;
                 }
             std::printf("]");
+            if (configured) {    // the atom's net charge Z - sum occ
+                double q = 0.;
+                for (int k = 0; k < cfgs[a].n_orbitals; ++k) q += cfgs[a].orb[k].occ;
+                std::printf(",\"charge\":%.17g", opts[a].Z - q);
+            }
             if (!quiet) {       // every "Step:" block of the reference's log, full precision
                 std::printf(",\"steps\":[");
                 for (int sp = 0; sp < R.n_steps; ++sp) {
@@ -306,9 +390,10 @@ int main(int argc, char** argv)
             else std::printf("********************************************************************************\n");
         }
         if (opts[a].method & 1) {
-            std::printf("Alpha: "); print_conf(R.sorted[0], R.n_levels[0]);
-            std::printf("\nBeta: "); print_conf(R.sorted[1], R.n_levels[1]);
-        } else print_conf(R.sorted[0], R.n_levels[0]);
+            const dftatom_config* cf = configured ? &cfgs[a] : nullptr;
+            std::printf("Alpha: "); print_conf(R.sorted[0], R.n_levels[0], 0, cf);
+            std::printf("\nBeta: "); print_conf(R.sorted[1], R.n_levels[1], 1, cf);
+        } else print_conf(R.sorted[0], R.n_levels[0], 0, configured ? &cfgs[a] : nullptr);
         std::printf("\n");
     }
     if (json && !framed) std::printf("]\n");

@@ -382,6 +382,7 @@ int dftatom_set_option(dftatom_ctx* c, const char* key, double value)
 }
 
 int dftatom_aufbau(int Z, dftatom_level* out, int max_out) { return dft::aufbau(Z, out, max_out); }
+int dftatom_config_aufbau(int Z, int method, double charge, dftatom_config* out) { return dft::config_aufbau(Z, method, charge, out); }
 int dftatom_split_spin(int Z, dftatom_level* a, int* na, dftatom_level* b, int* nb, int* ea, int* eb)
 {
     return dft::split_spin(Z, a, na, b, nb, ea, eb);
@@ -499,8 +500,8 @@ static int export_radial(dftatom_ctx* c, const GridDev& g, const ScfBuffers& b, 
 }
 
 // one group of atoms: its whole SCF, enqueued on the context's stream
-static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
-                       int steps_stride, const RadialDest* rd = nullptr)
+static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftatom_config* cfgs, int n_atoms, dftatom_result* out,
+                       dftatom_step* steps, int steps_stride, const RadialDest* rd = nullptr)
 {
     if (!c || !opts || !out || n_atoms <= 0) { set_error("bad argument"); return DFTATOM_E_ARG; }
     const bool host_dbg = getenv("DFTATOM_DEBUG_HOST") != nullptr;      // development aid: wall-clock of the host-side stages
@@ -531,7 +532,8 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
     std::vector<AtomDev> atoms(n_atoms);
     std::vector<AtomState> astate(n_atoms);
     std::vector<OrbitalDev> orbs;
-    std::vector<int> tab_of(2 * (size_t)n_atoms, -1), zbc(n_atoms);
+    std::vector<int> tab_of(2 * (size_t)n_atoms, -1);
+    std::vector<double> zbc(n_atoms);
     std::vector<std::vector<dftatom_level>> lev_a(n_atoms), lev_b(n_atoms);
     int n_tabs = 0, max_steps = 0, zmax = 1;
     for (int a = 0; a < n_atoms; ++a) {
@@ -542,20 +544,18 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
         at.mixing = opts[a].mixing;
         max_steps = std::max(max_steps, at.n_steps_max);
         zmax = std::max(zmax, at.Z);
-        zbc[a] = at.Z;
-        dftatom_level la[DFTATOM_MAX_LEVELS], lb[DFTATOM_MAX_LEVELS];
-        int na = 0, nb = 0, ea = at.Z, eb = 0;
-        if (at.method) { rc = split_spin(at.Z, la, &na, lb, &nb, &ea, &eb); if (rc) return rc; }
-        else { na = aufbau(at.Z, la, DFTATOM_MAX_LEVELS); if (na < 0) return na; }
-        lev_a[a].assign(la, la + na); lev_b[a].assign(lb, lb + nb);
-        at.n_el[0] = ea; at.n_el[1] = eb;
+        AtomLevels al;
+        if ((rc = atom_levels(a, opts[a], cfgs ? &cfgs[a] : nullptr, &al))) return rc;
+        lev_a[a] = al.lev[0]; lev_b[a] = al.lev[1];
+        at.n_el[0] = al.n_el[0]; at.n_el[1] = al.n_el[1];
+        zbc[a] = al.n_el[0] + al.n_el[1];                    // U(Rmax) = the electron count Q (Z for the neutral atom)
         for (int s = 0; s < at.n_spin; ++s) {
             tab_of[2 * a + s] = n_tabs;
             at.orb_begin[s] = (int)orbs.size();
-            const auto& L = s ? lev_b[a] : lev_a[a];
+            const auto& L = al.lev[s];
             at.orb_count[s] = (int)L.size();
-            for (const auto& x : L) {
-                OrbitalDev o; o.atom = a; o.spin = s; o.n0 = x.n - 1; o.l = x.l; o.occ = x.occ; o.want = x.nodes; o.tab = n_tabs;
+            for (size_t k = 0; k < L.size(); ++k) {
+                OrbitalDev o; o.atom = a; o.spin = s; o.n0 = L[k].n - 1; o.l = L[k].l; o.occ = al.occ[s][k]; o.want = L[k].nodes; o.tab = n_tabs;
                 orbs.push_back(o);
             }
             ++n_tabs;
@@ -567,7 +567,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
     const int stride = max_steps;
     c->last_graph_iterations = 0;
     c->last_h2d_bytes = (long long)(sizeof(AtomDev) * atoms.size() + sizeof(AtomState) * astate.size() + sizeof(OrbitalDev) * orbs.size()
-                                    + sizeof(int) * (tab_of.size() + zbc.size() + 2));
+                                    + sizeof(int) * (tab_of.size() + 2) + sizeof(double) * zbc.size());
 
     // ---- device buffers ----
     if ((rc = upload_arena_reset(c, (size_t)c->last_h2d_bytes + 64 * 8))) return rc;
@@ -613,7 +613,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
     b.atoms = c->atoms.as<AtomDev>(); b.astate = c->astate.as<AtomState>(); b.orbs = c->orbs.as<OrbitalDev>();
     b.ss = c->ss.as<SearchState>(); b.rho = c->rho.as<double>(); b.rhot = c->rhot.as<double>(); b.vpot = c->vpot.as<double>();
     b.atab = c->atab.as<double>(); b.psi = c->psi.as<double>(); b.match_pt = c->match_pt.as<int>(); b.inv_norm = c->inv_norm.as<double>(); b.epart = c->epart.as<double>(); b.eticket = c->eticket.as<int>();
-    b.phi = c->phi.as<double>(); b.src = c->src.as<double>(); b.U = c->ubuf.as<double>(); b.ldU = ldU; b.Zbc = c->zbc.as<int>(); b.tab_of = c->tab_of.as<int>();
+    b.phi = c->phi.as<double>(); b.src = c->src.as<double>(); b.U = c->ubuf.as<double>(); b.ldU = ldU; b.Zbc = c->zbc.as<double>(); b.tab_of = c->tab_of.as<int>();
     b.steps = c->steps.as<dftatom_step>(); b.steps_stride = stride; b.n_active = c->n_active.as<int>();
     b.run_to_cap = c->k.run_to_cap; b.adaptive_mixing = c->k.adaptive_mixing;
 
@@ -724,20 +724,20 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, int n_atoms,
     DFT_CHECK(cudaEventRecord(ev0, st));
     // initial guess -> U -> V   (DFTAtom.cpp:371-392)
     launch_initial_density(g, b, st); ++launches;
-    // The start density is n_el / volume on every node but the first and the boundary value is Z: A U = S is linear in Z.  One cold solve of
-    // the Z = 1 problem per grid (the same kernel, the same cycle), U_atom = Z U_1 afterwards.
+    // The start density is n_el / volume on every node but the first and the boundary value is the electron count Q: A U = S is linear in
+    // Q.  One cold solve of the Q = 1 problem per grid (the same kernel, the same cycle), U_atom = Q U_1 afterwards.
     const bool unit_guess = c->k.unit_guess && !exact && !stream && !g.uniform && g.L <= 14 && gentry != nullptr;
     if (unit_guess) {
         if (!gentry->u_unit_ok) {
             if ((rc = gentry->u_unit.ensure(sizeof(double) * (size_t)(2 * N + 2)))) return rc;
             double* u1 = gentry->u_unit.as<double>();
             double* rho1 = u1 + N;
-            int* one = reinterpret_cast<int*>(rho1 + N);
+            double* one = rho1 + N;
             std::vector<double> h1((size_t)N, 1. / (4. * M_PI / 3. * g.max_r * g.max_r * g.max_r));
             h1[0] = 0.;
-            const int h_one = 1;
+            const double h_one = 1.;
             DFT_CHECK(cudaMemcpyAsync(rho1, h1.data(), sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, st));
-            DFT_CHECK(cudaMemcpyAsync(one, &h_one, sizeof(int), cudaMemcpyHostToDevice, st));
+            DFT_CHECK(cudaMemcpyAsync(one, &h_one, sizeof(double), cudaMemcpyHostToDevice, st));
             DFT_CHECK(cudaStreamSynchronize(st));                       // (h1, h_one are pageable locals)
             PoissonArgs p1 = pa;
             p1.n_dens = 1; p1.rho = rho1; p1.src_nat = nullptr; p1.u_out = u1; p1.nat_stride = 0; p1.Zbc = one; p1.skip = nullptr; p1.skip_stride_bytes = 0;
@@ -970,7 +970,20 @@ int dftatom_solve_batch(dftatom_ctx* c, const dftatom_options* opts, int n_atoms
 int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
                                int steps_stride, const dftatom_radial* radial)
 {
+    return dftatom_solve_batch_config(c, opts, nullptr, n_atoms, out, steps, steps_stride, radial);
+}
+
+int dftatom_solve_batch_config(dftatom_ctx* c, const dftatom_options* opts, const dftatom_config* configs, int n_atoms, dftatom_result* out,
+                               dftatom_step* steps, int steps_stride, const dftatom_radial* radial)
+{
     if (!c || !opts || !out || n_atoms <= 0) { set_error("bad argument"); return DFTATOM_E_ARG; }
+    // every configuration is checked before anything is solved (solve_group checks them again per group)
+    if (configs)
+        for (int a = 0; a < n_atoms; ++a) {
+            int rc = validate(opts[a]);
+            AtomLevels al;
+            if (rc || (rc = atom_levels(a, opts[a], &configs[a], &al))) return rc;
+        }
     // radial export: the first orbital row of every atom in the caller's arrays, and the capacity check before anything is solved
     std::vector<int> dest_atom;
     std::vector<long long> dest_row;
@@ -979,13 +992,11 @@ int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int 
         for (int a = 0; a < n_atoms; ++a) {
             int rc = validate(opts[a]);
             if (rc) return rc;
-            dftatom_level la[DFTATOM_MAX_LEVELS], lb[DFTATOM_MAX_LEVELS];
-            int na = 0, nb = 0, ea = 0, eb = 0;
-            if (opts[a].method & 1) { rc = split_spin(opts[a].Z, la, &na, lb, &nb, &ea, &eb); if (rc) return rc; }
-            else { na = aufbau(opts[a].Z, la, DFTATOM_MAX_LEVELS); if (na < 0) return na; }
+            AtomLevels al;
+            if ((rc = atom_levels(a, opts[a], configs ? &configs[a] : nullptr, &al))) return rc;
             dest_atom.push_back(a);
             dest_row.push_back(rows);
-            rows += na + nb;
+            rows += (long long)(al.lev[0].size() + al.lev[1].size());
         }
         if ((radial->orbitals || radial->moments) && radial->orbital_rows < rows) {
             set_error("dftatom_radial.orbital_rows is " + std::to_string(radial->orbital_rows) + ", the batch has " + std::to_string(rows) + " orbitals");
@@ -994,8 +1005,8 @@ int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int 
     }
     const RadialDest rd_all{ radial, dest_atom.data(), dest_row.data(), true };
     const RadialDest* rd = radial ? &rd_all : nullptr;
-    if (c->stream_groups < 2 || n_atoms < 32) return solve_group(c, opts, n_atoms, out, steps, steps_stride, rd);
-    if (opts[0].levels > 14) return solve_group(c, opts, n_atoms, out, steps, steps_stride, rd);      // (large grids: one group - the stream-mode Poisson solver wants all densities in one launch)
+    if (c->stream_groups < 2 || n_atoms < 32) return solve_group(c, opts, configs, n_atoms, out, steps, steps_stride, rd);
+    if (opts[0].levels > 14) return solve_group(c, opts, configs, n_atoms, out, steps, steps_stride, rd);      // (large grids: one group - the stream-mode Poisson solver wants all densities in one launch)
     for (int a = 0; a < n_atoms; ++a) {
         int rc = validate(opts[a]);
         if (rc) return rc;
@@ -1012,7 +1023,8 @@ int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int 
         p->child->k = c->k; p->child->stream_groups = 1;
         ctxs.push_back(p->child);
     }
-    // deal the atoms in order of decreasing cost (orbital count ~ Z; LSDA doubles it) round-robin into the groups
+    // deal the atoms in order of decreasing cost (orbital count ~ Z; LSDA doubles it) round-robin into the groups; a configured atom keeps the
+    // key of its Z (it only balances the groups), so every batch of neutral atoms keeps its grouping
     std::vector<int> order(n_atoms);
     std::iota(order.begin(), order.end(), 0);
     std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return opts[x].Z * (1 + (opts[x].method & 1)) > opts[y].Z * (1 + (opts[y].method & 1)); });
@@ -1020,10 +1032,12 @@ int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int 
     for (int q = 0; q < n_atoms; ++q) idx[q % G].push_back(order[q]);
     for (auto& v : idx) std::sort(v.begin(), v.end());
     std::vector<std::vector<dftatom_options>> gopts(G);
+    std::vector<std::vector<dftatom_config>> gcfg(G);
     std::vector<std::vector<dftatom_result>> gout(G);
     std::vector<std::vector<dftatom_step>> gsteps(G);
     for (int gI = 0; gI < G; ++gI) {
         for (int a : idx[gI]) gopts[gI].push_back(opts[a]);
+        if (configs) for (int a : idx[gI]) gcfg[gI].push_back(configs[a]);
         gout[gI].resize(idx[gI].size());
         if (steps) gsteps[gI].resize(idx[gI].size() * (size_t)steps_stride);
     }
@@ -1040,11 +1054,11 @@ int dftatom_solve_batch_radial(dftatom_ctx* c, const dftatom_options* opts, int 
     std::vector<std::thread> th;
     for (int gI = 1; gI < G; ++gI)
         th.emplace_back([&, gI]() {
-            rcs[gI] = solve_group(ctxs[gI], gopts[gI].data(), (int)gopts[gI].size(), gout[gI].data(), steps ? gsteps[gI].data() : nullptr, steps_stride,
+            rcs[gI] = solve_group(ctxs[gI], gopts[gI].data(), configs ? gcfg[gI].data() : nullptr, (int)gopts[gI].size(), gout[gI].data(), steps ? gsteps[gI].data() : nullptr, steps_stride,
                                   radial ? &grd[gI] : nullptr);
             if (rcs[gI]) errs[gI] = g_err;
         });
-    rcs[0] = solve_group(c, gopts[0].data(), (int)gopts[0].size(), gout[0].data(), steps ? gsteps[0].data() : nullptr, steps_stride, radial ? &grd[0] : nullptr);
+    rcs[0] = solve_group(c, gopts[0].data(), configs ? gcfg[0].data() : nullptr, (int)gopts[0].size(), gout[0].data(), steps ? gsteps[0].data() : nullptr, steps_stride, radial ? &grd[0] : nullptr);
     for (auto& t : th) t.join();
     if (rcs[0]) return rcs[0];
     for (int gI = 1; gI < G; ++gI) if (rcs[gI]) { set_error(errs[gI]); return rcs[gI]; }
@@ -1248,12 +1262,13 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
     const PoissonLevels lv = make_levels(levels);
     DevBuf& dr = c->scratch[0]; DevBuf& dz = c->scratch[2]; DevBuf& dv = c->scratch[3];
-    if ((rc = dr.ensure(sizeof(double) * (size_t)n_dens * N)) || (rc = dz.ensure(sizeof(int) * n_dens)) || (rc = dv.ensure(sizeof(int) * n_dens))) return rc;
+    if ((rc = dr.ensure(sizeof(double) * (size_t)n_dens * N)) || (rc = dz.ensure(sizeof(double) * n_dens)) || (rc = dv.ensure(sizeof(int) * n_dens))) return rc;
     if ((rc = c->phi.ensure(sizeof(double) * (size_t)n_dens * lv.total)) || (rc = c->src.ensure(sizeof(double) * (size_t)n_dens * lv.total))) return rc;
+    const std::vector<double> zbc(Z, Z + n_dens);            // the solvers take the boundary value as a double (an electron count)
     DFT_CHECK(cudaMemcpyAsync(dr.p, rho, sizeof(double) * (size_t)n_dens * N, cudaMemcpyHostToDevice, st));
-    DFT_CHECK(cudaMemcpyAsync(dz.p, Z, sizeof(int) * n_dens, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dz.p, zbc.data(), sizeof(double) * n_dens, cudaMemcpyHostToDevice, st));
     PoissonArgs pa{};
-    pa.n_dens = n_dens; pa.rho = dr.as<double>(); pa.Zbc = dz.as<int>(); pa.phi = c->phi.as<double>(); pa.src = c->src.as<double>();
+    pa.n_dens = n_dens; pa.rho = dr.as<double>(); pa.Zbc = dz.as<double>(); pa.phi = c->phi.as<double>(); pa.src = c->src.as<double>();
     pa.max_vcycles = c->k.max_vcycles; pa.floor_stop = c->k.floor_stop; pa.vcycles_used = dv.as<int>();
     if ((rc = c->u0.ensure(sizeof(double) * (size_t)n_dens * N)) || (rc = c->ubuf.ensure(sizeof(double) * (size_t)n_dens * N))) return rc;
     pa.refine_vcycles = c->k.refine_vcycles; pa.u0 = c->u0.as<double>(); pa.u_out = c->ubuf.as<double>(); pa.coarse_op = g.coarse_op; pa.n_sm = c->n_sm;
@@ -1270,7 +1285,7 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
         if ((rc = c->exact_work.ensure(sizeof(double) * (size_t)n_dens * (size_t)exact_poisson_work_doubles(levels)))) return rc;
         ExactPoissonArgs xa{};
         xa.n_dens = n_dens; xa.L = levels; xa.delta = delta; xa.rho = dr.as<double>(); xa.rho_stride = N; xa.r = g.r; xa.pex = g.pex;
-        xa.Zbc = dz.as<int>(); xa.U = c->ubuf.as<double>(); xa.ldU = N; xa.work = c->exact_work.as<double>(); xa.max_vcycles = 100;
+        xa.Zbc = dz.as<double>(); xa.U = c->ubuf.as<double>(); xa.ldU = N; xa.work = c->exact_work.as<double>(); xa.max_vcycles = 100;
         xa.vcycles_used = dv.as<int>();
         launch_poisson_exact(xa, st);
         DFT_CHECK(cudaMemcpyAsync(U, c->ubuf.p, sizeof(double) * (size_t)n_dens * N, cudaMemcpyDeviceToHost, st));
@@ -1288,7 +1303,7 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
         if ((rc = c->ubuf.ensure(sizeof(double) * (size_t)n_dens * ld))) return rc;
         StreamSolveArgs sa{};
         sa.n_dens = n_dens; sa.rho = dr.as<double>(); sa.rho_stride = N; sa.psrc = g.psrc; sa.src0 = c->stream_src0.as<double>();
-        sa.U = c->ubuf.as<double>(); sa.ld0 = ld; sa.Zbc = dz.as<int>(); sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op;
+        sa.U = c->ubuf.as<double>(); sa.ld0 = ld; sa.Zbc = dz.as<double>(); sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op;
         sa.n_v = c->k.max_vcycles; sa.warm = 0; sa.variant = c->k.stream_variant;
         launch_poisson_stream_solve(splan, delta, sa, st, nullptr);
         DFT_CHECK(cudaMemcpy2DAsync(U, sizeof(double) * N, c->ubuf.p, sizeof(double) * ld, sizeof(double) * N, n_dens, cudaMemcpyDeviceToHost, st));

@@ -46,7 +46,8 @@ struct GridDev {
 
 // One orbital = one (atom, spin, n, l) level; also the unit of the batched energy search.
 struct OrbitalDev {
-    int atom, spin, n0, l, occ;
+    int atom, spin, n0, l;
+    double occ;          // electrons in this (spin) orbital; 0: solved and exported, not in the density
     int want;            // n0 - l = number of nodes (DFTAtom.cpp:497)
     int tab;             // index of the (atom,spin) table row
 };
@@ -69,7 +70,7 @@ struct AtomDev {
     int Z, method, n_spin, n_steps_max;
     double mixing;
     int orb_begin[2], orb_count[2];
-    int n_el[2];
+    double n_el[2];      // electrons per spin: the configuration's (Z for the neutral Aufbau atom)
 };
 
 struct AtomState {
@@ -145,7 +146,7 @@ struct PoissonArgs {
     const double* src_nat;  // [n_dens][N] Source_0 in natural node order, used when rho is NULL (or NULL)
     double* u_out;          // [n_dens][N] result U(r) = Phi_0 in natural node order (or NULL)
     long long nat_stride;   // row stride of rho / src_nat / u_out / u0 in doubles (0: N)
-    const int* Zbc;         // [n_dens] boundary value at Rmax (may be NULL: use hi_bc)
+    const double* Zbc;      // [n_dens] boundary value at Rmax = electron count (may be NULL: use hi_bc)
     double* phi; double* src;   // [n_dens][levels.total] the hierarchy, thread-major node order inside a level (poisson.cu)
     const int* skip;        // optional per-density skip flag (AtomState.done), stride given
     int skip_stride_bytes;
@@ -165,8 +166,8 @@ struct PoissonArgs {
 };
 void launch_coarse_op(int L, double delta, double* G, cudaStream_t st);
 void launch_poisson_full(const GridDev& g, const PoissonLevels& lv, const PoissonArgs& a, cudaStream_t st);
-// U[k][i] = Z[k] u1[i]: the Poisson solve of the SCF's start density from the solution of the Z = 1 problem (engine.cpp: unit_guess)
-void launch_scale_unit_potential(int N, int n_dens, int ldU, const double* u1, const int* Z, double* U, cudaStream_t st);
+// U[k][i] = Q[k] u1[i]: the Poisson solve of the SCF's start density from the solution of the Z = 1 problem (engine.cpp: unit_guess)
+void launch_scale_unit_potential(int N, int n_dens, int ldU, const double* u1, const double* Q, double* U, cudaStream_t st);
 void launch_poisson_vcycles(const PoissonLevels& lv, double delta, int n_dens, double* phi, double* src, double* phi_nat,
                             const double* src_nat, int n_cycles, double* last_err, cudaStream_t st);
 
@@ -209,7 +210,7 @@ struct StreamSolveArgs {
     int n_dens;
     const double* rho; long long rho_stride; const double* psrc;    // optional: densities [n_dens][rho_stride] and the grid's r 4 pi K table
     double* src0; double* U; long long ld0;                         // level 0: Source_0 and the solution U(r) = Phi_0, rows of ld0 doubles
-    const int* Zbc;                                                 // [n_dens] boundary value at Rmax
+    const double* Zbc;                                              // [n_dens] boundary value at Rmax
     double* scratch; const double* coarse_op;
     int n_v, warm, variant;
     const int* skip; int skip_stride_bytes;
@@ -222,7 +223,7 @@ struct ExactPoissonArgs {
     double delta;            // deltaGrid (0: uniform grid)
     const double* rho; long long rho_stride;    // [n_dens][rho_stride] densities, natural node order
     const double* r; const double* pex;         // grid tables (GridDev.r, GridDev.pex)
-    const int* Zbc;          // [n_dens] boundary value at Rmax
+    const double* Zbc;       // [n_dens] boundary value at Rmax
     double* U; long long ldU;                   // [n_dens][ldU] result
     double* work;            // n_dens * exact_poisson_work_doubles(L) doubles
     const int* skip; int skip_stride_bytes;
@@ -239,7 +240,7 @@ struct WarmPoissonArgs {
     double* rho_prev;                           // [n_dens][rho_stride], in / out: the density of the previous solve.  Increment form: the solve is
                                                 // A dU = -r 4 pi K (rho - rho_prev) from dU = 0 and U += dU (see scf.cu)
     double* U; long long ldU;                   // [n_dens][ldU] in: previous solution, out: U(r)
-    const int* Zbc;                             // [n_dens] boundary value at Rmax
+    const double* Zbc;                          // [n_dens] boundary value at Rmax
     const double* coarse_tri;                   // GridDev.coarse_tri (poisson_warm.cu): the levels below 2048 nodes are replaced by the exact solve of
                                                 // the 1024-node level (poisson_tri.cuh)
     const int* skip; int skip_stride_bytes;
@@ -289,7 +290,7 @@ struct ScfBuffers {
     double* phi; double* src;   // Poisson hierarchy [n_atoms][levels.total]
     double* U;        // [n_atoms][ldU] Hartree U(r) = r V_H, natural node order (output of the Poisson solve)
     int ldU;          // row stride of U (N, or N rounded up to a multiple of 4 when the stream-mode Poisson solver writes it)
-    int* Zbc;         // [n_atoms]
+    double* Zbc;      // [n_atoms] boundary value of the Poisson solves = electron count Q
     int* tab_of;      // [n_atoms][2] table row of (atom, spin) or -1
     dftatom_step* steps;  // [n_atoms][steps_stride]
     int steps_stride;
@@ -338,6 +339,15 @@ void launch_radial_fields(const GridDev& g, const ScfBuffers& b, double* rho_out
 // host rules (aufbau.cpp)
 int aufbau(int Z, dftatom_level* out, int max_out);
 int split_spin(int Z, dftatom_level* a, int* na, dftatom_level* b, int* nb, int* ea, int* eb);
+int config_aufbau(int Z, int method, double charge, dftatom_config* out);
+// the orbitals one atom is solved with: its configuration (cfg != NULL with n_orbitals > 0; validated, each spin sorted into (n, l)
+// order, level.occ = occ rounded) or the reference's Aufbau levels; occ = the exact occupations, n_el = electrons per spin
+struct AtomLevels {
+    std::vector<dftatom_level> lev[2];
+    std::vector<double> occ[2];
+    double n_el[2];
+};
+int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, AtomLevels* out);
 double estimate_cost(int Z, int method);
 int partition_atoms(const int* Z, const int* method, int n, int n_ranks, int* rank_of);
 

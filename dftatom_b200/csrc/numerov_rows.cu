@@ -624,12 +624,13 @@ __global__ void __launch_bounds__(32 * NW, NW == kRowWarps ? 3 : 1) search_rows_
         const int sc = astate[ob.atom].n_steps;
         const double mix = atoms[ob.atom].mixing;
         if (sc == 0 && !warm) {
-            // step 0: the initial density is a uniform sphere of radius MaxR (DFTAtom.cpp:371-376): V = -Z/r + 3Z/(2 MaxR) - Z r^2/(2 MaxR^3) + v_xc
-            // of a density of ~1e-3: hydrogenic levels shifted by 3Z/(2 MaxR) - ~0.1
+            // step 0: the initial density is a uniform sphere of Q electrons and radius MaxR (DFTAtom.cpp:371-376): V = -Z/r + 3Q/(2 MaxR)
+            // - Q r^2/(2 MaxR^3) + v_xc of a density of ~1e-3: hydrogenic levels shifted by 3Q/(2 MaxR) - ~0.1
             const double nq = (double)(ob.want + ob.l + 1);
             const double hyd = Z * Z / (2. * nq * nq);
+            const double Q = atoms[ob.atom].n_el[0] + atoms[ob.atom].n_el[1];
             b.mode = kLadder;
-            b.c_est = fmin(fmax(-hyd + 1.5 * Z / g.max_r - 0.1, b.lo), b.hi);
+            b.c_est = fmin(fmax(-hyd + 1.5 * Q / g.max_r - 0.1, b.lo), b.hi);
             b.inner = 0.1; b.radius = 0.4 + 0.002 * hyd;
         } else if (warm && sc == 1) {
             // step 1: the first real density screens the nucleus: every level rises by about (1 - mixing) x (|E| + 2); samples on that side only

@@ -1251,7 +1251,7 @@ __global__ void __launch_bounds__(kPT) poisson_full_kernel(GridDev g, PoissonLev
         if (leader) {
             if (threadIdx.x == 0) {
                 Ref::P(c).st(0, 0.);                                          // SetBoundaries(0, Z), PoissonSolver.h:76
-                Ref::P(c).st(g_sm.lc[c].n, a.Zbc ? (double)a.Zbc[k] : 0.);
+                Ref::P(c).st(g_sm.lc[c].n, a.Zbc ? a.Zbc[k] : 0.);
             }
             __syncthreads();
             if (dbg && threadIdx.x == 0) dbg[98] += clock64() - t_start;

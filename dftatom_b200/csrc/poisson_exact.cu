@@ -219,7 +219,7 @@ __global__ void __launch_bounds__(kXT, 1) poisson_exact_kernel(ExactPoissonArgs 
     XBuf b;
     b.A = a.work + (size_t)k * 3 * tot; b.B = b.A + tot; b.S = b.B + tot;
     const double* rho = a.rho + (size_t)k * a.rho_stride;
-    const double hi_bc = (double)a.Zbc[k];
+    const double hi_bc = a.Zbc[k];
 
     // Source_0 (PoissonSolver.h:55-74 / :22-43) and Initialize (.cpp:80-106)
     {

@@ -261,7 +261,7 @@ __global__ void __launch_bounds__(kAT) initial_density_kernel(GridDev g, ScfBuff
     for (int i = threadIdx.x; i < N; i += blockDim.x) {
         double tot = 0.;
         for (int s = 0; s < at.n_spin; ++s) {
-            const double c = (i == 0) ? 0. : (double)at.n_el[s] / volume;
+            const double c = (i == 0) ? 0. : at.n_el[s] / volume;
             b.rho[(size_t)b.tab_of[2 * a + s] * N + i] = c;
             tot += c;
         }
@@ -319,7 +319,7 @@ __global__ void __launch_bounds__(kDT) density_update_kernel(GridDev g, ScfBuffe
         const int s = q >= at.orb_count[0];
         const int k = s ? q - at.orb_count[0] : q;
         const int o = at.orb_begin[s] + k;
-        wgt[s * DFTATOM_MAX_LEVELS + k] = (double)b.orbs[o].occ * b.inv_norm[o];
+        wgt[s * DFTATOM_MAX_LEVELS + k] = b.orbs[o].occ * b.inv_norm[o];
     }
     __syncthreads();
     const int per = (N + (int)gridDim.y - 1) / (int)gridDim.y;
@@ -356,7 +356,7 @@ __global__ void __launch_bounds__(kDT) density_update_kernel(GridDev g, ScfBuffe
                 const int o = at.orb_begin[s] + k;
                 const SearchState& st = b.ss[o];
                 rec->E[s][k] = st.E;
-                eel += (double)b.orbs[o].occ * st.E;       // DFTAtom.cpp:561
+                eel += b.orbs[o].occ * st.E;       // DFTAtom.cpp:561
                 if (!st.converged) ok = 0;
             }
         rec->levels_converged = ok;
@@ -555,14 +555,14 @@ void launch_scf_loop_condition(const ScfLoopPhases& ph, int phase, int step_firs
     launch_step_kernel(scf_loop_condition_kernel, dim3(1), dim3(1), 0, st, ph, phase, step_first, step_end, n_active, iterations);
 }
 
-__global__ void scale_unit_potential_kernel(int N, int ldU, const double* __restrict__ u1, const int* __restrict__ Z, double* __restrict__ U)
+__global__ void scale_unit_potential_kernel(int N, int ldU, const double* __restrict__ u1, const double* __restrict__ Q, double* __restrict__ U)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < N) U[(size_t)blockIdx.y * ldU + i] = (double)Z[blockIdx.y] * u1[i];
+    if (i < N) U[(size_t)blockIdx.y * ldU + i] = Q[blockIdx.y] * u1[i];
 }
-void launch_scale_unit_potential(int N, int n_dens, int ldU, const double* u1, const int* Z, double* U, cudaStream_t st)
+void launch_scale_unit_potential(int N, int n_dens, int ldU, const double* u1, const double* Q, double* U, cudaStream_t st)
 {
-    scale_unit_potential_kernel<<<dim3((N + 255) / 256, n_dens), 256, 0, st>>>(N, ldU, u1, Z, U);
+    scale_unit_potential_kernel<<<dim3((N + 255) / 256, n_dens), 256, 0, st>>>(N, ldU, u1, Q, U);
 }
 
 // last "Step:" record of every atom, compact (what dftatom_solve_batch downloads when the caller did not ask for the steps)

@@ -82,7 +82,7 @@ def format_report(Z, method, steps, finished, final_alpha, final_beta=None, prec
             out += ["", "Finished!", ""]
         else:
             out.append(SEP)
-    conf = lambda lv: "".join(f"{n}{ORB[l]}{occ} " for (n, l, occ) in lv)
+    conf = lambda lv: "".join(f"{n}{ORB[l]}{occ:g} " for (n, l, occ) in lv)      # %g: integers as the reference prints them
     if lsda:
         out.append("Alpha: " + conf(final_alpha))
         out.append("Beta: " + conf(final_beta or []))

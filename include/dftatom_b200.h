@@ -54,7 +54,8 @@ typedef struct {
 typedef struct {
     int n;              /* principal quantum number, 1-based as printed */
     int l;              /* 0..3 -> s p d f */
-    int occ;            /* electrons in this (spin) subshell */
+    int occ;            /* electrons in this (spin) subshell; for an atom solved with a configuration (dftatom_solve_batch_config) the
+                           occupation rounded to the nearest integer - the exact value is the caller's entry with the same (n, l, spin) */
     int nodes;          /* n - l - 1, the "Num nodes" the reference prints */
     double E;           /* eigenvalue, Hartree */
 } dftatom_level;
@@ -139,12 +140,13 @@ const char* dftatom_version(void);
  *   "use_pdl"      (default 1) the kernels of an SCF step are launched with programmatic stream serialization (each starts with
  *                   griddepcontrol.wait before its first global read): the next kernel's blocks are scheduled while the previous one drains.
  *                   Same records; 0 = plain stream order.
- *   "unit_guess"   (default 1) the Poisson solve of the SCF's start density (DFTAtom.cpp:371-392: a uniform sphere of Z electrons, boundary value Z -
- *                   linear in Z) is done once per grid for Z = 1 by the cold multigrid kernel and scaled per atom (grids up to 16385 nodes);
+ *   "unit_guess"   (default 1) the Poisson solve of the SCF's start density (DFTAtom.cpp:371-392: a uniform sphere of Q electrons, boundary value Q -
+ *                   linear in the electron count Q, = Z for the neutral atom) is done once per grid for Q = 1 by the cold multigrid kernel and scaled
+ *                   per atom (grids up to 16385 nodes);
  *                   0 = one cold solve per atom and call.  Per-step parity with the reference unchanged (C3: 2.70e-6 vs 2.72e-6 Ha).
  *   "search_predict" (default 1) the production search starts every level of an SCF step from a ladder of 4 trial energies placed by what the
  *                   first steps of the reference's SCF are known to do: step 0 - hydrogenic levels of the initial potential (uniform sphere of
- *                   radius MaxR, DFTAtom.cpp:371-376: -Z^2/2n^2 + 3Z/(2 MaxR)); step 1 - one-sided (every level rises when the first real
+ *                   radius MaxR, DFTAtom.cpp:371-376: -Z^2/2n^2 + 3Q/(2 MaxR), Q = the electron count); step 1 - one-sided (every level rises when the first real
  *                   density screens the nucleus); step 2 - default decay ratio of the shifts; later - extrapolated shift, offsets scaled
  *                   with the shifts.  0 = cold section of [-Z^2-1, 50] at step 0 and the plain previous-eigenvalue ladder.  Same results
  *                   (every bracket is certified by the Sturm count), fewer rounds.
@@ -208,7 +210,8 @@ int dftatom_solve_batch(dftatom_ctx* ctx, const dftatom_options* opts, int n_ato
  * last node holds the orbital's value and is part of its normalisation; the density, like the reference's (DFTAtom.cpp:558-559), sums
  * occ u^2 / (4 pi r^2) over nodes 1 .. N-2 only.
  * Rows: atoms in call order, then spin (alpha, beta), then the (n, l) order of dftatom_result.levels; an atom has as many rows as
- * dftatom_aufbau (LDA) or dftatom_split_spin (n_alpha + n_beta levels, LSDA) gives it.  An `orbital_rows` smaller than the batch needs
+ * dftatom_aufbau (LDA) or dftatom_split_spin (n_alpha + n_beta levels, LSDA) gives it, a configured atom (dftatom_solve_batch_config) as
+ * many as its configuration has entries.  An `orbital_rows` smaller than the batch needs
  * (when `orbitals` or `moments` is given) returns DFTATOM_E_ARG before anything is solved.
  * Moments: sum_i wjac_i u_i^2 f(r_i) for f = 1/r (node 0 left out), r, r^2 - <1/r>, <r>, <r^2> of the normalised orbital.
  * atom_moments: sum_i wjac_i 4 pi r_i^2 rho_i (the electron count) and sum_i wjac_i 4 pi r_i^4 rho_i (<r^2> summed over the electrons),
@@ -228,6 +231,32 @@ typedef struct {                       /* HOST pointers; any may be NULL (not ex
 } dftatom_radial;
 int dftatom_solve_batch_radial(dftatom_ctx* ctx, const dftatom_options* opts, int n_atoms, dftatom_result* out, dftatom_step* steps,
                                int steps_stride, const dftatom_radial* radial);
+/* ---- L2 with electron configurations: ions, excited states, empty channels, fractional occupations ----
+ * A configuration is a list of orbitals (n, l, spin, occ), occ a double.  Every entry is one orbital the SCF solves (node count
+ * n - l - 1); occ = 0: the orbital is solved, reported and exported, but adds nothing to the density or to E_el = sum occ eps.
+ *   LDA  (methods 0, 2): spin = 0 and 0 <= occ <= 2 (2l + 1).   LSDA (methods 1, 3): spin = 0 (alpha) or 1 (beta), 0 <= occ <= 2l + 1.
+ *   1 <= n <= 8, 0 <= l <= min(3, n - 1); no duplicate (n, l, spin); at most DFTATOM_MAX_LEVELS entries per spin and at least one alpha
+ *   entry; every occ finite; the electron count Q = sum occ satisfies 0 < Q <= Z + 2.
+ * A violation returns DFTATOM_E_BAD_OPTION (the message names the atom and the entry) before anything is solved.  The entries of each
+ * spin are solved, reported (dftatom_result.levels, dftatom_step.E) and exported (radial rows) in (n, l) order, the order of
+ * dftatom_aufbau.  What depends on Q: the start density (a uniform sphere of Q_s electrons per spin) and the Hartree boundary value
+ * U(Rmax) = Q.  The nuclear charge stays Z: V = (-Z + U) / r, the energies, the search bracket [-Z^2 - 1, 50]. */
+typedef struct { int n, l, spin; double occ; } dftatom_occupation;
+typedef struct { int n_orbitals; dftatom_occupation orb[2 * DFTATOM_MAX_LEVELS]; } dftatom_config;
+/* The reference's configuration of atom Z (dftatom_aufbau / dftatom_split_spin: the same entries, empty beta levels omitted) ionised by
+ * `charge` electrons (may be fractional; < 0 = anion), alpha entries then beta entries, each in (n, l) order.
+ *   Cations lose electrons from the occupied subshell of largest n, among those of largest l, one subshell at a time (an emptied subshell
+ *   is dropped): Fe2+ = [Ar] 3d6, Cr+ = [Ar] 3d4 4s1 (the reference's Aufbau keeps Cr 3d4 4s2), Cu+ = [Ar] 3d9 4s1 (its Cu is 3d9 4s2;
+ *   pass [Ar] 3d10 explicitly for the other one).
+ *   Anions gain electrons in the reference's filling (Madelung) order from the first subshell that is not full: O- = 2p5, Ne- = ... 3s1.
+ *   LSDA: every subshell's total is split like dftatom_split_spin: alpha min(occ, 2l + 1), beta the rest, listed only when nonzero.
+ * charge == 0 reproduces dftatom_aufbau / dftatom_split_spin exactly.  -2 <= charge < Z, else DFTATOM_E_BAD_OPTION. */
+int dftatom_config_aufbau(int Z, int method, double charge, dftatom_config* out);
+/* = dftatom_solve_batch_radial with per-atom configurations: configs == NULL or configs[a].n_orbitals == 0: the Aufbau atom (bit for bit
+ * the result of dftatom_solve_batch_radial, which is this call with configs == NULL).  The radial export's rows of a configured atom are
+ * its configured entries. */
+int dftatom_solve_batch_config(dftatom_ctx* ctx, const dftatom_options* opts, const dftatom_config* configs, int n_atoms,
+                               dftatom_result* out, dftatom_step* steps, int steps_stride, const dftatom_radial* radial);
 /* The moment reduction of the export on caller-supplied orbitals u[n_rows][N] (HOST) of the grid (levels, delta, max_r; delta = 0: the
  * uniform grid): moments[n_rows][DFTATOM_N_MOMENTS] = sum_i wjac_i u_i^2 f(r_i), f = 1/r (node 0 left out), r, r^2.  The rows are used
  * as given (no normalisation, no sign). */
@@ -282,7 +311,8 @@ int dftatom_level_search(dftatom_ctx* ctx, const double* V, int levels, double d
 /* two-sided matched + normalised solution u(r) (Numerov.h:403-504 + DFTAtom.cpp:36-56) */
 int dftatom_numerov_orbital(dftatom_ctx* ctx, const double* V, int levels, double delta, double max_r,
                             int l, double E, double* u_out, int* match_point);
-/* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) */
+/* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) (the SCF passes the
+ * electron count as a double; Z[k] is converted exactly) */
 int dftatom_poisson_solve(dftatom_ctx* ctx, int levels, double delta, double max_r, int n_dens, const int* Z,
                           const double* rho, double* U, int* vcycles_used);
 /* n_cycles reference-shaped V-cycles (PoissonSolver.h:155-159) in place on phi[n_dens][N] with source src[n_dens][N] */
