@@ -53,6 +53,10 @@ class _CRadial(C.Structure):
                 ("atom_moments", C.POINTER(C.c_double))]
 
 
+class _CLogDeriv(C.Structure):
+    _fields_ = [("D", C.c_double), ("u", C.c_double), ("du", C.c_double), ("nodes", C.c_int), ("pad", C.c_int)]
+
+
 class _COccupation(C.Structure):
     _fields_ = [("n", C.c_int), ("l", C.c_int), ("spin", C.c_int), ("occ", C.c_double)]
 
@@ -108,6 +112,8 @@ def load_library():
     lib.dftatom_solve_batch_config.argtypes = [C.c_void_p, C.POINTER(_COptions), C.POINTER(_CConfig), C.c_int, C.POINTER(_CResult),
                                                C.POINTER(_CStep), C.c_int, C.POINTER(_CRadial)]
     lib.dftatom_radial_moments.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp]
+    lib.dftatom_log_derivatives.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _ip, _ip, _dp, C.c_int, _dp, C.c_int,
+                                            C.POINTER(_CLogDeriv), _dp]
     lib.dftatom_last_timing.argtypes = [C.c_void_p, _dp, C.POINTER(C.c_longlong)]
     lib.dftatom_last_graph_iterations.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
     lib.dftatom_last_transfer.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
@@ -276,6 +282,27 @@ class Radial:
     moments: List[np.ndarray]
     n_electrons: float
     r2: float
+
+
+@dataclass
+class LogDerivatives:
+    """Logarithmic derivatives of the outward radial solution (Context.log_derivatives; definition: dftatom_log_derivatives in
+    include/dftatom_b200.h).  D, u, du, nodes: [n_channels][n_energies]; D = u'(r_c) / u(r_c) in bohr^-1, u and du the value and slope
+    at r_c of the solution normalised to int_0^rc u^2 dr = 1; nodes = -1 (and NaN in D, u, du) where the grid is too coarse for the
+    energy.  r_c: [n_channels] the radii actually used (nearest grid node).  E: [n_energies]."""
+    D: np.ndarray
+    u: np.ndarray
+    du: np.ndarray
+    nodes: np.ndarray
+    r_c: np.ndarray
+    E: np.ndarray
+
+    @property
+    def phase(self) -> np.ndarray:
+        """pi nodes - atan(r_c D): continuous across the poles of D and increasing in E; NaN where nodes = -1."""
+        with np.errstate(invalid="ignore"):
+            ph = np.pi * self.nodes - np.arctan(self.r_c[:, None] * self.D)
+        return np.where(self.nodes < 0, np.nan, ph)
 
 
 def orbital_count(Z: int, method: int = 0, config=None, charge: float = 0.0) -> int:
@@ -625,6 +652,21 @@ class Context:
         out = np.zeros((u.shape[0], N_MOMENTS))
         _check(self._lib.dftatom_radial_moments(self._h, int(levels), float(delta), float(max_r), _d(u), u.shape[0], _d(out)))
         return out
+
+    def log_derivatives(self, V, levels, delta, max_r, pot, l, r_c, E) -> LogDerivatives:
+        """D_l(E) = u'(r_c) / u(r_c) of the outward radial solution for every (channel, energy) (dftatom_log_derivatives).  V: [n_pot][N]
+        potentials (one row may be given as [N]), e.g. rows of Result.radial.V; channel c = (V row pot[c], l[c], r_c[c] in bohr): pot, l
+        and r_c are broadcast against each other; E: energies shared by all channels."""
+        V = _f64(np.atleast_2d(V))
+        pot, l, r_c = np.broadcast_arrays(np.atleast_1d(pot), np.atleast_1d(l), np.atleast_1d(r_c))
+        pot = _i32(pot); l = _i32(l); r_c = _f64(r_c); E = _f64(np.atleast_1d(E))
+        nc, ne = len(pot), len(E)
+        out = np.zeros(nc * ne, dtype=np.dtype(_CLogDeriv))
+        used = np.zeros(nc)
+        _check(self._lib.dftatom_log_derivatives(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], _i(pot), _i(l), _d(r_c), nc,
+                                                 _d(E), ne, out.ctypes.data_as(C.POINTER(_CLogDeriv)), _d(used)))
+        out = out.reshape(nc, ne)
+        return LogDerivatives(out["D"].copy(), out["u"].copy(), out["du"].copy(), out["nodes"].copy(), used, E.copy())
 
     def integrate(self, rule, step, v):
         """Integral.h quadratures by rule: 0 Trapezoid, 1 SimpsonOneThird, 2 Simpson38, 3 Boole, 4 Romberg; one result per row of v."""

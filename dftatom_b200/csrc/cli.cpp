@@ -16,7 +16,12 @@
 //           < 0 = anion), e.g. --Z 1-92 --charge 1 for all cations.  --config "[Ne] 3s1 3p0": one atom (a single --Z) in that configuration
 //           (subshells "2p4.5", LSDA also "2p3/1" = alpha / beta, cores [He] .. [Rn]; the same string form as dftatom_b200.parse_config).
 //           Both are passed on to the shards of --gpus and select the rows of --radial.
+// --logderiv DIR --rc R [--energies lo:hi:n]: logarithmic derivatives D_l(E) = u'(R) / u(R) of every atom's converged potential, l = 0..3
+//           for each spin, at n energies from lo to hi (default -2:1:301), as a long table DIR/<index>_Z<Z>_logderiv.tsv with the columns
+//           spin, l, E, D, nodes, phase = pi nodes - atan(r_c D), u, du at 17 digits (dftatom_log_derivatives; r_c = the grid node nearest
+//           to R).  The potential is the one the radial export returns; --radial is not needed.  Works with --gpus, --charge and --config.
 #include <algorithm>
+#include <cmath>
 #include <cctype>
 #include <cstdio>
 #include <cstdlib>
@@ -233,12 +238,41 @@ static int write_radial(const std::string& dir, int index, const dftatom_options
     return 0;
 }
 
+// --logderiv: channels l = 0..3 of every spin on the atom's converged V (rows of dftatom_radial.v), one long table
+static int write_logderiv(dftatom_ctx* ctx, const std::string& dir, int index, const dftatom_options& o, int n_spin, const double* v,
+                          double rc, const std::vector<double>& E)
+{
+    const int nc = 4 * n_spin, ne = (int)E.size();
+    std::vector<int> pot(nc), l(nc);
+    std::vector<double> rcs(nc, rc), used(nc);
+    for (int c = 0; c < nc; ++c) { pot[c] = c / 4; l[c] = c % 4; }
+    std::vector<dftatom_logderiv> out((size_t)nc * ne);
+    if (dftatom_log_derivatives(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v, n_spin, pot.data(), l.data(), rcs.data(), nc, E.data(), ne,
+                                out.data(), used.data()) != DFTATOM_OK) {
+        std::fprintf(stderr, "dftatom: --logderiv Z=%d: %s\n", o.Z, dftatom_last_error());
+        return 1;
+    }
+    const std::string path = dir + "/" + std::to_string(index) + "_Z" + std::to_string(o.Z) + "_logderiv.tsv";
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) { std::perror(path.c_str()); return 1; }
+    std::fprintf(f, "# Z=%d method=%d r_c=%.17g\n# spin\tl\tE\tD\tnodes\tphase\tu\tdu\n", o.Z, o.method, used[0]);
+    for (int c = 0; c < nc; ++c)
+        for (int k = 0; k < ne; ++k) {
+            const dftatom_logderiv& q = out[(size_t)c * ne + k];
+            const double phase = q.nodes < 0 ? NAN : M_PI * q.nodes - std::atan(used[c] * q.D);
+            std::fprintf(f, "%d\t%d\t%.17g\t%.17g\t%d\t%.17g\t%.17g\t%.17g\n", pot[c], l[c], E[k], q.D, q.nodes, phase, q.u, q.du);
+        }
+    const bool bad = std::ferror(f) != 0;
+    if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
+    return 0;
+}
+
 int main(int argc, char** argv)
 {
     dftatom_options base = { 36, 12, 10.0, 0.001, 0.5, 0 };     // Options.cpp:6
     std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
-    std::string radial_dir, config_str;
-    double charge = 0.;
+    std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301";
+    double charge = 0., rc = NAN;
     int precision = 6, device = 0, gpus = 1;
     bool json = false, quiet = false, framed = false;      // framed: child of --gpus (one frame per atom on stdout)
     std::vector<std::string> passthrough;                   // flags a --gpus parent hands to its children unchanged
@@ -251,6 +285,9 @@ int main(int argc, char** argv)
         else if (a == "--framed") framed = true;
         else if (a == "--atom-index") atom_index = parse_z(next());
         else if (a == "--radial") radial_dir = next();
+        else if (a == "--logderiv") logderiv_dir = next();
+        else if (a == "--rc") rc = std::atof(next());
+        else if (a == "--energies") energies = next();
         else if (a == "--charge") charge = std::atof(next());
         else if (a == "--config") config_str = next();
         else if (a == "--levels") base.levels = std::atoi(next());
@@ -270,9 +307,14 @@ int main(int argc, char** argv)
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
                         "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR] [--charge Q] [--config \"...\"]\n"
+                        "               [--logderiv DIR --rc R [--energies lo:hi:n]]\n"
                         "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n"
                         "  --charge Q    solve every atom of --Z ionised by Q electrons (the reference's configuration; fractional allowed, < 0 = anion)\n"
-                        "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n");
+                        "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n"
+                        "  --logderiv DIR  write the logarithmic derivatives D_l(E) = u'(r_c)/u(r_c), l = 0..3 per spin, of every atom's converged V to\n"
+                        "                DIR/<index>_Z<Z>_logderiv.tsv (columns spin l E D nodes phase u du)\n"
+                        "  --rc R        radius of --logderiv in bohr (the nearest grid node is used)\n"
+                        "  --energies lo:hi:n  energies of --logderiv, n points from lo to hi Hartree (default -2:1:301)\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
         if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
@@ -281,6 +323,16 @@ int main(int argc, char** argv)
     if (!config_str.empty() && (zs.size() != 1 || charge != 0.)) { std::fprintf(stderr, "dftatom: --config needs a single --Z and no --charge\n"); return 2; }
     if (!atom_index.empty() && atom_index.size() != zs.size()) { std::fprintf(stderr, "dftatom: --atom-index needs one index per --Z entry\n"); return 2; }
     if (!radial_dir.empty() && mkdir(radial_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(radial_dir.c_str()); return 1; }
+    std::vector<double> ld_E;
+    if (!logderiv_dir.empty()) {
+        double lo = 0., hi = 0.; int ne = 0; char tail = 0;
+        if (std::sscanf(energies.c_str(), "%lf:%lf:%d%c", &lo, &hi, &ne, &tail) != 3 || ne < 1 || !std::isfinite(lo) || !std::isfinite(hi)) {
+            std::fprintf(stderr, "dftatom: --energies expects lo:hi:n with n >= 1, got '%s'\n", energies.c_str()); return 2;
+        }
+        for (int k = 0; k < ne; ++k) ld_E.push_back(k == ne - 1 && ne > 1 ? hi : lo + (hi - lo) * k / (ne > 1 ? ne - 1 : 1));
+        if (!(rc > 0.)) { std::fprintf(stderr, "dftatom: --logderiv needs --rc R (bohr)\n"); return 2; }
+        if (mkdir(logderiv_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(logderiv_dir.c_str()); return 1; }
+    }
     if (gpus > 1) {
         char self[4096];
         const ssize_t len = readlink("/proc/self/exe", self, sizeof self - 1);
@@ -320,11 +372,13 @@ int main(int argc, char** argv)
     std::vector<double> r_grid, rho, vks, vh, orb;
     dftatom_radial rad = {};
     if (!radial_dir.empty()) {
-        r_grid.resize(N); rho.resize((size_t)n * 2 * N); vks.resize((size_t)n * 2 * N); vh.resize((size_t)n * N); orb.resize((size_t)row0[n] * N);
-        rad.r = r_grid.data(); rad.rho = rho.data(); rad.v = vks.data(); rad.v_hartree = vh.data(); rad.orbitals = orb.data(); rad.orbital_rows = row0[n];
+        r_grid.resize(N); rho.resize((size_t)n * 2 * N); vh.resize((size_t)n * N); orb.resize((size_t)row0[n] * N);
+        rad.r = r_grid.data(); rad.rho = rho.data(); rad.v_hartree = vh.data(); rad.orbitals = orb.data(); rad.orbital_rows = row0[n];
     }
+    const bool export_v = !radial_dir.empty() || !logderiv_dir.empty();
+    if (export_v) { vks.resize((size_t)n * 2 * N); rad.v = vks.data(); }
     if (dftatom_solve_batch_config(ctx, opts.data(), configured ? cfgs.data() : nullptr, n, res.data(), steps.data(), stride,
-                                   radial_dir.empty() ? nullptr : &rad) != DFTATOM_OK) {
+                                   export_v ? &rad : nullptr) != DFTATOM_OK) {
         std::fprintf(stderr, "dftatom: %s\n", dftatom_last_error());
         dftatom_destroy(ctx);
         return 1;
@@ -334,6 +388,10 @@ int main(int argc, char** argv)
     for (int a = 0; a < n && !radial_dir.empty(); ++a)
         if (write_radial(radial_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a], N, r_grid.data(), &rho[(size_t)a * 2 * N], &vks[(size_t)a * 2 * N],
                          &vh[(size_t)a * N], &orb[(size_t)row0[a] * N])) { dftatom_destroy(ctx); return 1; }
+    for (int a = 0; a < n && !logderiv_dir.empty(); ++a)
+        if (write_logderiv(ctx, logderiv_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a].n_spin, &vks[(size_t)a * 2 * N], rc, ld_E)) {
+            dftatom_destroy(ctx); return 1;
+        }
 
     if (json && !framed) std::printf("[");
     for (int a = 0; a < n; ++a) {

@@ -1170,6 +1170,70 @@ int dftatom_numerov_lanes_timed(dftatom_ctx* c, const double* V, int levels, dou
                               lane_node_steps);
 }
 
+int dftatom_log_derivatives(dftatom_ctx* c, int levels, double delta, double max_r, const double* V, int n_pot, const int* pot, const int* l,
+                            const double* r_c, int n_channels, const double* E, int n_energies, dftatom_logderiv* out, double* r_used)
+{
+    if (!c || !V || !pot || !l || !r_c || !E || !out) { set_error("dftatom_log_derivatives: NULL argument"); return DFTATOM_E_ARG; }
+    if (n_pot < 1 || n_channels < 1 || n_energies < 1) { set_error("dftatom_log_derivatives: n_pot, n_channels and n_energies must be >= 1"); return DFTATOM_E_ARG; }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
+    if (N < 5) { set_error("dftatom_log_derivatives: the grid needs at least 5 nodes"); return DFTATOM_E_ARG; }
+    std::vector<double> r(N);             // the device's node radii: r_c is rounded to one of them
+    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    const auto where = [](const char* what, long long k) { return std::string("dftatom_log_derivatives: ") + what + " " + std::to_string(k) + ": "; };
+    std::vector<int> ic(n_channels);
+    for (int k = 0; k < n_channels; ++k) {
+        if (pot[k] < 0 || pot[k] >= n_pot) { set_error(where("channel", k) + "pot = " + std::to_string(pot[k]) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
+        if (l[k] < 0 || l[k] > 3) { set_error(where("channel", k) + "l = " + std::to_string(l[k]) + " outside 0..3"); return DFTATOM_E_ARG; }
+        if (!(r_c[k] >= r[2] && r_c[k] <= r[N - 2])) {
+            char b[160];
+            std::snprintf(b, sizeof b, "r_c = %.17g outside [r_2, r_(N-2)] = [%.17g, %.17g]", r_c[k], r[2], r[N - 2]);
+            set_error(where("channel", k) + b); return DFTATOM_E_ARG;
+        }
+        const int hi = (int)(std::lower_bound(r.begin() + 2, r.begin() + (N - 1), r_c[k]) - r.begin());      // first node >= r_c, 2..N-2
+        ic[k] = (hi > 2 && r_c[k] - r[hi - 1] <= r[hi] - r_c[k]) ? hi - 1 : hi;                           // nearest node, ties to the inner one
+    }
+    for (int k = 0; k < n_energies; ++k)
+        if (!std::isfinite(E[k])) { set_error(where("energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
+    for (int p = 0; p < n_pot; ++p)
+        for (int i = 1; i < N; ++i)
+            if (!std::isfinite(V[(size_t)p * N + i])) { set_error(where("potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    // one warp per (channel, block of 32 energies), dealt longest sweep first (stable: equal sweeps keep channel order)
+    const int eb = (n_energies + 31) / 32;
+    const long long n_warps_ll = (long long)n_channels * eb;
+    if (n_warps_ll > (1LL << 30)) { set_error("dftatom_log_derivatives: too many (channel, energy) lanes"); return DFTATOM_E_ARG; }
+    const int n_warps = (int)n_warps_ll;
+    std::vector<int> chan_order(n_channels);
+    std::iota(chan_order.begin(), chan_order.end(), 0);
+    std::stable_sort(chan_order.begin(), chan_order.end(), [&](int a, int b) { return ic[a] > ic[b]; });
+    std::vector<int> h_int(3 * (size_t)n_channels + n_warps);      // pot | l | ic | warp_item
+    std::copy(pot, pot + n_channels, h_int.begin());
+    std::copy(l, l + n_channels, h_int.begin() + n_channels);
+    std::copy(ic.begin(), ic.end(), h_int.begin() + 2 * (size_t)n_channels);
+    int* wi = h_int.data() + 3 * (size_t)n_channels;
+    for (int q = 0, w = 0; q < n_channels; ++q)
+        for (int b = 0; b < eb; ++b) wi[w++] = chan_order[q] * eb + b;
+    DevBuf& dV = c->scratch[0]; DevBuf& dA = c->scratch[1]; DevBuf& di = c->scratch[2]; DevBuf& dd = c->scratch[3]; DevBuf& dO = c->scratch[4];
+    const size_t nV = (size_t)n_pot * N, n_out = (size_t)n_channels * n_energies;
+    if ((rc = dV.ensure(sizeof(double) * nV)) || (rc = dA.ensure(sizeof(double) * nV)) || (rc = di.ensure(sizeof(int) * h_int.size())) ||
+        (rc = dd.ensure(sizeof(double) * n_energies)) || (rc = dO.ensure(sizeof(dftatom_logderiv) * n_out))) return rc;
+    DFT_CHECK(cudaMemcpyAsync(dV.p, V, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(di.p, h_int.data(), sizeof(int) * h_int.size(), cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dd.p, E, sizeof(double) * n_energies, cudaMemcpyHostToDevice, st));
+    launch_build_atab(g, dV.as<double>(), dA.as<double>(), n_pot, st);
+    const int* d_i = di.as<int>();
+    LogDerivArgs a{ dA.as<double>(), d_i, d_i + n_channels, d_i + 2 * (size_t)n_channels, dd.as<double>(), n_energies,
+                    d_i + 3 * (size_t)n_channels, n_warps, eb, dO.as<dftatom_logderiv>() };
+    launch_logderiv(g, a, st);
+    DFT_CHECK(cudaGetLastError());
+    DFT_CHECK(cudaMemcpyAsync(out, dO.p, sizeof(dftatom_logderiv) * n_out, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    if (r_used) for (int k = 0; k < n_channels; ++k) r_used[k] = r[ic[k]];
+    return 0;
+}
+
 // shared by level_search / numerov_orbital: one pseudo-atom with the given potential
 static int setup_single(dftatom_ctx* c, const GridDev& g, const double* V, int Z, const std::vector<OrbitalDev>& orbs,
                         AtomDev** d_atoms, AtomState** d_astate, OrbitalDev** d_orbs, SearchState** d_ss, double** d_atab)

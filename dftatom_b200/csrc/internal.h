@@ -336,6 +336,17 @@ void launch_radial_orbitals(const GridDev& g, const double* src, const double* i
 void launch_radial_fields(const GridDev& g, const ScfBuffers& b, double* rho_out, double* v_out, double* vh_out, double* atom_moments,
                           double* part, int* ticket, cudaStream_t st);
 
+// logarithmic derivatives (logderiv.cu): one warp per (channel, 32 energies); warp_item[w] = channel * energy_blocks + block, in the order
+// the warps are dealt (longest sweep first)
+struct LogDerivArgs {
+    const double* atab;                          // [n_pot][N] (launch_build_atab)
+    const int* pot; const int* l; const int* ic; // [n_channels] potential row, l, node index of r_c (2 <= ic <= N - 2)
+    const double* E; int n_energies;             // [n_energies], shared by all channels
+    const int* warp_item; int n_warps, energy_blocks;
+    dftatom_logderiv* out;                       // [n_channels][n_energies]
+};
+void launch_logderiv(const GridDev& g, const LogDerivArgs& a, cudaStream_t st);
+
 // host rules (aufbau.cpp)
 int aufbau(int Z, dftatom_level* out, int max_out);
 int split_spin(int Z, dftatom_level* a, int* na, dftatom_level* b, int* nb, int* ea, int* eb);

@@ -311,6 +311,29 @@ int dftatom_level_search(dftatom_ctx* ctx, const double* V, int levels, double d
 /* two-sided matched + normalised solution u(r) (Numerov.h:403-504 + DFTAtom.cpp:36-56) */
 int dftatom_numerov_orbital(dftatom_ctx* ctx, const double* V, int levels, double delta, double max_r,
                             int l, double E, double* u_out, int* match_point);
+/* Logarithmic derivatives D_l(E) = u'(r_c) / u(r_c) of the radial solution regular at the nucleus, for every (channel, energy) pair:
+ * the transferability diagnostic of pseudopotential generation, and the norm-conservation identity dD/dE = -2 int_0^rc u^2 dr / u(r_c)^2.
+ * Grid (levels, delta, max_r) as in the other component entries (delta = 0: the uniform grid of methods 2 / 3), N = 2^levels + 1.
+ * V[n_pot][N] HOST potentials (Hartree; node 0 ignored), e.g. rows of dftatom_radial.v.  Channel c = (V row pot[c], l[c], radius r_c[c]
+ * in bohr); E[n_energies] HOST energies shared by all channels, in any order.  out[n_channels][n_energies]; r_used[n_channels] (may be
+ * NULL) receives the radius actually used, the node r_(i_c) nearest to r_c[c].
+ * Definition: g_i = f_i / 12 = (2 K_i (V_i - E) + K_i l(l+1) / r_i^2 + delta^2 / 4) / 12, K_i = (Rp delta e^(delta i))^2 (uniform grid:
+ * K = h^2, no delta^2 / 4 term).  The outward Numerov solution starts from y_0 = 0, y_1 = r_1^(l+1) e^(-delta/2) (uniform grid: h^(l+1))
+ * and steps w_(i+1) = 2 w_i - w_(i-1) + 12 g_i y_i, w = (1 - g) y, through every turning point to i_c + 1; u = y e^(delta i / 2)
+ * (uniform grid: u = y).  u'(r_c) from the fourth-order index derivative y'_i = [(1 - 2 g_(i+1)) y_(i+1) - (1 - 2 g_(i-1)) y_(i-1)] / 2.
+ * int_0^rc u^2 dr by Simpson's 1/3 rule on nodes 0..i_c times dr/di (3/8 rule on the last three intervals when i_c is odd).
+ *   D      u'(r_c) / u(r_c), bohr^-1
+ *   u, du  u(r_c) and u'(r_c) of the solution scaled to int_0^rc u^2 dr = 1, u > 0 next to the nucleus
+ *   nodes  sign changes among the non-zero values of y_1 .. y_(i_c); the phase pi nodes - atan(r_c D) is continuous and increasing in E
+ * A lane whose grid is too coarse (1 - g_i <= 0 at some node 2 <= i <= i_c + 1) returns nodes = -1 and NaN in D, u, du.  Every other lane
+ * returns finite values (the sweep is rescaled by powers of two).
+ * Validation before anything runs on the device: a bad grid returns DFTATOM_E_BAD_OPTION; n_pot, n_channels, n_energies >= 1,
+ * 0 <= pot < n_pot, 0 <= l <= 3, r_2 <= r_c <= r_(N-2), every E finite and V finite at nodes 1..N-1, else DFTATOM_E_ARG naming the
+ * channel, energy or potential row. */
+typedef struct { double D, u, du; int nodes, pad; } dftatom_logderiv;      /* 32 bytes */
+int dftatom_log_derivatives(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, int n_pot,
+                            const int* pot, const int* l, const double* r_c, int n_channels,
+                            const double* E, int n_energies, dftatom_logderiv* out, double* r_used);
 /* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) (the SCF passes the
  * electron count as a double; Z[k] is converted exactly) */
 int dftatom_poisson_solve(dftatom_ctx* ctx, int levels, double delta, double max_r, int n_dens, const int* Z,
