@@ -57,6 +57,15 @@ class _CLogDeriv(C.Structure):
     _fields_ = [("D", C.c_double), ("u", C.c_double), ("du", C.c_double), ("nodes", C.c_int), ("pad", C.c_int)]
 
 
+class _CTmChannel(C.Structure):
+    _fields_ = [("pot", C.c_int), ("orbital", C.c_int), ("l", C.c_int), ("pad", C.c_int), ("eps", C.c_double), ("occ", C.c_double),
+                ("r_c", C.c_double)]
+
+
+class _CTmResult(C.Structure):
+    _fields_ = [("c", C.c_double * 7), ("r_c", C.c_double), ("q", C.c_double), ("status", C.c_int), ("pad", C.c_int)]
+
+
 class _COccupation(C.Structure):
     _fields_ = [("n", C.c_int), ("l", C.c_int), ("spin", C.c_int), ("occ", C.c_double)]
 
@@ -114,6 +123,9 @@ def load_library():
     lib.dftatom_radial_moments.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp]
     lib.dftatom_log_derivatives.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _ip, _ip, _dp, C.c_int, _dp, C.c_int,
                                             C.POINTER(_CLogDeriv), _dp]
+    lib.dftatom_grid_nodes.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp]
+    lib.dftatom_tm_pseudize.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp, C.c_int, C.POINTER(_CTmChannel), C.c_int,
+                                        C.POINTER(_CTmResult), _dp, _dp, _dp, _dp]
     lib.dftatom_last_timing.argtypes = [C.c_void_p, _dp, C.POINTER(C.c_longlong)]
     lib.dftatom_last_graph_iterations.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
     lib.dftatom_last_transfer.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
@@ -303,6 +315,29 @@ class LogDerivatives:
         with np.errstate(invalid="ignore"):
             ph = np.pi * self.nodes - np.arctan(self.r_c[:, None] * self.D)
         return np.where(self.nodes < 0, np.nan, ph)
+
+
+@dataclass
+class Pseudopotential:
+    """Troullier-Martins pseudopotentials (Context.tm_pseudize / Context.pseudize; definition: dftatom_tm_pseudize in include/dftatom_b200.h).
+    Per channel ([n_channels]): l, eps, occ, r_c (the radius actually used, a grid node), coefficients [n_channels][7] (c0, c2, ..., c12 of
+    p(r), bohr^-2k), q (all-electron norm inside r_c), status (0 ok, 1 no root on the ladder, 2 the sweep at eps failed, 3 the root
+    not refined to 1e-13), u (pseudo-orbital),
+    V_scr (screened potential) and V_ion (ionic potential), each [n_channels][N].  pot: the potential row of every channel; rho_val:
+    [n_pot][N] the valence density of each row.  r: [N] the grid."""
+    l: np.ndarray
+    eps: np.ndarray
+    occ: np.ndarray
+    r_c: np.ndarray
+    coefficients: np.ndarray
+    q: np.ndarray
+    status: np.ndarray
+    r: np.ndarray
+    u: np.ndarray
+    V_scr: np.ndarray
+    V_ion: np.ndarray
+    rho_val: np.ndarray
+    pot: np.ndarray
 
 
 def orbital_count(Z: int, method: int = 0, config=None, charge: float = 0.0) -> int:
@@ -667,6 +702,51 @@ class Context:
                                                  _d(E), ne, out.ctypes.data_as(C.POINTER(_CLogDeriv)), _d(used)))
         out = out.reshape(nc, ne)
         return LogDerivatives(out["D"].copy(), out["u"].copy(), out["du"].copy(), out["nodes"].copy(), used, E.copy())
+
+    def tm_pseudize(self, V, u, levels, delta, max_r, pot, orbital, l, eps, occ, r_c) -> Pseudopotential:
+        """Troullier-Martins pseudization and unscreening (dftatom_tm_pseudize).  V: [n_pot][N] potentials, u: [n_orb][N] all-electron
+        orbitals (one row of either may be given as [N]), e.g. rows of Result.radial.V and Result.radial.orbitals; channel c = (V row pot[c],
+        u row orbital[c], l[c], eigenvalue eps[c], occupation occ[c], radius r_c[c] in bohr), broadcast against each other.  The channels
+        sharing a potential row are one pseudo-atom for the unscreening."""
+        V = _f64(np.atleast_2d(V)); u = _f64(np.atleast_2d(u))
+        pot, orbital, l, eps, occ, r_c = np.broadcast_arrays(*(np.atleast_1d(x) for x in (pot, orbital, l, eps, occ, r_c)))
+        nc, N = len(pot), V.shape[1]
+        ch = np.zeros(nc, dtype=np.dtype(_CTmChannel))
+        ch["pot"], ch["orbital"], ch["l"], ch["eps"], ch["occ"], ch["r_c"] = pot, orbital, l, eps, occ, r_c
+        res = np.zeros(nc, dtype=np.dtype(_CTmResult))
+        u_ps, v_scr, v_ion = (np.zeros((nc, N)) for _ in range(3))
+        rho = np.zeros((V.shape[0], N))
+        _check(self._lib.dftatom_tm_pseudize(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], _d(u), u.shape[0],
+                                             ch.ctypes.data_as(C.POINTER(_CTmChannel)), nc, res.ctypes.data_as(C.POINTER(_CTmResult)),
+                                             _d(u_ps), _d(v_scr), _d(v_ion), _d(rho)))
+        rr = np.zeros(N)                                    # the engine's node radii
+        _check(self._lib.dftatom_grid_nodes(self._h, int(levels), float(delta), float(max_r), _d(rr)))
+        return Pseudopotential(_i32(l).copy(), _f64(eps).copy(), _f64(occ).copy(), res["r_c"].copy(), res["c"].copy(), res["q"].copy(),
+                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy())
+
+    def pseudize(self, result, r_c) -> Pseudopotential:
+        """Pseudopotentials of a solved LDA atom (Result of solve_batch(..., radial=True)): for every l of result.levels[0] the level of
+        largest n is the valence channel, with its eigenvalue and occupation.  r_c: one radius, a sequence indexed by l, or a dict {l: r_c}."""
+        o = result.options
+        if result.radial is None:
+            raise ValueError("pseudize needs the radial state: solve with radial=True")
+        if o.method & 1:
+            raise ValueError("pseudize needs an LDA atom (method 0 or 2): the unscreening is spin-unpolarised")
+        best = {}
+        for k, lev in enumerate(result.levels[0]):
+            if lev.l not in best or lev.n > result.levels[0][best[lev.l]].n:
+                best[lev.l] = k
+        ls = sorted(best)
+        if isinstance(r_c, dict):
+            rcs = [r_c[l] for l in ls]
+        elif np.ndim(r_c) == 0:
+            rcs = [float(r_c)] * len(ls)
+        else:
+            rcs = [r_c[l] for l in ls]
+        lev = [result.levels[0][best[l]] for l in ls]
+        rad = result.radial
+        return self.tm_pseudize(rad.V[0], rad.orbitals[0], o.MultigridLevels, 0.0 if o.method >= 2 else o.deltaGrid, o.MaxR, 0,
+                                [best[l] for l in ls], ls, [x.E for x in lev], [float(x.occ) for x in lev], rcs)
 
     def integrate(self, rule, step, v):
         """Integral.h quadratures by rule: 0 Trapezoid, 1 SimpsonOneThird, 2 Simpson38, 3 Boole, 4 Romberg; one result per row of v."""

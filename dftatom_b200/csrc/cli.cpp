@@ -20,6 +20,13 @@
 //           for each spin, at n energies from lo to hi (default -2:1:301), as a long table DIR/<index>_Z<Z>_logderiv.tsv with the columns
 //           spin, l, E, D, nodes, phase = pi nodes - atan(r_c D), u, du at 17 digits (dftatom_log_derivatives; r_c = the grid node nearest
 //           to R).  The potential is the one the radial export returns; --radial is not needed.  Works with --gpus, --charge and --config.
+// --pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf]: Troullier-Martins pseudopotentials of every (LDA) atom (dftatom_tm_pseudize): for every l of the
+//           atom's levels the level of largest n is the valence channel, at the radius given for that l (an l beyond the list takes the
+//           last radius), and all channels of the atom are unscreened together.  DIR/<index>_Z<Z>_pseudo.tsv holds one "#" line per
+//           channel (l n eps occ r_c status c0 .. c12) and the columns r, V_ion per l, V_scr per l, u per l and rho_val at 17 digits.
+//           With --logderiv DIR2 --rc R (R >= every pseudo radius) also DIR2/<index>_Z<Z>_pseudo_logderiv.tsv: the logarithmic
+//           derivatives of the V_scr channels at the --energies, in the columns of the all-electron table (spin 0).  LSDA atoms are an
+//           error; works with --gpus, --charge and --config and does not need --radial.
 #include <algorithm>
 #include <cmath>
 #include <cctype>
@@ -267,11 +274,87 @@ static int write_logderiv(dftatom_ctx* ctx, const std::string& dir, int index, c
     return 0;
 }
 
+// --pseudo: the valence channels of one LDA atom (largest n per l of its levels), pseudized and unscreened together; with --logderiv
+// also the logarithmic derivatives of their V_scr rows at the all-electron table's radius and energies
+static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::string& ld_dir, int index, const dftatom_options& o,
+                        const dftatom_result& R, const dftatom_config* cfg, int N, const double* r, const double* v, const double* orb,
+                        const std::vector<double>& rcs, double ld_rc, const std::vector<double>& E)
+{
+    int best[4] = { -1, -1, -1, -1 };
+    for (int k = 0; k < R.n_levels[0]; ++k) {
+        const dftatom_level& L = R.levels[0][k];
+        if (best[L.l] < 0 || L.n > R.levels[0][best[L.l]].n) best[L.l] = k;
+    }
+    std::vector<dftatom_tm_channel> ch;
+    for (int l = 0; l < 4; ++l) {
+        if (best[l] < 0) continue;
+        const dftatom_level& L = R.levels[0][best[l]];
+        dftatom_tm_channel c = {};
+        c.pot = 0; c.orbital = best[l]; c.l = l; c.eps = L.E; c.occ = exact_occ(L, 0, cfg);
+        c.r_c = rcs[std::min<size_t>(l, rcs.size() - 1)];
+        ch.push_back(c);
+    }
+    const int nc = (int)ch.size();
+    std::vector<dftatom_tm_result> out(nc);
+    std::vector<double> u_ps((size_t)nc * N), v_scr((size_t)nc * N), v_ion((size_t)nc * N), rho(N);
+    if (dftatom_tm_pseudize(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v, 1, orb, R.n_levels[0], ch.data(), nc, out.data(), u_ps.data(),
+                            v_scr.data(), v_ion.data(), rho.data()) != DFTATOM_OK) {
+        std::fprintf(stderr, "dftatom: --pseudo Z=%d: %s\n", o.Z, dftatom_last_error());
+        return 1;
+    }
+    const std::string stem = "/" + std::to_string(index) + "_Z" + std::to_string(o.Z) + "_pseudo";
+    const std::string path = dir + stem + ".tsv";
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) { std::perror(path.c_str()); return 1; }
+    std::fprintf(f, "# Z=%d method=%d channels: l n eps occ r_c status c0 c2 c4 c6 c8 c10 c12\n", o.Z, o.method);
+    for (int c = 0; c < nc; ++c) {
+        std::fprintf(f, "# %d\t%d\t%.17g\t%.17g\t%.17g\t%d", ch[c].l, R.levels[0][ch[c].orbital].n, ch[c].eps, ch[c].occ, out[c].r_c, out[c].status);
+        for (int k = 0; k < 7; ++k) std::fprintf(f, "\t%.17g", out[c].c[k]);
+        std::fprintf(f, "\n");
+    }
+    std::fprintf(f, "# r");
+    for (const char* q : { "V_ion", "V_scr", "u" })
+        for (int c = 0; c < nc; ++c) std::fprintf(f, "\t%s %c", q, kOrb[ch[c].l]);
+    std::fprintf(f, "\trho_val\n");
+    for (int i = 0; i < N; ++i) {
+        std::fprintf(f, "%.17g", r[i]);
+        for (const std::vector<double>* q : { &v_ion, &v_scr, &u_ps })
+            for (int c = 0; c < nc; ++c) std::fprintf(f, "\t%.17g", (*q)[(size_t)c * N + i]);
+        std::fprintf(f, "\t%.17g\n", rho[i]);
+    }
+    bool bad = std::ferror(f) != 0;
+    if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
+    if (ld_dir.empty()) return 0;
+    const int ne = (int)E.size();
+    std::vector<int> pot(nc), l(nc);
+    std::vector<double> lrc(nc, ld_rc), used(nc);
+    for (int c = 0; c < nc; ++c) { pot[c] = c; l[c] = ch[c].l; }
+    std::vector<dftatom_logderiv> ld((size_t)nc * ne);
+    if (dftatom_log_derivatives(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v_scr.data(), nc, pot.data(), l.data(), lrc.data(), nc, E.data(), ne,
+                                ld.data(), used.data()) != DFTATOM_OK) {
+        std::fprintf(stderr, "dftatom: --pseudo --logderiv Z=%d: %s\n", o.Z, dftatom_last_error());
+        return 1;
+    }
+    const std::string lpath = ld_dir + stem + "_logderiv.tsv";
+    f = std::fopen(lpath.c_str(), "w");
+    if (!f) { std::perror(lpath.c_str()); return 1; }
+    std::fprintf(f, "# Z=%d method=%d r_c=%.17g V_scr\n# spin\tl\tE\tD\tnodes\tphase\tu\tdu\n", o.Z, o.method, used[0]);
+    for (int c = 0; c < nc; ++c)
+        for (int k = 0; k < ne; ++k) {
+            const dftatom_logderiv& q = ld[(size_t)c * ne + k];
+            const double phase = q.nodes < 0 ? NAN : M_PI * q.nodes - std::atan(used[c] * q.D);
+            std::fprintf(f, "%d\t%d\t%.17g\t%.17g\t%d\t%.17g\t%.17g\t%.17g\n", 0, l[c], E[k], q.D, q.nodes, phase, q.u, q.du);
+        }
+    bad = std::ferror(f) != 0;
+    if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", lpath.c_str()); return 1; }
+    return 0;
+}
+
 int main(int argc, char** argv)
 {
     dftatom_options base = { 36, 12, 10.0, 0.001, 0.5, 0 };     // Options.cpp:6
     std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
-    std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301";
+    std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301", pseudo_dir, pseudo_rc;
     double charge = 0., rc = NAN;
     int precision = 6, device = 0, gpus = 1;
     bool json = false, quiet = false, framed = false;      // framed: child of --gpus (one frame per atom on stdout)
@@ -288,6 +371,8 @@ int main(int argc, char** argv)
         else if (a == "--logderiv") logderiv_dir = next();
         else if (a == "--rc") rc = std::atof(next());
         else if (a == "--energies") energies = next();
+        else if (a == "--pseudo") pseudo_dir = next();
+        else if (a == "--pseudo-rc") pseudo_rc = next();
         else if (a == "--charge") charge = std::atof(next());
         else if (a == "--config") config_str = next();
         else if (a == "--levels") base.levels = std::atoi(next());
@@ -307,14 +392,17 @@ int main(int argc, char** argv)
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
                         "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR] [--charge Q] [--config \"...\"]\n"
-                        "               [--logderiv DIR --rc R [--energies lo:hi:n]]\n"
+                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf]]\n"
                         "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n"
                         "  --charge Q    solve every atom of --Z ionised by Q electrons (the reference's configuration; fractional allowed, < 0 = anion)\n"
                         "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n"
                         "  --logderiv DIR  write the logarithmic derivatives D_l(E) = u'(r_c)/u(r_c), l = 0..3 per spin, of every atom's converged V to\n"
                         "                DIR/<index>_Z<Z>_logderiv.tsv (columns spin l E D nodes phase u du)\n"
                         "  --rc R        radius of --logderiv in bohr (the nearest grid node is used)\n"
-                        "  --energies lo:hi:n  energies of --logderiv, n points from lo to hi Hartree (default -2:1:301)\n");
+                        "  --energies lo:hi:n  energies of --logderiv, n points from lo to hi Hartree (default -2:1:301)\n"
+                        "  --pseudo DIR  write Troullier-Martins pseudopotentials of every LDA atom (valence = largest n per l) to DIR/<index>_Z<Z>_pseudo.tsv\n"
+                        "                (columns r, V_ion per l, V_scr per l, u per l, rho_val); with --logderiv also <index>_Z<Z>_pseudo_logderiv.tsv\n"
+                        "  --pseudo-rc Rs[,Rp,Rd,Rf]  radii of --pseudo in bohr by l (an l beyond the list takes the last one)\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
         if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
@@ -332,6 +420,24 @@ int main(int argc, char** argv)
         for (int k = 0; k < ne; ++k) ld_E.push_back(k == ne - 1 && ne > 1 ? hi : lo + (hi - lo) * k / (ne > 1 ? ne - 1 : 1));
         if (!(rc > 0.)) { std::fprintf(stderr, "dftatom: --logderiv needs --rc R (bohr)\n"); return 2; }
         if (mkdir(logderiv_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(logderiv_dir.c_str()); return 1; }
+    }
+    std::vector<double> ps_rc;
+    if (!pseudo_dir.empty()) {
+        if (base.method & 1) { std::fprintf(stderr, "dftatom: --pseudo needs an LDA atom (method 0 or 2): the unscreening is spin-unpolarised\n"); return 2; }
+        for (size_t p = 0; p < pseudo_rc.size();) {
+            const size_t q = std::min(pseudo_rc.find(',', p), pseudo_rc.size());
+            char* end = nullptr;
+            const std::string tok = pseudo_rc.substr(p, q - p);
+            const double x = std::strtod(tok.c_str(), &end);
+            if (tok.empty() || *end || !(x > 0.)) { std::fprintf(stderr, "dftatom: --pseudo-rc expects Rs[,Rp,Rd,Rf] in bohr, got '%s'\n", pseudo_rc.c_str()); return 2; }
+            ps_rc.push_back(x);
+            p = q + 1;
+        }
+        if (ps_rc.empty() || ps_rc.size() > 4) { std::fprintf(stderr, "dftatom: --pseudo needs --pseudo-rc Rs[,Rp,Rd,Rf] (1 to 4 radii)\n"); return 2; }
+        if (!logderiv_dir.empty() && rc < *std::max_element(ps_rc.begin(), ps_rc.end())) {
+            std::fprintf(stderr, "dftatom: with --pseudo, --rc must be >= every --pseudo-rc radius\n"); return 2;
+        }
+        if (mkdir(pseudo_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(pseudo_dir.c_str()); return 1; }
     }
     if (gpus > 1) {
         char self[4096];
@@ -361,7 +467,8 @@ int main(int argc, char** argv)
     // --radial: arrays of the whole batch, rows of the orbitals in call order (dftatom_radial)
     const int N = dftatom_n_nodes(base.levels);
     std::vector<long long> row0(n + 1, 0);
-    for (int k = 0; k < n && !radial_dir.empty(); ++k) {
+    const bool export_orb = !radial_dir.empty() || !pseudo_dir.empty();
+    for (int k = 0; k < n && export_orb; ++k) {
         dftatom_level la[DFTATOM_MAX_LEVELS], lb[DFTATOM_MAX_LEVELS];
         int na = 0, nb = 0, ea = 0, eb = 0;
         if (configured) na = cfgs[k].n_orbitals;
@@ -371,11 +478,11 @@ int main(int argc, char** argv)
     }
     std::vector<double> r_grid, rho, vks, vh, orb;
     dftatom_radial rad = {};
-    if (!radial_dir.empty()) {
+    if (export_orb) {
         r_grid.resize(N); rho.resize((size_t)n * 2 * N); vh.resize((size_t)n * N); orb.resize((size_t)row0[n] * N);
         rad.r = r_grid.data(); rad.rho = rho.data(); rad.v_hartree = vh.data(); rad.orbitals = orb.data(); rad.orbital_rows = row0[n];
     }
-    const bool export_v = !radial_dir.empty() || !logderiv_dir.empty();
+    const bool export_v = export_orb || !logderiv_dir.empty();
     if (export_v) { vks.resize((size_t)n * 2 * N); rad.v = vks.data(); }
     if (dftatom_solve_batch_config(ctx, opts.data(), configured ? cfgs.data() : nullptr, n, res.data(), steps.data(), stride,
                                    export_v ? &rad : nullptr) != DFTATOM_OK) {
@@ -390,6 +497,11 @@ int main(int argc, char** argv)
                          &vh[(size_t)a * N], &orb[(size_t)row0[a] * N])) { dftatom_destroy(ctx); return 1; }
     for (int a = 0; a < n && !logderiv_dir.empty(); ++a)
         if (write_logderiv(ctx, logderiv_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a].n_spin, &vks[(size_t)a * 2 * N], rc, ld_E)) {
+            dftatom_destroy(ctx); return 1;
+        }
+    for (int a = 0; a < n && !pseudo_dir.empty(); ++a)
+        if (write_pseudo(ctx, pseudo_dir, logderiv_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a], configured ? &cfgs[a] : nullptr, N,
+                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E)) {
             dftatom_destroy(ctx); return 1;
         }
 

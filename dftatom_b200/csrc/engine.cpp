@@ -1170,6 +1170,17 @@ int dftatom_numerov_lanes_timed(dftatom_ctx* c, const double* V, int levels, dou
                               lane_node_steps);
 }
 
+static int poisson_cold(dftatom_ctx* c, const GridDev& g, int n_dens, const double* d_rho, const double* d_zbc, int* d_vcycles, long long* ld_out,
+                        bool* streamed);
+
+// the node used for a radius r_2 <= r_c <= r_(N-2): the nearest one, ties to the inner one
+static int nearest_node(const std::vector<double>& r, double r_c)
+{
+    const int N = (int)r.size();
+    const int hi = (int)(std::lower_bound(r.begin() + 2, r.begin() + (N - 1), r_c) - r.begin());      // first node >= r_c, 2..N-2
+    return (hi > 2 && r_c - r[hi - 1] <= r[hi] - r_c) ? hi - 1 : hi;
+}
+
 int dftatom_log_derivatives(dftatom_ctx* c, int levels, double delta, double max_r, const double* V, int n_pot, const int* pot, const int* l,
                             const double* r_c, int n_channels, const double* E, int n_energies, dftatom_logderiv* out, double* r_used)
 {
@@ -1192,8 +1203,7 @@ int dftatom_log_derivatives(dftatom_ctx* c, int levels, double delta, double max
             std::snprintf(b, sizeof b, "r_c = %.17g outside [r_2, r_(N-2)] = [%.17g, %.17g]", r_c[k], r[2], r[N - 2]);
             set_error(where("channel", k) + b); return DFTATOM_E_ARG;
         }
-        const int hi = (int)(std::lower_bound(r.begin() + 2, r.begin() + (N - 1), r_c[k]) - r.begin());      // first node >= r_c, 2..N-2
-        ic[k] = (hi > 2 && r_c[k] - r[hi - 1] <= r[hi] - r_c[k]) ? hi - 1 : hi;                           // nearest node, ties to the inner one
+        ic[k] = nearest_node(r, r_c[k]);
     }
     for (int k = 0; k < n_energies; ++k)
         if (!std::isfinite(E[k])) { set_error(where("energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
@@ -1231,6 +1241,130 @@ int dftatom_log_derivatives(dftatom_ctx* c, int levels, double delta, double max
     DFT_CHECK(cudaMemcpyAsync(out, dO.p, sizeof(dftatom_logderiv) * n_out, cudaMemcpyDeviceToHost, st));
     DFT_CHECK(cudaStreamSynchronize(st));
     if (r_used) for (int k = 0; k < n_channels; ++k) r_used[k] = r[ic[k]];
+    return 0;
+}
+
+int dftatom_grid_nodes(dftatom_ctx* c, int levels, double delta, double max_r, double* r)
+{
+    if (!c || !r) { set_error("dftatom_grid_nodes: NULL argument"); return DFTATOM_E_ARG; }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    DFT_CHECK(cudaMemcpyAsync(r, gp->r, sizeof(double) * gp->N, cudaMemcpyDeviceToHost, c->stream));
+    DFT_CHECK(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, const double* V, int n_pot, const double* u, int n_orb,
+                        const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
+                        double* v_ion, double* rho_val)
+{
+    if (!c || !V || !u || !ch || !out) { set_error("dftatom_tm_pseudize: NULL argument"); return DFTATOM_E_ARG; }
+    if (n_pot < 1 || n_orb < 1 || n_channels < 1) { set_error("dftatom_tm_pseudize: n_pot, n_orb and n_channels must be >= 1"); return DFTATOM_E_ARG; }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
+    if (N < 7) { set_error("dftatom_tm_pseudize: the grid needs at least 7 nodes"); return DFTATOM_E_ARG; }
+    if ((long long)n_channels + n_pot > 65535 || (long long)std::max(n_pot, n_channels) * N >= (1LL << 31)) {
+        set_error("dftatom_tm_pseudize: too many channels or potential rows for one call"); return DFTATOM_E_ARG;
+    }
+    std::vector<double> r(N);             // the device's node radii: r_c is rounded to one of them
+    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    const auto where = [](const char* what, long long k) { return std::string("dftatom_tm_pseudize: ") + what + " " + std::to_string(k) + ": "; };
+    for (int p = 0; p < n_pot; ++p)
+        for (int i = 1; i < N; ++i)
+            if (!std::isfinite(V[(size_t)p * N + i])) { set_error(where("potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    for (int o = 0; o < n_orb; ++o)
+        for (int i = 1; i < N; ++i)
+            if (!std::isfinite(u[(size_t)o * N + i])) { set_error(where("orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    std::vector<int> ic(n_channels);
+    std::vector<unsigned> l_taken(n_pot, 0u);             // per potential row: bit l set once a channel takes l
+    for (int k = 0; k < n_channels; ++k) {
+        const dftatom_tm_channel& q = ch[k];
+        const std::string at = where("channel", k);
+        if (q.pot < 0 || q.pot >= n_pot) { set_error(at + "pot = " + std::to_string(q.pot) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
+        if (q.orbital < 0 || q.orbital >= n_orb) { set_error(at + "orbital = " + std::to_string(q.orbital) + " outside 0.." + std::to_string(n_orb - 1)); return DFTATOM_E_ARG; }
+        if (q.l < 0 || q.l > 3) { set_error(at + "l = " + std::to_string(q.l) + " outside 0..3"); return DFTATOM_E_ARG; }
+        if (l_taken[q.pot] & (1u << q.l)) { set_error(at + "l = " + std::to_string(q.l) + " already taken by another channel of potential row " + std::to_string(q.pot)); return DFTATOM_E_ARG; }
+        l_taken[q.pot] |= 1u << q.l;
+        if (!(q.r_c >= r[3] && q.r_c <= r[N - 3])) {      // i_c >= 3: the 5-point stencil of V' and V'' stays off node 0
+            char b[160];
+            std::snprintf(b, sizeof b, "r_c = %.17g outside [r_3, r_(N-3)] = [%.17g, %.17g]", q.r_c, r[3], r[N - 3]);
+            set_error(at + b); return DFTATOM_E_ARG;
+        }
+        if (!std::isfinite(q.eps)) { set_error(at + "eps is not finite"); return DFTATOM_E_ARG; }
+        if (!(q.occ >= 0. && q.occ <= 2. * (2 * q.l + 1))) { set_error(at + "occ is not finite or outside [0, 2(2l+1)]"); return DFTATOM_E_ARG; }
+        ic[k] = nearest_node(r, q.r_c);
+        const double* ur = u + (size_t)q.orbital * N;
+        if (ur[ic[k]] == 0.) { set_error(at + "u is 0 at r_c (node " + std::to_string(ic[k]) + ")"); return DFTATOM_E_ARG; }
+        const bool pos = ur[ic[k]] > 0.;
+        for (int i = ic[k] + 1; i < N; ++i)
+            if (pos ? ur[i] < 0. : ur[i] > 0.) { set_error(at + "u changes sign at node " + std::to_string(i) + " beyond r_c: r_c lies inside the outermost node"); return DFTATOM_E_ARG; }
+    }
+    // host tables: the channels dealt longest i_c first; the channels of each potential row; rows with electrons first (their Poisson solves)
+    std::vector<int> order(n_channels);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return ic[a] > ic[b]; });
+    std::vector<int> row_begin(n_pot + 1, 0), row_chan(n_channels), slot(n_pot);
+    std::vector<double> qv(n_pot, 0.), eps(n_channels), occ(n_channels);
+    for (int k = 0; k < n_channels; ++k) { ++row_begin[ch[k].pot + 1]; qv[ch[k].pot] += ch[k].occ; eps[k] = ch[k].eps; occ[k] = ch[k].occ; }
+    for (int p = 0; p < n_pot; ++p) row_begin[p + 1] += row_begin[p];
+    {
+        std::vector<int> fill(row_begin.begin(), row_begin.end() - 1);
+        for (int k = 0; k < n_channels; ++k) row_chan[fill[ch[k].pot]++] = k;
+    }
+    int n_solve = 0;
+    for (int p = 0; p < n_pot; ++p) if (qv[p] > 0.) slot[p] = n_solve++;
+    std::vector<double> zbc;
+    for (int p = 0; p < n_pot; ++p) if (qv[p] > 0.) zbc.push_back(qv[p]);
+    for (int p = 0, s = n_solve; p < n_pot; ++p) if (!(qv[p] > 0.)) slot[p] = s++;
+    std::vector<int> h_int;                                   // pot | orbital | l | ic | order | row_chan | row_begin | slot
+    for (int k = 0; k < n_channels; ++k) h_int.push_back(ch[k].pot);
+    for (int k = 0; k < n_channels; ++k) h_int.push_back(ch[k].orbital);
+    for (int k = 0; k < n_channels; ++k) h_int.push_back(ch[k].l);
+    h_int.insert(h_int.end(), ic.begin(), ic.end());
+    h_int.insert(h_int.end(), order.begin(), order.end());
+    h_int.insert(h_int.end(), row_chan.begin(), row_chan.end());
+    h_int.insert(h_int.end(), row_begin.begin(), row_begin.end());
+    h_int.insert(h_int.end(), slot.begin(), slot.end());
+    std::vector<double> h_dbl(eps);                           // eps | occ | zbc
+    h_dbl.insert(h_dbl.end(), occ.begin(), occ.end());
+    h_dbl.insert(h_dbl.end(), zbc.begin(), zbc.end());
+    const size_t nV = (size_t)n_pot * N, nU = (size_t)n_orb * N, nC = (size_t)n_channels * N;
+    DevBuf& dD = c->scratch[0]; DevBuf& dI = c->scratch[1]; DevBuf& dR = c->scratch[2]; DevBuf& dv = c->scratch[3];
+    const size_t n_dbl = 6 * nV + nU + 3 * nC + h_dbl.size();      // V atab rho rho_out vxc edif | u | u_ps v_scr v_ion | eps occ zbc
+    if ((rc = dD.ensure(sizeof(double) * n_dbl)) || (rc = dI.ensure(sizeof(int) * h_int.size())) || (rc = dR.ensure(sizeof(dftatom_tm_result) * n_channels)) ||
+        (rc = dv.ensure(sizeof(int) * n_pot))) return rc;
+    double* d = dD.as<double>();
+    double* dV = d; double* dA = dV + nV; double* drho = dA + nV; double* drho_out = drho + nV; double* dvxc = drho_out + nV; double* dedif = dvxc + nV;
+    double* du = dedif + nV; double* dups = du + nU; double* dvscr = dups + nC; double* dvion = dvscr + nC; double* dh = dvion + nC;
+    const int* di = dI.as<int>();
+    DFT_CHECK(cudaMemcpyAsync(dV, V, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(du, u, sizeof(double) * nU, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dh, h_dbl.data(), sizeof(double) * h_dbl.size(), cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dI.p, h_int.data(), sizeof(int) * h_int.size(), cudaMemcpyHostToDevice, st));
+    launch_build_atab(g, dV, dA, n_pot, st);
+    const size_t nc = (size_t)n_channels;
+    TmArgs ta{ dV, dA, du, di, di + nc, di + 2 * nc, di + 3 * nc, dh, di + 4 * nc, n_channels, dR.as<dftatom_tm_result>(), dups, dvscr };
+    launch_tm(g, ta, st);
+    TmRowArgs ra{ n_pot, n_channels, di + 6 * nc, di + 5 * nc, di, dh + nc, dR.as<dftatom_tm_result>(), dups, dvscr, di + 6 * nc + n_pot + 1, n_solve,
+                  drho, nullptr, N, dvxc, dvion, drho_out };
+    launch_tm_density(g, ra, st);
+    if (n_solve > 0) {
+        long long ld = N; bool streamed = false;
+        if ((rc = poisson_cold(c, g, n_solve, drho, dh + 2 * nc, dv.as<int>(), &ld, &streamed))) return rc;
+        ra.U = c->ubuf.as<double>(); ra.ldU = ld;
+    }
+    launch_vwn((int)nV, drho, nullptr, nullptr, nullptr, dvxc, dedif, st);
+    launch_tm_unscreen(g, ra, st);
+    DFT_CHECK(cudaGetLastError());
+    DFT_CHECK(cudaMemcpyAsync(out, dR.p, sizeof(dftatom_tm_result) * n_channels, cudaMemcpyDeviceToHost, st));
+    if (u_ps) DFT_CHECK(cudaMemcpyAsync(u_ps, dups, sizeof(double) * nC, cudaMemcpyDeviceToHost, st));
+    if (v_scr) DFT_CHECK(cudaMemcpyAsync(v_scr, dvscr, sizeof(double) * nC, cudaMemcpyDeviceToHost, st));
+    if (v_ion) DFT_CHECK(cudaMemcpyAsync(v_ion, dvion, sizeof(double) * nC, cudaMemcpyDeviceToHost, st));
+    if (rho_val) DFT_CHECK(cudaMemcpyAsync(rho_val, drho_out, sizeof(double) * nV, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
     return 0;
 }
 
@@ -1324,16 +1458,36 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
     DFT_CHECK(cudaSetDevice(c->device));
     GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
-    const PoissonLevels lv = make_levels(levels);
     DevBuf& dr = c->scratch[0]; DevBuf& dz = c->scratch[2]; DevBuf& dv = c->scratch[3];
     if ((rc = dr.ensure(sizeof(double) * (size_t)n_dens * N)) || (rc = dz.ensure(sizeof(double) * n_dens)) || (rc = dv.ensure(sizeof(int) * n_dens))) return rc;
-    if ((rc = c->phi.ensure(sizeof(double) * (size_t)n_dens * lv.total)) || (rc = c->src.ensure(sizeof(double) * (size_t)n_dens * lv.total))) return rc;
     const std::vector<double> zbc(Z, Z + n_dens);            // the solvers take the boundary value as a double (an electron count)
     DFT_CHECK(cudaMemcpyAsync(dr.p, rho, sizeof(double) * (size_t)n_dens * N, cudaMemcpyHostToDevice, st));
     DFT_CHECK(cudaMemcpyAsync(dz.p, zbc.data(), sizeof(double) * n_dens, cudaMemcpyHostToDevice, st));
+    long long ld = N; bool streamed = false;
+    if ((rc = poisson_cold(c, g, n_dens, dr.as<double>(), dz.as<double>(), dv.as<int>(), &ld, &streamed))) return rc;
+    if (ld != N) DFT_CHECK(cudaMemcpy2DAsync(U, sizeof(double) * N, c->ubuf.p, sizeof(double) * ld, sizeof(double) * N, n_dens, cudaMemcpyDeviceToHost, st));
+    else DFT_CHECK(cudaMemcpyAsync(U, c->ubuf.p, sizeof(double) * (size_t)n_dens * N, cudaMemcpyDeviceToHost, st));
+    if (vcycles_used && streamed) for (int k = 0; k < n_dens; ++k) vcycles_used[k] = c->k.max_vcycles;
+    else if (vcycles_used) DFT_CHECK(cudaMemcpyAsync(vcycles_used, dv.p, sizeof(int) * n_dens, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
+    return 0;
+}
+
+// The device part of dftatom_poisson_solve: the cold solve of n_dens densities d_rho [n_dens][N] with boundary values d_zbc [n_dens]
+// (device arrays).  U = r V_H lands in c->ubuf with row stride *ld; d_vcycles [n_dens] receives the V-cycles run, except in stream mode
+// (*streamed), which runs c->k.max_vcycles V-cycles for every density.
+static int poisson_cold(dftatom_ctx* c, const GridDev& g, int n_dens, const double* d_rho, const double* d_zbc, int* d_vcycles, long long* ld_out,
+                        bool* streamed)
+{
+    const int N = g.N, levels = g.L; const double delta = g.delta; cudaStream_t st = c->stream;
+    const PoissonLevels lv = make_levels(levels);
+    int rc;
+    *ld_out = N; *streamed = false;
+    if ((rc = c->phi.ensure(sizeof(double) * (size_t)n_dens * lv.total)) || (rc = c->src.ensure(sizeof(double) * (size_t)n_dens * lv.total))) return rc;
     PoissonArgs pa{};
-    pa.n_dens = n_dens; pa.rho = dr.as<double>(); pa.Zbc = dz.as<double>(); pa.phi = c->phi.as<double>(); pa.src = c->src.as<double>();
-    pa.max_vcycles = c->k.max_vcycles; pa.floor_stop = c->k.floor_stop; pa.vcycles_used = dv.as<int>();
+    pa.n_dens = n_dens; pa.rho = d_rho; pa.Zbc = d_zbc; pa.phi = c->phi.as<double>(); pa.src = c->src.as<double>();
+    pa.max_vcycles = c->k.max_vcycles; pa.floor_stop = c->k.floor_stop; pa.vcycles_used = d_vcycles;
     if ((rc = c->u0.ensure(sizeof(double) * (size_t)n_dens * N)) || (rc = c->ubuf.ensure(sizeof(double) * (size_t)n_dens * N))) return rc;
     pa.refine_vcycles = c->k.refine_vcycles; pa.u0 = c->u0.as<double>(); pa.u_out = c->ubuf.as<double>(); pa.coarse_op = g.coarse_op; pa.n_sm = c->n_sm;
     if ((rc = c->team_bar.ensure(sizeof(unsigned) * (size_t)n_dens))) return rc;
@@ -1348,14 +1502,10 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
         // bit-reproducible mode: the reference's FullCycle in its own operation order (poisson_exact.cu), 100 V-cycles
         if ((rc = c->exact_work.ensure(sizeof(double) * (size_t)n_dens * (size_t)exact_poisson_work_doubles(levels)))) return rc;
         ExactPoissonArgs xa{};
-        xa.n_dens = n_dens; xa.L = levels; xa.delta = delta; xa.rho = dr.as<double>(); xa.rho_stride = N; xa.r = g.r; xa.pex = g.pex;
-        xa.Zbc = dz.as<double>(); xa.U = c->ubuf.as<double>(); xa.ldU = N; xa.work = c->exact_work.as<double>(); xa.max_vcycles = 100;
-        xa.vcycles_used = dv.as<int>();
+        xa.n_dens = n_dens; xa.L = levels; xa.delta = delta; xa.rho = d_rho; xa.rho_stride = N; xa.r = g.r; xa.pex = g.pex;
+        xa.Zbc = d_zbc; xa.U = c->ubuf.as<double>(); xa.ldU = N; xa.work = c->exact_work.as<double>(); xa.max_vcycles = 100;
+        xa.vcycles_used = d_vcycles;
         launch_poisson_exact(xa, st);
-        DFT_CHECK(cudaMemcpyAsync(U, c->ubuf.p, sizeof(double) * (size_t)n_dens * N, cudaMemcpyDeviceToHost, st));
-        if (vcycles_used) DFT_CHECK(cudaMemcpyAsync(vcycles_used, dv.p, sizeof(int) * n_dens, cudaMemcpyDeviceToHost, st));
-        DFT_CHECK(cudaStreamSynchronize(st));
-        DFT_CHECK(cudaGetLastError());
         return 0;
     }
     const bool stream = c->k.stream_poisson && n_dens >= c->k.stream_min_dens && levels >= c->k.stream_min_levels && levels > c->k.stream_mid_levels && levels <= 22 && c->k.refine_vcycles == 0 && !c->k.floor_stop && !c->k.profile;
@@ -1366,14 +1516,11 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
         if ((rc = c->stream_src0.ensure(sizeof(double) * (size_t)n_dens * ld)) || (rc = c->stream_scratch.ensure(sizeof(double) * (size_t)splan.total))) return rc;
         if ((rc = c->ubuf.ensure(sizeof(double) * (size_t)n_dens * ld))) return rc;
         StreamSolveArgs sa{};
-        sa.n_dens = n_dens; sa.rho = dr.as<double>(); sa.rho_stride = N; sa.psrc = g.psrc; sa.src0 = c->stream_src0.as<double>();
-        sa.U = c->ubuf.as<double>(); sa.ld0 = ld; sa.Zbc = dz.as<double>(); sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op;
+        sa.n_dens = n_dens; sa.rho = d_rho; sa.rho_stride = N; sa.psrc = g.psrc; sa.src0 = c->stream_src0.as<double>();
+        sa.U = c->ubuf.as<double>(); sa.ld0 = ld; sa.Zbc = d_zbc; sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op;
         sa.n_v = c->k.max_vcycles; sa.warm = 0; sa.variant = c->k.stream_variant;
         launch_poisson_stream_solve(splan, delta, sa, st, nullptr);
-        DFT_CHECK(cudaMemcpy2DAsync(U, sizeof(double) * N, c->ubuf.p, sizeof(double) * ld, sizeof(double) * N, n_dens, cudaMemcpyDeviceToHost, st));
-        if (vcycles_used) for (int k = 0; k < n_dens; ++k) vcycles_used[k] = c->k.max_vcycles;
-        DFT_CHECK(cudaStreamSynchronize(st));
-        DFT_CHECK(cudaGetLastError());
+        *ld_out = ld; *streamed = true;
         return 0;
     }
     launch_poisson_full(g, lv, pa, st);
@@ -1395,10 +1542,6 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
                 fprintf(stderr, "  level %2d n=%7d  visits %9lld cycles (%lld visits)\n", l, (1 << (levels - l)), h[l], h[72 + l]);
         }
     }
-    DFT_CHECK(cudaMemcpyAsync(U, c->ubuf.p, sizeof(double) * (size_t)n_dens * N, cudaMemcpyDeviceToHost, st));
-    if (vcycles_used) DFT_CHECK(cudaMemcpyAsync(vcycles_used, dv.p, sizeof(int) * n_dens, cudaMemcpyDeviceToHost, st));
-    DFT_CHECK(cudaStreamSynchronize(st));
-    DFT_CHECK(cudaGetLastError());
     return 0;
 }
 

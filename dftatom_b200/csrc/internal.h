@@ -347,6 +347,30 @@ struct LogDerivArgs {
 };
 void launch_logderiv(const GridDev& g, const LogDerivArgs& a, cudaStream_t st);
 
+// Troullier-Martins pseudization (pseudo.cu): one CTA per channel, dealt in the order `order` (longest i_c first)
+struct TmArgs {
+    const double* V; const double* atab;          // [n_pot][N] potentials and their a-tables (launch_build_atab)
+    const double* u;                              // [n_orb][N] all-electron orbitals
+    const int* pot; const int* orbital; const int* l; const int* ic;   // [n_channels]; 2 <= ic <= N - 3
+    const double* eps;                            // [n_channels]
+    const int* order; int n_channels;
+    dftatom_tm_result* res;                       // [n_channels]
+    double* u_ps; double* v_scr;                  // [n_channels][N]
+};
+void launch_tm(const GridDev& g, const TmArgs& a, cudaStream_t st);
+// valence density and unscreening per potential row; the channels of row p are row_chan[row_begin[p] .. row_begin[p + 1]).  Row p's
+// density and V_xc are rows slot[p] of rho / vxc; its U = r V_H is row slot[p] of U when slot[p] < n_solve, else V_H = 0 (no electrons)
+struct TmRowArgs {
+    int n_pot, n_channels;
+    const int* row_begin; const int* row_chan; const int* pot; const double* occ;
+    const dftatom_tm_result* res; const double* u_ps; const double* v_scr;
+    const int* slot; int n_solve;
+    double* rho; const double* U; long long ldU; const double* vxc;
+    double* v_ion; double* rho_out;               // [n_channels][N], [n_pot][N]
+};
+void launch_tm_density(const GridDev& g, const TmRowArgs& a, cudaStream_t st);
+void launch_tm_unscreen(const GridDev& g, const TmRowArgs& a, cudaStream_t st);
+
 // host rules (aufbau.cpp)
 int aufbau(int Z, dftatom_level* out, int max_out);
 int split_spin(int Z, dftatom_level* a, int* na, dftatom_level* b, int* nb, int* ea, int* eb);

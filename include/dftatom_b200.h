@@ -334,6 +334,42 @@ typedef struct { double D, u, du; int nodes, pad; } dftatom_logderiv;      /* 32
 int dftatom_log_derivatives(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, int n_pot,
                             const int* pot, const int* l, const double* r_c, int n_channels,
                             const double* E, int n_energies, dftatom_logderiv* out, double* r_used);
+/* Troullier-Martins norm-conserving pseudization of all-electron valence orbitals, and unscreening to ionic semilocal potentials.
+ * Grid (levels, delta, max_r) and r_c rounding (the nearest node i_c, ties to the inner node), quadrature (Simpson 1/3 on nodes 0..i_c,
+ * the 3/8 rule on the last three intervals when i_c is odd) and outward sweep are those of dftatom_log_derivatives.
+ * V[n_pot][N] HOST potentials (node 0 ignored), u[n_orb][N] HOST all-electron orbitals u_nl(r) (e.g. rows of dftatom_radial.v and
+ * dftatom_radial.orbitals).  Channel c = ch[c]: potential row pot, orbital row orbital, l, eigenvalue eps, occupation occ, radius r_c.
+ * AE data at r_c: the sweep at E = eps on V[pot] gives D = u'/u and u_n(r_c) (solution normalised to int_0^rc u^2 dr = 1); a = |u(i_c)|,
+ * s = sign u(i_c), q = a^2 / u_n(r_c)^2 (the AE norm inside r_c); V' and V'' at r_c from 5-point central differences in the index with
+ * the chain rule: V' = V_i / J, V'' = (V_ii - delta V_i) / J^2, J = dr/di = delta (r + Rp) (uniform grid: J = h).
+ * Pseudo-orbital inside r_c: u_ps = r^(l+1) e^p(r), p = c0 + c2 r^2 + c4 r^4 + ... + c12 r^12, with
+ *   p = ln(a / r_c^(l+1)),  p' = D - (l+1)/r,  p'' = 2(V - eps) - 2(l+1)p'/r - p'^2,
+ *   p''' = 2V' + 2(l+1)p'/r^2 - 2(l+1)p''/r - 2p'p'',
+ *   p'''' = 2V'' - 4(l+1)p'/r^3 + 4(l+1)p''/r^2 - 2(l+1)p'''/r - 2p''^2 - 2p'p'''   at r_c,
+ *   c2^2 + (2l+5) c4 = 0 (V_scr''(0) = 0), and the norm F(c2) = ln S(c2) - ln q = 0, S = Simpson sum of r^(2l+2) e^(2p) dr/di over 0..i_c.
+ * For a given c2 the derivative conditions are linear in c6..c12.  Root: with x = c2 r_c^2 the ladder x = +-k/2 (k = 0..128) is scanned
+ * outward from 0, the negative interval first at each |x|; the root in the first interval where F changes sign, to 1e-13 relative in c2.
+ * out[c]: c0, c2, ..., c12 (bohr^-2k), r_c used, q, status: 0 ok, 1 no sign change on the ladder, 2 the sweep met 1 - g <= 0 (q = NaN),
+ * 3 the multisection stopped short of 1e-13 (no sub-interval of the bracket changed sign, e.g. F not finite inside it, or 40 rounds).
+ * Rows (each output may be NULL), node 0 = 0 in every row:
+ *   u_ps[n_channels][N]   r^(l+1) e^p for i <= i_c, s u(i) copied for i > i_c
+ *   v_scr[n_channels][N]  eps + [p'' + p'^2 + 2(l+1) p'/r] / 2 for i <= i_c (p'/r a polynomial), V[pot] copied for i > i_c
+ *   rho_val[n_pot][N]     valence density sum occ u_ps^2 / (4 pi r^2) of the channels sharing the row (0 for a row without channels)
+ *   v_ion[n_channels][N]  V_scr - V_H - V_xc: V_H = U / r from the cold Poisson solve of rho_val with boundary value Q_v = sum occ
+ *                         (V_H = 0 when Q_v = 0), V_xc the spin-unpolarised VWN LDA of the SCF
+ * A failed channel (status != 0) has NaN coefficients and NaN in u_ps, v_scr at nodes 1..i_c; its row's rho_val and every v_ion row of
+ * that potential row are NaN at nodes 1..N-1.
+ * Validation before anything runs on the device (outputs untouched): a bad grid returns DFTATOM_E_BAD_OPTION; DFTATOM_E_ARG, naming the
+ * channel or row, for NULL V, u, ch or out, n_pot, n_orb or n_channels < 1, pot or orbital out of range, l outside 0..3, two channels of
+ * one pot with the same l, r_c outside [r_3, r_(N-3)] (the 5-point stencil at i_c stays off node 0), eps not finite, occ not finite or outside [0, 2(2l+1)], V or u not finite at
+ * nodes 1..N-1, u(i_c) = 0, or a sign change among the non-zero values of u at nodes i_c..N-1 (r_c inside the outermost node). */
+typedef struct { int pot, orbital, l, pad; double eps, occ, r_c; } dftatom_tm_channel;      /* 40 bytes */
+typedef struct { double c[7], r_c, q; int status, pad; } dftatom_tm_result;               /* 80 bytes */
+int dftatom_tm_pseudize(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, int n_pot, const double* u, int n_orb,
+                        const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
+                        double* v_ion, double* rho_val);
+/* The node radii r[N] (HOST) of the grid (levels, delta, max_r; delta = 0: uniform) as the engine builds and uses them. */
+int dftatom_grid_nodes(dftatom_ctx* ctx, int levels, double delta, double max_r, double* r);
 /* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) (the SCF passes the
  * electron count as a double; Z[k] is converted exactly) */
 int dftatom_poisson_solve(dftatom_ctx* ctx, int levels, double delta, double max_r, int n_dens, const int* Z,
