@@ -66,6 +66,19 @@ class _CTmResult(C.Structure):
     _fields_ = [("c", C.c_double * 7), ("r_c", C.c_double), ("q", C.c_double), ("status", C.c_int), ("pad", C.c_int)]
 
 
+class _CKbChannel(C.Structure):
+    _fields_ = [("row", C.c_int), ("loc", C.c_int), ("l", C.c_int), ("pad", C.c_int), ("eps", C.c_double)]
+
+
+class _CKbResult(C.Structure):
+    _fields_ = [("E_KB", C.c_double), ("cos", C.c_double), ("eps_loc", C.c_double * 2), ("r_s", C.c_double), ("i_s", C.c_int),
+                ("ghost", C.c_int), ("status", C.c_int), ("pad", C.c_int)]
+
+
+class _CKbLdChannel(C.Structure):
+    _fields_ = [("pot", C.c_int), ("proj", C.c_int), ("l", C.c_int), ("pad", C.c_int), ("E_KB", C.c_double), ("r_c", C.c_double)]
+
+
 class _COccupation(C.Structure):
     _fields_ = [("n", C.c_int), ("l", C.c_int), ("spin", C.c_int), ("occ", C.c_double)]
 
@@ -126,6 +139,10 @@ def load_library():
     lib.dftatom_grid_nodes.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp]
     lib.dftatom_tm_pseudize.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp, C.c_int, C.POINTER(_CTmChannel), C.c_int,
                                         C.POINTER(_CTmResult), _dp, _dp, _dp, _dp]
+    lib.dftatom_kb_form.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, _dp, C.c_int, C.POINTER(_CKbChannel), C.c_int,
+                                    C.POINTER(_CKbResult), _dp]
+    lib.dftatom_kb_log_derivatives.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp, C.c_int, C.POINTER(_CKbLdChannel),
+                                               C.c_int, _dp, C.c_int, C.POINTER(_CLogDeriv), _dp]
     lib.dftatom_last_timing.argtypes = [C.c_void_p, _dp, C.POINTER(C.c_longlong)]
     lib.dftatom_last_graph_iterations.argtypes = [C.c_void_p, C.POINTER(C.c_longlong)]
     lib.dftatom_last_transfer.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]
@@ -338,6 +355,30 @@ class Pseudopotential:
     V_ion: np.ndarray
     rho_val: np.ndarray
     pot: np.ndarray
+    grid: Optional[tuple] = None        # (levels, delta, max_r) of the call, delta = 0: the uniform grid
+
+
+@dataclass
+class KleinmanBylander:
+    """Kleinman-Bylander form of semilocal pseudopotentials (Context.kb_form / Context.kleinman_bylander; definition: dftatom_kb_form in
+    include/dftatom_b200.h).  Per channel ([n_channels]): l, row (its potential / orbital row), loc (the row of its local potential), eps
+    (reference eigenvalue), E_KB (Hartree), cos (KB cosine), eps_loc [n_channels][2] (the local Hamiltonian's eigenvalues with 0 and 1
+    nodes), r_s / i_s (outermost node where V[row] != V[loc]), ghost (GSS verdict: 1 ghost below eps, 0 none, -1 undecided), status
+    (0 ok, 1 local channel, 2 no projector, 3 the local search did not converge); beta: [n_channels][N] projectors; r: [N] the grid."""
+    l: np.ndarray
+    loc: np.ndarray
+    E_KB: np.ndarray
+    cos: np.ndarray
+    eps_loc: np.ndarray
+    r_s: np.ndarray
+    ghost: np.ndarray
+    status: np.ndarray
+    beta: np.ndarray
+    r: np.ndarray
+    row: np.ndarray
+    eps: np.ndarray
+    i_s: np.ndarray
+    grid: tuple
 
 
 def orbital_count(Z: int, method: int = 0, config=None, charge: float = 0.0) -> int:
@@ -722,7 +763,7 @@ class Context:
         rr = np.zeros(N)                                    # the engine's node radii
         _check(self._lib.dftatom_grid_nodes(self._h, int(levels), float(delta), float(max_r), _d(rr)))
         return Pseudopotential(_i32(l).copy(), _f64(eps).copy(), _f64(occ).copy(), res["r_c"].copy(), res["c"].copy(), res["q"].copy(),
-                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy())
+                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy(), (int(levels), float(delta), float(max_r)))
 
     def pseudize(self, result, r_c) -> Pseudopotential:
         """Pseudopotentials of a solved LDA atom (Result of solve_batch(..., radial=True)): for every l of result.levels[0] the level of
@@ -747,6 +788,60 @@ class Context:
         rad = result.radial
         return self.tm_pseudize(rad.V[0], rad.orbitals[0], o.MultigridLevels, 0.0 if o.method >= 2 else o.deltaGrid, o.MaxR, 0,
                                 [best[l] for l in ls], ls, [x.E for x in lev], [float(x.occ) for x in lev], rcs)
+
+    def kb_form(self, V, u, levels, delta, max_r, row, loc, l, eps) -> KleinmanBylander:
+        """Kleinman-Bylander form and GSS ghost test (dftatom_kb_form).  V: [n_rows][N] screened potentials, u: [n_rows][N] pseudo-orbitals
+        (e.g. Pseudopotential.V_scr and .u); channel c = (row[c], local row loc[c], l[c], reference eigenvalue eps[c]), broadcast against
+        each other."""
+        V = _f64(np.atleast_2d(V)); u = _f64(np.atleast_2d(u))
+        row, loc, l, eps = np.broadcast_arrays(*(np.atleast_1d(x) for x in (row, loc, l, eps)))
+        nc, N = len(row), V.shape[1]
+        ch = np.zeros(nc, dtype=np.dtype(_CKbChannel))
+        ch["row"], ch["loc"], ch["l"], ch["eps"] = row, loc, l, eps
+        res = np.zeros(nc, dtype=np.dtype(_CKbResult))
+        beta = np.zeros((nc, N))
+        _check(self._lib.dftatom_kb_form(self._h, int(levels), float(delta), float(max_r), _d(V), _d(u), V.shape[0],
+                                         ch.ctypes.data_as(C.POINTER(_CKbChannel)), nc, res.ctypes.data_as(C.POINTER(_CKbResult)), _d(beta)))
+        rr = np.zeros(N)
+        _check(self._lib.dftatom_grid_nodes(self._h, int(levels), float(delta), float(max_r), _d(rr)))
+        return KleinmanBylander(_i32(l).copy(), _i32(loc).copy(), res["E_KB"].copy(), res["cos"].copy(), res["eps_loc"].copy(), res["r_s"].copy(),
+                                res["ghost"].copy(), res["status"].copy(), beta, rr, _i32(row).copy(), _f64(eps).copy(), res["i_s"].copy(),
+                                (int(levels), float(delta), float(max_r)))
+
+    def kleinman_bylander(self, pp, l_loc) -> KleinmanBylander:
+        """The KB form of a Pseudopotential (Context.tm_pseudize / Context.pseudize): within each potential row the channel of l = l_loc
+        is the local potential of the row's other channels."""
+        if pp.grid is None:
+            raise ValueError("kleinman_bylander needs a Pseudopotential of Context.tm_pseudize")
+        loc = np.empty(len(pp.l), np.int32)
+        for c, p in enumerate(pp.pot):
+            hit = np.nonzero((pp.pot == p) & (pp.l == int(l_loc)))[0]
+            if len(hit) == 0:
+                raise ValueError(f"l_loc = {l_loc} is not a channel of potential row {p} (channels l = {sorted(pp.l[pp.pot == p].tolist())})")
+            loc[c] = hit[0]
+        return self.kb_form(pp.V_scr, pp.u, *pp.grid, np.arange(len(pp.l)), loc, pp.l, pp.eps)
+
+    def kb_log_derivatives(self, kb, V_loc, r_c, E) -> LogDerivatives:
+        """Logarithmic derivatives of the KB Hamiltonian of every channel of `kb` (dftatom_kb_log_derivatives): local potential row
+        kb.loc[c] of V_loc (the V given to kb_form), projector kb.beta[c] with E_KB[c] (none for the local channels), l[c]; r_c broadcast
+        over the channels; E shared by all channels."""
+        if np.any(kb.status == 2):
+            raise ValueError("channels " + str(np.nonzero(kb.status == 2)[0].tolist()) + " have no KB projector (status 2)")
+        V = _f64(np.atleast_2d(V_loc)); E = _f64(np.atleast_1d(E))
+        nc, ne = len(kb.l), len(E)
+        local = kb.status == 1
+        ch = np.zeros(nc, dtype=np.dtype(_CKbLdChannel))
+        ch["pot"], ch["proj"], ch["l"] = kb.loc, np.where(local, -1, np.arange(nc)), kb.l
+        ch["E_KB"], ch["r_c"] = np.where(local, 0.0, kb.E_KB), np.broadcast_to(np.atleast_1d(r_c), (nc,))
+        beta = _f64(kb.beta)
+        out = np.zeros(nc * ne, dtype=np.dtype(_CLogDeriv))
+        used = np.zeros(nc)
+        levels, delta, max_r = kb.grid
+        _check(self._lib.dftatom_kb_log_derivatives(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], _d(beta), beta.shape[0],
+                                                    ch.ctypes.data_as(C.POINTER(_CKbLdChannel)), nc, _d(E), ne,
+                                                    out.ctypes.data_as(C.POINTER(_CLogDeriv)), _d(used)))
+        out = out.reshape(nc, ne)
+        return LogDerivatives(out["D"].copy(), out["u"].copy(), out["du"].copy(), out["nodes"].copy(), used, E.copy())
 
     def integrate(self, rule, step, v):
         """Integral.h quadratures by rule: 0 Trapezoid, 1 SimpsonOneThird, 2 Simpson38, 3 Boole, 4 Romberg; one result per row of v."""

@@ -27,6 +27,10 @@
 //           With --logderiv DIR2 --rc R (R >= every pseudo radius) also DIR2/<index>_Z<Z>_pseudo_logderiv.tsv: the logarithmic
 //           derivatives of the V_scr channels at the --energies, in the columns of the all-electron table (spin 0).  LSDA atoms are an
 //           error; works with --gpus, --charge and --config and does not need --radial.
+// --pseudo-local L: with --pseudo, the Kleinman-Bylander form of every atom's channels with the channel of l = L as the local potential
+//           (dftatom_kb_form): one "# kb" line per channel (l E_KB cos eps_loc0 eps_loc1 ghost status) after the channel lines and one
+//           beta column per channel after rho_val.  With --logderiv also DIR2/<index>_Z<Z>_pseudo_kb_logderiv.tsv, the KB logarithmic
+//           derivatives (dftatom_kb_log_derivatives) in the layout of the pseudo table.  An atom without a channel of l = L is an error.
 #include <algorithm>
 #include <cmath>
 #include <cctype>
@@ -278,7 +282,7 @@ static int write_logderiv(dftatom_ctx* ctx, const std::string& dir, int index, c
 // also the logarithmic derivatives of their V_scr rows at the all-electron table's radius and energies
 static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::string& ld_dir, int index, const dftatom_options& o,
                         const dftatom_result& R, const dftatom_config* cfg, int N, const double* r, const double* v, const double* orb,
-                        const std::vector<double>& rcs, double ld_rc, const std::vector<double>& E)
+                        const std::vector<double>& rcs, double ld_rc, const std::vector<double>& E, int kb_loc)
 {
     int best[4] = { -1, -1, -1, -1 };
     for (int k = 0; k < R.n_levels[0]; ++k) {
@@ -302,6 +306,19 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
         std::fprintf(stderr, "dftatom: --pseudo Z=%d: %s\n", o.Z, dftatom_last_error());
         return 1;
     }
+    // --pseudo-local: the Kleinman-Bylander form with the channel of l = kb_loc as the local potential
+    int loc = -1;
+    for (int c = 0; c < nc; ++c) if (ch[c].l == kb_loc) loc = c;
+    if (kb_loc >= 0 && loc < 0) { std::fprintf(stderr, "dftatom: --pseudo-local %d: Z=%d has no channel with l = %d\n", kb_loc, o.Z, kb_loc); return 1; }
+    std::vector<dftatom_kb_channel> kch(loc >= 0 ? nc : 0);
+    std::vector<dftatom_kb_result> kb(kch.size());
+    std::vector<double> beta(kch.size() * (size_t)N);
+    for (size_t c = 0; c < kch.size(); ++c) { kch[c] = dftatom_kb_channel{}; kch[c].row = (int)c; kch[c].loc = loc; kch[c].l = ch[c].l; kch[c].eps = ch[c].eps; }
+    if (loc >= 0 && dftatom_kb_form(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v_scr.data(), u_ps.data(), nc, kch.data(), nc, kb.data(),
+                                    beta.data()) != DFTATOM_OK) {
+        std::fprintf(stderr, "dftatom: --pseudo-local Z=%d: %s\n", o.Z, dftatom_last_error());
+        return 1;
+    }
     const std::string stem = "/" + std::to_string(index) + "_Z" + std::to_string(o.Z) + "_pseudo";
     const std::string path = dir + stem + ".tsv";
     FILE* f = std::fopen(path.c_str(), "w");
@@ -312,15 +329,22 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
         for (int k = 0; k < 7; ++k) std::fprintf(f, "\t%.17g", out[c].c[k]);
         std::fprintf(f, "\n");
     }
+    for (size_t c = 0; c < kb.size(); ++c)
+        std::fprintf(f, "# kb\t%d\t%.17g\t%.17g\t%.17g\t%.17g\t%d\t%d\n", ch[c].l, kb[c].E_KB, kb[c].cos, kb[c].eps_loc[0], kb[c].eps_loc[1], kb[c].ghost,
+                     kb[c].status);
     std::fprintf(f, "# r");
     for (const char* q : { "V_ion", "V_scr", "u" })
         for (int c = 0; c < nc; ++c) std::fprintf(f, "\t%s %c", q, kOrb[ch[c].l]);
-    std::fprintf(f, "\trho_val\n");
+    std::fprintf(f, "\trho_val");
+    for (size_t c = 0; c < kb.size(); ++c) std::fprintf(f, "\tbeta %c", kOrb[ch[c].l]);
+    std::fprintf(f, "\n");
     for (int i = 0; i < N; ++i) {
         std::fprintf(f, "%.17g", r[i]);
         for (const std::vector<double>* q : { &v_ion, &v_scr, &u_ps })
             for (int c = 0; c < nc; ++c) std::fprintf(f, "\t%.17g", (*q)[(size_t)c * N + i]);
-        std::fprintf(f, "\t%.17g\n", rho[i]);
+        std::fprintf(f, "\t%.17g", rho[i]);
+        for (size_t c = 0; c < kb.size(); ++c) std::fprintf(f, "\t%.17g", beta[c * N + i]);
+        std::fprintf(f, "\n");
     }
     bool bad = std::ferror(f) != 0;
     if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
@@ -347,6 +371,30 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
         }
     bad = std::ferror(f) != 0;
     if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", lpath.c_str()); return 1; }
+    if (loc < 0) return 0;
+    // the KB channels at the same radius and energies: local potential V_scr of l = kb_loc, projector of every other channel
+    std::vector<dftatom_kb_ld_channel> kl(nc);
+    for (int c = 0; c < nc; ++c) {
+        kl[c] = dftatom_kb_ld_channel{};
+        kl[c].pot = loc; kl[c].proj = kb[c].status == 1 ? -1 : c; kl[c].l = ch[c].l; kl[c].E_KB = kb[c].status == 1 ? 0. : kb[c].E_KB; kl[c].r_c = ld_rc;
+    }
+    if (dftatom_kb_log_derivatives(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v_scr.data(), nc, beta.data(), nc, kl.data(), nc, E.data(), ne,
+                                   ld.data(), used.data()) != DFTATOM_OK) {
+        std::fprintf(stderr, "dftatom: --pseudo-local --logderiv Z=%d: %s\n", o.Z, dftatom_last_error());
+        return 1;
+    }
+    const std::string kpath = ld_dir + stem + "_kb_logderiv.tsv";
+    f = std::fopen(kpath.c_str(), "w");
+    if (!f) { std::perror(kpath.c_str()); return 1; }
+    std::fprintf(f, "# Z=%d method=%d r_c=%.17g KB l_loc=%d\n# spin\tl\tE\tD\tnodes\tphase\tu\tdu\n", o.Z, o.method, used[0], kb_loc);
+    for (int c = 0; c < nc; ++c)
+        for (int k = 0; k < ne; ++k) {
+            const dftatom_logderiv& q = ld[(size_t)c * ne + k];
+            const double phase = q.nodes < 0 ? NAN : M_PI * q.nodes - std::atan(used[c] * q.D);
+            std::fprintf(f, "%d\t%d\t%.17g\t%.17g\t%d\t%.17g\t%.17g\t%.17g\n", 0, l[c], E[k], q.D, q.nodes, phase, q.u, q.du);
+        }
+    bad = std::ferror(f) != 0;
+    if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", kpath.c_str()); return 1; }
     return 0;
 }
 
@@ -356,6 +404,7 @@ int main(int argc, char** argv)
     std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
     std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301", pseudo_dir, pseudo_rc;
     double charge = 0., rc = NAN;
+    int pseudo_local = -1;
     int precision = 6, device = 0, gpus = 1;
     bool json = false, quiet = false, framed = false;      // framed: child of --gpus (one frame per atom on stdout)
     std::vector<std::string> passthrough;                   // flags a --gpus parent hands to its children unchanged
@@ -373,6 +422,11 @@ int main(int argc, char** argv)
         else if (a == "--energies") energies = next();
         else if (a == "--pseudo") pseudo_dir = next();
         else if (a == "--pseudo-rc") pseudo_rc = next();
+        else if (a == "--pseudo-local") {
+            const std::string v = next();
+            if (v.size() != 1 || v[0] < '0' || v[0] > '3') { std::fprintf(stderr, "dftatom: --pseudo-local expects l = 0, 1, 2 or 3, got '%s'\n", v.c_str()); return 2; }
+            pseudo_local = v[0] - '0';
+        }
         else if (a == "--charge") charge = std::atof(next());
         else if (a == "--config") config_str = next();
         else if (a == "--levels") base.levels = std::atoi(next());
@@ -392,7 +446,7 @@ int main(int argc, char** argv)
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
                         "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR] [--charge Q] [--config \"...\"]\n"
-                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf]]\n"
+                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf] [--pseudo-local L]]\n"
                         "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n"
                         "  --charge Q    solve every atom of --Z ionised by Q electrons (the reference's configuration; fractional allowed, < 0 = anion)\n"
                         "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n"
@@ -402,7 +456,9 @@ int main(int argc, char** argv)
                         "  --energies lo:hi:n  energies of --logderiv, n points from lo to hi Hartree (default -2:1:301)\n"
                         "  --pseudo DIR  write Troullier-Martins pseudopotentials of every LDA atom (valence = largest n per l) to DIR/<index>_Z<Z>_pseudo.tsv\n"
                         "                (columns r, V_ion per l, V_scr per l, u per l, rho_val); with --logderiv also <index>_Z<Z>_pseudo_logderiv.tsv\n"
-                        "  --pseudo-rc Rs[,Rp,Rd,Rf]  radii of --pseudo in bohr by l (an l beyond the list takes the last one)\n");
+                        "  --pseudo-rc Rs[,Rp,Rd,Rf]  radii of --pseudo in bohr by l (an l beyond the list takes the last one)\n"
+                        "  --pseudo-local L  Kleinman-Bylander form of --pseudo with the channel l = L local: one \"# kb\" line per channel (l E_KB cos\n"
+                        "                eps_loc0 eps_loc1 ghost status) and beta columns; with --logderiv also <index>_Z<Z>_pseudo_kb_logderiv.tsv\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
         if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
@@ -422,6 +478,7 @@ int main(int argc, char** argv)
         if (mkdir(logderiv_dir.c_str(), 0777) != 0 && errno != EEXIST) { std::perror(logderiv_dir.c_str()); return 1; }
     }
     std::vector<double> ps_rc;
+    if (pseudo_local >= 0 && pseudo_dir.empty()) { std::fprintf(stderr, "dftatom: --pseudo-local needs --pseudo DIR\n"); return 2; }
     if (!pseudo_dir.empty()) {
         if (base.method & 1) { std::fprintf(stderr, "dftatom: --pseudo needs an LDA atom (method 0 or 2): the unscreening is spin-unpolarised\n"); return 2; }
         for (size_t p = 0; p < pseudo_rc.size();) {
@@ -501,7 +558,7 @@ int main(int argc, char** argv)
         }
     for (int a = 0; a < n && !pseudo_dir.empty(); ++a)
         if (write_pseudo(ctx, pseudo_dir, logderiv_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a], configured ? &cfgs[a] : nullptr, N,
-                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E)) {
+                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E, pseudo_local)) {
             dftatom_destroy(ctx); return 1;
         }
 

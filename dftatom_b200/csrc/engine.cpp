@@ -1368,18 +1368,20 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
     return 0;
 }
 
-// shared by level_search / numerov_orbital: one pseudo-atom with the given potential
-static int setup_single(dftatom_ctx* c, const GridDev& g, const double* V, int Z, const std::vector<OrbitalDev>& orbs,
-                        AtomDev** d_atoms, AtomState** d_astate, OrbitalDev** d_orbs, SearchState** d_ss, double** d_atab)
+// shared by level_search / numerov_orbital / kb_form: n_rows pseudo-atoms, atom k with potential row k (V[n_rows][N]) and nuclear charge
+// Z[k] (which sets its search bracket [-Z^2 - 1, 50])
+static int setup_rows(dftatom_ctx* c, const GridDev& g, const double* V, int n_rows, const int* Z, const std::vector<OrbitalDev>& orbs,
+                      AtomDev** d_atoms, AtomState** d_astate, OrbitalDev** d_orbs, SearchState** d_ss, double** d_atab)
 {
-    const int N = g.N; cudaStream_t st = c->stream;
+    const size_t nV = (size_t)n_rows * g.N; cudaStream_t st = c->stream;
     int rc;
     DevBuf& dV = c->scratch[0]; DevBuf& dA = c->scratch[1];
-    if ((rc = dV.ensure(sizeof(double) * N)) || (rc = dA.ensure(sizeof(double) * N))) return rc;
-    DFT_CHECK(cudaMemcpyAsync(dV.p, V, sizeof(double) * N, cudaMemcpyHostToDevice, st));
-    launch_build_atab(g, dV.as<double>(), dA.as<double>(), 1, st);
-    std::vector<AtomDev> atoms(1); atoms[0] = AtomDev{}; atoms[0].Z = Z; atoms[0].n_spin = 1;
-    std::vector<AtomState> as(1); as[0] = AtomState{ 0., 0, 0, 0, 0 };
+    if ((rc = dV.ensure(sizeof(double) * nV)) || (rc = dA.ensure(sizeof(double) * nV))) return rc;
+    DFT_CHECK(cudaMemcpyAsync(dV.p, V, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
+    launch_build_atab(g, dV.as<double>(), dA.as<double>(), n_rows, st);
+    std::vector<AtomDev> atoms(n_rows);
+    for (int k = 0; k < n_rows; ++k) { atoms[k] = AtomDev{}; atoms[k].Z = Z[k]; atoms[k].n_spin = 1; }
+    std::vector<AtomState> as(n_rows, AtomState{ 0., 0, 0, 0, 0 });
     if ((rc = upload(c, c->scratch[4], atoms)) || (rc = upload(c, c->scratch[5], as)) || (rc = upload(c, c->scratch[6], orbs))) return rc;
     if ((rc = c->scratch[7].ensure(sizeof(SearchState) * orbs.size()))) return rc;
     *d_atoms = c->scratch[4].as<AtomDev>(); *d_astate = c->scratch[5].as<AtomState>(); *d_orbs = c->scratch[6].as<OrbitalDev>();
@@ -1387,19 +1389,23 @@ static int setup_single(dftatom_ctx* c, const GridDev& g, const double* V, int Z
     return 0;
 }
 
-int dftatom_level_search(dftatom_ctx* c, const double* V, int levels, double delta, double max_r, int Z, int n_levels,
-                         const int* n, const int* l, double* E_out, int* converged_out)
+static int setup_single(dftatom_ctx* c, const GridDev& g, const double* V, int Z, const std::vector<OrbitalDev>& orbs,
+                        AtomDev** d_atoms, AtomState** d_astate, OrbitalDev** d_orbs, SearchState** d_ss, double** d_atab)
 {
-    if (!c || !V || n_levels <= 0) return DFTATOM_E_ARG;
-    DFT_CHECK(cudaSetDevice(c->device));
-    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
-    const GridDev g = *gp; cudaStream_t st = c->stream;
-    std::vector<OrbitalDev> orbs(n_levels);
-    for (int k = 0; k < n_levels; ++k) { orbs[k] = OrbitalDev{ 0, 0, n[k] - 1, l[k], 1, n[k] - 1 - l[k], 0 }; }
+    return setup_rows(c, g, V, 1, &Z, orbs, d_atoms, d_astate, d_orbs, d_ss, d_atab);
+}
+
+// the production energy search of every orbital (OrbitalDev.atom = .tab = its potential row) on the rows V[n_rows][N]; E_out / converged_out
+// (may be NULL) as dftatom_level_search returns them
+static int search_levels(dftatom_ctx* c, const GridDev& g, const double* V, int n_rows, const int* Z, const std::vector<OrbitalDev>& orbs,
+                         double* E_out, int* converged_out)
+{
+    const int n_levels = (int)orbs.size(); cudaStream_t st = c->stream;
     AtomDev* da; AtomState* ds; OrbitalDev* dorb; SearchState* dss; double* datab;
-    if ((rc = setup_single(c, g, V, Z, orbs, &da, &ds, &dorb, &dss, &datab))) return rc;
+    int rc;
+    if ((rc = setup_rows(c, g, V, n_rows, Z, orbs, &da, &ds, &dorb, &dss, &datab))) return rc;
     launch_search_init(g, da, ds, dorb, dss, n_levels, st);
-    const int rounds = search_rounds_needed(Z);
+    const int rounds = search_rounds_needed(*std::max_element(Z, Z + n_rows));
     if (c->k.search_mode == 0 && c->k.search_kernel == 0 && !g.uniform) launch_search_rows(g, datab, da, dorb, ds, dss, n_levels, nullptr, 0, c->k.rows_cfg, 0, 0, 1 << 30, st);
     else if (c->k.search_mode == 0 && c->segments(g.N) > 1) launch_search_seg(g, datab, da, dorb, ds, dss, n_levels, nullptr, c->segments(g.N), nullptr, 0, 0, st);
     else if (c->k.search_mode == 0) launch_search_fused(g, datab, da, dorb, ds, dss, n_levels, nullptr, nullptr, 0, 0, st);
@@ -1413,6 +1419,197 @@ int dftatom_level_search(dftatom_ctx* c, const double* V, int levels, double del
         if (E_out) E_out[k] = fin ? h[k].E : (h[k].stage == 0 ? h[k].dn_hi : h[k].bot);
         if (converged_out) converged_out[k] = fin ? h[k].converged : 0;
     }
+    return 0;
+}
+
+int dftatom_level_search(dftatom_ctx* c, const double* V, int levels, double delta, double max_r, int Z, int n_levels,
+                         const int* n, const int* l, double* E_out, int* converged_out)
+{
+    if (!c || !V || n_levels <= 0) return DFTATOM_E_ARG;
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp;
+    std::vector<OrbitalDev> orbs(n_levels);
+    for (int k = 0; k < n_levels; ++k) { orbs[k] = OrbitalDev{ 0, 0, n[k] - 1, l[k], 1, n[k] - 1 - l[k], 0 }; }
+    return search_levels(c, g, V, 1, &Z, orbs, E_out, converged_out);
+}
+
+int dftatom_kb_form(dftatom_ctx* c, int levels, double delta, double max_r, const double* V, const double* u, int n_rows,
+                    const dftatom_kb_channel* ch, int n_channels, dftatom_kb_result* out, double* beta)
+{
+    if (!c || !V || !u || !ch || !out) { set_error("dftatom_kb_form: NULL argument"); return DFTATOM_E_ARG; }
+    if (n_rows < 1 || n_channels < 1) { set_error("dftatom_kb_form: n_rows and n_channels must be >= 1"); return DFTATOM_E_ARG; }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
+    if (N < 7) { set_error("dftatom_kb_form: the grid needs at least 7 nodes"); return DFTATOM_E_ARG; }
+    if (n_channels > 65535 || (long long)std::max(n_rows, n_channels) * N >= (1LL << 31)) {
+        set_error("dftatom_kb_form: too many channels or rows for one call"); return DFTATOM_E_ARG;
+    }
+    const auto where = [](const char* what, long long k) { return std::string("dftatom_kb_form: ") + what + " " + std::to_string(k) + ": "; };
+    for (int p = 0; p < n_rows; ++p)
+        for (int i = 1; i < N; ++i) {
+            if (!std::isfinite(V[(size_t)p * N + i])) { set_error(where("row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+            if (!std::isfinite(u[(size_t)p * N + i])) { set_error(where("row", p) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+        }
+    // i_s per channel, the search bracket of every local row, and the (loc, l) searches of the non-local channels (each searched once)
+    std::vector<int> is(n_channels, 0), zb(n_rows, 0), srow_of(n_rows, -1), search_of(n_channels, -1), srows;
+    std::map<std::pair<int, int>, int> searches;
+    std::vector<OrbitalDev> orbs;
+    for (int k = 0; k < n_channels; ++k) {
+        const dftatom_kb_channel& q = ch[k];
+        const std::string at = where("channel", k);
+        if (q.row < 0 || q.row >= n_rows) { set_error(at + "row = " + std::to_string(q.row) + " outside 0.." + std::to_string(n_rows - 1)); return DFTATOM_E_ARG; }
+        if (q.loc < 0 || q.loc >= n_rows) { set_error(at + "loc = " + std::to_string(q.loc) + " outside 0.." + std::to_string(n_rows - 1)); return DFTATOM_E_ARG; }
+        if (q.l < 0 || q.l > 3) { set_error(at + "l = " + std::to_string(q.l) + " outside 0..3"); return DFTATOM_E_ARG; }
+        if (!std::isfinite(q.eps)) { set_error(at + "eps is not finite"); return DFTATOM_E_ARG; }
+        if (q.row == q.loc) continue;
+        const double* a = V + (size_t)q.row * N; const double* b = V + (size_t)q.loc * N;
+        for (int i = N - 1; i >= 1 && !is[k]; --i) if (a[i] != b[i]) is[k] = i;
+        if (is[k] > N - 3) { set_error(at + "V[row] differs from V[loc] at node " + std::to_string(is[k]) + " > N - 3"); return DFTATOM_E_ARG; }
+        if (!zb[q.loc]) {
+            double vmin = b[1];
+            for (int i = 2; i < N; ++i) vmin = std::min(vmin, b[i]);
+            int z = 1;
+            while (z <= 118 && -(double)z * z - 1. > vmin) ++z;
+            if (z > 118) { set_error(at + "local potential too deep (min V[loc] = " + std::to_string(vmin) + " below -118^2 - 1)"); return DFTATOM_E_ARG; }
+            zb[q.loc] = z;
+        }
+        if (srow_of[q.loc] < 0) { srow_of[q.loc] = (int)srows.size(); srows.push_back(q.loc); }
+        const auto key = std::make_pair(q.loc, q.l);
+        auto it = searches.find(key);
+        if (it == searches.end()) {
+            it = searches.emplace(key, (int)orbs.size() / 2).first;
+            const int sr = srow_of[q.loc];
+            for (int w = 0; w < 2; ++w) orbs.push_back(OrbitalDev{ sr, 0, q.l + w, q.l, 1, w, sr });
+        }
+        search_of[k] = it->second;
+    }
+    std::vector<double> eloc(orbs.size(), NAN);
+    std::vector<int> conv(orbs.size(), 0);
+    if (!orbs.empty()) {
+        std::vector<double> vs(srows.size() * (size_t)N);
+        std::vector<int> zs(srows.size());
+        for (size_t k = 0; k < srows.size(); ++k) { std::copy(V + (size_t)srows[k] * N, V + (size_t)(srows[k] + 1) * N, vs.begin() + k * N); zs[k] = zb[srows[k]]; }
+        if ((rc = search_levels(c, g, vs.data(), (int)srows.size(), zs.data(), orbs, eloc.data(), conv.data()))) return rc;
+    }
+    std::vector<int> h_int(3 * (size_t)n_channels);                // row | loc | is
+    for (int k = 0; k < n_channels; ++k) { h_int[k] = ch[k].row; h_int[n_channels + k] = ch[k].loc; h_int[2 * n_channels + k] = is[k]; }
+    const size_t nV = (size_t)n_rows * N, nB = (size_t)n_channels * N;
+    DevBuf& dD = c->scratch[0]; DevBuf& dI = c->scratch[1]; DevBuf& dR = c->scratch[2];
+    if ((rc = dD.ensure(sizeof(double) * (2 * nV + nB))) || (rc = dI.ensure(sizeof(int) * h_int.size())) ||
+        (rc = dR.ensure(sizeof(dftatom_kb_result) * n_channels))) return rc;
+    double* dV = dD.as<double>(); double* du = dV + nV; double* dB = du + nV;
+    DFT_CHECK(cudaMemcpyAsync(dV, V, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(du, u, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dI.p, h_int.data(), sizeof(int) * h_int.size(), cudaMemcpyHostToDevice, st));
+    const int* di = dI.as<int>();
+    KbFormArgs ka{ dV, du, di, di + n_channels, di + 2 * (size_t)n_channels, n_channels, dR.as<dftatom_kb_result>(), dB };
+    launch_kb_form(g, ka, st);
+    DFT_CHECK(cudaGetLastError());
+    std::vector<dftatom_kb_result> res(n_channels);
+    DFT_CHECK(cudaMemcpyAsync(res.data(), dR.p, sizeof(dftatom_kb_result) * n_channels, cudaMemcpyDeviceToHost, st));
+    if (beta) DFT_CHECK(cudaMemcpyAsync(beta, dB, sizeof(double) * nB, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
+    // the GSS verdict (nodeless reference state): a ghost below eps iff eps lies above the local level with 1 node (E_KB > 0) or 0 nodes (E_KB < 0)
+    for (int k = 0; k < n_channels; ++k) {
+        dftatom_kb_result& r = res[k];
+        r.pad = 0;
+        if (r.status == 1) { r.eps_loc[0] = r.eps_loc[1] = NAN; r.ghost = 0; continue; }
+        const int s = search_of[k];
+        r.eps_loc[0] = eloc[2 * s]; r.eps_loc[1] = eloc[2 * s + 1];
+        if (r.status == 0 && !(conv[2 * s] && conv[2 * s + 1])) r.status = 3;
+        if (r.status != 0) { r.ghost = -1; continue; }
+        r.ghost = r.E_KB > 0. ? (ch[k].eps > r.eps_loc[1]) : (ch[k].eps > r.eps_loc[0]);
+    }
+    std::copy(res.begin(), res.end(), out);
+    return 0;
+}
+
+int dftatom_kb_log_derivatives(dftatom_ctx* c, int levels, double delta, double max_r, const double* V_loc, int n_pot,
+                               const double* beta, int n_proj, const dftatom_kb_ld_channel* ch, int n_channels,
+                               const double* E, int n_energies, dftatom_logderiv* out, double* r_used)
+{
+    if (!c || !V_loc || !ch || !E || !out || (n_proj > 0 && !beta)) { set_error("dftatom_kb_log_derivatives: NULL argument"); return DFTATOM_E_ARG; }
+    if (n_pot < 1 || n_channels < 1 || n_energies < 1 || n_proj < 0) {
+        set_error("dftatom_kb_log_derivatives: n_pot, n_channels and n_energies must be >= 1, n_proj >= 0"); return DFTATOM_E_ARG;
+    }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
+    if (N < 5) { set_error("dftatom_kb_log_derivatives: the grid needs at least 5 nodes"); return DFTATOM_E_ARG; }
+    if (n_proj > 65535) { set_error("dftatom_kb_log_derivatives: too many projectors for one call"); return DFTATOM_E_ARG; }
+    std::vector<double> r(N);
+    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    const auto where = [](const char* what, long long k) { return std::string("dftatom_kb_log_derivatives: ") + what + " " + std::to_string(k) + ": "; };
+    std::vector<int> ic(n_channels), is(std::max(n_proj, 1), 0);
+    for (int p = 0; p < n_proj; ++p) {
+        const double* b = beta + (size_t)p * N;
+        for (int i = 0; i < N; ++i) {
+            if (!std::isfinite(b[i])) { set_error(where("projector", p) + "beta is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+            if (b[i] != 0.) is[p] = i;
+        }
+        if (is[p] > N - 3) { set_error(where("projector", p) + "beta is not 0 at node " + std::to_string(is[p]) + " > N - 3"); return DFTATOM_E_ARG; }
+    }
+    for (int k = 0; k < n_channels; ++k) {
+        const dftatom_kb_ld_channel& q = ch[k];
+        const std::string at = where("channel", k);
+        if (q.pot < 0 || q.pot >= n_pot) { set_error(at + "pot = " + std::to_string(q.pot) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
+        if (q.proj < -1 || q.proj >= n_proj) { set_error(at + "proj = " + std::to_string(q.proj) + " outside -1.." + std::to_string(n_proj - 1)); return DFTATOM_E_ARG; }
+        if (q.l < 0 || q.l > 3) { set_error(at + "l = " + std::to_string(q.l) + " outside 0..3"); return DFTATOM_E_ARG; }
+        if (!std::isfinite(q.E_KB)) { set_error(at + "E_KB is not finite"); return DFTATOM_E_ARG; }
+        if (!(q.r_c >= r[2] && q.r_c <= r[N - 2])) {
+            char b[160];
+            std::snprintf(b, sizeof b, "r_c = %.17g outside [r_2, r_(N-2)] = [%.17g, %.17g]", q.r_c, r[2], r[N - 2]);
+            set_error(at + b); return DFTATOM_E_ARG;
+        }
+        ic[k] = nearest_node(r, q.r_c);
+    }
+    for (int k = 0; k < n_energies; ++k)
+        if (!std::isfinite(E[k])) { set_error(where("energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
+    for (int p = 0; p < n_pot; ++p)
+        for (int i = 1; i < N; ++i)
+            if (!std::isfinite(V_loc[(size_t)p * N + i])) { set_error(where("potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    // warps dealt longest sweep first: a channel with a projector sweeps to max(i_c, i_s) + 1 and again to i_c
+    const int eb = (n_energies + 31) / 32;
+    const long long n_warps_ll = (long long)n_channels * eb;
+    if (n_warps_ll > (1LL << 30)) { set_error("dftatom_kb_log_derivatives: too many (channel, energy) lanes"); return DFTATOM_E_ARG; }
+    const int n_warps = (int)n_warps_ll;
+    std::vector<long long> cost(n_channels);
+    for (int k = 0; k < n_channels; ++k) cost[k] = ch[k].proj < 0 ? ic[k] : (long long)std::max(ic[k], is[ch[k].proj]) + ic[k];
+    std::vector<int> chan_order(n_channels);
+    std::iota(chan_order.begin(), chan_order.end(), 0);
+    std::stable_sort(chan_order.begin(), chan_order.end(), [&](int a, int b) { return cost[a] > cost[b]; });
+    const size_t nc = (size_t)n_channels, np = (size_t)std::max(n_proj, 1);
+    std::vector<int> h_int(4 * nc + np + n_warps);             // pot | l | ic | proj | is | warp_item
+    for (size_t k = 0; k < nc; ++k) { h_int[k] = ch[k].pot; h_int[nc + k] = ch[k].l; h_int[2 * nc + k] = ic[k]; h_int[3 * nc + k] = ch[k].proj; }
+    std::copy(is.begin(), is.end(), h_int.begin() + 4 * nc);
+    int* wi = h_int.data() + 4 * nc + np;
+    for (int q = 0, w = 0; q < n_channels; ++q)
+        for (int b = 0; b < eb; ++b) wi[w++] = chan_order[q] * eb + b;
+    std::vector<double> h_dbl(E, E + n_energies);                // E | E_KB
+    for (int k = 0; k < n_channels; ++k) h_dbl.push_back(ch[k].E_KB);
+    const size_t nV = (size_t)n_pot * N, nP = (size_t)n_proj * N, n_out = nc * n_energies;
+    DevBuf& dD = c->scratch[0]; DevBuf& dI = c->scratch[1]; DevBuf& dO = c->scratch[2];
+    if ((rc = dD.ensure(sizeof(double) * (2 * nV + 3 * nP + h_dbl.size()))) || (rc = dI.ensure(sizeof(int) * h_int.size())) ||
+        (rc = dO.ensure(sizeof(dftatom_logderiv) * n_out))) return rc;
+    double* dV = dD.as<double>(); double* dA = dV + nV; double* dB = dA + nV; double* dS = dB + nP; double* dH = dS + nP; double* dE = dH + nP;
+    DFT_CHECK(cudaMemcpyAsync(dV, V_loc, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
+    if (n_proj > 0) DFT_CHECK(cudaMemcpyAsync(dB, beta, sizeof(double) * nP, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dE, h_dbl.data(), sizeof(double) * h_dbl.size(), cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dI.p, h_int.data(), sizeof(int) * h_int.size(), cudaMemcpyHostToDevice, st));
+    launch_build_atab(g, dV, dA, n_pot, st);
+    const int* d_i = dI.as<int>();
+    if (n_proj > 0) launch_kb_proj(g, KbProjArgs{ dB, d_i + 4 * nc, n_proj, dS, dH }, st);
+    KbLogDerivArgs a{ dA, d_i, d_i + nc, d_i + 2 * nc, d_i + 3 * nc, dE + n_energies, dS, dH, d_i + 4 * nc, dE, n_energies,
+                      d_i + 4 * nc + np, n_warps, eb, dO.as<dftatom_logderiv>() };
+    launch_kb_logderiv(g, a, st);
+    DFT_CHECK(cudaGetLastError());
+    DFT_CHECK(cudaMemcpyAsync(out, dO.p, sizeof(dftatom_logderiv) * n_out, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    if (r_used) for (int k = 0; k < n_channels; ++k) r_used[k] = r[ic[k]];
     return 0;
 }
 

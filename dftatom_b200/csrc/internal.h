@@ -371,6 +371,31 @@ struct TmRowArgs {
 void launch_tm_density(const GridDev& g, const TmRowArgs& a, cudaStream_t st);
 void launch_tm_unscreen(const GridDev& g, const TmRowArgs& a, cudaStream_t st);
 
+// Kleinman-Bylander form (kb.cu): one CTA per channel; is[c] = i_s of the channel (host: the largest node with V[row] != V[loc])
+struct KbFormArgs {
+    const double* V; const double* u;             // [n_rows][N] screened potentials, pseudo-orbitals
+    const int* row; const int* loc; const int* is; int n_channels;
+    dftatom_kb_result* res;                       // [n_channels]: E_KB, cos, r_s, i_s, status (eps_loc and ghost are the host's)
+    double* beta;                                 // [n_channels][N]
+};
+void launch_kb_form(const GridDev& g, const KbFormArgs& a, cudaStream_t st);
+// source and projection rows of every projector of dftatom_kb_log_derivatives
+struct KbProjArgs {
+    const double* beta; const int* is; int n_proj;    // [n_proj][N], [n_proj]
+    double* src; double* hw;                          // [n_proj][N]
+};
+void launch_kb_proj(const GridDev& g, const KbProjArgs& a, cudaStream_t st);
+// KB logarithmic derivatives: LogDerivArgs plus per channel the projector (-1: none, the plain sweep) and E_KB
+struct KbLogDerivArgs {
+    const double* atab;                           // [n_pot][N]
+    const int* pot; const int* l; const int* ic; const int* proj; const double* ekb;     // [n_channels]
+    const double* src; const double* hw; const int* is;                                // rows and i_s of the projectors
+    const double* E; int n_energies;
+    const int* warp_item; int n_warps, energy_blocks;
+    dftatom_logderiv* out;                        // [n_channels][n_energies]
+};
+void launch_kb_logderiv(const GridDev& g, const KbLogDerivArgs& a, cudaStream_t st);
+
 // host rules (aufbau.cpp)
 int aufbau(int Z, dftatom_level* out, int max_out);
 int split_spin(int Z, dftatom_level* a, int* na, dftatom_level* b, int* nb, int* ea, int* eb);

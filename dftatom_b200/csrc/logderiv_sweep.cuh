@@ -17,6 +17,16 @@ constexpr double kBig = 0x1p128;       // rescale threshold of |y|, checked ever
 constexpr double kDown = 0x1p-256;     // scale of y and w at a rescale (the norm sum takes its square)
 }
 
+// Simpson weight of node i of 0..n (1/3 rule on 0..m, the 3/8 rule on m..n when n is odd), the rule of the sweep's norm
+__device__ __forceinline__ double simpson_weight(int i, int n)
+{
+    const int m = (n & 1) ? n - 3 : n;
+    double w = 0.;
+    if (m > 0 && i <= m) w = (i == 0 || i == m) ? 1. / 3. : ((i & 1) ? 4. / 3. : 2. / 3.);
+    if ((n & 1) && i >= m) w += (i == m || i == n) ? 0.375 : 1.125;
+    return w;
+}
+
 // D, u, du and the node count at node n = i_c of the outward solution at energy E on the a-table row `atab`; nodes = -1 and NaN in
 // D, u, du when 1 - g <= 0 at some node 2..n+1
 __device__ __forceinline__ dftatom_logderiv logderiv_sweep(const GridDev& g, const double* __restrict__ atab, int l, int n, double E)

@@ -53,16 +53,6 @@ __device__ __forceinline__ double tm_p(const double d[7], double t2)
 
 __device__ __forceinline__ double pow_l1(double r, int l) { double v = r; for (int k = 0; k < l; ++k) v *= r; return v; }
 
-// Simpson weight of node i of 0..n (1/3 rule on 0..m, the 3/8 rule on m..n when n is odd), as logderiv_sweep
-__device__ __forceinline__ double simpson_weight(int i, int n)
-{
-    const int m = (n & 1) ? n - 3 : n;
-    double w = 0.;
-    if (m > 0 && i <= m) w = (i == 0 || i == m) ? 1. / 3. : ((i & 1) ? 4. / 3. : 2. / 3.);
-    if ((n & 1) && i >= m) w += (i == m || i == n) ? 0.375 : 1.125;
-    return w;
-}
-
 // ln S(x) - ln q, S = sum_i w_i r_i^(2l+2) e^(2 p(r_i)) (dr/di)_i over nodes 0..n, reduced over the warp
 __device__ double tm_norm_F(const GridDev& g, const TmShared& s, double x, int l, int n, double inv_rc)
 {

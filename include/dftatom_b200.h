@@ -368,6 +368,48 @@ typedef struct { double c[7], r_c, q; int status, pad; } dftatom_tm_result;     
 int dftatom_tm_pseudize(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, int n_pot, const double* u, int n_orb,
                         const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
                         double* v_ion, double* rho_val);
+/* Kleinman-Bylander (KB) form of semilocal pseudopotentials: one local potential plus one separable projector per other channel,
+ * V_NL = |beta> E_KB <beta|, with the Gonze-Stumpf-Scheffler (GSS) ghost-state test.  Grid (levels, delta, max_r) and the "sweep rule on
+ * 0..n" (Simpson 1/3 on nodes 0..m, the 3/8 rule on the last three intervals when n is odd, times dr/di) are those of
+ * dftatom_log_derivatives / dftatom_tm_pseudize.
+ * V[n_rows][N] HOST screened potentials (node 0 ignored), u[n_rows][N] HOST pseudo-orbitals, e.g. v_scr and u_ps of dftatom_tm_pseudize.
+ * Channel c = ch[c]: projects V[row] against the local potential V[loc] at angular momentum l, reference eigenvalue eps.
+ *   dV_i = V[row]_i - V[loc]_i (nodes >= 1); i_s = the largest node with dV_i != 0 (0 if none), r_s = r_(i_s)
+ *   a = sum w_i u_i^2 dV_i, b = sum w_i u_i^2 dV_i^2 (sweep rule on 0..i_s); E_KB = b / a; cos = a / sqrt(<u|u> b), <u|u> = sum over all
+ *   nodes of the wjac weights of the radial export times u^2; beta_i = dV_i u_i / sqrt(b) (sum w beta^2 = 1 with the same rule)
+ *   eps_loc[0], eps_loc[1]: the eigenvalues with 0 and 1 nodes of -1/2 u'' + [V[loc] + l(l+1)/2r^2] u in the box u(max_r) = 0, found by
+ *   the energy search of the SCF (dftatom_level_search) with the bracket bottom -Z_b^2 - 1, Z_b the smallest integer >= 1 with
+ *   -Z_b^2 - 1 <= min over nodes 1..N-1 of V[loc] (Z_b > 118: DFTATOM_E_ARG, "local potential too deep")
+ *   ghost (GSS, nodeless reference state): E_KB > 0: 1 iff eps > eps_loc[1]; E_KB < 0: 1 iff eps > eps_loc[0]; else 0
+ *   status: 0 ok; 1 local channel (row == loc): beta = 0, E_KB = 0, cos = 1, ghost = 0, eps_loc NaN; 2 a = 0 or i_s < 3: E_KB and cos
+ *   NaN, beta = 0, ghost = -1; 3 the search did not converge for eps_loc[0] or [1]: eps_loc holds what it found, ghost = -1
+ * beta[n_channels][N] (may be NULL): the projectors, 0 outside nodes 1..i_s.
+ * Validation before anything runs on the device (outputs untouched): a bad grid returns DFTATOM_E_BAD_OPTION; DFTATOM_E_ARG, naming the
+ * channel or row, for NULL V, u, ch or out, n_rows or n_channels < 1, row or loc out of range, l outside 0..3, eps not finite, V or u
+ * not finite at nodes 1..N-1, i_s > N - 3, or a local potential too deep. */
+typedef struct { int row, loc, l, pad; double eps; } dftatom_kb_channel;                                   /* 24 bytes */
+typedef struct { double E_KB, cos, eps_loc[2], r_s; int i_s, ghost, status, pad; } dftatom_kb_result;     /* 56 bytes */
+int dftatom_kb_form(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, const double* u, int n_rows,
+                    const dftatom_kb_channel* ch, int n_channels, dftatom_kb_result* out, double* beta);
+/* Logarithmic derivatives of the KB Hamiltonian: the solution regular at the nucleus of
+ *   -1/2 u'' + [V_loc + l(l+1)/2r^2 - E] u + E_KB beta <beta|u> = 0
+ * for every (channel, energy).  V_loc[n_pot][N] HOST local potentials, beta[n_proj][N] HOST projectors (e.g. of dftatom_kb_form),
+ * channel c = ch[c]: potential row pot, projector proj (-1: none), l, E_KB, radius r_c.  E, out, r_used, the rounding of r_c and the
+ * meaning of D, u, du and nodes are those of dftatom_log_derivatives; a channel with proj = -1 is computed by its sweep (bit for bit).
+ * With a projector: u_h = the outward homogeneous solution of dftatom_log_derivatives; u_p = the outward solution driven by -beta, from
+ * y_0 = y_1 = 0, with the Numerov source (s_(i-1) + 10 s_i + s_(i+1)) / 12, s_i = 2 K_i beta_i e^(-delta i / 2) (uniform grid: 2 h^2 beta_i),
+ * in the index variable of the sweep; h_x = <beta|u_x> by the sweep rule on 0..i_s (i_s = the largest node with beta != 0);
+ * u = (1 - E_KB h_p) u_h + E_KB h_h u_p.  Both solutions run to max(i_c, i_s) + 1, each rescaled by exact powers of two (u_p with its
+ * source), and are combined in one common scale.  u'(r_c) is the fourth-order index derivative of dftatom_log_derivatives less the
+ * source term E_KB h_h (s_(i_c+1) - s_(i_c-1)) / 12; int_0^rc u^2 dr is assembled from the running sums of u_h^2, u_h u_p and u_p^2;
+ * nodes = sign changes among the non-zero values of u at nodes 1..i_c, and u > 0 at the first of them.  1 - g_i <= 0 at some node
+ * 2..max(i_c, i_s) + 1: nodes = -1, NaN.
+ * Validation: that of dftatom_log_derivatives (pot, l, r_c, E, V_loc) plus NULL beta with a projector, n_proj < 0, proj outside
+ * -1..n_proj-1, E_KB not finite, beta not finite, or i_s > N - 3. */
+typedef struct { int pot, proj, l, pad; double E_KB, r_c; } dftatom_kb_ld_channel;                         /* 32 bytes */
+int dftatom_kb_log_derivatives(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V_loc, int n_pot,
+                               const double* beta, int n_proj, const dftatom_kb_ld_channel* ch, int n_channels,
+                               const double* E, int n_energies, dftatom_logderiv* out, double* r_used);
 /* The node radii r[N] (HOST) of the grid (levels, delta, max_r; delta = 0: uniform) as the engine builds and uses them. */
 int dftatom_grid_nodes(dftatom_ctx* ctx, int levels, double delta, double max_r, double* r);
 /* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) (the SCF passes the
