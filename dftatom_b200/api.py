@@ -87,6 +87,11 @@ class _CConfig(C.Structure):
     _fields_ = [("n_orbitals", C.c_int), ("orb", _COccupation * (2 * MAX_LEVELS))]
 
 
+class _CPseudoAtom(C.Structure):
+    _fields_ = [("row", C.c_int * 4), ("n_ref", C.c_int * 4), ("z_val", C.c_double), ("mixing", C.c_double), ("method", C.c_int),
+                ("pad", C.c_int)]
+
+
 _RESULT_DTYPE = np.dtype(_CResult)      # numpy views of the C structs (same layout: built from the ctypes definitions)
 _STEP_DTYPE = np.dtype(_CStep)
 _LEVEL_IDX = np.arange(MAX_LEVELS)[None, None, :]
@@ -133,6 +138,8 @@ def load_library():
     lib.dftatom_config_aufbau.argtypes = [C.c_int, C.c_int, C.c_double, C.POINTER(_CConfig)]
     lib.dftatom_solve_batch_config.argtypes = [C.c_void_p, C.POINTER(_COptions), C.POINTER(_CConfig), C.c_int, C.POINTER(_CResult),
                                                C.POINTER(_CStep), C.c_int, C.POINTER(_CRadial)]
+    lib.dftatom_solve_pseudo_batch.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, C.POINTER(_CPseudoAtom),
+                                               C.POINTER(_CConfig), C.c_int, C.POINTER(_CResult), C.POINTER(_CStep), C.c_int, C.POINTER(_CRadial)]
     lib.dftatom_radial_moments.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp]
     lib.dftatom_log_derivatives.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _ip, _ip, _dp, C.c_int, _dp, C.c_int,
                                             C.POINTER(_CLogDeriv), _dp]
@@ -341,7 +348,8 @@ class Pseudopotential:
     p(r), bohr^-2k), q (all-electron norm inside r_c), status (0 ok, 1 no root on the ladder, 2 the sweep at eps failed, 3 the root
     not refined to 1e-13), u (pseudo-orbital),
     V_scr (screened potential) and V_ion (ionic potential), each [n_channels][N].  pot: the potential row of every channel; rho_val:
-    [n_pot][N] the valence density of each row.  r: [N] the grid."""
+    [n_pot][N] the valence density of each row.  r: [N] the grid.  n: [n_channels] the all-electron principal number of every channel's
+    reference state (None when not given), which Context.solve_pseudo_batch needs."""
     l: np.ndarray
     eps: np.ndarray
     occ: np.ndarray
@@ -356,6 +364,7 @@ class Pseudopotential:
     rho_val: np.ndarray
     pot: np.ndarray
     grid: Optional[tuple] = None        # (levels, delta, max_r) of the call, delta = 0: the uniform grid
+    n: Optional[np.ndarray] = None
 
 
 @dataclass
@@ -508,6 +517,71 @@ def n_nodes(levels: int) -> int:
     return load_library().dftatom_n_nodes(int(levels))
 
 
+def _radial_buffers(n, N, rows):
+    """One allocation for the radial export of n atoms with `rows` orbital rows: (the views of _decode, the _CRadial over them)."""
+    buf = np.zeros(N + n * 5 * N + n * 2 + rows * (N + N_MOMENTS))      # r | rho | V | V_H | atom moments | orbitals | moments
+    r = buf[:N]
+    rho = buf[N:N + 2 * n * N].reshape(n, 2, N)
+    V = buf[N + 2 * n * N:N + 4 * n * N].reshape(n, 2, N)
+    VH = buf[N + 4 * n * N:N + 5 * n * N].reshape(n, N)
+    am = buf[N + 5 * n * N:N + 5 * n * N + 2 * n].reshape(n, 2)
+    q = N + 5 * n * N + 2 * n
+    orb = buf[q:q + rows * N].reshape(rows, N)
+    mom = buf[q + rows * N:].reshape(rows, N_MOMENTS)
+    return (r, rho, V, VH, am, orb, mom), _CRadial(_d(r), _d(rho), _d(V), _d(VH), _d(orb), rows, _d(mom), _d(am))
+
+
+def _decode(options, entries, cres, csteps, stride, radial):
+    """Result objects of n = len(options) C records (csteps: None or [n][stride] step records; radial: None or the arrays of the
+    export (r, rho, V, V_H, atom moments, orbitals, moments)); entries[a]: the (n, l, spin, occ) configuration of atom a or None."""
+    n = len(options)
+    keep_steps = csteps is not None
+    # host structs -> Python objects in bulk (numpy structured views of the ctypes arrays: one pass in C instead of a ctypes
+    # attribute access per field)
+    ra = np.frombuffer(cres, dtype=_RESULT_DTYPE, count=n)
+    head = ra[["status", "n_steps", "n_spin", "Etotal", "Ekin", "Ecoul", "Eenuc", "Exc"]].tolist()
+    nlv = ra["n_levels"]
+    used = (_LEVEL_IDX < nlv[:, :, None]) & (_SPIN_IDX < ra["n_spin"][:, None, None])        # [atom][spin][k]
+    lev, sor = ra["levels"][used].tolist(), ra["sorted"][used].tolist()                        # flat, (n, l, occ, nodes, E) each
+    n_levels = nlv.tolist()
+    sa = np.frombuffer(csteps, dtype=_STEP_DTYPE, count=n * stride) if keep_steps else None
+    out = []
+    p = 0
+    for a in range(n):
+        status, n_steps, n_spin, etot, ekin, ecoul, eenuc, exc = head[a]
+        nl = n_levels[a]
+        lv, sl = [], []
+        for s in range(n_spin):
+            q = p + nl[s]
+            lv.append(lev[p:q]); sl.append(sor[p:q])
+            p = q
+        if entries[a] is not None:         # the exact occupations (the C records hold them rounded)
+            occ = {(x[0], x[1], x[2]): x[3] for x in entries[a]}
+            lv = [[(t[0], t[1], occ[(t[0], t[1], s)]) + tuple(t[3:]) for t in ch] for s, ch in enumerate(lv)]
+            sl = [[(t[0], t[1], occ[(t[0], t[1], s)]) + tuple(t[3:]) for t in ch] for s, ch in enumerate(sl)]
+        steps = []
+        if keep_steps and n_steps:
+            blk = sa[a * stride:a * stride + n_steps]
+            E = blk["E"].tolist()
+            rest = blk[["Etotal", "Ekin", "Ecoul", "Eenuc", "Exc", "levels_converged", "stop_criterion_met"]].tolist()
+            for k in range(n_steps):
+                r_ = rest[k]
+                steps.append(Step([E[k][s][:nl[s]] for s in range(n_spin)], r_[0], r_[1], r_[2], r_[3], r_[4], bool(r_[5]), bool(r_[6])))
+        out.append(Result(options[a], status, n_steps, lv, sl, etot, ekin, ecoul, eenuc, exc, steps))
+    if radial is not None:
+        r, rho, V, VH, am, orb, mom = radial
+        row = 0
+        for a, res in enumerate(out):
+            ns = 2 if options[a].method & 1 else 1
+            orbs, moms = [], []
+            for s in range(ns):
+                k = n_levels[a][s]
+                orbs.append(orb[row:row + k]); moms.append(mom[row:row + k])
+                row += k
+            res.radial = Radial(r, rho[a, :ns], V[a, :ns], VH[a], orbs, moms, float(am[a, 0]), float(am[a, 1]))
+    return out
+
+
 class Context:
     """Owns the CUDA device state behind an opaque dftatom_ctx* (one per GPU / host thread)."""
 
@@ -558,67 +632,77 @@ class Context:
         cres = (_CResult * n)()
         stride = MAX_STEPS_LSDA if any(o.method for o in options) else MAX_STEPS_LDA
         csteps = (_CStep * (n * stride))() if keep_steps else None
+        views = None
         if radial and n:
             N = n_nodes(options[0].MultigridLevels)
             rows = sum(len(e) if e is not None else orbital_count(o.Z, o.method) for o, e in zip(options, entries))
-            buf = np.zeros(N + n * 5 * N + n * 2 + rows * (N + N_MOMENTS))      # r | rho | V | V_H | atom moments | orbitals | moments
-            r = buf[:N]
-            rho = buf[N:N + 2 * n * N].reshape(n, 2, N)
-            V = buf[N + 2 * n * N:N + 4 * n * N].reshape(n, 2, N)
-            VH = buf[N + 4 * n * N:N + 5 * n * N].reshape(n, N)
-            am = buf[N + 5 * n * N:N + 5 * n * N + 2 * n].reshape(n, 2)
-            q = N + 5 * n * N + 2 * n
-            orb = buf[q:q + rows * N].reshape(rows, N)
-            mom = buf[q + rows * N:].reshape(rows, N_MOMENTS)
-            crad = _CRadial(_d(r), _d(rho), _d(V), _d(VH), _d(orb), rows, _d(mom), _d(am))
+            views, crad = _radial_buffers(n, N, rows)
             _check(self._lib.dftatom_solve_batch_config(self._h, copts, ccfg, n, cres, csteps, stride if keep_steps else 0, C.byref(crad)))
         elif ccfg is not None:
             _check(self._lib.dftatom_solve_batch_config(self._h, copts, ccfg, n, cres, csteps, stride if keep_steps else 0, None))
         else:
             _check(self._lib.dftatom_solve_batch(self._h, copts, n, cres, csteps, stride if keep_steps else 0))
-        # host structs -> Python objects in bulk (numpy structured views of the ctypes arrays: one pass in C instead of a ctypes
-        # attribute access per field)
-        ra = np.frombuffer(cres, dtype=_RESULT_DTYPE, count=n)
-        head = ra[["status", "n_steps", "n_spin", "Etotal", "Ekin", "Ecoul", "Eenuc", "Exc"]].tolist()
-        nlv = ra["n_levels"]
-        used = (_LEVEL_IDX < nlv[:, :, None]) & (_SPIN_IDX < ra["n_spin"][:, None, None])        # [atom][spin][k]
-        lev, sor = ra["levels"][used].tolist(), ra["sorted"][used].tolist()                        # flat, (n, l, occ, nodes, E) each
-        n_levels = nlv.tolist()
-        sa = np.frombuffer(csteps, dtype=_STEP_DTYPE, count=n * stride) if keep_steps else None
-        out = []
-        p = 0
-        for a in range(n):
-            status, n_steps, n_spin, etot, ekin, ecoul, eenuc, exc = head[a]
-            nl = n_levels[a]
-            lv, sl = [], []
-            for s in range(n_spin):
-                q = p + nl[s]
-                lv.append(lev[p:q]); sl.append(sor[p:q])
-                p = q
-            if entries[a] is not None:         # the exact occupations (the C records hold them rounded)
-                occ = {(x[0], x[1], x[2]): x[3] for x in entries[a]}
-                lv = [[(t[0], t[1], occ[(t[0], t[1], s)]) + tuple(t[3:]) for t in ch] for s, ch in enumerate(lv)]
-                sl = [[(t[0], t[1], occ[(t[0], t[1], s)]) + tuple(t[3:]) for t in ch] for s, ch in enumerate(sl)]
-            steps = []
-            if keep_steps and n_steps:
-                blk = sa[a * stride:a * stride + n_steps]
-                E = blk["E"].tolist()
-                rest = blk[["Etotal", "Ekin", "Ecoul", "Eenuc", "Exc", "levels_converged", "stop_criterion_met"]].tolist()
-                for k in range(n_steps):
-                    r_ = rest[k]
-                    steps.append(Step([E[k][s][:nl[s]] for s in range(n_spin)], r_[0], r_[1], r_[2], r_[3], r_[4], bool(r_[5]), bool(r_[6])))
-            out.append(Result(options[a], status, n_steps, lv, sl, etot, ekin, ecoul, eenuc, exc, steps))
-        if radial and n:
-            row = 0
-            for a, res in enumerate(out):
-                ns = 2 if options[a].method & 1 else 1
-                orbs, moms = [], []
-                for s in range(ns):
-                    k = n_levels[a][s]
-                    orbs.append(orb[row:row + k]); moms.append(mom[row:row + k])
-                    row += k
-                res.radial = Radial(r, rho[a, :ns], V[a, :ns], VH[a], orbs, moms, float(am[a, 0]), float(am[a, 1]))
-        return out
+        return _decode(options, entries, cres, csteps if keep_steps else None, stride, views)
+
+    def solve_pseudo_batch(self, pseudos, configs, mixing: float = 0.5, method: int = 0, keep_steps: bool = True,
+                           radial: bool = False) -> List[Result]:
+        """Self-consistent pseudo-atoms (dftatom_solve_pseudo_batch).  pseudos: Pseudopotential objects (Context.tm_pseudize /
+        Context.pseudize, with `n` set), one pseudo-atom each: its channels (one per l) with ionic potentials V_ion, reference principal
+        numbers n and ionic charge z_val = sum of the channels' occupations.  configs: valence configurations with all-electron labels,
+        parse_config strings or entry lists ((n, l, occ) for LDA, (n, l, spin, occ) for LSDA), broadcast against pseudos.  All pseudos
+        share one grid (the logarithmic grid).  Returns one Result per pseudo-atom: levels with the all-electron n and nodes = n - n_ref,
+        Eenuc = E_ion, Ecoul = E_H, Exc, Ekin and Etotal as documented there; options = Options(Z = round(z_val), the grid, mixing,
+        method, config = the entries).  radial=True: Result.radial with V = the screening V_H + V_xc per spin."""
+        pseudos = list(pseudos) if isinstance(pseudos, (list, tuple)) else [pseudos]
+        one = isinstance(configs, str) or (len(configs) > 0 and all(isinstance(e, (list, tuple)) and len(e) in (3, 4)
+                                                                     and not isinstance(e[0], (list, tuple, str)) for e in configs))
+        configs = [configs] if one else list(configs)
+        n = max(len(pseudos), len(configs))
+        if len(pseudos) not in (1, n) or len(configs) not in (1, n):
+            raise DFTAtomError(f"solve_pseudo_batch: {len(pseudos)} pseudopotentials and {len(configs)} configurations do not broadcast")
+        pseudos = pseudos * (n // len(pseudos)); configs = configs * (n // len(configs))
+        grid = pseudos[0].grid
+        if grid is None or any(pp.grid != grid for pp in pseudos):
+            raise DFTAtomError("solve_pseudo_batch: every Pseudopotential must come from Context.tm_pseudize on one grid")
+        levels, delta, max_r = grid
+        rows, row_of, catoms = [], {}, (_CPseudoAtom * n)()
+        for a, pp in enumerate(pseudos):
+            if pp.n is None:
+                raise DFTAtomError(f"solve_pseudo_batch: pseudopotential {a} has no reference principal numbers (Pseudopotential.n)")
+            if len(set(pp.l.tolist())) != len(pp.l):
+                raise DFTAtomError(f"solve_pseudo_batch: pseudopotential {a} has two channels of one l")
+            key = id(pp)
+            if key not in row_of:
+                row_of[key] = len(rows)
+                rows += [pp.V_ion[c] for c in range(len(pp.l))]
+            base = row_of[key]
+            catoms[a].row[:] = [-1] * 4
+            catoms[a].n_ref[:] = [0] * 4
+            for c, l in enumerate(pp.l.tolist()):
+                catoms[a].row[l] = base + c
+                catoms[a].n_ref[l] = int(pp.n[c])
+            catoms[a].z_val = float(np.sum(pp.occ))
+            catoms[a].mixing = float(mixing)
+            catoms[a].method = int(method)
+        entries = [[_entry4(e, method) for e in (parse_config(c, method) if isinstance(c, str) else c)] for c in configs]
+        ccfg = (_CConfig * n)()
+        for a, e in enumerate(entries):
+            if len(e) > 2 * MAX_LEVELS:
+                raise DFTAtomError(f"atom {a}: {len(e)} configuration entries, at most {2 * MAX_LEVELS}")
+            ccfg[a].n_orbitals = len(e)
+            for k, x in enumerate(e):
+                ccfg[a].orb[k] = _COccupation(*x)
+        V = _f64(np.array(rows))
+        cres = (_CResult * n)()
+        stride = MAX_STEPS_LSDA if method & 1 else MAX_STEPS_LDA
+        csteps = (_CStep * (n * stride))() if keep_steps else None
+        views, crad = _radial_buffers(n, V.shape[1], sum(len(e) for e in entries)) if radial else (None, None)
+        _check(self._lib.dftatom_solve_pseudo_batch(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], catoms, ccfg, n, cres,
+                                                    csteps, stride if keep_steps else 0, C.byref(crad) if radial else None))
+        options = [Options(int(round(catoms[a].z_val)), int(levels), float(max_r), float(delta), float(mixing), int(method),
+                           config=_as_method_form(entries[a], method)) for a in range(n)]
+        return _decode(options, entries, cres, csteps, stride, views)
+
 
     def last_timing(self):
         ms, n = C.c_double(), C.c_longlong()
@@ -744,11 +828,12 @@ class Context:
         out = out.reshape(nc, ne)
         return LogDerivatives(out["D"].copy(), out["u"].copy(), out["du"].copy(), out["nodes"].copy(), used, E.copy())
 
-    def tm_pseudize(self, V, u, levels, delta, max_r, pot, orbital, l, eps, occ, r_c) -> Pseudopotential:
+    def tm_pseudize(self, V, u, levels, delta, max_r, pot, orbital, l, eps, occ, r_c, n=None) -> Pseudopotential:
         """Troullier-Martins pseudization and unscreening (dftatom_tm_pseudize).  V: [n_pot][N] potentials, u: [n_orb][N] all-electron
         orbitals (one row of either may be given as [N]), e.g. rows of Result.radial.V and Result.radial.orbitals; channel c = (V row pot[c],
         u row orbital[c], l[c], eigenvalue eps[c], occupation occ[c], radius r_c[c] in bohr), broadcast against each other.  The channels
-        sharing a potential row are one pseudo-atom for the unscreening."""
+        sharing a potential row are one pseudo-atom for the unscreening.  n (optional, broadcast likewise): the all-electron principal
+        number of every channel's reference state, kept as Pseudopotential.n."""
         V = _f64(np.atleast_2d(V)); u = _f64(np.atleast_2d(u))
         pot, orbital, l, eps, occ, r_c = np.broadcast_arrays(*(np.atleast_1d(x) for x in (pot, orbital, l, eps, occ, r_c)))
         nc, N = len(pot), V.shape[1]
@@ -762,8 +847,9 @@ class Context:
                                              _d(u_ps), _d(v_scr), _d(v_ion), _d(rho)))
         rr = np.zeros(N)                                    # the engine's node radii
         _check(self._lib.dftatom_grid_nodes(self._h, int(levels), float(delta), float(max_r), _d(rr)))
+        nn = None if n is None else _i32(np.broadcast_to(np.atleast_1d(n), (nc,))).copy()
         return Pseudopotential(_i32(l).copy(), _f64(eps).copy(), _f64(occ).copy(), res["r_c"].copy(), res["c"].copy(), res["q"].copy(),
-                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy(), (int(levels), float(delta), float(max_r)))
+                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy(), (int(levels), float(delta), float(max_r)), nn)
 
     def pseudize(self, result, r_c) -> Pseudopotential:
         """Pseudopotentials of a solved LDA atom (Result of solve_batch(..., radial=True)): for every l of result.levels[0] the level of
@@ -787,7 +873,7 @@ class Context:
         lev = [result.levels[0][best[l]] for l in ls]
         rad = result.radial
         return self.tm_pseudize(rad.V[0], rad.orbitals[0], o.MultigridLevels, 0.0 if o.method >= 2 else o.deltaGrid, o.MaxR, 0,
-                                [best[l] for l in ls], ls, [x.E for x in lev], [float(x.occ) for x in lev], rcs)
+                                [best[l] for l in ls], ls, [x.E for x in lev], [float(x.occ) for x in lev], rcs, [x.n for x in lev])
 
     def kb_form(self, V, u, levels, delta, max_r, row, loc, l, eps) -> KleinmanBylander:
         """Kleinman-Bylander form and GSS ghost test (dftatom_kb_form).  V: [n_rows][N] screened potentials, u: [n_rows][N] pseudo-orbitals

@@ -140,7 +140,7 @@ int config_aufbau(int Z, int method, double charge, dftatom_config* out)
     return 0;
 }
 
-int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, AtomLevels* out)
+int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, AtomLevels* out, double z_val)
 {
     const bool lsda = o.method & 1;
     for (int s = 0; s < 2; ++s) { out->lev[s].clear(); out->occ[s].clear(); }
@@ -155,7 +155,7 @@ int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, A
         return 0;
     }
     auto bad = [&](int k, const std::string& why) {
-        std::string e = "atom " + std::to_string(atom) + " (Z = " + std::to_string(o.Z) + "): configuration";
+        std::string e = "atom " + std::to_string(atom) + (z_val > 0. ? " (z_val = " + std::to_string(z_val) : " (Z = " + std::to_string(o.Z)) + "): configuration";
         if (k >= 0) {
             const dftatom_occupation& x = cfg->orb[k];
             e += " entry " + std::to_string(k) + " (n = " + std::to_string(x.n) + ", l = " + std::to_string(x.l) + ", spin = " + std::to_string(x.spin)
@@ -183,7 +183,8 @@ int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, A
     if (ord[0].empty()) return bad(-1, "has no alpha (spin 0) entry");
     for (int s = 0; s < 2; ++s)
         if ((int)ord[s].size() > DFTATOM_MAX_LEVELS) return bad(-1, "more than DFTATOM_MAX_LEVELS entries of one spin");
-    if (!(q > 0. && q <= o.Z + 2.)) return bad(-1, "electron count " + std::to_string(q) + " outside (0, Z + 2]");
+    if (z_val > 0. ? !(q > 0. && q <= z_val + 2.) : !(q > 0. && q <= o.Z + 2.))
+        return bad(-1, "electron count " + std::to_string(q) + (z_val > 0. ? " outside (0, z_val + 2]" : " outside (0, Z + 2]"));
     for (int s = 0; s < 2; ++s) {
         std::stable_sort(ord[s].begin(), ord[s].end(), [&](int x, int y) {
             const dftatom_occupation &a = cfg->orb[x], &b = cfg->orb[y];

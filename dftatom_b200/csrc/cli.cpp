@@ -31,6 +31,11 @@
 //           (dftatom_kb_form): one "# kb" line per channel (l E_KB cos eps_loc0 eps_loc1 ghost status) after the channel lines and one
 //           beta column per channel after rho_val.  With --logderiv also DIR2/<index>_Z<Z>_pseudo_kb_logderiv.tsv, the KB logarithmic
 //           derivatives (dftatom_kb_log_derivatives) in the layout of the pseudo table.  An atom without a channel of l = L is an error.
+// --pseudo-test "3s1 3p3;3s2 3p1": with --pseudo and a single --Z, the transferability test of its pseudopotentials: the pseudo-atom
+//           (dftatom_solve_pseudo_batch) in the reference valence configuration and in each listed one, and the all-electron atom in core +
+//           each of them (the core: every reference entry whose n is below its channel's reference n, or whose l has no channel).
+//           DIR/<index>_Z<Z>_pseudo_test.tsv: one row per configuration (config Q E_AE E_PS dE_AE dE_PS dE_PS-dE_AE status_AE status_PS;
+//           dE against the reference configuration), then one "# level" line per level (config n l spin occ eps_AE eps_PS).
 #include <algorithm>
 #include <cmath>
 #include <cctype>
@@ -278,11 +283,86 @@ static int write_logderiv(dftatom_ctx* ctx, const std::string& dir, int index, c
     return 0;
 }
 
+// --pseudo-test: the pseudo-atom of the channels ch (rows of v_ion) against the all-electron atom in the reference configuration and in
+// every configuration of `tests`
+static int pseudo_test(dftatom_ctx* ctx, const std::string& path, const dftatom_options& o, const dftatom_result& R, const dftatom_config* cfg,
+                       const std::vector<dftatom_tm_channel>& ch, const std::vector<double>& v_ion, const std::vector<std::string>& tests)
+{
+    dftatom_pseudo_atom pa = {};
+    for (int l = 0; l < 4; ++l) pa.row[l] = -1;
+    for (size_t c = 0; c < ch.size(); ++c) { pa.row[ch[c].l] = (int)c; pa.n_ref[ch[c].l] = R.levels[0][ch[c].orbital].n; pa.z_val += ch[c].occ; }
+    pa.mixing = o.mixing; pa.method = 0;
+    // the reference configuration split into core and valence; its valence string
+    dftatom_config core = {}, ref = {};
+    std::string ref_str;
+    for (int k = 0; k < R.n_levels[0]; ++k) {
+        const dftatom_level& L = R.levels[0][k];
+        const dftatom_occupation e = { L.n, L.l, 0, exact_occ(L, 0, cfg) };
+        if (pa.row[L.l] < 0 || L.n < pa.n_ref[L.l]) core.orb[core.n_orbitals++] = e;
+        else {
+            ref.orb[ref.n_orbitals++] = e;
+            char b[64];
+            std::snprintf(b, sizeof b, "%s%d%c%.17g", ref_str.empty() ? "" : " ", L.n, kOrb[L.l], e.occ);
+            ref_str += b;
+        }
+    }
+    std::vector<std::string> names(1, ref_str);
+    std::vector<dftatom_config> ps(1, ref);
+    for (const std::string& t : tests) {
+        dftatom_config c = {};
+        if (!parse_config(t, 0, &c)) return 2;
+        for (int k = 0; k < c.n_orbitals; ++k)
+            if (pa.row[c.orb[k].l] < 0) {
+                std::fprintf(stderr, "dftatom: --pseudo-test \"%s\": Z=%d has no pseudopotential channel with l = %d\n", t.c_str(), o.Z, c.orb[k].l);
+                return 2;
+            }
+        names.push_back(t);
+        ps.push_back(c);
+    }
+    const int n = (int)ps.size();
+    std::vector<dftatom_config> ae(n, core);
+    for (int q = 0; q < n; ++q)
+        for (int k = 0; k < ps[q].n_orbitals; ++k) ae[q].orb[ae[q].n_orbitals++] = ps[q].orb[k];
+    std::vector<dftatom_pseudo_atom> pas(n, pa);
+    std::vector<dftatom_options> opts(n, o);
+    std::vector<dftatom_result> r_ps(n), r_ae(n);
+    if (dftatom_solve_pseudo_batch(ctx, o.levels, o.delta, o.max_r, v_ion.data(), (int)ch.size(), pas.data(), ps.data(), n, r_ps.data(), nullptr, 0,
+                                   nullptr) != DFTATOM_OK ||
+        dftatom_solve_batch_config(ctx, opts.data(), ae.data(), n, r_ae.data(), nullptr, 0, nullptr) != DFTATOM_OK) {
+        std::fprintf(stderr, "dftatom: --pseudo-test Z=%d: %s\n", o.Z, dftatom_last_error());
+        return 1;
+    }
+    FILE* f = std::fopen(path.c_str(), "w");
+    if (!f) { std::perror(path.c_str()); return 1; }
+    std::fprintf(f, "# Z=%d method=%d pseudo-atom test; dE against the reference configuration (row 1)\n", o.Z, o.method);
+    std::fprintf(f, "# config\tQ\tE_AE\tE_PS\tdE_AE\tdE_PS\tdE_PS-dE_AE\tstatus_AE\tstatus_PS\n");
+    for (int q = 0; q < n; ++q) {
+        double Q = 0.;
+        for (int k = 0; k < ps[q].n_orbitals; ++k) Q += ps[q].orb[k].occ;
+        const double dae = r_ae[q].Etotal - r_ae[0].Etotal, dps = r_ps[q].Etotal - r_ps[0].Etotal;
+        std::fprintf(f, "%s\t%.17g\t%.17g\t%.17g\t%.17g\t%.17g\t%.17g\t%d\t%d\n", names[q].c_str(), Q, r_ae[q].Etotal, r_ps[q].Etotal, dae, dps, dps - dae,
+                     r_ae[q].status, r_ps[q].status);
+    }
+    std::fprintf(f, "# level\tconfig\tn\tl\tspin\tocc\teps_AE\teps_PS\n");
+    for (int q = 0; q < n; ++q)
+        for (int k = 0; k < r_ps[q].n_levels[0]; ++k) {
+            const dftatom_level& L = r_ps[q].levels[0][k];
+            double e_ae = NAN;
+            for (int j = 0; j < r_ae[q].n_levels[0]; ++j)
+                if (r_ae[q].levels[0][j].n == L.n && r_ae[q].levels[0][j].l == L.l) e_ae = r_ae[q].levels[0][j].E;
+            std::fprintf(f, "# level\t%s\t%d\t%d\t%d\t%.17g\t%.17g\t%.17g\n", names[q].c_str(), L.n, L.l, 0, exact_occ(L, 0, &ps[q]), e_ae, L.E);
+        }
+    const bool bad = std::ferror(f) != 0;
+    if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
+    return 0;
+}
+
 // --pseudo: the valence channels of one LDA atom (largest n per l of its levels), pseudized and unscreened together; with --logderiv
 // also the logarithmic derivatives of their V_scr rows at the all-electron table's radius and energies
 static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::string& ld_dir, int index, const dftatom_options& o,
                         const dftatom_result& R, const dftatom_config* cfg, int N, const double* r, const double* v, const double* orb,
-                        const std::vector<double>& rcs, double ld_rc, const std::vector<double>& E, int kb_loc)
+                        const std::vector<double>& rcs, double ld_rc, const std::vector<double>& E, int kb_loc,
+                        const std::vector<std::string>& tests)
 {
     int best[4] = { -1, -1, -1, -1 };
     for (int k = 0; k < R.n_levels[0]; ++k) {
@@ -348,6 +428,10 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
     }
     bool bad = std::ferror(f) != 0;
     if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
+    if (!tests.empty()) {
+        const int rc_t = pseudo_test(ctx, dir + stem + "_test.tsv", o, R, cfg, ch, v_ion, tests);
+        if (rc_t) return rc_t;
+    }
     if (ld_dir.empty()) return 0;
     const int ne = (int)E.size();
     std::vector<int> pot(nc), l(nc);
@@ -402,7 +486,7 @@ int main(int argc, char** argv)
 {
     dftatom_options base = { 36, 12, 10.0, 0.001, 0.5, 0 };     // Options.cpp:6
     std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
-    std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301", pseudo_dir, pseudo_rc;
+    std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301", pseudo_dir, pseudo_rc, pseudo_test;
     double charge = 0., rc = NAN;
     int pseudo_local = -1;
     int precision = 6, device = 0, gpus = 1;
@@ -422,6 +506,7 @@ int main(int argc, char** argv)
         else if (a == "--energies") energies = next();
         else if (a == "--pseudo") pseudo_dir = next();
         else if (a == "--pseudo-rc") pseudo_rc = next();
+        else if (a == "--pseudo-test") pseudo_test = next();
         else if (a == "--pseudo-local") {
             const std::string v = next();
             if (v.size() != 1 || v[0] < '0' || v[0] > '3') { std::fprintf(stderr, "dftatom: --pseudo-local expects l = 0, 1, 2 or 3, got '%s'\n", v.c_str()); return 2; }
@@ -446,7 +531,7 @@ int main(int argc, char** argv)
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
                         "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR] [--charge Q] [--config \"...\"]\n"
-                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf] [--pseudo-local L]]\n"
+                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf] [--pseudo-local L] [--pseudo-test \"C1;C2\"]]\n"
                         "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n"
                         "  --charge Q    solve every atom of --Z ionised by Q electrons (the reference's configuration; fractional allowed, < 0 = anion)\n"
                         "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n"
@@ -458,7 +543,10 @@ int main(int argc, char** argv)
                         "                (columns r, V_ion per l, V_scr per l, u per l, rho_val); with --logderiv also <index>_Z<Z>_pseudo_logderiv.tsv\n"
                         "  --pseudo-rc Rs[,Rp,Rd,Rf]  radii of --pseudo in bohr by l (an l beyond the list takes the last one)\n"
                         "  --pseudo-local L  Kleinman-Bylander form of --pseudo with the channel l = L local: one \"# kb\" line per channel (l E_KB cos\n"
-                        "                eps_loc0 eps_loc1 ghost status) and beta columns; with --logderiv also <index>_Z<Z>_pseudo_kb_logderiv.tsv\n");
+                        "                eps_loc0 eps_loc1 ghost status) and beta columns; with --logderiv also <index>_Z<Z>_pseudo_kb_logderiv.tsv\n"
+                        "  --pseudo-test \"C1;C2\"  with --pseudo and a single --Z: solve the pseudo-atom in the reference valence configuration and in\n"
+                        "                each valence configuration Ck (e.g. \"3s1 3p3;3s2 3p1\"), the all-electron atom in core + each, and write\n"
+                        "                <index>_Z<Z>_pseudo_test.tsv (config Q E_AE E_PS dE_AE dE_PS dE_PS-dE_AE statuses, then eps_AE / eps_PS per level)\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
         if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
@@ -479,6 +567,21 @@ int main(int argc, char** argv)
     }
     std::vector<double> ps_rc;
     if (pseudo_local >= 0 && pseudo_dir.empty()) { std::fprintf(stderr, "dftatom: --pseudo-local needs --pseudo DIR\n"); return 2; }
+    std::vector<std::string> ps_tests;
+    if (!pseudo_test.empty()) {
+        if (pseudo_dir.empty() || zs.size() != 1) { std::fprintf(stderr, "dftatom: --pseudo-test needs --pseudo DIR and a single --Z\n"); return 2; }
+        if (base.method & 2) { std::fprintf(stderr, "dftatom: --pseudo-test needs the logarithmic grid (method 0)\n"); return 2; }
+        for (size_t p = 0; p <= pseudo_test.size();) {
+            const size_t q = std::min(pseudo_test.find(';', p), pseudo_test.size());
+            const std::string t = pseudo_test.substr(p, q - p);
+            dftatom_config c = {};
+            if (t.find_first_not_of(" \t") == std::string::npos || !parse_config(t, 0, &c) || c.n_orbitals == 0) {
+                std::fprintf(stderr, "dftatom: --pseudo-test: cannot read the configuration '%s'\n", t.c_str()); return 2;
+            }
+            ps_tests.push_back(t);
+            p = q + 1;
+        }
+    }
     if (!pseudo_dir.empty()) {
         if (base.method & 1) { std::fprintf(stderr, "dftatom: --pseudo needs an LDA atom (method 0 or 2): the unscreening is spin-unpolarised\n"); return 2; }
         for (size_t p = 0; p < pseudo_rc.size();) {
@@ -558,7 +661,7 @@ int main(int argc, char** argv)
         }
     for (int a = 0; a < n && !pseudo_dir.empty(); ++a)
         if (write_pseudo(ctx, pseudo_dir, logderiv_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a], configured ? &cfgs[a] : nullptr, N,
-                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E, pseudo_local)) {
+                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E, pseudo_local, ps_tests)) {
             dftatom_destroy(ctx); return 1;
         }
 

@@ -130,6 +130,7 @@ struct dftatom_ctx {
     DevBuf atoms, astate, orbs, ss, rho, rhot, vpot, atab, psi, match_pt, inv_norm, epart, eticket, team_bar, phi, src, u0, ubuf, zbc, tab_of, steps, n_active;
     DevBuf scratch[8];
     DevBuf radial, radial_part, radial_ticket;     // export of the radial state (dftatom_solve_batch_radial): staging, partial sums, tickets
+    DevBuf pseudo_atoms, pseudo_v;                 // dftatom_solve_pseudo_batch: per-atom channel rows, the ionic potentials
     int* h_active = nullptr;       // pinned
     char* h_up = nullptr; size_t h_up_cap = 0, h_up_used = 0;      // pinned staging of the descriptor uploads of one solve (reset at its start)
     // timing of the last solve
@@ -326,6 +327,7 @@ void dftatom_destroy(dftatom_ctx* c)
     for (DevBuf* b : all) b->release();
     for (DevBuf& b : c->scratch) b.release();
     c->radial.release(); c->radial_part.release(); c->radial_ticket.release();
+    c->pseudo_atoms.release(); c->pseudo_v.release();
     c->stream_G.release(); c->stream_src0.release(); c->stream_scratch.release(); c->exact_work.release(); c->last_steps.release(); c->rho_prev.release(); c->d_src.release(); c->d_u.release();
     if (c->h_active) cudaFreeHost(c->h_active);
     if (c->h_up) cudaFreeHost(c->h_up);
@@ -499,9 +501,15 @@ static int export_radial(dftatom_ctx* c, const GridDev& g, const ScfBuffers& b, 
     return 0;
 }
 
-// one group of atoms: its whole SCF, enqueued on the context's stream
+// A group of pseudo-atoms (dftatom_solve_pseudo_batch, validated there): the HOST ionic potentials and the atoms' descriptors
+struct PseudoGroup {
+    const double* v_ion; int n_rows;
+    const dftatom_pseudo_atom* atoms;
+};
+
+// one group of atoms: its whole SCF, enqueued on the context's stream (pg: pseudo-atoms, opts[a].Z = their Z_b)
 static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftatom_config* cfgs, int n_atoms, dftatom_result* out,
-                       dftatom_step* steps, int steps_stride, const RadialDest* rd = nullptr)
+                       dftatom_step* steps, int steps_stride, const RadialDest* rd = nullptr, const PseudoGroup* pg = nullptr)
 {
     if (!c || !opts || !out || n_atoms <= 0) { set_error("bad argument"); return DFTATOM_E_ARG; }
     const bool host_dbg = getenv("DFTATOM_DEBUG_HOST") != nullptr;      // development aid: wall-clock of the host-side stages
@@ -535,6 +543,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     std::vector<int> tab_of(2 * (size_t)n_atoms, -1);
     std::vector<double> zbc(n_atoms);
     std::vector<std::vector<dftatom_level>> lev_a(n_atoms), lev_b(n_atoms);
+    std::vector<PseudoAtomDev> patoms(pg ? n_atoms : 0);
     int n_tabs = 0, max_steps = 0, zmax = 1;
     for (int a = 0; a < n_atoms; ++a) {
         AtomDev& at = atoms[a];
@@ -545,7 +554,8 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
         max_steps = std::max(max_steps, at.n_steps_max);
         zmax = std::max(zmax, at.Z);
         AtomLevels al;
-        if ((rc = atom_levels(a, opts[a], cfgs ? &cfgs[a] : nullptr, &al))) return rc;
+        if ((rc = atom_levels(a, opts[a], cfgs ? &cfgs[a] : nullptr, &al, pg ? pg->atoms[a].z_val : 0.))) return rc;
+        if (pg) for (auto& L : al.lev) for (dftatom_level& x : L) x.nodes = x.n - pg->atoms[a].n_ref[x.l];
         lev_a[a] = al.lev[0]; lev_b[a] = al.lev[1];
         at.n_el[0] = al.n_el[0]; at.n_el[1] = al.n_el[1];
         zbc[a] = al.n_el[0] + al.n_el[1];                    // U(Rmax) = the electron count Q (Z for the neutral atom)
@@ -561,6 +571,14 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
             ++n_tabs;
         }
         if (at.n_spin == 1) { at.orb_begin[1] = 0; at.orb_count[1] = 0; }
+        if (pg) {       // one row per (spin, channel) after the atom's density rows; its orbitals are solved in the row of their l
+            PseudoAtomDev& p = patoms[a];
+            for (int l = 0; l < 4; ++l) {
+                p.vrow[l] = pg->atoms[a].row[l];
+                for (int s = 0; s < 2; ++s) p.tab[s][l] = (p.vrow[l] >= 0 && s < at.n_spin) ? n_tabs++ : -1;
+            }
+            for (size_t q = (size_t)at.orb_begin[0]; q < orbs.size(); ++q) orbs[q].tab = p.tab[orbs[q].spin][orbs[q].l];
+        }
         astate[a] = AtomState{ 0., 0, 0, 0, DFTATOM_MAX_STEPS, opts[a].mixing, 0., 0., 0, 0 };
     }
     const int n_orbs = (int)orbs.size();
@@ -569,8 +587,10 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     c->last_h2d_bytes = (long long)(sizeof(AtomDev) * atoms.size() + sizeof(AtomState) * astate.size() + sizeof(OrbitalDev) * orbs.size()
                                     + sizeof(int) * (tab_of.size() + 2) + sizeof(double) * zbc.size());
 
+    const size_t pseudo_bytes = pg ? sizeof(PseudoAtomDev) * patoms.size() + sizeof(double) * (size_t)pg->n_rows * N : 0;
+
     // ---- device buffers ----
-    if ((rc = upload_arena_reset(c, (size_t)c->last_h2d_bytes + 64 * 8))) return rc;
+    if ((rc = upload_arena_reset(c, (size_t)c->last_h2d_bytes + pseudo_bytes + 64 * 8))) return rc;
     if ((rc = upload(c, c->atoms, atoms))) return rc;
     if ((rc = upload(c, c->astate, astate))) return rc;
     if ((rc = upload(c, c->orbs, orbs))) return rc;
@@ -603,6 +623,13 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     if ((rc = c->steps.ensure(sizeof(dftatom_step) * (size_t)n_atoms * stride))) return rc;
     if ((rc = c->last_steps.ensure(sizeof(dftatom_step) * (size_t)n_atoms))) return rc;
     if ((rc = c->n_active.ensure(sizeof(int) * 2))) return rc;
+    PseudoArgs pargs{};
+    if (pg) {
+        if ((rc = upload(c, c->pseudo_atoms, patoms))) return rc;
+        if ((rc = upload(c, c->pseudo_v, std::vector<double>(pg->v_ion, pg->v_ion + (size_t)pg->n_rows * N)))) return rc;
+        pargs.atoms = c->pseudo_atoms.as<PseudoAtomDev>(); pargs.v_ion = c->pseudo_v.as<double>();
+        c->last_h2d_bytes += (long long)pseudo_bytes;
+    }
     DFT_CHECK(cudaMemsetAsync(c->steps.p, 0, sizeof(dftatom_step) * (size_t)n_atoms * stride, st));
     DFT_CHECK(cudaMemsetAsync(c->ss.p, 0, sizeof(SearchState) * (size_t)n_orbs, st));
     const int h_counts[2] = { n_atoms, n_orbs };        // atoms / orbitals still iterating, kept up to date by potential_energy_kernel
@@ -750,7 +777,9 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     } else {
         poisson_solve(0, launches);
     }
-    launch_potential_energy(g, lv, b, 1, st); ++launches;
+    if (pg) launch_pseudo_potential_energy(g, b, pargs, 1, st);
+    else launch_potential_energy(g, lv, b, 1, st);
+    ++launches;
 
     const int rounds = search_rounds_needed(zmax);
     int steps_enqueued = 0;
@@ -798,7 +827,9 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
         poisson_solve(sp >= c->k.warm_after ? c->k.warm_vcycles : 0, nl);
         end_phase();
         begin_phase(DFTATOM_K_POTENTIAL);
-        launch_potential_energy(g, lv, b, 0, st); ++nl;
+        if (pg) launch_pseudo_potential_energy(g, b, pargs, 0, st);
+        else launch_potential_energy(g, lv, b, 0, st);
+        ++nl;
         end_phase();
         nvtxRangePop();
     };
@@ -1076,6 +1107,85 @@ int dftatom_solve_batch_config(dftatom_ctx* c, const dftatom_options* opts, cons
         for (int k = 0; k < DFTATOM_K_COUNT; ++k) { c->prof[k].ms += ch->prof[k].ms; c->prof[k].launches += ch->prof[k].launches; c->prof[k].work += ch->prof[k].work; }
     }
     return 0;
+}
+
+int dftatom_solve_pseudo_batch(dftatom_ctx* c, int levels, double delta, double max_r, const double* v_ion, int n_rows,
+                               const dftatom_pseudo_atom* atoms, const dftatom_config* configs, int n_atoms, dftatom_result* out,
+                               dftatom_step* steps, int steps_stride, const dftatom_radial* radial)
+{
+    if (!c || !v_ion || !atoms || !configs || !out) { set_error("dftatom_solve_pseudo_batch: NULL argument"); return DFTATOM_E_ARG; }
+    if (n_rows < 1 || n_atoms < 1) { set_error("dftatom_solve_pseudo_batch: n_rows and n_atoms must be >= 1"); return DFTATOM_E_ARG; }
+    if (delta == 0.) { set_error("dftatom_solve_pseudo_batch: the uniform grid (delta = 0) is not supported"); return DFTATOM_E_BAD_OPTION; }
+    const auto where = [](int a) { return "dftatom_solve_pseudo_batch: atom " + std::to_string(a) + ": "; };
+    const int N = (1 << std::min(std::max(levels, 0), 20)) + 1;
+    std::vector<dftatom_options> opts(n_atoms);
+    std::vector<char> row_ok(n_rows, 0);
+    long long orb_rows = 0;
+    int rc;
+    for (int a = 0; a < n_atoms; ++a) {
+        const dftatom_pseudo_atom& pa = atoms[a];
+        if (pa.method != 0 && pa.method != 1) { set_error(where(a) + "method must be 0 (LDA) or 1 (LSDA)"); return DFTATOM_E_BAD_OPTION; }
+        dftatom_options& o = opts[a];
+        o.Z = 1; o.levels = levels; o.max_r = max_r; o.delta = delta; o.mixing = pa.mixing; o.method = pa.method;
+        if ((rc = validate(o))) { set_error(where(a) + dftatom_last_error()); return rc; }
+        if (!(std::isfinite(pa.z_val) && pa.z_val > 0.)) { set_error(where(a) + "z_val must be finite and > 0"); return DFTATOM_E_BAD_OPTION; }
+        int n_ch = 0;
+        for (int l = 0; l < 4; ++l) {
+            if (pa.row[l] < -1 || pa.row[l] >= n_rows) {
+                set_error(where(a) + "row[" + std::to_string(l) + "] = " + std::to_string(pa.row[l]) + " outside -1.." + std::to_string(n_rows - 1));
+                return DFTATOM_E_BAD_OPTION;
+            }
+            if (pa.row[l] < 0) continue;
+            ++n_ch;
+            if (pa.n_ref[l] < l + 1 || pa.n_ref[l] > 8) {
+                set_error(where(a) + "n_ref[" + std::to_string(l) + "] = " + std::to_string(pa.n_ref[l]) + " outside " + std::to_string(l + 1) + "..8");
+                return DFTATOM_E_BAD_OPTION;
+            }
+        }
+        if (!n_ch) { set_error(where(a) + "no channel (every row is -1)"); return DFTATOM_E_BAD_OPTION; }
+        const dftatom_config& cf = configs[a];
+        if (cf.n_orbitals == 0) { set_error(where(a) + "empty configuration"); return DFTATOM_E_BAD_OPTION; }
+        AtomLevels al;
+        if ((rc = atom_levels(a, o, &cf, &al, pa.z_val))) { set_error(where(a) + dftatom_last_error()); return rc; }
+        for (int k = 0; k < cf.n_orbitals; ++k) {
+            const dftatom_occupation& x = cf.orb[k];
+            const std::string at = where(a) + "configuration entry " + std::to_string(k) + " (n = " + std::to_string(x.n) + ", l = " + std::to_string(x.l) + "): ";
+            if (pa.row[x.l] < 0) { set_error(at + "l has no channel"); return DFTATOM_E_BAD_OPTION; }
+            if (x.n < pa.n_ref[x.l]) { set_error(at + "n below n_ref = " + std::to_string(pa.n_ref[x.l])); return DFTATOM_E_BAD_OPTION; }
+        }
+        orb_rows += cf.n_orbitals;
+        // the bracket of the energy search: -Z_b^2 - 1 at least 10 Ha below the deepest ionic potential of the atom
+        double vmin = INFINITY;
+        for (int l = 0; l < 4; ++l) {
+            if (pa.row[l] < 0) continue;
+            const double* v = v_ion + (size_t)pa.row[l] * N;
+            for (int i = 1; i < N; ++i) {
+                if (!row_ok[pa.row[l]] && !std::isfinite(v[i])) {
+                    set_error(where(a) + "v_ion row " + std::to_string(pa.row[l]) + " is not finite at node " + std::to_string(i));
+                    return DFTATOM_E_BAD_OPTION;
+                }
+                vmin = std::min(vmin, v[i]);
+            }
+            row_ok[pa.row[l]] = 1;
+        }
+        int zb = 1;
+        while (zb <= 118 && -(double)zb * zb - 1. > vmin - 10.) ++zb;
+        if (zb > 118) { set_error(where(a) + "ionic potential too deep (min V_ion = " + std::to_string(vmin) + " below -118^2 + 9)"); return DFTATOM_E_BAD_OPTION; }
+        o.Z = zb;
+    }
+    std::vector<int> dest_atom;
+    std::vector<long long> dest_row;
+    if (radial) {
+        if ((radial->orbitals || radial->moments) && radial->orbital_rows < orb_rows) {
+            set_error("dftatom_radial.orbital_rows is " + std::to_string(radial->orbital_rows) + ", the batch has " + std::to_string(orb_rows) + " orbitals");
+            return DFTATOM_E_ARG;
+        }
+        long long rows = 0;
+        for (int a = 0; a < n_atoms; ++a) { dest_atom.push_back(a); dest_row.push_back(rows); rows += configs[a].n_orbitals; }
+    }
+    const RadialDest rd{ radial, dest_atom.data(), dest_row.data(), true };
+    const PseudoGroup pg{ v_ion, n_rows, atoms };
+    return solve_group(c, opts.data(), configs, n_atoms, out, steps, steps_stride, radial ? &rd : nullptr, &pg);
 }
 
 // ---------------------------------------------------------------------------------------------------------

@@ -328,6 +328,19 @@ void launch_initial_density(const GridDev& g, const ScfBuffers& b, cudaStream_t 
 void launch_orbital_norms(const GridDev& g, const ScfBuffers& b, cudaStream_t st);
 void launch_density_update(const GridDev& g, const ScfBuffers& b, cudaStream_t st);
 void launch_potential_energy(const GridDev& g, const PoissonLevels& lv, const ScfBuffers& b, int first, cudaStream_t st);
+// pseudo-atoms (dftatom_solve_pseudo_batch): the SCF of ScfBuffers with one atab / vpot row per (atom, spin, channel l), which
+// OrbitalDev.tab points at; the row tab_of[2 a + s] keeps the density of (a, s) and, in vpot, the screening V_H + V_xc,s
+struct PseudoAtomDev {
+    int vrow[4];          // v_ion row of channel l, -1 = no channel
+    int tab[2][4];        // atab / vpot row of (spin, l), -1 = none
+};
+struct PseudoArgs {
+    const PseudoAtomDev* atoms;     // [n_atoms]
+    const double* v_ion;            // [n_rows][N]
+};
+// V_l,s = V_ion,l + U / r + V_xc,s into every channel row, the energies of dftatom_solve_pseudo_batch and the stop test of
+// potential_energy_kernel; first != 0: only the initial potential
+void launch_pseudo_potential_energy(const GridDev& g, const ScfBuffers& b, const PseudoArgs& p, int first, cudaStream_t st);
 
 // export of the radial state (radial.cu): part / ticket: radial_part_doubles(N, rows) doubles / rows ints (tickets zero before the launch)
 long long radial_part_doubles(int N, int n_rows);
@@ -407,7 +420,8 @@ struct AtomLevels {
     std::vector<double> occ[2];
     double n_el[2];
 };
-int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, AtomLevels* out);
+// z_val > 0 (a pseudo-atom): the electron count is bounded by z_val + 2 instead of Z + 2, and the messages name z_val
+int atom_levels(int atom, const dftatom_options& o, const dftatom_config* cfg, AtomLevels* out, double z_val = 0.);
 double estimate_cost(int Z, int method);
 int partition_atoms(const int* Z, const int* method, int n, int n_ranks, int* rank_of);
 

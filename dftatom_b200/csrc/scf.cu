@@ -583,4 +583,143 @@ void launch_potential_energy(const GridDev& g, const PoissonLevels& lv, const Sc
     launch_step_kernel(potential_energy_kernel, dim3(b.n_atoms, node_chunks(g.N)), dim3(kPT2), 0, st, g, lv, b, first);
 }
 
+// The potential-and-energy step of a pseudo-atom (dftatom_solve_pseudo_batch): grid, per-atom ticket, fixed-order sum, stop test and
+// adaptive mixing of potential_energy_kernel (the tail is repeated here so that kernel's code stays as it is).  Every channel row gets
+// V_l,s = V_ion,l + U / r + V_xc,s and its a-table; the row tab_of[2 a + s] gets the screening U / r + V_xc,s (the radial export's v).
+// The integrals: E_ion = sum occ <u|V_ion,l|u> and sum occ <u|V_l,s|u> over the orbitals in psi (occ x inv_norm x wjac x u^2), and
+// the xc / Hartree integrals of the density as in the all-electron kernel.
+__global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g, ScfBuffers b, PseudoArgs p, int first)
+{
+    DFT_PDL_WAIT();
+    __shared__ double sm[5 * 32];
+    __shared__ double wgt[2 * DFTATOM_MAX_LEVELS];          // occupation / norm of every orbital
+    __shared__ int orb_l[2 * DFTATOM_MAX_LEVELS];
+    __shared__ int is_last;
+    const int a = blockIdx.x;
+    AtomState& as = b.astate[a];
+    if (as.done) return;
+    const AtomDev at = b.atoms[a];
+    const PseudoAtomDev pd = p.atoms[a];
+    const int N = g.N;
+    const int n_orb = at.orb_count[0] + at.orb_count[1];
+    if (!first)
+        for (int q = threadIdx.x; q < n_orb; q += blockDim.x) {
+            const int o = at.orb_begin[0] + q;          // the beta orbitals follow the alpha ones
+            wgt[q] = b.orbs[o].occ * b.inv_norm[o];
+            orb_l[q] = b.orbs[o].l;
+        }
+    __syncthreads();
+    const double* U = b.U + (size_t)a * b.ldU;
+    const double* rt = b.rhot + (size_t)a * N;
+    const int ta = b.tab_of[2 * a], tb = b.tab_of[2 * a + 1];
+    const double q = g.delta * g.delta * 0.25;
+
+    double e[5] = { 0., 0., 0., 0., 0. };   // E_ion, exccor, eexcDeriv, hartree, sum occ <u|V_l|u>
+    const int kPotChunks = (int)gridDim.y;
+    const int per = (N + kPotChunks - 1) / kPotChunks;
+    const int i0 = blockIdx.y * per, i1 = min(i0 + per, N);
+    for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        double S[2] = { 0., 0. };                           // screening per spin
+        if (i >= 1) {
+            const double r = g.r[i];
+            const double vh = U[i] / r;
+            const double rho = rt[i];
+            const double wj = g.wjac[i];
+            const double rd = r * rho * wj;
+            const double r2d = r * rd;
+            double vexc, edif;
+            if (at.n_spin == 2) {
+                const XcLsda x = xc_lsda(b.rho[(size_t)ta * N + i], b.rho[(size_t)tb * N + i]);
+                S[0] = vh + x.va; S[1] = vh + x.vb;
+                vexc = x.vexc; edif = x.edif;
+            } else {
+                const XcLda x = xc_lda(rho);
+                S[0] = vh + x.vexc;
+                vexc = x.vexc; edif = x.edif;
+            }
+            e[1] = fma(r2d, vexc, e[1]);
+            e[2] = fma(r2d, edif, e[2]);
+            e[3] = fma(rd, U[i], e[3]);
+            if (!first) {
+                const double sq = g.sqex[i];
+                for (int k = 0; k < n_orb; ++k) {
+                    const int o = at.orb_begin[0] + k;
+                    const double u = b.psi[(size_t)o * N + i] * sq;
+                    const double w = wgt[k] * wj * u * u;
+                    const double vi = p.v_ion[(size_t)pd.vrow[orb_l[k]] * N + i];
+                    e[0] = fma(w, vi, e[0]);
+                    e[4] = fma(w, vi + S[k >= at.orb_count[0]], e[4]);
+                }
+            }
+        }
+        for (int s = 0; s < at.n_spin; ++s) b.vpot[(size_t)(s ? tb : ta) * N + i] = S[s];
+#pragma unroll
+        for (int l = 0; l < 4; ++l) {
+            if (pd.vrow[l] < 0) continue;
+            const double vi = i >= 1 ? p.v_ion[(size_t)pd.vrow[l] * N + i] : 0.;
+            for (int s = 0; s < at.n_spin; ++s) {
+                const double V = i >= 1 ? vi + S[s] : 0.;
+                const int t = pd.tab[s][l];
+                b.vpot[(size_t)t * N + i] = V;
+                b.atab[(size_t)t * N + i] = (g.k2[i] * V + q) * (1. / 12.);
+            }
+        }
+    }
+    if (first) return;
+    block_sum_n<5>(e, sm);
+    if (threadIdx.x == 0) {
+        double* part = b.epart + ((size_t)a * kPotChunks + blockIdx.y) * 5;
+        for (int c = 0; c < 5; ++c) part[c] = e[c];
+        __threadfence();
+        const int ticket = atomicAdd(b.eticket + a, 1);
+        is_last = (ticket == kPotChunks - 1);
+        if (is_last) b.eticket[a] = 0;
+    }
+    __syncthreads();
+    if (!is_last) return;
+    if (threadIdx.x < 5) {
+        __threadfence();
+        const double* part = b.epart + (size_t)a * kPotChunks * 5 + threadIdx.x;
+        double t = 0.;
+        for (int c = 0; c < kPotChunks; ++c) t += __ldcg(part + c * 5);
+        sm[threadIdx.x] = t;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int c = 0; c < 5; ++c) e[c] = sm[c];
+        dftatom_step* rec = b.steps + (size_t)a * b.steps_stride + as.n_steps;
+        const double eel = rec->Ekin;                      // parked by density_update_kernel
+        const double e_dif = kFourPi * e[2];
+        const double e_xc = kFourPi * e[1] + e_dif;
+        const double e_har = -0.5 * kFourPi * e[3];
+        const double etot = eel + e_har + e_dif;
+        rec->Etotal = etot; rec->Ekin = eel - e[4]; rec->Ecoul = -e_har; rec->Eenuc = e[0]; rec->Exc = e_xc;
+        const int ok = rec->levels_converged;
+        int done = 0, status = DFTATOM_MAX_STEPS;
+        const int crit = fabs((as.e_old - etot) / etot) < kTotalEnergyTol && ok && as.prev_ok;
+        rec->stop_criterion_met = crit;
+        if (crit && !b.run_to_cap) { done = 1; status = DFTATOM_CONVERGED; }
+        if (b.adaptive_mixing) {                           // potential_energy_kernel's opt-in damping
+            const double d0 = etot - as.e_old;
+            if (as.hold > 0) --as.hold;
+            else if (as.n_steps >= 6 && as.n_raised < 3 && d0 * as.d1 < 0. && as.d1 * as.d2 < 0. && fabs(d0) > 0.5 * fabs(as.d1) && fabs(as.d1) > 0.5 * fabs(as.d2)) {
+                as.mix = 0.5 * (1. + as.mix);
+                as.hold = 4; as.n_raised += 1;
+            }
+            as.d2 = as.d1; as.d1 = d0;
+        }
+        as.e_old = etot;
+        as.prev_ok = ok;
+        as.n_steps += 1;
+        if (!done && as.n_steps >= at.n_steps_max) { done = 1; status = DFTATOM_MAX_STEPS; }
+        if (!done && !(fabs(etot) <= 1.7e308)) { done = 1; status = DFTATOM_NUMERIC_FAILURE; }
+        if (done) { as.done = 1; as.status = status; atomicAdd(b.n_active, -1); atomicAdd(b.n_active + 1, -n_orb); }
+    }
+}
+
+void launch_pseudo_potential_energy(const GridDev& g, const ScfBuffers& b, const PseudoArgs& p, int first, cudaStream_t st)
+{
+    launch_step_kernel(pseudo_potential_energy_kernel, dim3(b.n_atoms, node_chunks(g.N)), dim3(kPT2), 0, st, g, b, p, first);
+}
+
 }  // namespace dft

@@ -410,6 +410,38 @@ typedef struct { int pot, proj, l, pad; double E_KB, r_c; } dftatom_kb_ld_channe
 int dftatom_kb_log_derivatives(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V_loc, int n_pot,
                                const double* beta, int n_proj, const dftatom_kb_ld_channel* ch, int n_channels,
                                const double* E, int n_energies, dftatom_logderiv* out, double* r_used);
+/* Self-consistent pseudo-atoms: the valence-only atom of semilocal ionic pseudopotentials (e.g. v_ion of dftatom_tm_pseudize), solved
+ * in any valence configuration by the SCF of dftatom_solve_batch_config - the transferability test of a pseudopotential: total-energy
+ * differences and eigenvalues between configurations against the all-electron atom in the same configurations.
+ * Grid (levels, delta, max_r): the logarithmic grid of the SCF (delta = 0, the uniform grid, returns DFTATOM_E_BAD_OPTION).
+ * v_ion[n_rows][N] HOST ionic potentials (node 0 ignored).  Atom a = atoms[a]: row[l] the v_ion row of channel l (-1 = no channel),
+ * n_ref[l] the all-electron principal number of the channel's reference state (3 for Si 3s), z_val the ionic charge, mixing and method
+ * (0 = LDA, 1 = LSDA) as in dftatom_options.  configs[a]: its valence configuration, entries (n, l, spin, occ) with all-electron labels
+ * and the occupation rules of dftatom_solve_batch_config; an entry is solved with n - n_ref[l] nodes.
+ * Every SCF step runs the all-electron loop in the same order with
+ *   V_l,s = V_ion,l + U / r + V_xc,s(rho),  U the Poisson solution of the valence density with boundary value Q = sum occ, V_xc the
+ *   VWN LDA (method 0) or LSDA (method 1) of the SCF;
+ * every entry is solved in its V_l,s, then the density is built and mixed as in the all-electron SCF.  The stop test, the step caps (100
+ * LDA / 150 LSDA), the mixing, the start density (a uniform sphere of Q electrons) and the option "adaptive_mixing" are those of the
+ * all-electron SCF.  The energy search brackets [-Z_b^2 - 1, 50], Z_b the smallest integer >= 1 with -Z_b^2 - 1 at least 10 Ha below
+ * min over the atom's channels and nodes 1..N-1 of V_ion,l (the margin covers V_xc); its step-0 ladder uses Z_b in place of Z.
+ * Reported energies (dftatom_result / dftatom_step):
+ *   Eenuc  E_ion = sum occ <u|V_ion,l|u>          Ecoul  E_H            Exc  E_xc
+ *   Ekin   sum occ eps - sum occ <u|V_l,s|u>     Etotal sum occ eps - E_H + int rho (eps_xc - v_xc), the all-electron formula; at
+ *          convergence Etotal = Ekin + Eenuc + Ecoul + Exc
+ *   (<u|f|u> = sum over nodes 1..N-1 of wjac_i u_i^2 f_i with the normalised orbital of the step and the potential built in the step.)
+ * dftatom_result.levels[s][k]: n the all-electron label, nodes = n - n_ref[l].  steps, steps_stride and radial as in
+ * dftatom_solve_batch_config; the radial export's `v` holds the l-independent screening V_H + V_xc,s per spin (V_l,s = v_ion row + v).
+ * The atoms of one call are solved in one group (no stream-group split): a pseudo-atom's records do not depend on the batch.
+ * Validation before anything runs on the device (outputs untouched): DFTATOM_E_BAD_OPTION, naming the atom and the entry, for a bad grid or
+ * mixing, a method other than 0 / 1, no channel, a row outside -1..n_rows-1, n_ref[l] outside l+1..8, z_val not finite or <= 0, an empty
+ * configuration, the occupation ranges and duplicates of dftatom_solve_batch_config, an entry whose l has no channel or with n < n_ref[l],
+ * Q outside (0, z_val + 2], V_ion not finite at nodes 1..N-1, or Z_b > 118; DFTATOM_E_ARG for NULL pointers, n_rows or n_atoms < 1 and a
+ * too small radial orbital_rows. */
+typedef struct { int row[4], n_ref[4]; double z_val, mixing; int method, pad; } dftatom_pseudo_atom;      /* 56 bytes */
+int dftatom_solve_pseudo_batch(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* v_ion, int n_rows,
+                               const dftatom_pseudo_atom* atoms, const dftatom_config* configs, int n_atoms, dftatom_result* out,
+                               dftatom_step* steps, int steps_stride, const dftatom_radial* radial);
 /* The node radii r[N] (HOST) of the grid (levels, delta, max_r; delta = 0: uniform) as the engine builds and uses them. */
 int dftatom_grid_nodes(dftatom_ctx* ctx, int levels, double delta, double max_r, double* r);
 /* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) (the SCF passes the
