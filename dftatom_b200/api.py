@@ -161,6 +161,7 @@ def load_library():
     lib.dftatom_level_search.argtypes = [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, _ip, _ip, _dp, _ip]
     lib.dftatom_numerov_orbital.argtypes = [C.c_void_p, _dp, C.c_int, C.c_double, C.c_double, C.c_int, C.c_double, _dp, _ip]
     lib.dftatom_poisson_solve.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_int, _ip, _dp, _dp, _ip]
+    lib.dftatom_poisson_increment.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_int, _dp, _dp, _dp, _ip, C.c_int, C.c_int]
     lib.dftatom_poisson_vcycles.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_int, _dp, _dp, C.c_int, _dp]
     lib.dftatom_vwn.argtypes = [C.c_void_p, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp]
     lib.dftatom_simpson38.argtypes = [C.c_void_p, C.c_double, _dp, C.c_int, C.c_int, _dp]
@@ -769,6 +770,19 @@ class Context:
         U = np.zeros_like(rho); used = np.zeros(len(Z), np.int32)
         _check(self._lib.dftatom_poisson_solve(self._h, int(levels), float(delta), float(max_r), len(Z), _i(Z), _d(rho), _d(U), _i(used)))
         return U, used
+
+    def poisson_increment(self, levels, delta, max_r, rho, rho_prev, U, skip=None, solver=0, n_vcycles=7):
+        """One warm Poisson solve of the SCF in increment form (dftatom_poisson_increment): solver 0 direct, 1 warm V-cycles,
+        2 V-cycles of the cold solvers.  Returns (U + dU, rho_prev after the call = rho except where skipped); the inputs are not changed."""
+        rho = _f64(np.atleast_2d(rho)); rho_prev = _f64(np.atleast_2d(rho_prev)).copy(); U = _f64(np.atleast_2d(U)).copy()
+        if rho.shape != rho_prev.shape or rho.shape != U.shape or rho.shape[1] != (1 << int(levels)) + 1:
+            raise ValueError("rho, rho_prev and U must have the same shape [n_dens][2^levels + 1]")
+        sk = None if skip is None else _i32(np.asarray(skip).astype(np.int32))
+        if sk is not None and len(sk) != rho.shape[0]:
+            raise ValueError("skip must have one entry per density")
+        _check(self._lib.dftatom_poisson_increment(self._h, int(levels), float(delta), float(max_r), rho.shape[0], _d(rho), _d(rho_prev), _d(U),
+                                                   None if sk is None else _i(sk), int(solver), int(n_vcycles)))
+        return U, rho_prev
 
     def poisson_vcycles(self, levels, delta, phi, src, n_cycles):
         phi = _f64(np.atleast_2d(phi)).copy(); src = _f64(np.atleast_2d(src))

@@ -507,6 +507,51 @@ struct PseudoGroup {
     const dftatom_pseudo_atom* atoms;
 };
 
+// The three ways of a warm Poisson solve in increment form (selected by solve_group's poisson_solve; dftatom_poisson_increment's `solver`)
+enum { kIncDirect = 0, kIncWarmVcycles = 1, kIncColdForm = 2 };
+
+// One warm Poisson solve in increment form of the densities ca.rho: A dU = S(rho) - S(rho_prev) with dU = 0 at both ends, U += dU,
+// rho_prev = rho (ca.rho_prev, ca.U, ca.skip; ca.ldU is the row stride of U, d_src and d_u).  path kIncDirect: poisson_direct.cu (d_u is its
+// scratch above 14 levels); kIncWarmVcycles: n_vcycles V-cycles of poisson_warm.cu in pa's hierarchy; kIncColdForm: n_vcycles V-cycles of
+// the cold solvers (sa and splan: the stream solver when `stream`; else pa: poisson_full_kernel) on (d_src, d_u) between
+// poisson_delta_prepare and poisson_delta_apply.  Shared by the SCF and dftatom_poisson_increment.
+static void poisson_increment(int path, const GridDev& g, const PoissonLevels& lv, bool stream, const StreamPlan& splan, WarmPoissonArgs ca,
+                              const PoissonArgs& pa, const StreamSolveArgs& sa, double* d_src, double* d_u, int n_vcycles, cudaStream_t st,
+                              long long& n_launch)
+{
+    const int n_dens = ca.n_dens;
+    const long long ldU = ca.ldU;
+    ca.work = pa.work;
+    if (path == kIncDirect) {
+        ca.scratch = d_u; ca.scratch_stride = ldU;
+        launch_poisson_direct(g, ca, st);
+        ++n_launch;
+    } else if (path == kIncWarmVcycles) {
+        ca.n_vcycles = n_vcycles;
+        launch_poisson_warm(g, ca, pa.phi, pa.src, lv.total, st);
+        ++n_launch;
+    } else {
+        // increment form around the existing solvers: dS, dU = 0 -> V-cycles on (dS, dU) with zero boundary values -> U += dU
+        launch_poisson_delta_prepare(g, n_dens, ldU, ca.rho, ca.rho_prev, d_src, d_u, ca.skip, ca.skip_stride_bytes, st);
+        if (stream) {
+            StreamSolveArgs sd = sa;
+            sd.rho = nullptr; sd.src0 = d_src; sd.U = d_u; sd.Zbc = nullptr; sd.warm = 1; sd.n_v = n_vcycles;
+            long long nl = 0;
+            launch_poisson_stream_solve(splan, g.delta, sd, st, &nl);
+            n_launch += nl;
+        } else {
+            PoissonArgs pd = pa;
+            pd.rho = nullptr; pd.src_nat = d_src; pd.u_out = d_u; pd.nat_stride = ldU == g.N ? 0 : ldU; pd.Zbc = nullptr; pd.warm_vcycles = n_vcycles;
+            // (team mode keeps Phi_0 in place in the hierarchy between warm solves: it must start from the zero increment too)
+            cudaMemsetAsync(pa.phi, 0, sizeof(double) * (size_t)n_dens * lv.total, st);
+            launch_poisson_full(g, lv, pd, st);
+            ++n_launch;
+        }
+        launch_poisson_delta_apply(g, n_dens, ldU, ca.U, d_u, ca.skip, ca.skip_stride_bytes, st);
+        n_launch += 2;
+    }
+}
+
 // one group of atoms: its whole SCF, enqueued on the context's stream (pg: pseudo-atoms, opts[a].Z = their Z_b)
 static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftatom_config* cfgs, int n_atoms, dftatom_result* out,
                        dftatom_step* steps, int steps_stride, const RadialDest* rd = nullptr, const PseudoGroup* pg = nullptr)
@@ -658,7 +703,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     xa.max_vcycles = 100;                                       // PoissonSolver.h:117
     WarmPoissonArgs ca{};
     ca.n_dens = n_atoms; ca.rho = b.rhot; ca.rho_stride = N; ca.U = b.U; ca.ldU = ldU; ca.Zbc = b.Zbc; ca.coarse_tri = g.coarse_tri;
-    ca.skip = &b.astate[0].done; ca.skip_stride_bytes = (int)sizeof(AtomState);
+    ca.skip = &b.astate[0].done; ca.skip_stride_bytes = (int)sizeof(AtomState); ca.rho_prev = c->rho_prev.as<double>();
     StreamSolveArgs sa{};
     sa.n_dens = n_atoms; sa.rho = b.rhot; sa.rho_stride = N; sa.psrc = g.psrc; sa.src0 = c->stream_src0.as<double>(); sa.U = b.U; sa.ld0 = ldU;
     sa.Zbc = b.Zbc; sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op; sa.variant = c->k.stream_variant;
@@ -676,33 +721,9 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
         if (exact) {
             launch_poisson_exact(xa, st);
             ++n_launch;
-        } else if (warm && direct_ok && cur_step >= c->k.direct_after) {
-            ca.work = pa.work; ca.rho_prev = rho_prev; ca.scratch = d_u; ca.scratch_stride = ldU;
-            launch_poisson_direct(g, ca, st);
-            ++n_launch;
-        } else if (warm && warm_ok) {
-            ca.n_vcycles = warm_vcycles; ca.work = pa.work; ca.rho_prev = rho_prev;
-            launch_poisson_warm(g, ca, pa.phi, pa.src, lv.total, st);
-            ++n_launch;
         } else if (warm && delta) {
-            // increment form around the existing solvers: dS, dU = 0 -> V-cycles on (dS, dU) with zero boundary values -> U += dU
-            launch_poisson_delta_prepare(g, n_atoms, ldU, b.rhot, rho_prev, d_src, d_u, skip_p, skip_stride, st);
-            if (stream) {
-                StreamSolveArgs sd = sa;
-                sd.rho = nullptr; sd.src0 = d_src; sd.U = d_u; sd.Zbc = nullptr; sd.warm = 1; sd.n_v = warm_vcycles;
-                long long nl = 0;
-                launch_poisson_stream_solve(splan, g.delta, sd, st, &nl);
-                n_launch += nl;
-            } else {
-                PoissonArgs pd = pa;
-                pd.rho = nullptr; pd.src_nat = d_src; pd.u_out = d_u; pd.nat_stride = ldU == N ? 0 : ldU; pd.Zbc = nullptr; pd.warm_vcycles = warm_vcycles;
-                // (team mode keeps Phi_0 in place in the hierarchy between warm solves: it must start from the zero increment too)
-                cudaMemsetAsync(pa.phi, 0, sizeof(double) * (size_t)n_atoms * lv.total, st);
-                launch_poisson_full(g, lv, pd, st);
-                ++n_launch;
-            }
-            launch_poisson_delta_apply(g, n_atoms, ldU, b.U, d_u, skip_p, skip_stride, st);
-            n_launch += 2;
+            const int path = direct_ok && cur_step >= c->k.direct_after ? kIncDirect : warm_ok ? kIncWarmVcycles : kIncColdForm;
+            poisson_increment(path, g, lv, stream, splan, ca, pa, sa, d_src, d_u, warm_vcycles, st, n_launch);
         } else if (stream) {
             sa.warm = warm; sa.n_v = warm ? warm_vcycles : c->k.max_vcycles;
             long long nl = 0;
@@ -1776,6 +1797,59 @@ int dftatom_poisson_solve(dftatom_ctx* c, int levels, double delta, double max_r
     else DFT_CHECK(cudaMemcpyAsync(U, c->ubuf.p, sizeof(double) * (size_t)n_dens * N, cudaMemcpyDeviceToHost, st));
     if (vcycles_used && streamed) for (int k = 0; k < n_dens; ++k) vcycles_used[k] = c->k.max_vcycles;
     else if (vcycles_used) DFT_CHECK(cudaMemcpyAsync(vcycles_used, dv.p, sizeof(int) * n_dens, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int dftatom_poisson_increment(dftatom_ctx* c, int levels, double delta, double max_r, int n_dens, const double* rho, double* rho_prev,
+                              double* U, const int* skip, int solver, int n_vcycles)
+{
+    if (!c || !rho || !rho_prev || !U || n_dens <= 0 || n_dens > 65535) { set_error("bad argument"); return DFTATOM_E_ARG; }
+    if (levels < 8 || levels > 20) { set_error("levels must be in 8..20 (the SCF's range)"); return DFTATOM_E_BAD_OPTION; }
+    if (solver < kIncDirect || solver > kIncColdForm) { set_error("solver must be 0 (direct), 1 (warm V-cycles) or 2 (increment form around the cold solvers)"); return DFTATOM_E_ARG; }
+    if (solver != kIncDirect && (n_vcycles < 1 || n_vcycles > 1000)) { set_error("n_vcycles must be in 1..1000"); return DFTATOM_E_ARG; }
+    if (c->k.poisson_exact || c->k.refine_vcycles || c->k.floor_stop) { set_error("the SCF solves no increment with poisson_exact, refine_vcycles or floor_stop set"); return DFTATOM_E_ARG; }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
+    const PoissonLevels lv = make_levels(levels);
+    // the SCF's choices for a batch of n_dens atoms (solve_group)
+    const bool stream = c->k.stream_poisson && n_dens >= c->k.stream_min_dens && levels >= c->k.stream_min_levels && levels > c->k.stream_mid_levels;
+    const long long ldU = stream ? ((N + 3) & ~3) : N;
+    if (solver == kIncDirect && g.coarse_direct == nullptr) { set_error("the direct solve needs 11..20 levels"); return DFTATOM_E_ARG; }
+    if (solver == kIncWarmVcycles && (stream || !poisson_warm_supported(levels, delta) || g.coarse_tri == nullptr || (long long)lv.total < poisson_warm_scratch_doubles(levels))) {
+        set_error("the warm V-cycle kernel needs 11..14 levels, delta > 0 and no stream-mode solver");
+        return DFTATOM_E_ARG;
+    }
+    const StreamPlan splan = stream ? make_stream_plan(levels, n_dens, c->k.stream_mid_levels) : StreamPlan{};
+    const size_t nN = (size_t)n_dens * N, nL = (size_t)n_dens * ldU;
+    DevBuf& dr = c->scratch[0]; DevBuf& dp = c->scratch[1]; DevBuf& ds = c->scratch[2];
+    if ((rc = dr.ensure(sizeof(double) * nN)) || (rc = dp.ensure(sizeof(double) * nN)) || (rc = ds.ensure(sizeof(int) * n_dens))
+        || (rc = c->ubuf.ensure(sizeof(double) * nL)) || (rc = c->d_src.ensure(sizeof(double) * nL)) || (rc = c->d_u.ensure(sizeof(double) * nL))
+        || (rc = c->phi.ensure(sizeof(double) * (size_t)n_dens * lv.total)) || (rc = c->src.ensure(sizeof(double) * (size_t)n_dens * lv.total))
+        || (rc = c->team_bar.ensure(sizeof(unsigned) * (size_t)n_dens))) return rc;
+    if (stream && (rc = c->stream_scratch.ensure(sizeof(double) * (size_t)splan.total))) return rc;
+    DFT_CHECK(cudaMemcpyAsync(dr.p, rho, sizeof(double) * nN, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dp.p, rho_prev, sizeof(double) * nN, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpy2DAsync(c->ubuf.p, sizeof(double) * ldU, U, sizeof(double) * N, sizeof(double) * N, n_dens, cudaMemcpyHostToDevice, st));
+    if (skip) DFT_CHECK(cudaMemcpyAsync(ds.p, skip, sizeof(int) * n_dens, cudaMemcpyHostToDevice, st));
+    // the arguments solve_group sets (the skip flags here: one int per density)
+    PoissonArgs pa{};
+    pa.n_dens = n_dens; pa.phi = c->phi.as<double>(); pa.src = c->src.as<double>(); pa.coarse_op = g.coarse_op;
+    pa.skip = skip ? ds.as<int>() : nullptr; pa.skip_stride_bytes = (int)sizeof(int);
+    pa.max_vcycles = c->k.max_vcycles; pa.u0 = c->u0.as<double>(); pa.n_sm = c->n_sm;
+    pa.team_bar = c->k.team_poisson ? c->team_bar.as<unsigned>() : nullptr;
+    WarmPoissonArgs ca{};
+    ca.n_dens = n_dens; ca.rho = dr.as<double>(); ca.rho_stride = N; ca.rho_prev = dp.as<double>(); ca.U = c->ubuf.as<double>(); ca.ldU = ldU;
+    ca.coarse_tri = g.coarse_tri; ca.skip = pa.skip; ca.skip_stride_bytes = pa.skip_stride_bytes;
+    StreamSolveArgs sa{};
+    sa.n_dens = n_dens; sa.rho_stride = N; sa.psrc = g.psrc; sa.ld0 = ldU; sa.scratch = c->stream_scratch.as<double>(); sa.coarse_op = g.coarse_op;
+    sa.variant = c->k.stream_variant; sa.skip = pa.skip; sa.skip_stride_bytes = pa.skip_stride_bytes;
+    long long nl = 0;
+    poisson_increment(solver, g, lv, stream, splan, ca, pa, sa, c->d_src.as<double>(), c->d_u.as<double>(), n_vcycles, st, nl);
+    DFT_CHECK(cudaMemcpy2DAsync(U, sizeof(double) * N, c->ubuf.p, sizeof(double) * ldU, sizeof(double) * N, n_dens, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaMemcpyAsync(rho_prev, dp.p, sizeof(double) * nN, cudaMemcpyDeviceToHost, st));
     DFT_CHECK(cudaStreamSynchronize(st));
     DFT_CHECK(cudaGetLastError());
     return 0;

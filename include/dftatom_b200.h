@@ -448,6 +448,19 @@ int dftatom_grid_nodes(dftatom_ctx* ctx, int levels, double delta, double max_r,
  * electron count as a double; Z[k] is converted exactly) */
 int dftatom_poisson_solve(dftatom_ctx* ctx, int levels, double delta, double max_r, int n_dens, const int* Z,
                           const double* rho, double* U, int* vcycles_used);
+/* One warm Poisson solve of the SCF in increment form for n_dens densities on the grid (levels 8..20, delta, max_r; delta = 0: uniform):
+ *     -a dU_{i-1} + dU_i - b dU_{i+1} = psrc_i (rho_i - rho_prev_i) / 2,   a = (1 + delta/2)/2,  b = (1 - delta/2)/2,  dU_0 = dU_{N-1} = 0,
+ * then U += dU and rho_prev = rho (psrc_i = r_i 4 pi K_i, the source factor of dftatom_poisson_solve).  rho[n_dens][N]; rho_prev[n_dens][N] and
+ * U[n_dens][N] are in / out.  skip (optional, [n_dens]): a density with skip[k] != 0 is left untouched.  solver selects the path the SCF takes:
+ *   0  the direct solve (poisson_direct.cu: Thomas algorithm as block scans; 11..20 levels), the SCF's from step "direct_after" on;
+ *   1  n_vcycles V-cycles of the warm kernel (poisson_warm.cu; 11..14 levels, delta > 0), the SCF's earlier warm steps there;
+ *   2  n_vcycles V-cycles of the cold solvers on the increment (poisson_delta_prepare, poisson_full_kernel or - under the SCF's condition
+ *      for a batch of n_dens atoms - the stream-mode solver, poisson_delta_apply), the SCF's warm steps everywhere else.
+ * With the launches and arguments of the SCF (the same code); a component entry point for tests.  DFTATOM_E_ARG where the SCF never runs
+ * that solver (solver 0 below 11 levels, solver 1 outside 11..14 levels, on the uniform grid or in stream mode, any solver with
+ * "poisson_exact", "refine_vcycles" or "floor_stop" set), for NULL pointers and for n_vcycles outside 1..1000 (solvers 1, 2). */
+int dftatom_poisson_increment(dftatom_ctx* ctx, int levels, double delta, double max_r, int n_dens, const double* rho, double* rho_prev,
+                              double* U, const int* skip, int solver, int n_vcycles);
 /* n_cycles reference-shaped V-cycles (PoissonSolver.h:155-159) in place on phi[n_dens][N] with source src[n_dens][N] */
 int dftatom_poisson_vcycles(dftatom_ctx* ctx, int levels, double delta, int n_dens, double* phi, const double* src,
                             int n_cycles, double* last_err);

@@ -17,7 +17,7 @@ def _potential(kind, Z, r):
 
 
 @pytest.mark.parametrize("kind,L,delta,rmax,Z", [("coulomb", 12, 0.001, 15.0, 18), ("screened", 13, 0.0008, 30.0, 64),
-                                                 ("coulomb", 10, 0.004, 15.0, 92)])
+                                                 ("coulomb", 10, 0.004, 15.0, 92), ("screened", 20, 1.25e-5, 50.0, 36)])
 def test_numerov_lanes_match_oracle(ctx, kind, L, delta, rmax, Z):
     """(sign y0, node count) of SolutionInZero / CountNodes: bit-exact except where |y0| is at its rounding floor."""
     N, rp, r = O.grid(L, delta, rmax)
@@ -32,11 +32,13 @@ def test_numerov_lanes_match_oracle(ctx, kind, L, delta, rmax, Z):
     sign, lg, cnt = ctx.numerov_lanes(V, L, delta, rmax, ls, Es, lim, impl=1)
     assert np.array_equal(cnt, cnt_o)
     assert np.array_equal(sign, (y0 > 0).astype(np.int32))
-    np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=1e-6)     # |y0| to ~1e-6 relative (1e15 guard needs a factor 2)
+    # |y0| to ~1e-6 relative (1e15 guard needs a factor 2); at 1048577 nodes the rounding of the longer sweep: 4.4e-6 measured on a B200
+    atol = 1e-6 if L <= 17 else 1e-5
+    np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=atol)
     # production tile-staged sweep: same y0, and the full Sturm count (all sign changes, no early exit)
     sign, lg, cnt = ctx.numerov_lanes(V, L, delta, rmax, ls, Es, lim, impl=0)
     assert np.array_equal(sign, (y0 > 0).astype(np.int32))
-    np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=1e-6)
+    np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=atol)
     assert np.array_equal(cnt, O.numerov_count_all(V, delta, rmax, ls, Es))
     # the same through the parallel-in-r sweep (cluster per 32 lanes, 8 / 32 radial segments)
     try:
@@ -44,7 +46,7 @@ def test_numerov_lanes_match_oracle(ctx, kind, L, delta, rmax, Z):
             ctx.set_option("r_segments", segs)
             sign, lg, cnt = ctx.numerov_lanes(V, L, delta, rmax, ls, Es, lim, impl=2)
             assert np.array_equal(sign, (y0 > 0).astype(np.int32))
-            np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=1e-6)
+            np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=atol)
             assert np.array_equal(cnt, O.numerov_count_all(V, delta, rmax, ls, Es))
     finally:
         ctx.set_option("r_segments", -1)
@@ -52,7 +54,7 @@ def test_numerov_lanes_match_oracle(ctx, kind, L, delta, rmax, Z):
     for impl in (4, 5, 6):
         sign, lg, cnt = ctx.numerov_lanes(V, L, delta, rmax, ls, Es, lim, impl=impl)
         assert np.array_equal(sign, (y0 > 0).astype(np.int32)), impl
-        np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=1e-6)
+        np.testing.assert_allclose(lg, np.log2(np.abs(y0)), atol=atol)
         assert np.array_equal(cnt, O.numerov_count_all(V, delta, rmax, ls, Es)), impl
 
 
@@ -100,7 +102,8 @@ def test_level_search_matches_oracle(ctx, kind, L, delta, rmax, Z):
         np.testing.assert_allclose(E_g, [-Z * Z / (2.0 * n * n) for n in ns], atol=5e-5)
 
 
-@pytest.mark.parametrize("L,delta,rmax,Z", [(12, 0.001, 15.0, 18), (16, 0.0002, 50.0, 30), (17, 0.0001, 50.0, 86)])
+@pytest.mark.parametrize("L,delta,rmax,Z", [(12, 0.001, 15.0, 18), (16, 0.0002, 50.0, 30), (17, 0.0001, 50.0, 86), (18, 5e-5, 50.0, 54),
+                                         (20, 1.25e-5, 50.0, 92)])
 def test_orbital_matches_oracle(ctx, L, delta, rmax, Z):
     """Two-sided matched + normalised solution (Numerov.h:403-504, DFTAtom.cpp:36-56).  16, 17 levels: the grid does not fit
     in shared memory and the production kernel works through it window by window (match_win_kernel)."""
@@ -116,12 +119,14 @@ def test_orbital_matches_oracle(ctx, L, delta, rmax, Z):
             u_g, mp_g = ctx.numerov_orbital(V, L, delta, rmax, l, E)
             ctx.set_option("match_mode", 0)
             assert abs(mp_g - mp_o) <= (0 if mode == 1 else 1)      # the match point is an argmax: rounding may move it by one node
-            # rounding accumulates with the number of nodes: 2e-10 observed at 131073 nodes (relative 1e-10)
-            np.testing.assert_allclose(u_g, u_o, rtol=0, atol=1e-10 if L <= 14 else 1e-9)
+            # rounding accumulates with the number of nodes: 2e-10 observed at 131073 nodes (relative 1e-10); measured on a B200:
+            # 4.8e-10 at 262145 nodes, 3.0e-9 at 1048577
+            np.testing.assert_allclose(u_g, u_o, rtol=0, atol=1e-10 if L <= 14 else 1e-9 if L <= 18 else 1e-8)
 
 
 @pytest.mark.parametrize("L,delta,rmax,stream", [(10, 0.004, 15.0, 0), (14, 0.0005, 25.0, 0), (16, 0.0002, 50.0, 0), (14, 0.0005, 25.0, 1),
-                                                 (15, 0.0004, 50.0, 1), (16, 0.0002, 50.0, 1), (17, 0.0001, 50.0, 1)])
+                                                 (15, 0.0004, 50.0, 1), (16, 0.0002, 50.0, 1), (17, 0.0001, 50.0, 1), (18, 5e-5, 50.0, 0),
+                                                 (18, 5e-5, 50.0, 1), (20, 1.25e-5, 50.0, 0), (20, 1.25e-5, 50.0, 1)])
 def test_poisson_matches_oracle_and_analytic(ctx, L, delta, rmax, stream):
     """U(r) of FMG + V-cycles vs the reference algorithm (oracle, 100 V-cycles) and vs the analytic Hartree potential.
     stream: the solver for many densities on grids beyond the chip (poisson_stream.cu) instead of one CTA / team per density."""
@@ -142,9 +147,12 @@ def test_poisson_matches_oracle_and_analytic(ctx, L, delta, rmax, stream):
     for j, (Z, k) in enumerate(zip(Zs, a)):
         U_o, errs = O.poisson(L, delta, rmax, Z, rho[j], max_vcycles=100 if L <= 14 else 12)
         U_x = Z * (1 - np.exp(-2 * k * r) * (1 + k * r))
-        # both are the same discrete solution up to their FP64 rounding floors (SURVEY fact 3: 7e-10 at L=14)
-        assert np.max(np.abs(U[j] - U_o)) < 2e-9 * max(1, Z) * (4 if L > 14 else 1)
-        assert abs(np.max(np.abs(U[j] - U_x)) - np.max(np.abs(U_o - U_x))) < 1e-8 * Z
+        # both are the same discrete solution up to their FP64 rounding floors (SURVEY fact 3: 7e-10 at L=14), which grow like
+        # eps N^1.5: above 17 levels the bars of 17 levels scaled so.  Measured on a B200, per unit of Z: 4.8e-9 at 18 levels, 4.7e-8 at 20
+        # (bars 2.3e-8, 1.8e-7); the gap to the analytic potential 2.1e-9 at 18, 4.1e-8 at 20 (bars 2.8e-8, 2.3e-7)
+        grow = max(1.0, (N / 131073.0) ** 1.5)
+        assert np.max(np.abs(U[j] - U_o)) < 2e-9 * max(1, Z) * (4 if L > 14 else 1) * grow
+        assert abs(np.max(np.abs(U[j] - U_x)) - np.max(np.abs(U_o - U_x))) < 1e-8 * Z * grow
         assert U[j][0] == 0.0 and U[j][-1] == Z
 
 
@@ -291,7 +299,7 @@ def test_poisson_uniform_grid_matches_oracle(ctx, L, rmax):
 
 
 @pytest.mark.parametrize("L,delta,rmax", [(8, 0.02, 10.0), (10, 0.004, 15.0), (14, 0.0005, 25.0), (16, 0.0002, 50.0), (17, 0.0001, 50.0),
-                                          (12, 0.0, 15.0), (14, 0.0, 25.0)])
+                                          (18, 5e-5, 50.0), (20, 1.25e-5, 50.0), (12, 0.0, 15.0), (14, 0.0, 25.0)])
 def test_poisson_exact_mode_is_bit_identical(ctx, L, delta, rmax):
     """set_option("poisson_exact", 1): the reference's FullCycle (Initialize, FMG ramp with its 1e-3 early exits, 100 V-cycles) in the
     reference's own floating-point operation order (PoissonSolver.cpp:40-157, .h:51-124), chunk-parallel with a 128-node warm-up halo:

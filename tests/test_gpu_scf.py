@@ -379,6 +379,35 @@ def test_radon_c2_every_step(ctx):
     np.testing.assert_allclose(res.steps[n_ref - 1].E[0], readme, rtol=0, atol=EIG_TOL + 5e-7)
 
 
+@pytest.mark.parametrize("case", ["H_L18", "He_L19", "Li_L20", "batch_L18"])
+def test_fine_grids_every_step(ctx, case):
+    """18 .. 20 levels (262145 .. 1048577 nodes; the reference's dialog offers up to 20): the first steps of the SCF against the C
+    restatement oracle (tests/golden/fine_grid.json, scripts/make_fine_grid_fixture.py: the reference itself does not stop within its cap
+    here, so no stop step is compared).  One or three atoms: cold Poisson solves by one team of CTAs per density; the batch of four: the
+    stream solver.  Eigenvalues at 1e-6 Ha and energies at 1e-5 Ha, unless the fixture shows that the oracle's own Poisson floor at this
+    size (100 against 12 V-cycles per solve) is not that precise (then: twice that floor)."""
+    atoms = golden("fine_grid")["cases"][case]
+    n = atoms[0]["n_steps"]
+    ctx.set_option("run_to_cap", 1)
+    ctx.set_option("step_cap", n)
+    try:
+        res = ctx.solve_batch([_opt(a["options"]) for a in atoms])
+    finally:
+        ctx.set_option("run_to_cap", 0)
+        ctx.set_option("step_cap", 0)
+    for r, a in zip(res, atoms):
+        eig_tol = EIG_TOL if a["floor_eig"] <= 0.5 * EIG_TOL else 2.0 * a["floor_eig"]
+        en_tol = ENERGY_TOL if a["floor_energy"] <= 0.5 * ENERGY_TOL else 2.0 * a["floor_energy"]
+        assert r.n_steps == a["n_steps"] == n
+        assert [(L.n, L.l, L.occ) for chan in r.levels for L in chan] == [(x["n"], x["l"], x["occ"]) for x in a["levels"]]
+        for k in range(n):
+            s = r.steps[k]
+            np.testing.assert_allclose([x for chan in s.E for x in chan], a["eig_per_step"][k], rtol=0, atol=eig_tol,
+                                       err_msg=f"{case} Z={a['options']['Z']} step {k}")
+            for j, key in enumerate(KEYS):
+                assert abs(getattr(s, key) - a["energies_per_step"][k][j]) <= en_tol, (case, a["options"]["Z"], k, key)
+
+
 def test_radon_c2_default_path(ctx):
     """C2 on the production path (8 V-cycles, FMA, warm start): eigenvalues at 1e-6 Ha at every step, shell structure exact; the
     energies are reported (bench.py `parity`) and must stay within the reference's own reproducibility (fixture-derived)."""
