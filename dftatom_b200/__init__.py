@@ -14,6 +14,7 @@ from .api import (  # noqa: F401
     Level,
     LogDerivatives,
     Options,
+    PartialCore,
     Pseudopotential,
     Radial,
     Result,
@@ -33,7 +34,7 @@ from .api import (  # noqa: F401
 from .report import format_report, parse_report  # noqa: F401
 
 __all__ = [
-    "Context", "DFTAtom", "DFTAtomError", "KleinmanBylander", "Level", "LogDerivatives", "Options", "Pseudopotential", "Radial", "Result", "Step", "aufbau", "split_spin", "n_nodes",
+    "Context", "DFTAtom", "DFTAtomError", "KleinmanBylander", "Level", "LogDerivatives", "Options", "PartialCore", "Pseudopotential", "Radial", "Result", "Step", "aufbau", "split_spin", "n_nodes",
     "lib_path", "load_library", "format_report", "parse_report", "estimate_cost", "partition", "orbital_count",
     "config_aufbau", "parse_config", "format_config",
 ]

@@ -79,6 +79,15 @@ class _CKbLdChannel(C.Structure):
     _fields_ = [("pot", C.c_int), ("proj", C.c_int), ("l", C.c_int), ("pad", C.c_int), ("E_KB", C.c_double), ("r_c", C.c_double)]
 
 
+class _CCoreOrbital(C.Structure):
+    _fields_ = [("row", C.c_int), ("orbital", C.c_int), ("occ", C.c_double)]
+
+
+class _CPccResult(C.Structure):
+    _fields_ = [("r_pc", C.c_double), ("A", C.c_double), ("B", C.c_double), ("n_core", C.c_double), ("n_pc", C.c_double),
+                ("i_pc", C.c_int), ("status", C.c_int), ("pad", C.c_int)]
+
+
 class _COccupation(C.Structure):
     _fields_ = [("n", C.c_int), ("l", C.c_int), ("spin", C.c_int), ("occ", C.c_double)]
 
@@ -140,12 +149,16 @@ def load_library():
                                                C.POINTER(_CStep), C.c_int, C.POINTER(_CRadial)]
     lib.dftatom_solve_pseudo_batch.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, C.POINTER(_CPseudoAtom),
                                                C.POINTER(_CConfig), C.c_int, C.POINTER(_CResult), C.POINTER(_CStep), C.c_int, C.POINTER(_CRadial)]
+    lib.dftatom_solve_pseudo_batch_core.argtypes = lib.dftatom_solve_pseudo_batch.argtypes + [_dp, C.c_int, _ip]
     lib.dftatom_radial_moments.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp]
     lib.dftatom_log_derivatives.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _ip, _ip, _dp, C.c_int, _dp, C.c_int,
                                             C.POINTER(_CLogDeriv), _dp]
     lib.dftatom_grid_nodes.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp]
     lib.dftatom_tm_pseudize.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp, C.c_int, C.POINTER(_CTmChannel), C.c_int,
                                         C.POINTER(_CTmResult), _dp, _dp, _dp, _dp]
+    lib.dftatom_tm_pseudize_core.argtypes = lib.dftatom_tm_pseudize.argtypes + [_dp]
+    lib.dftatom_partial_core.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, C.POINTER(_CCoreOrbital), C.c_int, _dp,
+                                         C.c_int, C.POINTER(_CPccResult), _dp, _dp]
     lib.dftatom_kb_form.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, _dp, C.c_int, C.POINTER(_CKbChannel), C.c_int,
                                     C.POINTER(_CKbResult), _dp]
     lib.dftatom_kb_log_derivatives.argtypes = [C.c_void_p, C.c_int, C.c_double, C.c_double, _dp, C.c_int, _dp, C.c_int, C.POINTER(_CKbLdChannel),
@@ -366,6 +379,27 @@ class Pseudopotential:
     pot: np.ndarray
     grid: Optional[tuple] = None        # (levels, delta, max_r) of the call, delta = 0: the uniform grid
     n: Optional[np.ndarray] = None
+    rho_core: Optional[np.ndarray] = None   # [n_pot][N] core density (Context.pseudize with r_pc)
+    rho_pc: Optional[np.ndarray] = None     # [n_pot][N] partial core the unscreening used; solve_pseudo_batch solves with it
+    core: Optional["PartialCore"] = None    # the partial core's parameters (Context.pseudize with r_pc)
+
+
+@dataclass
+class PartialCore:
+    """Core densities and their Louie-Froyen-Cohen partial cores (Context.partial_core; definition: dftatom_partial_core in
+    include/dftatom_b200.h).  Per row ([n_rows]): r_pc (the node radius used, 0 = full core), i_pc, A, B (rho_pc = A sin(B r) / r inside
+    r_pc), n_core, n_pc (electrons in rho_core / rho_pc), status (0 ok, 1 the core density does not decrease at r_pc: NaN rows);
+    rho_core, rho_pc: [n_rows][N]; r: [N] the grid."""
+    r_pc: np.ndarray
+    i_pc: np.ndarray
+    A: np.ndarray
+    B: np.ndarray
+    n_core: np.ndarray
+    n_pc: np.ndarray
+    status: np.ndarray
+    rho_core: np.ndarray
+    rho_pc: np.ndarray
+    r: np.ndarray
 
 
 @dataclass
@@ -653,7 +687,8 @@ class Context:
         parse_config strings or entry lists ((n, l, occ) for LDA, (n, l, spin, occ) for LSDA), broadcast against pseudos.  All pseudos
         share one grid (the logarithmic grid).  Returns one Result per pseudo-atom: levels with the all-electron n and nodes = n - n_ref,
         Eenuc = E_ion, Ecoul = E_H, Exc, Ekin and Etotal as documented there; options = Options(Z = round(z_val), the grid, mixing,
-        method, config = the entries).  radial=True: Result.radial with V = the screening V_H + V_xc per spin."""
+        method, config = the entries).  radial=True: Result.radial with V = the screening V_H + V_xc per spin.  A pseudopotential with
+        rho_pc (unscreened with a partial core) is solved with that core (dftatom_solve_pseudo_batch_core); batches may mix both kinds."""
         pseudos = list(pseudos) if isinstance(pseudos, (list, tuple)) else [pseudos]
         one = isinstance(configs, str) or (len(configs) > 0 and all(isinstance(e, (list, tuple)) and len(e) in (3, 4)
                                                                      and not isinstance(e[0], (list, tuple, str)) for e in configs))
@@ -667,6 +702,7 @@ class Context:
             raise DFTAtomError("solve_pseudo_batch: every Pseudopotential must come from Context.tm_pseudize on one grid")
         levels, delta, max_r = grid
         rows, row_of, catoms = [], {}, (_CPseudoAtom * n)()
+        pc_rows, pc_of, pc_row = [], {}, np.full(n, -1, dtype=np.int32)
         for a, pp in enumerate(pseudos):
             if pp.n is None:
                 raise DFTAtomError(f"solve_pseudo_batch: pseudopotential {a} has no reference principal numbers (Pseudopotential.n)")
@@ -682,6 +718,14 @@ class Context:
             for c, l in enumerate(pp.l.tolist()):
                 catoms[a].row[l] = base + c
                 catoms[a].n_ref[l] = int(pp.n[c])
+            if pp.rho_pc is not None:
+                pots = set(np.asarray(pp.pot).tolist())
+                if len(pots) != 1:
+                    raise DFTAtomError(f"solve_pseudo_batch: pseudopotential {a} with a core has channels on several potential rows")
+                if key not in pc_of:
+                    pc_of[key] = len(pc_rows)
+                    pc_rows.append(np.asarray(pp.rho_pc)[pots.pop()])
+                pc_row[a] = pc_of[key]
             catoms[a].z_val = float(np.sum(pp.occ))
             catoms[a].mixing = float(mixing)
             catoms[a].method = int(method)
@@ -698,8 +742,14 @@ class Context:
         stride = MAX_STEPS_LSDA if method & 1 else MAX_STEPS_LDA
         csteps = (_CStep * (n * stride))() if keep_steps else None
         views, crad = _radial_buffers(n, V.shape[1], sum(len(e) for e in entries)) if radial else (None, None)
-        _check(self._lib.dftatom_solve_pseudo_batch(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], catoms, ccfg, n, cres,
-                                                    csteps, stride if keep_steps else 0, C.byref(crad) if radial else None))
+        if pc_rows:
+            PC = _f64(np.array(pc_rows))
+            _check(self._lib.dftatom_solve_pseudo_batch_core(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], catoms, ccfg, n,
+                                                             cres, csteps, stride if keep_steps else 0, C.byref(crad) if radial else None,
+                                                             _d(PC), PC.shape[0], _i(pc_row)))
+        else:
+            _check(self._lib.dftatom_solve_pseudo_batch(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], catoms, ccfg, n,
+                                                        cres, csteps, stride if keep_steps else 0, C.byref(crad) if radial else None))
         options = [Options(int(round(catoms[a].z_val)), int(levels), float(max_r), float(delta), float(mixing), int(method),
                            config=_as_method_form(entries[a], method)) for a in range(n)]
         return _decode(options, entries, cres, csteps, stride, views)
@@ -842,13 +892,17 @@ class Context:
         out = out.reshape(nc, ne)
         return LogDerivatives(out["D"].copy(), out["u"].copy(), out["du"].copy(), out["nodes"].copy(), used, E.copy())
 
-    def tm_pseudize(self, V, u, levels, delta, max_r, pot, orbital, l, eps, occ, r_c, n=None) -> Pseudopotential:
+    def tm_pseudize(self, V, u, levels, delta, max_r, pot, orbital, l, eps, occ, r_c, n=None, rho_pc=None) -> Pseudopotential:
         """Troullier-Martins pseudization and unscreening (dftatom_tm_pseudize).  V: [n_pot][N] potentials, u: [n_orb][N] all-electron
         orbitals (one row of either may be given as [N]), e.g. rows of Result.radial.V and Result.radial.orbitals; channel c = (V row pot[c],
         u row orbital[c], l[c], eigenvalue eps[c], occupation occ[c], radius r_c[c] in bohr), broadcast against each other.  The channels
         sharing a potential row are one pseudo-atom for the unscreening.  n (optional, broadcast likewise): the all-electron principal
-        number of every channel's reference state, kept as Pseudopotential.n."""
+        number of every channel's reference state, kept as Pseudopotential.n.  rho_pc (optional, [n_pot][N]): a partial core density per
+        potential row; the unscreening then removes V_xc(rho_val + rho_pc) (dftatom_tm_pseudize_core), kept as Pseudopotential.rho_pc."""
         V = _f64(np.atleast_2d(V)); u = _f64(np.atleast_2d(u))
+        pc = None if rho_pc is None else _f64(np.atleast_2d(rho_pc))
+        if pc is not None and pc.shape != V.shape:
+            raise ValueError(f"tm_pseudize: rho_pc has shape {pc.shape}, V {V.shape}")
         pot, orbital, l, eps, occ, r_c = np.broadcast_arrays(*(np.atleast_1d(x) for x in (pot, orbital, l, eps, occ, r_c)))
         nc, N = len(pot), V.shape[1]
         ch = np.zeros(nc, dtype=np.dtype(_CTmChannel))
@@ -856,18 +910,42 @@ class Context:
         res = np.zeros(nc, dtype=np.dtype(_CTmResult))
         u_ps, v_scr, v_ion = (np.zeros((nc, N)) for _ in range(3))
         rho = np.zeros((V.shape[0], N))
-        _check(self._lib.dftatom_tm_pseudize(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], _d(u), u.shape[0],
-                                             ch.ctypes.data_as(C.POINTER(_CTmChannel)), nc, res.ctypes.data_as(C.POINTER(_CTmResult)),
-                                             _d(u_ps), _d(v_scr), _d(v_ion), _d(rho)))
+        _check(self._lib.dftatom_tm_pseudize_core(self._h, int(levels), float(delta), float(max_r), _d(V), V.shape[0], _d(u), u.shape[0],
+                                                  ch.ctypes.data_as(C.POINTER(_CTmChannel)), nc, res.ctypes.data_as(C.POINTER(_CTmResult)),
+                                                  _d(u_ps), _d(v_scr), _d(v_ion), _d(rho), None if pc is None else _d(pc)))
         rr = np.zeros(N)                                    # the engine's node radii
         _check(self._lib.dftatom_grid_nodes(self._h, int(levels), float(delta), float(max_r), _d(rr)))
         nn = None if n is None else _i32(np.broadcast_to(np.atleast_1d(n), (nc,))).copy()
         return Pseudopotential(_i32(l).copy(), _f64(eps).copy(), _f64(occ).copy(), res["r_c"].copy(), res["c"].copy(), res["q"].copy(),
-                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy(), (int(levels), float(delta), float(max_r)), nn)
+                               res["status"].copy(), rr, u_ps, v_scr, v_ion, rho, _i32(pot).copy(), (int(levels), float(delta), float(max_r)), nn,
+                               None, None if pc is None else pc.copy())
 
-    def pseudize(self, result, r_c) -> Pseudopotential:
+    def partial_core(self, u, levels, delta, max_r, row, orbital, occ, r_pc) -> PartialCore:
+        """Core densities and Louie-Froyen-Cohen partial cores (dftatom_partial_core).  u: [n_orb][N] all-electron orbitals; core entry k =
+        (output row row[k], u row orbital[k], occupation occ[k]), broadcast against each other; r_pc: [n_rows] radii (0 = the full core),
+        one per output row."""
+        u = _f64(np.atleast_2d(u))
+        r_pc = _f64(np.atleast_1d(r_pc))
+        row, orbital, occ = np.broadcast_arrays(*(np.atleast_1d(x) for x in (row, orbital, occ)))
+        nr, N = len(r_pc), u.shape[1]
+        ce = np.zeros(len(row), dtype=np.dtype(_CCoreOrbital))
+        ce["row"], ce["orbital"], ce["occ"] = row, orbital, occ
+        res = np.zeros(nr, dtype=np.dtype(_CPccResult))
+        rho_core, rho_pc = np.zeros((nr, N)), np.zeros((nr, N))
+        _check(self._lib.dftatom_partial_core(self._h, int(levels), float(delta), float(max_r), _d(u), u.shape[0],
+                                              ce.ctypes.data_as(C.POINTER(_CCoreOrbital)), len(ce), _d(r_pc), nr,
+                                              res.ctypes.data_as(C.POINTER(_CPccResult)), _d(rho_core), _d(rho_pc)))
+        rr = np.zeros(N)
+        _check(self._lib.dftatom_grid_nodes(self._h, int(levels), float(delta), float(max_r), _d(rr)))
+        return PartialCore(res["r_pc"].copy(), res["i_pc"].copy(), res["A"].copy(), res["B"].copy(), res["n_core"].copy(), res["n_pc"].copy(),
+                           res["status"].copy(), rho_core, rho_pc, rr)
+
+    def pseudize(self, result, r_c, r_pc=None) -> Pseudopotential:
         """Pseudopotentials of a solved LDA atom (Result of solve_batch(..., radial=True)): for every l of result.levels[0] the level of
-        largest n is the valence channel, with its eigenvalue and occupation.  r_c: one radius, a sequence indexed by l, or a dict {l: r_c}."""
+        largest n is the valence channel, with its eigenvalue and occupation.  r_c: one radius, a sequence indexed by l, or a dict {l: r_c}.
+        r_pc (optional; 0 = the full core): unscreen with the nonlinear core correction, the partial core of the other (core) levels at
+        r_pc (Context.partial_core); the result carries rho_core, rho_pc and core.  DFTAtomError when the core density does not decrease at
+        r_pc (no partial core there)."""
         o = result.options
         if result.radial is None:
             raise ValueError("pseudize needs the radial state: solve with radial=True")
@@ -886,8 +964,18 @@ class Context:
             rcs = [r_c[l] for l in ls]
         lev = [result.levels[0][best[l]] for l in ls]
         rad = result.radial
-        return self.tm_pseudize(rad.V[0], rad.orbitals[0], o.MultigridLevels, 0.0 if o.method >= 2 else o.deltaGrid, o.MaxR, 0,
-                                [best[l] for l in ls], ls, [x.E for x in lev], [float(x.occ) for x in lev], rcs, [x.n for x in lev])
+        grid = (o.MultigridLevels, 0.0 if o.method >= 2 else o.deltaGrid, o.MaxR)
+        pc = None
+        if r_pc is not None:
+            core = [k for k, x in enumerate(result.levels[0]) if k not in best.values()]
+            pc = self.partial_core(rad.orbitals[0], *grid, 0, core, [float(result.levels[0][k].occ) for k in core], [float(r_pc)])
+            if pc.status[0] != 0:
+                raise DFTAtomError(f"pseudize: the core density does not decrease at r_pc = {pc.r_pc[0]!r}: no partial core there")
+        pp = self.tm_pseudize(rad.V[0], rad.orbitals[0], *grid, 0, [best[l] for l in ls], ls, [x.E for x in lev], [float(x.occ) for x in lev],
+                              rcs, [x.n for x in lev], rho_pc=None if pc is None else pc.rho_pc)
+        if pc is not None:
+            pp.rho_core, pp.core = pc.rho_core, pc
+        return pp
 
     def kb_form(self, V, u, levels, delta, max_r, row, loc, l, eps) -> KleinmanBylander:
         """Kleinman-Bylander form and GSS ghost test (dftatom_kb_form).  V: [n_rows][N] screened potentials, u: [n_rows][N] pseudo-orbitals

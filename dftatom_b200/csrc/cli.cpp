@@ -36,6 +36,11 @@
 //           each of them (the core: every reference entry whose n is below its channel's reference n, or whose l has no channel).
 //           DIR/<index>_Z<Z>_pseudo_test.tsv: one row per configuration (config Q E_AE E_PS dE_AE dE_PS dE_PS-dE_AE status_AE status_PS;
 //           dE against the reference configuration), then one "# level" line per level (config n l spin occ eps_AE eps_PS).
+// --pseudo-core R: with --pseudo, the nonlinear core correction: the core density of the atom's other (core) levels, its Louie-Froyen-
+//           Cohen partial core at radius R (0 = the full core, dftatom_partial_core), and the unscreening with it
+//           (dftatom_tm_pseudize_core); --pseudo-test then solves the pseudo-atoms with it (dftatom_solve_pseudo_batch_core).  The pseudo
+//           table gains a "# core" line (r_pc i_pc A B n_core n_pc status) after the channel and kb lines and the columns rho_core and
+//           rho_pc after the others.
 #include <algorithm>
 #include <cmath>
 #include <cctype>
@@ -286,7 +291,8 @@ static int write_logderiv(dftatom_ctx* ctx, const std::string& dir, int index, c
 // --pseudo-test: the pseudo-atom of the channels ch (rows of v_ion) against the all-electron atom in the reference configuration and in
 // every configuration of `tests`
 static int pseudo_test(dftatom_ctx* ctx, const std::string& path, const dftatom_options& o, const dftatom_result& R, const dftatom_config* cfg,
-                       const std::vector<dftatom_tm_channel>& ch, const std::vector<double>& v_ion, const std::vector<std::string>& tests)
+                       const std::vector<dftatom_tm_channel>& ch, const std::vector<double>& v_ion, const std::vector<std::string>& tests,
+                       const std::vector<double>& rho_pc)
 {
     dftatom_pseudo_atom pa = {};
     for (int l = 0; l < 4; ++l) pa.row[l] = -1;
@@ -326,8 +332,9 @@ static int pseudo_test(dftatom_ctx* ctx, const std::string& path, const dftatom_
     std::vector<dftatom_pseudo_atom> pas(n, pa);
     std::vector<dftatom_options> opts(n, o);
     std::vector<dftatom_result> r_ps(n), r_ae(n);
-    if (dftatom_solve_pseudo_batch(ctx, o.levels, o.delta, o.max_r, v_ion.data(), (int)ch.size(), pas.data(), ps.data(), n, r_ps.data(), nullptr, 0,
-                                   nullptr) != DFTATOM_OK ||
+    const std::vector<int> pc_row(n, 0);          // with --pseudo-core every pseudo-atom takes the one partial core row
+    if (dftatom_solve_pseudo_batch_core(ctx, o.levels, o.delta, o.max_r, v_ion.data(), (int)ch.size(), pas.data(), ps.data(), n, r_ps.data(), nullptr, 0,
+                                        nullptr, rho_pc.empty() ? nullptr : rho_pc.data(), 1, rho_pc.empty() ? nullptr : pc_row.data()) != DFTATOM_OK ||
         dftatom_solve_batch_config(ctx, opts.data(), ae.data(), n, r_ae.data(), nullptr, 0, nullptr) != DFTATOM_OK) {
         std::fprintf(stderr, "dftatom: --pseudo-test Z=%d: %s\n", o.Z, dftatom_last_error());
         return 1;
@@ -362,7 +369,7 @@ static int pseudo_test(dftatom_ctx* ctx, const std::string& path, const dftatom_
 static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::string& ld_dir, int index, const dftatom_options& o,
                         const dftatom_result& R, const dftatom_config* cfg, int N, const double* r, const double* v, const double* orb,
                         const std::vector<double>& rcs, double ld_rc, const std::vector<double>& E, int kb_loc,
-                        const std::vector<std::string>& tests)
+                        const std::vector<std::string>& tests, double r_pc)
 {
     int best[4] = { -1, -1, -1, -1 };
     for (int k = 0; k < R.n_levels[0]; ++k) {
@@ -381,8 +388,23 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
     const int nc = (int)ch.size();
     std::vector<dftatom_tm_result> out(nc);
     std::vector<double> u_ps((size_t)nc * N), v_scr((size_t)nc * N), v_ion((size_t)nc * N), rho(N);
-    if (dftatom_tm_pseudize(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v, 1, orb, R.n_levels[0], ch.data(), nc, out.data(), u_ps.data(),
-                            v_scr.data(), v_ion.data(), rho.data()) != DFTATOM_OK) {
+    // --pseudo-core: the partial core of the levels that are not valence channels
+    const bool with_core = !std::isnan(r_pc);
+    dftatom_pcc_result pcc = {};
+    std::vector<double> rho_core(with_core ? N : 0), rho_pc(with_core ? N : 0);
+    if (with_core) {
+        std::vector<dftatom_core_orbital> core;
+        for (int k = 0; k < R.n_levels[0]; ++k)
+            if (k != best[R.levels[0][k].l]) core.push_back(dftatom_core_orbital{ 0, k, exact_occ(R.levels[0][k], 0, cfg) });
+        if (dftatom_partial_core(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, orb, R.n_levels[0], core.data(), (int)core.size(), &r_pc, 1, &pcc,
+                                 rho_core.data(), rho_pc.data()) != DFTATOM_OK) {
+            std::fprintf(stderr, "dftatom: --pseudo-core Z=%d: %s\n", o.Z, dftatom_last_error());
+            return 1;
+        }
+        if (pcc.status != 0) { std::fprintf(stderr, "dftatom: --pseudo-core Z=%d: the core density does not decrease at r_pc = %.17g\n", o.Z, pcc.r_pc); return 1; }
+    }
+    if (dftatom_tm_pseudize_core(ctx, o.levels, o.method >= 2 ? 0. : o.delta, o.max_r, v, 1, orb, R.n_levels[0], ch.data(), nc, out.data(), u_ps.data(),
+                                 v_scr.data(), v_ion.data(), rho.data(), with_core ? rho_pc.data() : nullptr) != DFTATOM_OK) {
         std::fprintf(stderr, "dftatom: --pseudo Z=%d: %s\n", o.Z, dftatom_last_error());
         return 1;
     }
@@ -412,11 +434,14 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
     for (size_t c = 0; c < kb.size(); ++c)
         std::fprintf(f, "# kb\t%d\t%.17g\t%.17g\t%.17g\t%.17g\t%d\t%d\n", ch[c].l, kb[c].E_KB, kb[c].cos, kb[c].eps_loc[0], kb[c].eps_loc[1], kb[c].ghost,
                      kb[c].status);
+    if (with_core)
+        std::fprintf(f, "# core\t%.17g\t%d\t%.17g\t%.17g\t%.17g\t%.17g\t%d\n", pcc.r_pc, pcc.i_pc, pcc.A, pcc.B, pcc.n_core, pcc.n_pc, pcc.status);
     std::fprintf(f, "# r");
     for (const char* q : { "V_ion", "V_scr", "u" })
         for (int c = 0; c < nc; ++c) std::fprintf(f, "\t%s %c", q, kOrb[ch[c].l]);
     std::fprintf(f, "\trho_val");
     for (size_t c = 0; c < kb.size(); ++c) std::fprintf(f, "\tbeta %c", kOrb[ch[c].l]);
+    if (with_core) std::fprintf(f, "\trho_core\trho_pc");
     std::fprintf(f, "\n");
     for (int i = 0; i < N; ++i) {
         std::fprintf(f, "%.17g", r[i]);
@@ -424,12 +449,13 @@ static int write_pseudo(dftatom_ctx* ctx, const std::string& dir, const std::str
             for (int c = 0; c < nc; ++c) std::fprintf(f, "\t%.17g", (*q)[(size_t)c * N + i]);
         std::fprintf(f, "\t%.17g", rho[i]);
         for (size_t c = 0; c < kb.size(); ++c) std::fprintf(f, "\t%.17g", beta[c * N + i]);
+        if (with_core) std::fprintf(f, "\t%.17g\t%.17g", rho_core[i], rho_pc[i]);
         std::fprintf(f, "\n");
     }
     bool bad = std::ferror(f) != 0;
     if (std::fclose(f) != 0 || bad) { std::fprintf(stderr, "dftatom: write error on %s\n", path.c_str()); return 1; }
     if (!tests.empty()) {
-        const int rc_t = pseudo_test(ctx, dir + stem + "_test.tsv", o, R, cfg, ch, v_ion, tests);
+        const int rc_t = pseudo_test(ctx, dir + stem + "_test.tsv", o, R, cfg, ch, v_ion, tests, rho_pc);
         if (rc_t) return rc_t;
     }
     if (ld_dir.empty()) return 0;
@@ -487,7 +513,7 @@ int main(int argc, char** argv)
     dftatom_options base = { 36, 12, 10.0, 0.001, 0.5, 0 };     // Options.cpp:6
     std::vector<int> zs, atom_index;                        // atom_index: positions of this shard's atoms in the parent's --Z list (--gpus children)
     std::string radial_dir, config_str, logderiv_dir, energies = "-2:1:301", pseudo_dir, pseudo_rc, pseudo_test;
-    double charge = 0., rc = NAN;
+    double charge = 0., rc = NAN, pseudo_core = NAN;
     int pseudo_local = -1;
     int precision = 6, device = 0, gpus = 1;
     bool json = false, quiet = false, framed = false;      // framed: child of --gpus (one frame per atom on stdout)
@@ -512,6 +538,14 @@ int main(int argc, char** argv)
             if (v.size() != 1 || v[0] < '0' || v[0] > '3') { std::fprintf(stderr, "dftatom: --pseudo-local expects l = 0, 1, 2 or 3, got '%s'\n", v.c_str()); return 2; }
             pseudo_local = v[0] - '0';
         }
+        else if (a == "--pseudo-core") {
+            const std::string v = next();
+            char* end = nullptr;
+            pseudo_core = std::strtod(v.c_str(), &end);
+            if (v.empty() || *end || !std::isfinite(pseudo_core) || pseudo_core < 0.) {
+                std::fprintf(stderr, "dftatom: --pseudo-core expects a radius >= 0 in bohr (0 = the full core), got '%s'\n", v.c_str()); return 2;
+            }
+        }
         else if (a == "--charge") charge = std::atof(next());
         else if (a == "--config") config_str = next();
         else if (a == "--levels") base.levels = std::atoi(next());
@@ -531,7 +565,8 @@ int main(int argc, char** argv)
         else if (a == "--help" || a == "-h") {
             std::printf("usage: dftatom [--Z 18|1-92|a,b,c] [--levels L] [--delta d] [--mixing a] [--rmax R] [--method 0|1] "
                         "[--precision p] [--json] [--quiet-steps] [--device k] [--gpus N] [--ini file] [--radial DIR] [--charge Q] [--config \"...\"]\n"
-                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf] [--pseudo-local L] [--pseudo-test \"C1;C2\"]]\n"
+                        "               [--logderiv DIR --rc R [--energies lo:hi:n]] [--pseudo DIR --pseudo-rc Rs[,Rp,Rd,Rf] [--pseudo-local L] [--pseudo-test \"C1;C2\"]\n"
+                        "               [--pseudo-core R]]\n"
                         "  --radial DIR  write the converged r, rho, V, V_H and orbitals u(r) of every atom to DIR/<index>_Z<Z>.tsv\n"
                         "  --charge Q    solve every atom of --Z ionised by Q electrons (the reference's configuration; fractional allowed, < 0 = anion)\n"
                         "  --config C    solve one atom (a single --Z) in configuration C, e.g. \"[Ar] 3d10\", \"1s2 2s2 2p4.5\", LSDA \"[He] 2s1 2p3/1\"\n"
@@ -546,7 +581,9 @@ int main(int argc, char** argv)
                         "                eps_loc0 eps_loc1 ghost status) and beta columns; with --logderiv also <index>_Z<Z>_pseudo_kb_logderiv.tsv\n"
                         "  --pseudo-test \"C1;C2\"  with --pseudo and a single --Z: solve the pseudo-atom in the reference valence configuration and in\n"
                         "                each valence configuration Ck (e.g. \"3s1 3p3;3s2 3p1\"), the all-electron atom in core + each, and write\n"
-                        "                <index>_Z<Z>_pseudo_test.tsv (config Q E_AE E_PS dE_AE dE_PS dE_PS-dE_AE statuses, then eps_AE / eps_PS per level)\n");
+                        "                <index>_Z<Z>_pseudo_test.tsv (config Q E_AE E_PS dE_AE dE_PS dE_PS-dE_AE statuses, then eps_AE / eps_PS per level)\n"
+                        "  --pseudo-core R  nonlinear core correction of --pseudo: unscreen with the partial core of the other levels at R bohr (0 = the\n"
+                        "                full core); --pseudo-test solves with it; adds a \"# core\" line and rho_core, rho_pc columns\n");
             return 0;
         } else { std::fprintf(stderr, "unknown flag %s\n", a.c_str()); return 2; }
         if (a != "--Z" && a != "--gpus" && a != "--device" && a != "--framed" && a != "--atom-index") for (int q = i_flag; q <= i; ++q) passthrough.push_back(argv[q]);
@@ -567,6 +604,7 @@ int main(int argc, char** argv)
     }
     std::vector<double> ps_rc;
     if (pseudo_local >= 0 && pseudo_dir.empty()) { std::fprintf(stderr, "dftatom: --pseudo-local needs --pseudo DIR\n"); return 2; }
+    if (!std::isnan(pseudo_core) && pseudo_dir.empty()) { std::fprintf(stderr, "dftatom: --pseudo-core needs --pseudo DIR\n"); return 2; }
     std::vector<std::string> ps_tests;
     if (!pseudo_test.empty()) {
         if (pseudo_dir.empty() || zs.size() != 1) { std::fprintf(stderr, "dftatom: --pseudo-test needs --pseudo DIR and a single --Z\n"); return 2; }
@@ -661,7 +699,7 @@ int main(int argc, char** argv)
         }
     for (int a = 0; a < n && !pseudo_dir.empty(); ++a)
         if (write_pseudo(ctx, pseudo_dir, logderiv_dir, atom_index.empty() ? a : atom_index[a], opts[a], res[a], configured ? &cfgs[a] : nullptr, N,
-                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E, pseudo_local, ps_tests)) {
+                         r_grid.data(), &vks[(size_t)a * 2 * N], &orb[(size_t)row0[a] * N], ps_rc, rc, ld_E, pseudo_local, ps_tests, pseudo_core)) {
             dftatom_destroy(ctx); return 1;
         }
 

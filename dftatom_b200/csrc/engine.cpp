@@ -131,6 +131,7 @@ struct dftatom_ctx {
     DevBuf scratch[8];
     DevBuf radial, radial_part, radial_ticket;     // export of the radial state (dftatom_solve_batch_radial): staging, partial sums, tickets
     DevBuf pseudo_atoms, pseudo_v;                 // dftatom_solve_pseudo_batch: per-atom channel rows, the ionic potentials
+    DevBuf pseudo_pc, pseudo_pc_row;               // dftatom_solve_pseudo_batch_core: partial core rows, the row of each atom
     int* h_active = nullptr;       // pinned
     char* h_up = nullptr; size_t h_up_cap = 0, h_up_used = 0;      // pinned staging of the descriptor uploads of one solve (reset at its start)
     // timing of the last solve
@@ -327,7 +328,7 @@ void dftatom_destroy(dftatom_ctx* c)
     for (DevBuf* b : all) b->release();
     for (DevBuf& b : c->scratch) b.release();
     c->radial.release(); c->radial_part.release(); c->radial_ticket.release();
-    c->pseudo_atoms.release(); c->pseudo_v.release();
+    c->pseudo_atoms.release(); c->pseudo_v.release(); c->pseudo_pc.release(); c->pseudo_pc_row.release();
     c->stream_G.release(); c->stream_src0.release(); c->stream_scratch.release(); c->exact_work.release(); c->last_steps.release(); c->rho_prev.release(); c->d_src.release(); c->d_u.release();
     if (c->h_active) cudaFreeHost(c->h_active);
     if (c->h_up) cudaFreeHost(c->h_up);
@@ -505,6 +506,8 @@ static int export_radial(dftatom_ctx* c, const GridDev& g, const ScfBuffers& b, 
 struct PseudoGroup {
     const double* v_ion; int n_rows;
     const dftatom_pseudo_atom* atoms;
+    const double* rho_pc; int n_pc_rows;      // partial cores (dftatom_solve_pseudo_batch_core); NULL when no atom has one
+    const int* pc_row;                        // [n_atoms], -1 = none (only read with rho_pc)
 };
 
 // The three ways of a warm Poisson solve in increment form (selected by solve_group's poisson_solve; dftatom_poisson_increment's `solver`)
@@ -632,7 +635,9 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     c->last_h2d_bytes = (long long)(sizeof(AtomDev) * atoms.size() + sizeof(AtomState) * astate.size() + sizeof(OrbitalDev) * orbs.size()
                                     + sizeof(int) * (tab_of.size() + 2) + sizeof(double) * zbc.size());
 
-    const size_t pseudo_bytes = pg ? sizeof(PseudoAtomDev) * patoms.size() + sizeof(double) * (size_t)pg->n_rows * N : 0;
+    const bool core = pg && pg->rho_pc;
+    const size_t pseudo_bytes = pg ? sizeof(PseudoAtomDev) * patoms.size() + sizeof(double) * (size_t)pg->n_rows * N
+                                     + (core ? sizeof(double) * (size_t)pg->n_pc_rows * N + sizeof(int) * (size_t)n_atoms : 0) : 0;
 
     // ---- device buffers ----
     if ((rc = upload_arena_reset(c, (size_t)c->last_h2d_bytes + pseudo_bytes + 64 * 8))) return rc;
@@ -649,7 +654,7 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     if ((rc = c->psi.ensure(sizeof(double) * (size_t)n_orbs * N))) return rc;
     if ((rc = c->match_pt.ensure(sizeof(int) * (size_t)n_orbs))) return rc;
     if ((rc = c->inv_norm.ensure(sizeof(double) * (size_t)n_orbs))) return rc;
-    if ((rc = c->epart.ensure(sizeof(double) * (size_t)n_atoms * 64 * 5)) || (rc = c->eticket.ensure(sizeof(int) * (size_t)n_atoms))) return rc;
+    if ((rc = c->epart.ensure(sizeof(double) * (size_t)n_atoms * 64 * (core ? 6 : 5))) || (rc = c->eticket.ensure(sizeof(int) * (size_t)n_atoms))) return rc;
     DFT_CHECK(cudaMemsetAsync(c->eticket.p, 0, sizeof(int) * (size_t)n_atoms, st));
     if ((rc = c->phi.ensure(sizeof(double) * (size_t)n_atoms * lv.total))) return rc;
     if ((rc = c->src.ensure(sizeof(double) * (size_t)n_atoms * lv.total))) return rc;
@@ -673,6 +678,11 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
         if ((rc = upload(c, c->pseudo_atoms, patoms))) return rc;
         if ((rc = upload(c, c->pseudo_v, std::vector<double>(pg->v_ion, pg->v_ion + (size_t)pg->n_rows * N)))) return rc;
         pargs.atoms = c->pseudo_atoms.as<PseudoAtomDev>(); pargs.v_ion = c->pseudo_v.as<double>();
+        if (core) {
+            if ((rc = upload(c, c->pseudo_pc, std::vector<double>(pg->rho_pc, pg->rho_pc + (size_t)pg->n_pc_rows * N)))) return rc;
+            if ((rc = upload(c, c->pseudo_pc_row, std::vector<int>(pg->pc_row, pg->pc_row + n_atoms)))) return rc;
+            pargs.rho_pc = c->pseudo_pc.as<double>(); pargs.pc_row = c->pseudo_pc_row.as<int>();
+        }
         c->last_h2d_bytes += (long long)pseudo_bytes;
     }
     DFT_CHECK(cudaMemsetAsync(c->steps.p, 0, sizeof(dftatom_step) * (size_t)n_atoms * stride, st));
@@ -1134,6 +1144,15 @@ int dftatom_solve_pseudo_batch(dftatom_ctx* c, int levels, double delta, double 
                                const dftatom_pseudo_atom* atoms, const dftatom_config* configs, int n_atoms, dftatom_result* out,
                                dftatom_step* steps, int steps_stride, const dftatom_radial* radial)
 {
+    return dftatom_solve_pseudo_batch_core(c, levels, delta, max_r, v_ion, n_rows, atoms, configs, n_atoms, out, steps, steps_stride, radial,
+                                           nullptr, 0, nullptr);
+}
+
+int dftatom_solve_pseudo_batch_core(dftatom_ctx* c, int levels, double delta, double max_r, const double* v_ion, int n_rows,
+                                    const dftatom_pseudo_atom* atoms, const dftatom_config* configs, int n_atoms, dftatom_result* out,
+                                    dftatom_step* steps, int steps_stride, const dftatom_radial* radial, const double* rho_pc,
+                                    int n_pc_rows, const int* pc_row)
+{
     if (!c || !v_ion || !atoms || !configs || !out) { set_error("dftatom_solve_pseudo_batch: NULL argument"); return DFTATOM_E_ARG; }
     if (n_rows < 1 || n_atoms < 1) { set_error("dftatom_solve_pseudo_batch: n_rows and n_atoms must be >= 1"); return DFTATOM_E_ARG; }
     if (delta == 0.) { set_error("dftatom_solve_pseudo_batch: the uniform grid (delta = 0) is not supported"); return DFTATOM_E_BAD_OPTION; }
@@ -1193,6 +1212,22 @@ int dftatom_solve_pseudo_batch(dftatom_ctx* c, int levels, double delta, double 
         while (zb <= 118 && -(double)zb * zb - 1. > vmin - 10.) ++zb;
         if (zb > 118) { set_error(where(a) + "ionic potential too deep (min V_ion = " + std::to_string(vmin) + " below -118^2 + 9)"); return DFTATOM_E_BAD_OPTION; }
         o.Z = zb;
+        if (pc_row && (pc_row[a] < -1 || pc_row[a] >= (rho_pc ? n_pc_rows : 0))) {
+            set_error(where(a) + "pc_row = " + std::to_string(pc_row[a]) + " outside -1.." + std::to_string((rho_pc ? n_pc_rows : 0) - 1));
+            return DFTATOM_E_BAD_OPTION;
+        }
+    }
+    bool any_core = false;
+    for (int a = 0; pc_row && a < n_atoms; ++a) any_core |= pc_row[a] >= 0;
+    if (any_core) {
+        for (int q = 0; q < n_pc_rows; ++q)
+            for (int i = 1; i < N; ++i) {
+                const double x = rho_pc[(size_t)q * N + i];
+                if (!(std::isfinite(x) && x >= 0.)) {
+                    set_error("dftatom_solve_pseudo_batch: rho_pc row " + std::to_string(q) + " is not finite or negative at node " + std::to_string(i));
+                    return DFTATOM_E_BAD_OPTION;
+                }
+            }
     }
     std::vector<int> dest_atom;
     std::vector<long long> dest_row;
@@ -1205,7 +1240,7 @@ int dftatom_solve_pseudo_batch(dftatom_ctx* c, int levels, double delta, double 
         for (int a = 0; a < n_atoms; ++a) { dest_atom.push_back(a); dest_row.push_back(rows); rows += configs[a].n_orbitals; }
     }
     const RadialDest rd{ radial, dest_atom.data(), dest_row.data(), true };
-    const PseudoGroup pg{ v_ion, n_rows, atoms };
+    const PseudoGroup pg{ v_ion, n_rows, atoms, any_core ? rho_pc : nullptr, any_core ? n_pc_rows : 0, pc_row };
     return solve_group(c, opts.data(), configs, n_atoms, out, steps, steps_stride, radial ? &rd : nullptr, &pg);
 }
 
@@ -1389,6 +1424,13 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
                         const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
                         double* v_ion, double* rho_val)
 {
+    return dftatom_tm_pseudize_core(c, levels, delta, max_r, V, n_pot, u, n_orb, ch, n_channels, out, u_ps, v_scr, v_ion, rho_val, nullptr);
+}
+
+int dftatom_tm_pseudize_core(dftatom_ctx* c, int levels, double delta, double max_r, const double* V, int n_pot, const double* u, int n_orb,
+                             const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
+                             double* v_ion, double* rho_val, const double* rho_pc)
+{
     if (!c || !V || !u || !ch || !out) { set_error("dftatom_tm_pseudize: NULL argument"); return DFTATOM_E_ARG; }
     if (n_pot < 1 || n_orb < 1 || n_channels < 1) { set_error("dftatom_tm_pseudize: n_pot, n_orb and n_channels must be >= 1"); return DFTATOM_E_ARG; }
     DFT_CHECK(cudaSetDevice(c->device));
@@ -1408,6 +1450,11 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
     for (int o = 0; o < n_orb; ++o)
         for (int i = 1; i < N; ++i)
             if (!std::isfinite(u[(size_t)o * N + i])) { set_error(where("orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    for (int p = 0; rho_pc && p < n_pot; ++p)
+        for (int i = 1; i < N; ++i) {
+            const double x = rho_pc[(size_t)p * N + i];
+            if (!(std::isfinite(x) && x >= 0.)) { set_error(where("rho_pc row", p) + "not finite or negative at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+        }
     std::vector<int> ic(n_channels);
     std::vector<unsigned> l_taken(n_pot, 0u);             // per potential row: bit l set once a channel takes l
     for (int k = 0; k < n_channels; ++k) {
@@ -1463,7 +1510,7 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
     h_dbl.insert(h_dbl.end(), zbc.begin(), zbc.end());
     const size_t nV = (size_t)n_pot * N, nU = (size_t)n_orb * N, nC = (size_t)n_channels * N;
     DevBuf& dD = c->scratch[0]; DevBuf& dI = c->scratch[1]; DevBuf& dR = c->scratch[2]; DevBuf& dv = c->scratch[3];
-    const size_t n_dbl = 6 * nV + nU + 3 * nC + h_dbl.size();      // V atab rho rho_out vxc edif | u | u_ps v_scr v_ion | eps occ zbc
+    const size_t n_dbl = 6 * nV + nU + 3 * nC + h_dbl.size() + (rho_pc ? 2 * nV : 0);      // V atab rho rho_out vxc edif | u | u_ps v_scr v_ion | eps occ zbc | rho_pc rho_xc
     if ((rc = dD.ensure(sizeof(double) * n_dbl)) || (rc = dI.ensure(sizeof(int) * h_int.size())) || (rc = dR.ensure(sizeof(dftatom_tm_result) * n_channels)) ||
         (rc = dv.ensure(sizeof(int) * n_pot))) return rc;
     double* d = dD.as<double>();
@@ -1474,6 +1521,8 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
     DFT_CHECK(cudaMemcpyAsync(du, u, sizeof(double) * nU, cudaMemcpyHostToDevice, st));
     DFT_CHECK(cudaMemcpyAsync(dh, h_dbl.data(), sizeof(double) * h_dbl.size(), cudaMemcpyHostToDevice, st));
     DFT_CHECK(cudaMemcpyAsync(dI.p, h_int.data(), sizeof(int) * h_int.size(), cudaMemcpyHostToDevice, st));
+    double* dpc = dh + h_dbl.size(); double* dxc = dpc + nV;
+    if (rho_pc) DFT_CHECK(cudaMemcpyAsync(dpc, rho_pc, sizeof(double) * nV, cudaMemcpyHostToDevice, st));
     launch_build_atab(g, dV, dA, n_pot, st);
     const size_t nc = (size_t)n_channels;
     TmArgs ta{ dV, dA, du, di, di + nc, di + 2 * nc, di + 3 * nc, dh, di + 4 * nc, n_channels, dR.as<dftatom_tm_result>(), dups, dvscr };
@@ -1486,7 +1535,12 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
         if ((rc = poisson_cold(c, g, n_solve, drho, dh + 2 * nc, dv.as<int>(), &ld, &streamed))) return rc;
         ra.U = c->ubuf.as<double>(); ra.ldU = ld;
     }
-    launch_vwn((int)nV, drho, nullptr, nullptr, nullptr, dvxc, dedif, st);
+    if (rho_pc) {           // V_xc of rho_val + rho_pc; V_H and rho_out keep reading rho_val
+        launch_core_xc_density(g, n_pot, di + 6 * nc + n_pot + 1, drho, dpc, dxc, st);
+        launch_vwn((int)nV, dxc, nullptr, nullptr, nullptr, dvxc, dedif, st);
+    } else {
+        launch_vwn((int)nV, drho, nullptr, nullptr, nullptr, dvxc, dedif, st);
+    }
     launch_tm_unscreen(g, ra, st);
     DFT_CHECK(cudaGetLastError());
     DFT_CHECK(cudaMemcpyAsync(out, dR.p, sizeof(dftatom_tm_result) * n_channels, cudaMemcpyDeviceToHost, st));
@@ -1494,6 +1548,71 @@ int dftatom_tm_pseudize(dftatom_ctx* c, int levels, double delta, double max_r, 
     if (v_scr) DFT_CHECK(cudaMemcpyAsync(v_scr, dvscr, sizeof(double) * nC, cudaMemcpyDeviceToHost, st));
     if (v_ion) DFT_CHECK(cudaMemcpyAsync(v_ion, dvion, sizeof(double) * nC, cudaMemcpyDeviceToHost, st));
     if (rho_val) DFT_CHECK(cudaMemcpyAsync(rho_val, drho_out, sizeof(double) * nV, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    DFT_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int dftatom_partial_core(dftatom_ctx* c, int levels, double delta, double max_r, const double* u, int n_orb, const dftatom_core_orbital* core,
+                         int n_core, const double* r_pc, int n_rows, dftatom_pcc_result* out, double* rho_core, double* rho_pc)
+{
+    if (!c || !u || !r_pc || !out || (n_core > 0 && !core)) { set_error("dftatom_partial_core: NULL argument"); return DFTATOM_E_ARG; }
+    if (n_orb < 1 || n_rows < 1 || n_core < 0) { set_error("dftatom_partial_core: n_orb and n_rows must be >= 1, n_core >= 0"); return DFTATOM_E_ARG; }
+    DFT_CHECK(cudaSetDevice(c->device));
+    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
+    if (N < 7) { set_error("dftatom_partial_core: the grid needs at least 7 nodes"); return DFTATOM_E_ARG; }
+    if (n_rows > 65535 || (long long)std::max(n_rows, n_orb) * N >= (1LL << 31)) { set_error("dftatom_partial_core: too many rows for one call"); return DFTATOM_E_ARG; }
+    std::vector<double> r(N);
+    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
+    DFT_CHECK(cudaStreamSynchronize(st));
+    const auto where = [](const char* what, long long k) { return std::string("dftatom_partial_core: ") + what + " " + std::to_string(k) + ": "; };
+    std::vector<int> ipc(n_rows, 0);
+    for (int p = 0; p < n_rows; ++p) {
+        const double x = r_pc[p];
+        if (!(std::isfinite(x) && x >= 0.) || (x > 0. && x < r[3]) || x > r[N - 3]) {
+            char b[160];
+            std::snprintf(b, sizeof b, "r_pc = %.17g is neither 0 nor in [r_3, r_(N-3)] = [%.17g, %.17g]", x, r[3], r[N - 3]);
+            set_error(where("row", p) + b); return DFTATOM_E_ARG;
+        }
+        if (x > 0.) ipc[p] = nearest_node(r, x);
+    }
+    std::vector<int> begin(n_rows + 1, 0), orb(n_core);
+    std::vector<double> occ(n_core);
+    for (int k = 0; k < n_core; ++k) {
+        const dftatom_core_orbital& e = core[k];
+        const std::string at = where("core entry", k);
+        if (e.row < 0 || e.row >= n_rows) { set_error(at + "row = " + std::to_string(e.row) + " outside 0.." + std::to_string(n_rows - 1)); return DFTATOM_E_ARG; }
+        if (e.orbital < 0 || e.orbital >= n_orb) { set_error(at + "orbital = " + std::to_string(e.orbital) + " outside 0.." + std::to_string(n_orb - 1)); return DFTATOM_E_ARG; }
+        if (!(e.occ >= 0. && e.occ <= 14.)) { set_error(at + "occ is not finite or outside [0, 14]"); return DFTATOM_E_ARG; }
+        ++begin[e.row + 1];
+    }
+    for (int o = 0; o < n_orb; ++o)
+        for (int i = 1; i < N; ++i)
+            if (!std::isfinite(u[(size_t)o * N + i])) { set_error(where("orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    for (int p = 0; p < n_rows; ++p) begin[p + 1] += begin[p];
+    {
+        std::vector<int> fill(begin.begin(), begin.end() - 1);
+        for (int k = 0; k < n_core; ++k) { const int q = fill[core[k].row]++; orb[q] = core[k].orbital; occ[q] = core[k].occ; }
+    }
+    std::vector<int> h_int(begin);                               // core_begin | core_orb | ipc
+    h_int.insert(h_int.end(), orb.begin(), orb.end());
+    h_int.insert(h_int.end(), ipc.begin(), ipc.end());
+    const size_t nU = (size_t)n_orb * N, nR = (size_t)n_rows * N;
+    DevBuf& dD = c->scratch[0]; DevBuf& dI = c->scratch[1]; DevBuf& dR = c->scratch[2];
+    if ((rc = dD.ensure(sizeof(double) * (nU + 2 * nR + std::max(n_core, 1)))) || (rc = dI.ensure(sizeof(int) * h_int.size())) ||
+        (rc = dR.ensure(sizeof(dftatom_pcc_result) * n_rows))) return rc;
+    double* du = dD.as<double>(); double* dcore = du + nU; double* dpc = dcore + nR; double* docc = dpc + nR;
+    DFT_CHECK(cudaMemcpyAsync(du, u, sizeof(double) * nU, cudaMemcpyHostToDevice, st));
+    if (n_core) DFT_CHECK(cudaMemcpyAsync(docc, occ.data(), sizeof(double) * n_core, cudaMemcpyHostToDevice, st));
+    DFT_CHECK(cudaMemcpyAsync(dI.p, h_int.data(), sizeof(int) * h_int.size(), cudaMemcpyHostToDevice, st));
+    const int* di = dI.as<int>();
+    PcArgs pa{ du, di, di + n_rows + 1, docc, di + n_rows + 1 + n_core, n_rows, dR.as<dftatom_pcc_result>(), dcore, dpc };
+    launch_partial_core(g, pa, st);
+    DFT_CHECK(cudaGetLastError());
+    DFT_CHECK(cudaMemcpyAsync(out, dR.p, sizeof(dftatom_pcc_result) * n_rows, cudaMemcpyDeviceToHost, st));
+    if (rho_core) DFT_CHECK(cudaMemcpyAsync(rho_core, dcore, sizeof(double) * nR, cudaMemcpyDeviceToHost, st));
+    if (rho_pc) DFT_CHECK(cudaMemcpyAsync(rho_pc, dpc, sizeof(double) * nR, cudaMemcpyDeviceToHost, st));
     DFT_CHECK(cudaStreamSynchronize(st));
     DFT_CHECK(cudaGetLastError());
     return 0;

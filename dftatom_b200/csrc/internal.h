@@ -337,9 +337,12 @@ struct PseudoAtomDev {
 struct PseudoArgs {
     const PseudoAtomDev* atoms;     // [n_atoms]
     const double* v_ion;            // [n_rows][N]
+    const double* rho_pc;           // [n_pc_rows][N] partial core densities (dftatom_solve_pseudo_batch_core); NULL: no atom has a core
+    const int* pc_row;              // [n_atoms] rho_pc row of each atom, -1 = none (read only when rho_pc != NULL)
 };
 // V_l,s = V_ion,l + U / r + V_xc,s into every channel row, the energies of dftatom_solve_pseudo_batch and the stop test of
-// potential_energy_kernel; first != 0: only the initial potential
+// potential_energy_kernel; first != 0: only the initial potential.  With p.rho_pc the core-corrected instance runs (V_xc,s of
+// rho_s + rho_pc / 2, one more energy integral: b.epart then needs 6 doubles per atom and node range)
 void launch_pseudo_potential_energy(const GridDev& g, const ScfBuffers& b, const PseudoArgs& p, int first, cudaStream_t st);
 
 // export of the radial state (radial.cu): part / ticket: radial_part_doubles(N, rows) doubles / rows ints (tickets zero before the launch)
@@ -383,6 +386,18 @@ struct TmRowArgs {
 };
 void launch_tm_density(const GridDev& g, const TmRowArgs& a, cudaStream_t st);
 void launch_tm_unscreen(const GridDev& g, const TmRowArgs& a, cudaStream_t st);
+// rho_xc[slot[p]] = rho[slot[p]] + rho_pc[p] for the n_pot potential rows: the V_xc argument of the core-corrected unscreening
+void launch_core_xc_density(const GridDev& g, int n_pot, const int* slot, const double* rho, const double* rho_pc, double* rho_xc, cudaStream_t st);
+// Louie-Froyen-Cohen partial core (pseudo.cu): one CTA per row; the entries of row p are core_orb / core_occ[core_begin[p] ..
+// core_begin[p + 1]); ipc[p] = i_pc (0: the full core)
+struct PcArgs {
+    const double* u;                              // [n_orb][N] all-electron orbitals
+    const int* core_begin; const int* core_orb; const double* core_occ;
+    const int* ipc; int n_rows;
+    dftatom_pcc_result* res;                      // [n_rows]
+    double* rho_core; double* rho_pc;             // [n_rows][N]
+};
+void launch_partial_core(const GridDev& g, const PcArgs& a, cudaStream_t st);
 
 // Kleinman-Bylander form (kb.cu): one CTA per channel; is[c] = i_s of the channel (host: the largest node with V[row] != V[loc])
 struct KbFormArgs {

@@ -9,6 +9,7 @@
 // nodes 0..i_c; the ladder x = 0, -1/2, +1/2, -1, +1, ... is evaluated 8 candidates per round until the first interval (in the
 // order of the definition) with a sign change, which 8-point multisection then shrinks to 1e-13 relative.
 // tm_density_kernel / tm_unscreen_kernel: the valence density of each potential row and V_ion = V_scr - V_H - V_xc per channel.
+// partial_core_kernel (dftatom_partial_core): the core density and its Louie-Froyen-Cohen partial core per row.
 #include "logderiv_sweep.cuh"
 
 namespace dft {
@@ -249,6 +250,98 @@ __global__ void tm_unscreen_kernel(GridDev g, TmRowArgs a)
     }
 }
 
+// Louie-Froyen-Cohen partial core (dftatom_partial_core): one CTA per row.  The threads build rho_core = sum occ u^2 / (4 pi r^2) over
+// the row's core entries at nodes 1..N-2; thread 0 takes the 5-point index derivative at i_pc, t = 1 + r rho' / rho, and the root x of
+// x cos x - t sin x on (0, pi) by bisection to the last bit; then every thread writes its nodes of rho_pc, and n_core / n_pc are reduced
+// in shared memory in a fixed tree order.
+constexpr int kPcThreads = 256;
+__global__ void __launch_bounds__(kPcThreads) partial_core_kernel(GridDev g, PcArgs a)
+{
+    __shared__ double red[2][kPcThreads];
+    __shared__ double sA, sB;
+    __shared__ int s_ok;
+    const int p = blockIdx.x, N = g.N, t = threadIdx.x;
+    const int e0 = a.core_begin[p], e1 = a.core_begin[p + 1], ipc = a.ipc[p];
+    double* __restrict__ rc = a.rho_core + (size_t)p * N;
+    double* __restrict__ rpc = a.rho_pc + (size_t)p * N;
+    for (int i = t; i < N; i += kPcThreads) {
+        double acc = 0.;
+        if (i >= 1 && i <= N - 2)
+            for (int k = e0; k < e1; ++k) {
+                const double u = a.u[(size_t)a.core_orb[k] * N + i];
+                acc = fma(a.core_occ[k] * u, u, acc);
+            }
+        rc[i] = acc * g.inv4pr2[i];
+    }
+    __syncthreads();                      // rho_core is read back below by other threads of the CTA
+    if (t == 0) {
+        dftatom_pcc_result* res = a.res + p;
+        double A = 0., B = 0.;
+        int ok = 1;
+        if (ipc > 0) {
+            const double r = g.r[ipc], rho = rc[ipc];
+            const double di = ((rc[ipc - 2] - 8. * rc[ipc - 1]) + (8. * rc[ipc + 1] - rc[ipc + 2])) / 12.;
+            const double J = g.uniform ? g.h : g.delta * (r + g.rp);
+            const double tt = 1. + r * (di / J) / rho;
+            ok = rho > 0. && tt < 1.;
+            if (ok) {
+                // x cot x falls from 1 to -inf on (0, pi): f = x cos x - t sin x is > 0 left of the root, < 0 right of it
+                double lo = 0., hi = 3.14159265358979323846;
+                for (int it = 0; it < 2000; ++it) {
+                    const double mid = 0.5 * (lo + hi);
+                    if (mid <= lo || mid >= hi) break;
+                    if (mid * cos(mid) - tt * sin(mid) > 0.) lo = mid; else hi = mid;
+                }
+                const double x = 0.5 * (lo + hi);
+                B = x / r; A = rho * r / sin(x);
+            } else {
+                A = nan_value(); B = nan_value();
+            }
+            res->r_pc = r;
+        } else {
+            res->r_pc = 0.;
+        }
+        res->A = A; res->B = B; res->i_pc = ipc; res->status = ok ? 0 : 1;
+        sA = A; sB = B; s_ok = ok;
+    }
+    __syncthreads();
+    const double A = sA, B = sB;
+    const bool ok = s_ok;
+    double nc = 0., np = 0.;
+    for (int i = t; i < N; i += kPcThreads) {
+        const double c = rc[i];
+        double v;
+        if (i == 0) v = 0.;
+        else if (!ok) v = nan_value();
+        else if (i < ipc) { const double r = g.r[i]; v = A * sin(B * r) / r; }
+        else v = c;
+        rpc[i] = v;
+        const double w = g.wjac[i] * (4. * 3.14159265358979323846) * (g.r[i] * g.r[i]);
+        nc = fma(w, c, nc);
+        np = fma(w, v, np);
+    }
+    red[0][t] = nc; red[1][t] = np;
+    __syncthreads();
+    for (int s = kPcThreads / 2; s > 0; s >>= 1) {
+        if (t < s) { red[0][t] += red[0][t + s]; red[1][t] += red[1][t + s]; }
+        __syncthreads();
+    }
+    if (t == 0) { a.res[p].n_core = red[0][0]; a.res[p].n_pc = red[1][0]; a.res[p].pad = 0; }
+}
+
+// the xc argument of the core-corrected unscreening: out[slot[p]] = rho[slot[p]] + rho_pc[p] per potential row (blockIdx.y)
+__global__ void core_xc_density_kernel(int N, const int* slot, const double* rho, const double* rho_pc, double* out)
+{
+    const int p = blockIdx.y;
+    const size_t s = (size_t)slot[p] * N;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) out[s + i] = rho[s + i] + rho_pc[(size_t)p * N + i];
+}
+
+void launch_partial_core(const GridDev& g, const PcArgs& a, cudaStream_t st)
+{
+    partial_core_kernel<<<a.n_rows, kPcThreads, 0, st>>>(g, a);
+}
+
 void launch_tm(const GridDev& g, const TmArgs& a, cudaStream_t st)
 {
     tm_kernel<<<a.n_channels, kTmWarps * 32, 0, st>>>(g, a);
@@ -264,6 +357,11 @@ void launch_tm_density(const GridDev& g, const TmRowArgs& a, cudaStream_t st)
 void launch_tm_unscreen(const GridDev& g, const TmRowArgs& a, cudaStream_t st)
 {
     tm_unscreen_kernel<<<dim3(tm_row_chunks(g.N), a.n_channels + a.n_pot), 256, 0, st>>>(g, a);
+}
+
+void launch_core_xc_density(const GridDev& g, int n_pot, const int* slot, const double* rho, const double* rho_pc, double* rho_xc, cudaStream_t st)
+{
+    core_xc_density_kernel<<<dim3(tm_row_chunks(g.N), n_pot), 256, 0, st>>>(g.N, slot, rho, rho_pc, rho_xc);
 }
 
 }  // namespace dft

@@ -588,10 +588,18 @@ void launch_potential_energy(const GridDev& g, const PoissonLevels& lv, const Sc
 // V_l,s = V_ion,l + U / r + V_xc,s and its a-table; the row tab_of[2 a + s] gets the screening U / r + V_xc,s (the radial export's v).
 // The integrals: E_ion = sum occ <u|V_ion,l|u> and sum occ <u|V_l,s|u> over the orbitals in psi (occ x inv_norm x wjac x u^2), and
 // the xc / Hartree integrals of the density as in the all-electron kernel.
-__global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g, ScfBuffers b, PseudoArgs p, int first)
+// kCore (dftatom_solve_pseudo_batch_core; launched when some atom of the group has a core): an atom with p.pc_row[a] >= 0 takes V_xc,s of
+// rho_s + rho_pc / 2 and the energies of the core-corrected definition - e[1] = sum_s rho_s v_xc,s, e[2] = rho eps_xc - e[1]'s integrand,
+// e[5] = rho_pc eps_xc - so Etotal uses 4 pi (e[2] + e[5]); an atom without a core takes the operations and roundings of the kCore =
+// false instance (its energy tail written out in explicit roundings below), so its records do not depend on the batch.
+// Launch bounds: kCore = false keeps the plain (kPT2) bound (minimum 0 = none: the parent kernel's code, 128 registers); kCore = true
+// asks for 1 CTA per SM, which lets ptxas use 188 registers without spills (at the 128 of 2 CTAs per SM it spills 68 B).
+template <bool kCore>
+__global__ void __launch_bounds__(kPT2, kCore ? 1 : 0) pseudo_potential_energy_kernel(GridDev g, ScfBuffers b, PseudoArgs p, int first)
 {
     DFT_PDL_WAIT();
-    __shared__ double sm[5 * 32];
+    constexpr int NE = kCore ? 6 : 5;
+    __shared__ double sm[NE * 32];
     __shared__ double wgt[2 * DFTATOM_MAX_LEVELS];          // occupation / norm of every orbital
     __shared__ int orb_l[2 * DFTATOM_MAX_LEVELS];
     __shared__ int is_last;
@@ -613,8 +621,10 @@ __global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g
     const double* rt = b.rhot + (size_t)a * N;
     const int ta = b.tab_of[2 * a], tb = b.tab_of[2 * a + 1];
     const double q = g.delta * g.delta * 0.25;
+    const double* pc = nullptr;
+    if (kCore) { const int pr = p.pc_row[a]; if (pr >= 0) pc = p.rho_pc + (size_t)pr * N; }
 
-    double e[5] = { 0., 0., 0., 0., 0. };   // E_ion, exccor, eexcDeriv, hartree, sum occ <u|V_l|u>
+    double e[NE] = {};                      // E_ion, exccor, eexcDeriv, hartree, sum occ <u|V_l|u> (, core exccor)
     const int kPotChunks = (int)gridDim.y;
     const int per = (N + kPotChunks - 1) / kPotChunks;
     const int i0 = blockIdx.y * per, i1 = min(i0 + per, N);
@@ -629,16 +639,29 @@ __global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g
             const double r2d = r * rd;
             double vexc, edif;
             if (at.n_spin == 2) {
-                const XcLsda x = xc_lsda(b.rho[(size_t)ta * N + i], b.rho[(size_t)tb * N + i]);
+                const double ra = b.rho[(size_t)ta * N + i], rb = b.rho[(size_t)tb * N + i];
+                double xa = ra, xb = rb;
+                if (kCore && pc) { const double h = 0.5 * pc[i]; xa += h; xb += h; }
+                const XcLsda x = xc_lsda(xa, xb);
                 S[0] = vh + x.va; S[1] = vh + x.vb;
                 vexc = x.vexc; edif = x.edif;
+                if (kCore && pc) {          // sum_s rho_s v_xc,s is no longer rho vexc
+                    const double sv = ra * x.va + rb * x.vb, rw = r * r * wj;
+                    e[1] = fma(rw, sv, e[1]);
+                    e[2] = fma(rw, rho * (vexc + edif) - sv, e[2]);
+                }
             } else {
-                const XcLda x = xc_lda(rho);
+                const XcLda x = xc_lda((kCore && pc) ? rho + pc[i] : rho);
                 S[0] = vh + x.vexc;
                 vexc = x.vexc; edif = x.edif;
             }
-            e[1] = fma(r2d, vexc, e[1]);
-            e[2] = fma(r2d, edif, e[2]);
+            if (kCore && pc) {
+                e[5] = fma(r * r * wj * pc[i], vexc + edif, e[5]);
+                if (at.n_spin == 1) { e[1] = fma(r2d, vexc, e[1]); e[2] = fma(r2d, edif, e[2]); }
+            } else {
+                e[1] = fma(r2d, vexc, e[1]);
+                e[2] = fma(r2d, edif, e[2]);
+            }
             e[3] = fma(rd, U[i], e[3]);
             if (!first) {
                 const double sq = g.sqex[i];
@@ -666,10 +689,10 @@ __global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g
         }
     }
     if (first) return;
-    block_sum_n<5>(e, sm);
+    block_sum_n<NE>(e, sm);
     if (threadIdx.x == 0) {
-        double* part = b.epart + ((size_t)a * kPotChunks + blockIdx.y) * 5;
-        for (int c = 0; c < 5; ++c) part[c] = e[c];
+        double* part = b.epart + ((size_t)a * kPotChunks + blockIdx.y) * NE;
+        for (int c = 0; c < NE; ++c) part[c] = e[c];
         __threadfence();
         const int ticket = atomicAdd(b.eticket + a, 1);
         is_last = (ticket == kPotChunks - 1);
@@ -677,22 +700,34 @@ __global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g
     }
     __syncthreads();
     if (!is_last) return;
-    if (threadIdx.x < 5) {
+    if (threadIdx.x < NE) {
         __threadfence();
-        const double* part = b.epart + (size_t)a * kPotChunks * 5 + threadIdx.x;
+        const double* part = b.epart + (size_t)a * kPotChunks * NE + threadIdx.x;
         double t = 0.;
-        for (int c = 0; c < kPotChunks; ++c) t += __ldcg(part + c * 5);
+        for (int c = 0; c < kPotChunks; ++c) t += __ldcg(part + c * NE);
         sm[threadIdx.x] = t;
     }
     __syncthreads();
     if (threadIdx.x == 0) {
-        for (int c = 0; c < 5; ++c) e[c] = sm[c];
+        for (int c = 0; c < NE; ++c) e[c] = sm[c];
         dftatom_step* rec = b.steps + (size_t)a * b.steps_stride + as.n_steps;
         const double eel = rec->Ekin;                      // parked by density_update_kernel
-        const double e_dif = kFourPi * e[2];
-        const double e_xc = kFourPi * e[1] + e_dif;
         const double e_har = -0.5 * kFourPi * e[3];
-        const double etot = eel + e_har + e_dif;
+        double e_xc, etot;
+        if constexpr (!kCore) {
+            const double e_dif = kFourPi * e[2];
+            e_xc = kFourPi * e[1] + e_dif;
+            etot = eel + e_har + e_dif;
+        } else if (pc) {
+            const double e_dif = kFourPi * e[2] + kFourPi * e[5];
+            e_xc = kFourPi * e[1] + e_dif;
+            etot = eel + e_har + e_dif;
+        } else {
+            // an atom without a core: the roundings ptxas gives the kCore = false instance above (4 pi e[2] fused into both sums), written
+            // out so that such an atom's records are bit-identical to dftatom_solve_pseudo_batch's
+            e_xc = __fma_rn(e[2], kFourPi, __dmul_rn(kFourPi, e[1]));
+            etot = __fma_rn(e[2], kFourPi, __dadd_rn(eel, e_har));
+        }
         rec->Etotal = etot; rec->Ekin = eel - e[4]; rec->Ecoul = -e_har; rec->Eenuc = e[0]; rec->Exc = e_xc;
         const int ok = rec->levels_converged;
         int done = 0, status = DFTATOM_MAX_STEPS;
@@ -719,7 +754,8 @@ __global__ void __launch_bounds__(kPT2) pseudo_potential_energy_kernel(GridDev g
 
 void launch_pseudo_potential_energy(const GridDev& g, const ScfBuffers& b, const PseudoArgs& p, int first, cudaStream_t st)
 {
-    launch_step_kernel(pseudo_potential_energy_kernel, dim3(b.n_atoms, node_chunks(g.N)), dim3(kPT2), 0, st, g, b, p, first);
+    if (p.rho_pc) launch_step_kernel(pseudo_potential_energy_kernel<true>, dim3(b.n_atoms, node_chunks(g.N)), dim3(kPT2), 0, st, g, b, p, first);
+    else launch_step_kernel(pseudo_potential_energy_kernel<false>, dim3(b.n_atoms, node_chunks(g.N)), dim3(kPT2), 0, st, g, b, p, first);
 }
 
 }  // namespace dft

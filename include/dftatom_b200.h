@@ -368,6 +368,33 @@ typedef struct { double c[7], r_c, q; int status, pad; } dftatom_tm_result;     
 int dftatom_tm_pseudize(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, int n_pot, const double* u, int n_orb,
                         const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
                         double* v_ion, double* rho_val);
+/* Nonlinear core correction (Louie, Froyen and Cohen 1982): the core density, its partial core, and the unscreening with it.
+ * Grid (levels, delta, max_r; delta = 0: uniform), rounding to the nearest node (ties to the inner one) and the index derivative with
+ * J = dr/di = delta (r + Rp) (uniform grid: J = h) are those of dftatom_tm_pseudize.
+ * u[n_orb][N] HOST all-electron orbitals.  Core entry k = core[k]: output row `row`, orbital row `orbital`, occupation occ.
+ *   rho_core[p] = sum occ u^2 / (4 pi r^2) over the entries of row p at nodes 1..N-2 (the SCF's density convention), 0 at nodes 0, N-1.
+ * Partial core of row p with radius r_pc[p] >= 0:
+ *   r_pc = 0: the full core, rho_pc = rho_core, i_pc = 0, A = B = 0.
+ *   else i_pc = the nearest node, rho = rho_core(i_pc), rho' = its 5-point index derivative / J, t = 1 + r rho' / rho at r = r_(i_pc);
+ *   x the root in (0, pi) of x cos x - t sin x = 0 (unique for t < 1: x cot x falls from 1 to -inf), found by bisection to the last
+ *   bit; B = x / r, A = rho r / sin x; rho_pc = A sin(B r_i) / r_i for 1 <= i < i_pc, rho_core for i >= i_pc, 0 at node 0 (value and
+ *   slope of rho_core at r_pc).
+ * out[p]: r_pc used (the node radius, 0 for the full core), A, B, n_core = sum wjac 4 pi r^2 rho_core, n_pc likewise of rho_pc (wjac the
+ * weights of the radial export), i_pc, status: 0 ok, 1 rho <= 0 or t >= 1 (the core density does not decrease at r_pc): A, B and
+ * rho_pc at nodes 1..N-1 NaN.  rho_core, rho_pc [n_rows][N] may be NULL.
+ * Validation before anything runs on the device (outputs untouched): a bad grid returns DFTATOM_E_BAD_OPTION; DFTATOM_E_ARG, naming the
+ * row or entry, for NULL u, r_pc or out (core with n_core > 0), n_orb or n_rows < 1, n_core < 0, r_pc not finite, negative, in (0, r_3)
+ * or above r_(N-3), an entry's row or orbital out of range, occ not finite or outside [0, 14], u not finite at nodes 1..N-1. */
+typedef struct { int row, orbital; double occ; } dftatom_core_orbital;                                     /* 16 bytes */
+typedef struct { double r_pc, A, B, n_core, n_pc; int i_pc, status, pad; } dftatom_pcc_result;           /* 56 bytes */
+int dftatom_partial_core(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* u, int n_orb, const dftatom_core_orbital* core,
+                         int n_core, const double* r_pc, int n_rows, dftatom_pcc_result* out, double* rho_core, double* rho_pc);
+/* dftatom_tm_pseudize with the core-corrected unscreening V_ion,l = V_scr,l - V_H[rho_val] - V_xc(rho_val + rho_pc): rho_pc[n_pot][N]
+ * HOST, one row per potential row (e.g. of dftatom_partial_core); V_H and rho_val stay those of the valence density.  rho_pc = NULL is
+ * dftatom_tm_pseudize.  Validation adds DFTATOM_E_ARG for a rho_pc row that is not finite or negative at nodes 1..N-1. */
+int dftatom_tm_pseudize_core(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* V, int n_pot, const double* u, int n_orb,
+                             const dftatom_tm_channel* ch, int n_channels, dftatom_tm_result* out, double* u_ps, double* v_scr,
+                             double* v_ion, double* rho_val, const double* rho_pc);
 /* Kleinman-Bylander (KB) form of semilocal pseudopotentials: one local potential plus one separable projector per other channel,
  * V_NL = |beta> E_KB <beta|, with the Gonze-Stumpf-Scheffler (GSS) ghost-state test.  Grid (levels, delta, max_r) and the "sweep rule on
  * 0..n" (Simpson 1/3 on nodes 0..m, the 3/8 rule on the last three intervals when n is odd, times dr/di) are those of
@@ -442,6 +469,18 @@ typedef struct { int row[4], n_ref[4]; double z_val, mixing; int method, pad; } 
 int dftatom_solve_pseudo_batch(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* v_ion, int n_rows,
                                const dftatom_pseudo_atom* atoms, const dftatom_config* configs, int n_atoms, dftatom_result* out,
                                dftatom_step* steps, int steps_stride, const dftatom_radial* radial);
+/* dftatom_solve_pseudo_batch with nonlinear core corrections: rho_pc[n_pc_rows][N] HOST partial core densities, pc_row[n_atoms] the row
+ * of each atom (-1 = none; pc_row = NULL: no atom has one, which is dftatom_solve_pseudo_batch).  An atom with a core uses
+ *   V_l,s = V_ion,l + U / r + V_xc,s(rho_a + rho_pc / 2, rho_b + rho_pc / 2)   (LDA: V_xc(rho + rho_pc)),
+ *   Exc = int (rho + rho_pc) eps_xc 4 pi r^2 dr,  Etotal = sum occ eps - E_H - sum_s int rho_s v_xc,s 4 pi r^2 dr + Exc;
+ * Eenuc, Ecoul and Ekin as before (at convergence Etotal = Ekin + Eenuc + Ecoul + Exc still holds); the radial export's `v` includes the
+ * core in V_xc and `rho` stays the valence density.  An atom without a core is solved exactly as by dftatom_solve_pseudo_batch.
+ * Validation adds DFTATOM_E_BAD_OPTION, naming the atom or row, for a pc_row outside -1..n_pc_rows-1 (rho_pc = NULL counts as no row)
+ * and, when some atom has a core, for a rho_pc row that is not finite or negative at nodes 1..N-1. */
+int dftatom_solve_pseudo_batch_core(dftatom_ctx* ctx, int levels, double delta, double max_r, const double* v_ion, int n_rows,
+                                    const dftatom_pseudo_atom* atoms, const dftatom_config* configs, int n_atoms, dftatom_result* out,
+                                    dftatom_step* steps, int steps_stride, const dftatom_radial* radial, const double* rho_pc,
+                                    int n_pc_rows, const int* pc_row);
 /* The node radii r[N] (HOST) of the grid (levels, delta, max_r; delta = 0: uniform) as the engine builds and uses them. */
 int dftatom_grid_nodes(dftatom_ctx* ctx, int levels, double delta, double max_r, double* r);
 /* SolvePoissonNonUniform (PoissonSolver.h:51-81) for n_dens densities rho[n_dens][N] with boundary values (0, Z[k]) (the SCF passes the
