@@ -43,6 +43,7 @@ struct GridKey {
 
 struct GridEntry {
     GridDev dev; DevBuf mem;
+    std::vector<double> r;                      // the node radii dev.r holds, as uploaded (host checks of radii round to these nodes)
     DevBuf u_unit; bool u_unit_ok = false;      // U of the SCF's start density for Z = 1 (solve_group: unit_guess), [N] doubles + one int (= 1)
 };
 
@@ -195,6 +196,7 @@ static int get_grid(dftatom_ctx* c, int L, double delta, double max_r, GridDev**
         }
     }
     GridEntry& e = c->grids[key];
+    e.r.assign(r, r + N);
     int rc = e.mem.ensure((h.size() + 32 * 32 + 3 * 1024 + (size_t)poisson_direct_table_doubles(L)) * sizeof(double));
     if (rc) { c->grids.erase(key); return rc; }
     DFT_CHECK(cudaMemcpyAsync(e.mem.p, h.data(), h.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
@@ -236,6 +238,77 @@ static int validate(const dftatom_options& o)
     if (o.method < 0 || o.method > 3) { set_error("method must be 0 (LDA), 1 (LSDA), 2 (LDA, uniform grid) or 3 (LSDA, uniform grid)"); return DFTATOM_E_BAD_OPTION; }
     if (o.method < 2 && !(o.delta > 0. && o.delta <= 1.)) { set_error("delta must be in (0,1]"); return DFTATOM_E_BAD_OPTION; }      // unused on the uniform grid
     if (!(o.mixing >= 0. && o.mixing <= 1.)) { set_error("mixing must be in [0,1]"); return DFTATOM_E_BAD_OPTION; }
+    return 0;
+}
+
+// ---- argument checks shared by the entry points ----
+
+// the message prefix "fn: what k: "
+static std::string where(const char* fn, const char* what, long long k)
+{
+    return std::string(fn) + ": " + what + " " + std::to_string(k) + ": ";
+}
+
+// the first node in 1..N-1 of row[N] that is not finite (or, with `negative`, also below 0); 0 if there is none
+static int bad_node(const double* row, int N, bool negative = false)
+{
+    for (int i = 1; i < N; ++i)
+        if (!std::isfinite(row[i]) || (negative && row[i] < 0.)) return i;
+    return 0;
+}
+
+// the node used for a radius r_2 <= r_c <= r_(N-2): the nearest one, ties to the inner one
+static int nearest_node(const std::vector<double>& r, double r_c)
+{
+    const int N = (int)r.size();
+    const int hi = (int)(std::lower_bound(r.begin() + 2, r.begin() + (N - 1), r_c) - r.begin());      // first node >= r_c, 2..N-2
+    return (hi > 2 && r_c - r[hi - 1] <= r[hi] - r_c) ? hi - 1 : hi;
+}
+
+// the node of the radius `name` = x, which must lie in [r_k, r_(N-k)] (k >= 2); -1 with the error set (prefix `at`) if it does not
+static int radius_node(const std::vector<double>& r, double x, int k, const std::string& at, const char* name)
+{
+    const int N = (int)r.size();
+    if (!(x >= r[k] && x <= r[N - k])) {
+        char b[160];
+        std::snprintf(b, sizeof b, "%s = %.17g outside [r_%d, r_(N-%d)] = [%.17g, %.17g]", name, x, k, k, r[k], r[N - k]);
+        set_error(at + b);
+        return -1;
+    }
+    return nearest_node(r, x);
+}
+
+// the bottom -Z_b^2 - 1 of the energy search's bracket on a potential with minimum vmin: the smallest Z_b in 1..118 with -Z_b^2 - 1 at
+// least `margin` below vmin; 0 if there is none
+static int bracket_z(double vmin, double margin)
+{
+    for (int z = 1; z <= 118; ++z)
+        if (-(double)z * z - 1. <= vmin - margin) return z;
+    return 0;
+}
+
+// one warp per (channel, block of eb energies), dealt longest sweep first (stable: equal costs keep channel order): the item
+// channel * eb + block of every warp
+static std::vector<int> warp_order(const std::vector<long long>& cost, int eb)
+{
+    std::vector<int> order(cost.size()), item;
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return cost[a] > cost[b]; });
+    for (int q : order)
+        for (int b = 0; b < eb; ++b) item.push_back(q * eb + b);
+    return item;
+}
+
+// the radial export of a whole batch: atom a goes to index a of the caller's arrays and its orb_rows[a] orbitals to the rows after those
+// of atoms 0..a-1; radial.orbital_rows must hold them all
+static int batch_rows(const dftatom_radial& radial, const std::vector<long long>& orb_rows, std::vector<int>& atom, std::vector<long long>& row)
+{
+    long long rows = 0;
+    for (size_t a = 0; a < orb_rows.size(); ++a) { atom.push_back((int)a); row.push_back(rows); rows += orb_rows[a]; }
+    if ((radial.orbitals || radial.moments) && radial.orbital_rows < rows) {
+        set_error("dftatom_radial.orbital_rows is " + std::to_string(radial.orbital_rows) + ", the batch has " + std::to_string(rows) + " orbitals");
+        return DFTATOM_E_ARG;
+    }
     return 0;
 }
 
@@ -555,7 +628,8 @@ static void poisson_increment(int path, const GridDev& g, const PoissonLevels& l
     }
 }
 
-// one group of atoms: its whole SCF, enqueued on the context's stream (pg: pseudo-atoms, opts[a].Z = their Z_b)
+// one group of atoms: its whole SCF, enqueued on the context's stream (pg: pseudo-atoms, opts[a].Z = their Z_b).  The callers have
+// validated every atom's options and checked that all atoms share atom 0's grid.
 static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftatom_config* cfgs, int n_atoms, dftatom_result* out,
                        dftatom_step* steps, int steps_stride, const RadialDest* rd = nullptr, const PseudoGroup* pg = nullptr)
 {
@@ -565,16 +639,6 @@ static int solve_group(dftatom_ctx* c, const dftatom_options* opts, const dftato
     const double th0 = now();
     double th1 = 0., th2 = 0., th3 = 0., th4 = 0.;
     DFT_CHECK(cudaSetDevice(c->device));
-    for (int a = 0; a < n_atoms; ++a) {
-        int rc = validate(opts[a]);
-        if (rc) return rc;
-        // methods 2 / 3 (CalculateUniformLDA / LSDA, DFTAtom.h:15,18) run on the uniform grid: delta is not used (grid key: delta = 0)
-        const bool uni_a = opts[a].method >= 2, uni_0 = opts[0].method >= 2;
-        if (opts[a].levels != opts[0].levels || uni_a != uni_0 || (!uni_a && opts[a].delta != opts[0].delta) || opts[a].max_r != opts[0].max_r) {
-            set_error("all atoms of one batch must share (levels, delta, max_r) and the kind of grid");
-            return DFTATOM_E_MIXED_GRID;
-        }
-    }
     GridDev* gp = nullptr;
     GridEntry* gentry = nullptr;
     int rc = get_grid(c, opts[0].levels, opts[0].method >= 2 ? 0. : opts[0].delta, opts[0].max_r, &gp, &gentry);
@@ -1039,44 +1103,29 @@ int dftatom_solve_batch_config(dftatom_ctx* c, const dftatom_options* opts, cons
                                dftatom_step* steps, int steps_stride, const dftatom_radial* radial)
 {
     if (!c || !opts || !out || n_atoms <= 0) { set_error("bad argument"); return DFTATOM_E_ARG; }
-    // every configuration is checked before anything is solved (solve_group checks them again per group)
-    if (configs)
-        for (int a = 0; a < n_atoms; ++a) {
-            int rc = validate(opts[a]);
-            AtomLevels al;
-            if (rc || (rc = atom_levels(a, opts[a], &configs[a], &al))) return rc;
+    // one pass over the batch before anything is solved: per atom its options, atom 0's grid, its levels (configuration) and orbital rows
+    std::vector<long long> orb_rows;
+    for (int a = 0; a < n_atoms; ++a) {
+        int rc = validate(opts[a]);
+        if (rc) return rc;
+        // methods 2 / 3 (CalculateUniformLDA / LSDA, DFTAtom.h:15,18) run on the uniform grid: delta is not used (grid key: delta = 0)
+        const bool uni_a = opts[a].method >= 2, uni_0 = opts[0].method >= 2;
+        if (opts[a].levels != opts[0].levels || uni_a != uni_0 || (!uni_a && opts[a].delta != opts[0].delta) || opts[a].max_r != opts[0].max_r) {
+            set_error("all atoms of one batch must share (levels, delta, max_r) and the kind of grid");
+            return DFTATOM_E_MIXED_GRID;
         }
-    // radial export: the first orbital row of every atom in the caller's arrays, and the capacity check before anything is solved
+        AtomLevels al;
+        if ((rc = atom_levels(a, opts[a], configs ? &configs[a] : nullptr, &al))) return rc;
+        if (radial) orb_rows.push_back((long long)(al.lev[0].size() + al.lev[1].size()));
+    }
+    // radial export: the first orbital row of every atom in the caller's arrays
     std::vector<int> dest_atom;
     std::vector<long long> dest_row;
-    if (radial) {
-        long long rows = 0;
-        for (int a = 0; a < n_atoms; ++a) {
-            int rc = validate(opts[a]);
-            if (rc) return rc;
-            AtomLevels al;
-            if ((rc = atom_levels(a, opts[a], configs ? &configs[a] : nullptr, &al))) return rc;
-            dest_atom.push_back(a);
-            dest_row.push_back(rows);
-            rows += (long long)(al.lev[0].size() + al.lev[1].size());
-        }
-        if ((radial->orbitals || radial->moments) && radial->orbital_rows < rows) {
-            set_error("dftatom_radial.orbital_rows is " + std::to_string(radial->orbital_rows) + ", the batch has " + std::to_string(rows) + " orbitals");
-            return DFTATOM_E_ARG;
-        }
-    }
+    if (radial) { int rc = batch_rows(*radial, orb_rows, dest_atom, dest_row); if (rc) return rc; }
     const RadialDest rd_all{ radial, dest_atom.data(), dest_row.data(), true };
     const RadialDest* rd = radial ? &rd_all : nullptr;
     if (c->stream_groups < 2 || n_atoms < 32) return solve_group(c, opts, configs, n_atoms, out, steps, steps_stride, rd);
     if (opts[0].levels > 14) return solve_group(c, opts, configs, n_atoms, out, steps, steps_stride, rd);      // (large grids: one group - the stream-mode Poisson solver wants all densities in one launch)
-    for (int a = 0; a < n_atoms; ++a) {
-        int rc = validate(opts[a]);
-        if (rc) return rc;
-        if (opts[a].levels != opts[0].levels || (opts[a].method >= 2) != (opts[0].method >= 2) || (opts[a].method < 2 && opts[a].delta != opts[0].delta) || opts[a].max_r != opts[0].max_r) {
-            set_error("all atoms of one batch must share (levels, delta, max_r) and the kind of grid");
-            return DFTATOM_E_MIXED_GRID;
-        }
-    }
     // G groups: this context and a chain of G - 1 child contexts (each its own stream and buffers)
     const int G = std::min(c->stream_groups, std::max(1, n_atoms / 16));
     std::vector<dftatom_ctx*> ctxs(1, c);
@@ -1156,89 +1205,76 @@ int dftatom_solve_pseudo_batch_core(dftatom_ctx* c, int levels, double delta, do
     if (!c || !v_ion || !atoms || !configs || !out) { set_error("dftatom_solve_pseudo_batch: NULL argument"); return DFTATOM_E_ARG; }
     if (n_rows < 1 || n_atoms < 1) { set_error("dftatom_solve_pseudo_batch: n_rows and n_atoms must be >= 1"); return DFTATOM_E_ARG; }
     if (delta == 0.) { set_error("dftatom_solve_pseudo_batch: the uniform grid (delta = 0) is not supported"); return DFTATOM_E_BAD_OPTION; }
-    const auto where = [](int a) { return "dftatom_solve_pseudo_batch: atom " + std::to_string(a) + ": "; };
+    static const char* const fn = "dftatom_solve_pseudo_batch";
     const int N = (1 << std::min(std::max(levels, 0), 20)) + 1;
     std::vector<dftatom_options> opts(n_atoms);
     std::vector<char> row_ok(n_rows, 0);
-    long long orb_rows = 0;
+    std::vector<long long> orb_rows;
     int rc;
     for (int a = 0; a < n_atoms; ++a) {
         const dftatom_pseudo_atom& pa = atoms[a];
-        if (pa.method != 0 && pa.method != 1) { set_error(where(a) + "method must be 0 (LDA) or 1 (LSDA)"); return DFTATOM_E_BAD_OPTION; }
+        const std::string at_a = where(fn, "atom", a);
+        if (pa.method != 0 && pa.method != 1) { set_error(at_a + "method must be 0 (LDA) or 1 (LSDA)"); return DFTATOM_E_BAD_OPTION; }
         dftatom_options& o = opts[a];
         o.Z = 1; o.levels = levels; o.max_r = max_r; o.delta = delta; o.mixing = pa.mixing; o.method = pa.method;
-        if ((rc = validate(o))) { set_error(where(a) + dftatom_last_error()); return rc; }
-        if (!(std::isfinite(pa.z_val) && pa.z_val > 0.)) { set_error(where(a) + "z_val must be finite and > 0"); return DFTATOM_E_BAD_OPTION; }
+        if ((rc = validate(o))) { set_error(at_a + dftatom_last_error()); return rc; }
+        if (!(std::isfinite(pa.z_val) && pa.z_val > 0.)) { set_error(at_a + "z_val must be finite and > 0"); return DFTATOM_E_BAD_OPTION; }
         int n_ch = 0;
         for (int l = 0; l < 4; ++l) {
             if (pa.row[l] < -1 || pa.row[l] >= n_rows) {
-                set_error(where(a) + "row[" + std::to_string(l) + "] = " + std::to_string(pa.row[l]) + " outside -1.." + std::to_string(n_rows - 1));
+                set_error(at_a + "row[" + std::to_string(l) + "] = " + std::to_string(pa.row[l]) + " outside -1.." + std::to_string(n_rows - 1));
                 return DFTATOM_E_BAD_OPTION;
             }
             if (pa.row[l] < 0) continue;
             ++n_ch;
             if (pa.n_ref[l] < l + 1 || pa.n_ref[l] > 8) {
-                set_error(where(a) + "n_ref[" + std::to_string(l) + "] = " + std::to_string(pa.n_ref[l]) + " outside " + std::to_string(l + 1) + "..8");
+                set_error(at_a + "n_ref[" + std::to_string(l) + "] = " + std::to_string(pa.n_ref[l]) + " outside " + std::to_string(l + 1) + "..8");
                 return DFTATOM_E_BAD_OPTION;
             }
         }
-        if (!n_ch) { set_error(where(a) + "no channel (every row is -1)"); return DFTATOM_E_BAD_OPTION; }
+        if (!n_ch) { set_error(at_a + "no channel (every row is -1)"); return DFTATOM_E_BAD_OPTION; }
         const dftatom_config& cf = configs[a];
-        if (cf.n_orbitals == 0) { set_error(where(a) + "empty configuration"); return DFTATOM_E_BAD_OPTION; }
+        if (cf.n_orbitals == 0) { set_error(at_a + "empty configuration"); return DFTATOM_E_BAD_OPTION; }
         AtomLevels al;
-        if ((rc = atom_levels(a, o, &cf, &al, pa.z_val))) { set_error(where(a) + dftatom_last_error()); return rc; }
+        if ((rc = atom_levels(a, o, &cf, &al, pa.z_val))) { set_error(at_a + dftatom_last_error()); return rc; }
         for (int k = 0; k < cf.n_orbitals; ++k) {
             const dftatom_occupation& x = cf.orb[k];
-            const std::string at = where(a) + "configuration entry " + std::to_string(k) + " (n = " + std::to_string(x.n) + ", l = " + std::to_string(x.l) + "): ";
+            const std::string at = at_a + "configuration entry " + std::to_string(k) + " (n = " + std::to_string(x.n) + ", l = " + std::to_string(x.l) + "): ";
             if (pa.row[x.l] < 0) { set_error(at + "l has no channel"); return DFTATOM_E_BAD_OPTION; }
             if (x.n < pa.n_ref[x.l]) { set_error(at + "n below n_ref = " + std::to_string(pa.n_ref[x.l])); return DFTATOM_E_BAD_OPTION; }
         }
-        orb_rows += cf.n_orbitals;
+        orb_rows.push_back(cf.n_orbitals);
         // the bracket of the energy search: -Z_b^2 - 1 at least 10 Ha below the deepest ionic potential of the atom
         double vmin = INFINITY;
         for (int l = 0; l < 4; ++l) {
             if (pa.row[l] < 0) continue;
             const double* v = v_ion + (size_t)pa.row[l] * N;
-            for (int i = 1; i < N; ++i) {
-                if (!row_ok[pa.row[l]] && !std::isfinite(v[i])) {
-                    set_error(where(a) + "v_ion row " + std::to_string(pa.row[l]) + " is not finite at node " + std::to_string(i));
+            if (!row_ok[pa.row[l]]) {
+                if (const int i = bad_node(v, N)) {
+                    set_error(at_a + "v_ion row " + std::to_string(pa.row[l]) + " is not finite at node " + std::to_string(i));
                     return DFTATOM_E_BAD_OPTION;
                 }
-                vmin = std::min(vmin, v[i]);
+                row_ok[pa.row[l]] = 1;
             }
-            row_ok[pa.row[l]] = 1;
+            for (int i = 1; i < N; ++i) vmin = std::min(vmin, v[i]);
         }
-        int zb = 1;
-        while (zb <= 118 && -(double)zb * zb - 1. > vmin - 10.) ++zb;
-        if (zb > 118) { set_error(where(a) + "ionic potential too deep (min V_ion = " + std::to_string(vmin) + " below -118^2 + 9)"); return DFTATOM_E_BAD_OPTION; }
-        o.Z = zb;
+        o.Z = bracket_z(vmin, 10.);
+        if (!o.Z) { set_error(at_a + "ionic potential too deep (min V_ion = " + std::to_string(vmin) + " below -118^2 + 9)"); return DFTATOM_E_BAD_OPTION; }
         if (pc_row && (pc_row[a] < -1 || pc_row[a] >= (rho_pc ? n_pc_rows : 0))) {
-            set_error(where(a) + "pc_row = " + std::to_string(pc_row[a]) + " outside -1.." + std::to_string((rho_pc ? n_pc_rows : 0) - 1));
+            set_error(at_a + "pc_row = " + std::to_string(pc_row[a]) + " outside -1.." + std::to_string((rho_pc ? n_pc_rows : 0) - 1));
             return DFTATOM_E_BAD_OPTION;
         }
     }
     bool any_core = false;
     for (int a = 0; pc_row && a < n_atoms; ++a) any_core |= pc_row[a] >= 0;
-    if (any_core) {
-        for (int q = 0; q < n_pc_rows; ++q)
-            for (int i = 1; i < N; ++i) {
-                const double x = rho_pc[(size_t)q * N + i];
-                if (!(std::isfinite(x) && x >= 0.)) {
-                    set_error("dftatom_solve_pseudo_batch: rho_pc row " + std::to_string(q) + " is not finite or negative at node " + std::to_string(i));
-                    return DFTATOM_E_BAD_OPTION;
-                }
-            }
-    }
+    for (int q = 0; any_core && q < n_pc_rows; ++q)
+        if (const int i = bad_node(rho_pc + (size_t)q * N, N, true)) {
+            set_error(where(fn, "rho_pc row", q) + "not finite or negative at node " + std::to_string(i));
+            return DFTATOM_E_BAD_OPTION;
+        }
     std::vector<int> dest_atom;
     std::vector<long long> dest_row;
-    if (radial) {
-        if ((radial->orbitals || radial->moments) && radial->orbital_rows < orb_rows) {
-            set_error("dftatom_radial.orbital_rows is " + std::to_string(radial->orbital_rows) + ", the batch has " + std::to_string(orb_rows) + " orbitals");
-            return DFTATOM_E_ARG;
-        }
-        long long rows = 0;
-        for (int a = 0; a < n_atoms; ++a) { dest_atom.push_back(a); dest_row.push_back(rows); rows += configs[a].n_orbitals; }
-    }
+    if (radial && (rc = batch_rows(*radial, orb_rows, dest_atom, dest_row))) return rc;
     const RadialDest rd{ radial, dest_atom.data(), dest_row.data(), true };
     const PseudoGroup pg{ v_ion, n_rows, atoms, any_core ? rho_pc : nullptr, any_core ? n_pc_rows : 0, pc_row };
     return solve_group(c, opts.data(), configs, n_atoms, out, steps, steps_stride, radial ? &rd : nullptr, &pg);
@@ -1339,58 +1375,37 @@ int dftatom_numerov_lanes_timed(dftatom_ctx* c, const double* V, int levels, dou
 static int poisson_cold(dftatom_ctx* c, const GridDev& g, int n_dens, const double* d_rho, const double* d_zbc, int* d_vcycles, long long* ld_out,
                         bool* streamed);
 
-// the node used for a radius r_2 <= r_c <= r_(N-2): the nearest one, ties to the inner one
-static int nearest_node(const std::vector<double>& r, double r_c)
-{
-    const int N = (int)r.size();
-    const int hi = (int)(std::lower_bound(r.begin() + 2, r.begin() + (N - 1), r_c) - r.begin());      // first node >= r_c, 2..N-2
-    return (hi > 2 && r_c - r[hi - 1] <= r[hi] - r_c) ? hi - 1 : hi;
-}
-
 int dftatom_log_derivatives(dftatom_ctx* c, int levels, double delta, double max_r, const double* V, int n_pot, const int* pot, const int* l,
                             const double* r_c, int n_channels, const double* E, int n_energies, dftatom_logderiv* out, double* r_used)
 {
     if (!c || !V || !pot || !l || !r_c || !E || !out) { set_error("dftatom_log_derivatives: NULL argument"); return DFTATOM_E_ARG; }
     if (n_pot < 1 || n_channels < 1 || n_energies < 1) { set_error("dftatom_log_derivatives: n_pot, n_channels and n_energies must be >= 1"); return DFTATOM_E_ARG; }
     DFT_CHECK(cudaSetDevice(c->device));
-    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    GridDev* gp; GridEntry* ge; int rc = get_grid(c, levels, delta, max_r, &gp, &ge); if (rc) return rc;
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
     if (N < 5) { set_error("dftatom_log_derivatives: the grid needs at least 5 nodes"); return DFTATOM_E_ARG; }
-    std::vector<double> r(N);             // the device's node radii: r_c is rounded to one of them
-    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
-    DFT_CHECK(cudaStreamSynchronize(st));
-    const auto where = [](const char* what, long long k) { return std::string("dftatom_log_derivatives: ") + what + " " + std::to_string(k) + ": "; };
+    static const char* const fn = "dftatom_log_derivatives";
+    const std::vector<double>& r = ge->r;
     std::vector<int> ic(n_channels);
     for (int k = 0; k < n_channels; ++k) {
-        if (pot[k] < 0 || pot[k] >= n_pot) { set_error(where("channel", k) + "pot = " + std::to_string(pot[k]) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
-        if (l[k] < 0 || l[k] > 3) { set_error(where("channel", k) + "l = " + std::to_string(l[k]) + " outside 0..3"); return DFTATOM_E_ARG; }
-        if (!(r_c[k] >= r[2] && r_c[k] <= r[N - 2])) {
-            char b[160];
-            std::snprintf(b, sizeof b, "r_c = %.17g outside [r_2, r_(N-2)] = [%.17g, %.17g]", r_c[k], r[2], r[N - 2]);
-            set_error(where("channel", k) + b); return DFTATOM_E_ARG;
-        }
-        ic[k] = nearest_node(r, r_c[k]);
+        const std::string at = where(fn, "channel", k);
+        if (pot[k] < 0 || pot[k] >= n_pot) { set_error(at + "pot = " + std::to_string(pot[k]) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
+        if (l[k] < 0 || l[k] > 3) { set_error(at + "l = " + std::to_string(l[k]) + " outside 0..3"); return DFTATOM_E_ARG; }
+        if ((ic[k] = radius_node(r, r_c[k], 2, at, "r_c")) < 0) return DFTATOM_E_ARG;
     }
     for (int k = 0; k < n_energies; ++k)
-        if (!std::isfinite(E[k])) { set_error(where("energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
+        if (!std::isfinite(E[k])) { set_error(where(fn, "energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
     for (int p = 0; p < n_pot; ++p)
-        for (int i = 1; i < N; ++i)
-            if (!std::isfinite(V[(size_t)p * N + i])) { set_error(where("potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
-    // one warp per (channel, block of 32 energies), dealt longest sweep first (stable: equal sweeps keep channel order)
+        if (const int i = bad_node(V + (size_t)p * N, N)) { set_error(where(fn, "potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
     const int eb = (n_energies + 31) / 32;
     const long long n_warps_ll = (long long)n_channels * eb;
     if (n_warps_ll > (1LL << 30)) { set_error("dftatom_log_derivatives: too many (channel, energy) lanes"); return DFTATOM_E_ARG; }
     const int n_warps = (int)n_warps_ll;
-    std::vector<int> chan_order(n_channels);
-    std::iota(chan_order.begin(), chan_order.end(), 0);
-    std::stable_sort(chan_order.begin(), chan_order.end(), [&](int a, int b) { return ic[a] > ic[b]; });
-    std::vector<int> h_int(3 * (size_t)n_channels + n_warps);      // pot | l | ic | warp_item
-    std::copy(pot, pot + n_channels, h_int.begin());
-    std::copy(l, l + n_channels, h_int.begin() + n_channels);
-    std::copy(ic.begin(), ic.end(), h_int.begin() + 2 * (size_t)n_channels);
-    int* wi = h_int.data() + 3 * (size_t)n_channels;
-    for (int q = 0, w = 0; q < n_channels; ++q)
-        for (int b = 0; b < eb; ++b) wi[w++] = chan_order[q] * eb + b;
+    std::vector<int> h_int(pot, pot + n_channels);                  // pot | l | ic | warp_item
+    h_int.insert(h_int.end(), l, l + n_channels);
+    h_int.insert(h_int.end(), ic.begin(), ic.end());
+    const std::vector<int> wi = warp_order(std::vector<long long>(ic.begin(), ic.end()), eb);
+    h_int.insert(h_int.end(), wi.begin(), wi.end());
     DevBuf& dV = c->scratch[0]; DevBuf& dA = c->scratch[1]; DevBuf& di = c->scratch[2]; DevBuf& dd = c->scratch[3]; DevBuf& dO = c->scratch[4];
     const size_t nV = (size_t)n_pot * N, n_out = (size_t)n_channels * n_energies;
     if ((rc = dV.ensure(sizeof(double) * nV)) || (rc = dA.ensure(sizeof(double) * nV)) || (rc = di.ensure(sizeof(int) * h_int.size())) ||
@@ -1414,9 +1429,8 @@ int dftatom_grid_nodes(dftatom_ctx* c, int levels, double delta, double max_r, d
 {
     if (!c || !r) { set_error("dftatom_grid_nodes: NULL argument"); return DFTATOM_E_ARG; }
     DFT_CHECK(cudaSetDevice(c->device));
-    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
-    DFT_CHECK(cudaMemcpyAsync(r, gp->r, sizeof(double) * gp->N, cudaMemcpyDeviceToHost, c->stream));
-    DFT_CHECK(cudaStreamSynchronize(c->stream));
+    GridDev* gp; GridEntry* ge; int rc = get_grid(c, levels, delta, max_r, &gp, &ge); if (rc) return rc;
+    std::copy(ge->r.begin(), ge->r.end(), r);
     return 0;
 }
 
@@ -1434,45 +1448,33 @@ int dftatom_tm_pseudize_core(dftatom_ctx* c, int levels, double delta, double ma
     if (!c || !V || !u || !ch || !out) { set_error("dftatom_tm_pseudize: NULL argument"); return DFTATOM_E_ARG; }
     if (n_pot < 1 || n_orb < 1 || n_channels < 1) { set_error("dftatom_tm_pseudize: n_pot, n_orb and n_channels must be >= 1"); return DFTATOM_E_ARG; }
     DFT_CHECK(cudaSetDevice(c->device));
-    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    GridDev* gp; GridEntry* ge; int rc = get_grid(c, levels, delta, max_r, &gp, &ge); if (rc) return rc;
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
     if (N < 7) { set_error("dftatom_tm_pseudize: the grid needs at least 7 nodes"); return DFTATOM_E_ARG; }
     if ((long long)n_channels + n_pot > 65535 || (long long)std::max(n_pot, n_channels) * N >= (1LL << 31)) {
         set_error("dftatom_tm_pseudize: too many channels or potential rows for one call"); return DFTATOM_E_ARG;
     }
-    std::vector<double> r(N);             // the device's node radii: r_c is rounded to one of them
-    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
-    DFT_CHECK(cudaStreamSynchronize(st));
-    const auto where = [](const char* what, long long k) { return std::string("dftatom_tm_pseudize: ") + what + " " + std::to_string(k) + ": "; };
+    static const char* const fn = "dftatom_tm_pseudize";
+    const std::vector<double>& r = ge->r;
     for (int p = 0; p < n_pot; ++p)
-        for (int i = 1; i < N; ++i)
-            if (!std::isfinite(V[(size_t)p * N + i])) { set_error(where("potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+        if (const int i = bad_node(V + (size_t)p * N, N)) { set_error(where(fn, "potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
     for (int o = 0; o < n_orb; ++o)
-        for (int i = 1; i < N; ++i)
-            if (!std::isfinite(u[(size_t)o * N + i])) { set_error(where("orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+        if (const int i = bad_node(u + (size_t)o * N, N)) { set_error(where(fn, "orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
     for (int p = 0; rho_pc && p < n_pot; ++p)
-        for (int i = 1; i < N; ++i) {
-            const double x = rho_pc[(size_t)p * N + i];
-            if (!(std::isfinite(x) && x >= 0.)) { set_error(where("rho_pc row", p) + "not finite or negative at node " + std::to_string(i)); return DFTATOM_E_ARG; }
-        }
+        if (const int i = bad_node(rho_pc + (size_t)p * N, N, true)) { set_error(where(fn, "rho_pc row", p) + "not finite or negative at node " + std::to_string(i)); return DFTATOM_E_ARG; }
     std::vector<int> ic(n_channels);
     std::vector<unsigned> l_taken(n_pot, 0u);             // per potential row: bit l set once a channel takes l
     for (int k = 0; k < n_channels; ++k) {
         const dftatom_tm_channel& q = ch[k];
-        const std::string at = where("channel", k);
+        const std::string at = where(fn, "channel", k);
         if (q.pot < 0 || q.pot >= n_pot) { set_error(at + "pot = " + std::to_string(q.pot) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
         if (q.orbital < 0 || q.orbital >= n_orb) { set_error(at + "orbital = " + std::to_string(q.orbital) + " outside 0.." + std::to_string(n_orb - 1)); return DFTATOM_E_ARG; }
         if (q.l < 0 || q.l > 3) { set_error(at + "l = " + std::to_string(q.l) + " outside 0..3"); return DFTATOM_E_ARG; }
         if (l_taken[q.pot] & (1u << q.l)) { set_error(at + "l = " + std::to_string(q.l) + " already taken by another channel of potential row " + std::to_string(q.pot)); return DFTATOM_E_ARG; }
         l_taken[q.pot] |= 1u << q.l;
-        if (!(q.r_c >= r[3] && q.r_c <= r[N - 3])) {      // i_c >= 3: the 5-point stencil of V' and V'' stays off node 0
-            char b[160];
-            std::snprintf(b, sizeof b, "r_c = %.17g outside [r_3, r_(N-3)] = [%.17g, %.17g]", q.r_c, r[3], r[N - 3]);
-            set_error(at + b); return DFTATOM_E_ARG;
-        }
+        if ((ic[k] = radius_node(r, q.r_c, 3, at, "r_c")) < 0) return DFTATOM_E_ARG;      // i_c >= 3: the 5-point stencil of V' and V'' stays off node 0
         if (!std::isfinite(q.eps)) { set_error(at + "eps is not finite"); return DFTATOM_E_ARG; }
         if (!(q.occ >= 0. && q.occ <= 2. * (2 * q.l + 1))) { set_error(at + "occ is not finite or outside [0, 2(2l+1)]"); return DFTATOM_E_ARG; }
-        ic[k] = nearest_node(r, q.r_c);
         const double* ur = u + (size_t)q.orbital * N;
         if (ur[ic[k]] == 0.) { set_error(at + "u is 0 at r_c (node " + std::to_string(ic[k]) + ")"); return DFTATOM_E_ARG; }
         const bool pos = ur[ic[k]] > 0.;
@@ -1559,37 +1561,26 @@ int dftatom_partial_core(dftatom_ctx* c, int levels, double delta, double max_r,
     if (!c || !u || !r_pc || !out || (n_core > 0 && !core)) { set_error("dftatom_partial_core: NULL argument"); return DFTATOM_E_ARG; }
     if (n_orb < 1 || n_rows < 1 || n_core < 0) { set_error("dftatom_partial_core: n_orb and n_rows must be >= 1, n_core >= 0"); return DFTATOM_E_ARG; }
     DFT_CHECK(cudaSetDevice(c->device));
-    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    GridDev* gp; GridEntry* ge; int rc = get_grid(c, levels, delta, max_r, &gp, &ge); if (rc) return rc;
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
     if (N < 7) { set_error("dftatom_partial_core: the grid needs at least 7 nodes"); return DFTATOM_E_ARG; }
     if (n_rows > 65535 || (long long)std::max(n_rows, n_orb) * N >= (1LL << 31)) { set_error("dftatom_partial_core: too many rows for one call"); return DFTATOM_E_ARG; }
-    std::vector<double> r(N);
-    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
-    DFT_CHECK(cudaStreamSynchronize(st));
-    const auto where = [](const char* what, long long k) { return std::string("dftatom_partial_core: ") + what + " " + std::to_string(k) + ": "; };
+    static const char* const fn = "dftatom_partial_core";
     std::vector<int> ipc(n_rows, 0);
-    for (int p = 0; p < n_rows; ++p) {
-        const double x = r_pc[p];
-        if (!(std::isfinite(x) && x >= 0.) || (x > 0. && x < r[3]) || x > r[N - 3]) {
-            char b[160];
-            std::snprintf(b, sizeof b, "r_pc = %.17g is neither 0 nor in [r_3, r_(N-3)] = [%.17g, %.17g]", x, r[3], r[N - 3]);
-            set_error(where("row", p) + b); return DFTATOM_E_ARG;
-        }
-        if (x > 0.) ipc[p] = nearest_node(r, x);
-    }
+    for (int p = 0; p < n_rows; ++p)       // r_pc = 0: the full core
+        if (r_pc[p] != 0. && (ipc[p] = radius_node(ge->r, r_pc[p], 3, where(fn, "row", p), "r_pc")) < 0) return DFTATOM_E_ARG;
     std::vector<int> begin(n_rows + 1, 0), orb(n_core);
     std::vector<double> occ(n_core);
     for (int k = 0; k < n_core; ++k) {
         const dftatom_core_orbital& e = core[k];
-        const std::string at = where("core entry", k);
+        const std::string at = where(fn, "core entry", k);
         if (e.row < 0 || e.row >= n_rows) { set_error(at + "row = " + std::to_string(e.row) + " outside 0.." + std::to_string(n_rows - 1)); return DFTATOM_E_ARG; }
         if (e.orbital < 0 || e.orbital >= n_orb) { set_error(at + "orbital = " + std::to_string(e.orbital) + " outside 0.." + std::to_string(n_orb - 1)); return DFTATOM_E_ARG; }
         if (!(e.occ >= 0. && e.occ <= 14.)) { set_error(at + "occ is not finite or outside [0, 14]"); return DFTATOM_E_ARG; }
         ++begin[e.row + 1];
     }
     for (int o = 0; o < n_orb; ++o)
-        for (int i = 1; i < N; ++i)
-            if (!std::isfinite(u[(size_t)o * N + i])) { set_error(where("orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+        if (const int i = bad_node(u + (size_t)o * N, N)) { set_error(where(fn, "orbital row", o) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
     for (int p = 0; p < n_rows; ++p) begin[p + 1] += begin[p];
     {
         std::vector<int> fill(begin.begin(), begin.end() - 1);
@@ -1637,12 +1628,6 @@ static int setup_rows(dftatom_ctx* c, const GridDev& g, const double* V, int n_r
     *d_atoms = c->scratch[4].as<AtomDev>(); *d_astate = c->scratch[5].as<AtomState>(); *d_orbs = c->scratch[6].as<OrbitalDev>();
     *d_ss = c->scratch[7].as<SearchState>(); *d_atab = dA.as<double>();
     return 0;
-}
-
-static int setup_single(dftatom_ctx* c, const GridDev& g, const double* V, int Z, const std::vector<OrbitalDev>& orbs,
-                        AtomDev** d_atoms, AtomState** d_astate, OrbitalDev** d_orbs, SearchState** d_ss, double** d_atab)
-{
-    return setup_rows(c, g, V, 1, &Z, orbs, d_atoms, d_astate, d_orbs, d_ss, d_atab);
 }
 
 // the production energy search of every orbital (OrbitalDev.atom = .tab = its potential row) on the rows V[n_rows][N]; E_out / converged_out
@@ -1696,19 +1681,18 @@ int dftatom_kb_form(dftatom_ctx* c, int levels, double delta, double max_r, cons
     if (n_channels > 65535 || (long long)std::max(n_rows, n_channels) * N >= (1LL << 31)) {
         set_error("dftatom_kb_form: too many channels or rows for one call"); return DFTATOM_E_ARG;
     }
-    const auto where = [](const char* what, long long k) { return std::string("dftatom_kb_form: ") + what + " " + std::to_string(k) + ": "; };
-    for (int p = 0; p < n_rows; ++p)
-        for (int i = 1; i < N; ++i) {
-            if (!std::isfinite(V[(size_t)p * N + i])) { set_error(where("row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
-            if (!std::isfinite(u[(size_t)p * N + i])) { set_error(where("row", p) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
-        }
+    static const char* const fn = "dftatom_kb_form";
+    for (int p = 0; p < n_rows; ++p) {
+        if (const int i = bad_node(V + (size_t)p * N, N)) { set_error(where(fn, "row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+        if (const int i = bad_node(u + (size_t)p * N, N)) { set_error(where(fn, "row", p) + "u is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
+    }
     // i_s per channel, the search bracket of every local row, and the (loc, l) searches of the non-local channels (each searched once)
     std::vector<int> is(n_channels, 0), zb(n_rows, 0), srow_of(n_rows, -1), search_of(n_channels, -1), srows;
     std::map<std::pair<int, int>, int> searches;
     std::vector<OrbitalDev> orbs;
     for (int k = 0; k < n_channels; ++k) {
         const dftatom_kb_channel& q = ch[k];
-        const std::string at = where("channel", k);
+        const std::string at = where(fn, "channel", k);
         if (q.row < 0 || q.row >= n_rows) { set_error(at + "row = " + std::to_string(q.row) + " outside 0.." + std::to_string(n_rows - 1)); return DFTATOM_E_ARG; }
         if (q.loc < 0 || q.loc >= n_rows) { set_error(at + "loc = " + std::to_string(q.loc) + " outside 0.." + std::to_string(n_rows - 1)); return DFTATOM_E_ARG; }
         if (q.l < 0 || q.l > 3) { set_error(at + "l = " + std::to_string(q.l) + " outside 0..3"); return DFTATOM_E_ARG; }
@@ -1720,10 +1704,7 @@ int dftatom_kb_form(dftatom_ctx* c, int levels, double delta, double max_r, cons
         if (!zb[q.loc]) {
             double vmin = b[1];
             for (int i = 2; i < N; ++i) vmin = std::min(vmin, b[i]);
-            int z = 1;
-            while (z <= 118 && -(double)z * z - 1. > vmin) ++z;
-            if (z > 118) { set_error(at + "local potential too deep (min V[loc] = " + std::to_string(vmin) + " below -118^2 - 1)"); return DFTATOM_E_ARG; }
-            zb[q.loc] = z;
+            if (!(zb[q.loc] = bracket_z(vmin, 0.))) { set_error(at + "local potential too deep (min V[loc] = " + std::to_string(vmin) + " below -118^2 - 1)"); return DFTATOM_E_ARG; }
         }
         if (srow_of[q.loc] < 0) { srow_of[q.loc] = (int)srows.size(); srows.push_back(q.loc); }
         const auto key = std::make_pair(q.loc, q.l);
@@ -1786,59 +1767,46 @@ int dftatom_kb_log_derivatives(dftatom_ctx* c, int levels, double delta, double 
         set_error("dftatom_kb_log_derivatives: n_pot, n_channels and n_energies must be >= 1, n_proj >= 0"); return DFTATOM_E_ARG;
     }
     DFT_CHECK(cudaSetDevice(c->device));
-    GridDev* gp; int rc = get_grid(c, levels, delta, max_r, &gp); if (rc) return rc;
+    GridDev* gp; GridEntry* ge; int rc = get_grid(c, levels, delta, max_r, &gp, &ge); if (rc) return rc;
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
     if (N < 5) { set_error("dftatom_kb_log_derivatives: the grid needs at least 5 nodes"); return DFTATOM_E_ARG; }
     if (n_proj > 65535) { set_error("dftatom_kb_log_derivatives: too many projectors for one call"); return DFTATOM_E_ARG; }
-    std::vector<double> r(N);
-    DFT_CHECK(cudaMemcpyAsync(r.data(), g.r, sizeof(double) * N, cudaMemcpyDeviceToHost, st));
-    DFT_CHECK(cudaStreamSynchronize(st));
-    const auto where = [](const char* what, long long k) { return std::string("dftatom_kb_log_derivatives: ") + what + " " + std::to_string(k) + ": "; };
+    static const char* const fn = "dftatom_kb_log_derivatives";
+    const std::vector<double>& r = ge->r;
     std::vector<int> ic(n_channels), is(std::max(n_proj, 1), 0);
     for (int p = 0; p < n_proj; ++p) {
         const double* b = beta + (size_t)p * N;
-        for (int i = 0; i < N; ++i) {
-            if (!std::isfinite(b[i])) { set_error(where("projector", p) + "beta is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
-            if (b[i] != 0.) is[p] = i;
-        }
-        if (is[p] > N - 3) { set_error(where("projector", p) + "beta is not 0 at node " + std::to_string(is[p]) + " > N - 3"); return DFTATOM_E_ARG; }
+        const int bad = std::isfinite(b[0]) ? bad_node(b, N) : 0;      // (beta is checked from node 0 on)
+        if (bad || !std::isfinite(b[0])) { set_error(where(fn, "projector", p) + "beta is not finite at node " + std::to_string(bad)); return DFTATOM_E_ARG; }
+        for (int i = 0; i < N; ++i) if (b[i] != 0.) is[p] = i;
+        if (is[p] > N - 3) { set_error(where(fn, "projector", p) + "beta is not 0 at node " + std::to_string(is[p]) + " > N - 3"); return DFTATOM_E_ARG; }
     }
     for (int k = 0; k < n_channels; ++k) {
         const dftatom_kb_ld_channel& q = ch[k];
-        const std::string at = where("channel", k);
+        const std::string at = where(fn, "channel", k);
         if (q.pot < 0 || q.pot >= n_pot) { set_error(at + "pot = " + std::to_string(q.pot) + " outside 0.." + std::to_string(n_pot - 1)); return DFTATOM_E_ARG; }
         if (q.proj < -1 || q.proj >= n_proj) { set_error(at + "proj = " + std::to_string(q.proj) + " outside -1.." + std::to_string(n_proj - 1)); return DFTATOM_E_ARG; }
         if (q.l < 0 || q.l > 3) { set_error(at + "l = " + std::to_string(q.l) + " outside 0..3"); return DFTATOM_E_ARG; }
         if (!std::isfinite(q.E_KB)) { set_error(at + "E_KB is not finite"); return DFTATOM_E_ARG; }
-        if (!(q.r_c >= r[2] && q.r_c <= r[N - 2])) {
-            char b[160];
-            std::snprintf(b, sizeof b, "r_c = %.17g outside [r_2, r_(N-2)] = [%.17g, %.17g]", q.r_c, r[2], r[N - 2]);
-            set_error(at + b); return DFTATOM_E_ARG;
-        }
-        ic[k] = nearest_node(r, q.r_c);
+        if ((ic[k] = radius_node(r, q.r_c, 2, at, "r_c")) < 0) return DFTATOM_E_ARG;
     }
     for (int k = 0; k < n_energies; ++k)
-        if (!std::isfinite(E[k])) { set_error(where("energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
+        if (!std::isfinite(E[k])) { set_error(where(fn, "energy", k) + "E is not finite"); return DFTATOM_E_ARG; }
     for (int p = 0; p < n_pot; ++p)
-        for (int i = 1; i < N; ++i)
-            if (!std::isfinite(V_loc[(size_t)p * N + i])) { set_error(where("potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
-    // warps dealt longest sweep first: a channel with a projector sweeps to max(i_c, i_s) + 1 and again to i_c
+        if (const int i = bad_node(V_loc + (size_t)p * N, N)) { set_error(where(fn, "potential row", p) + "V is not finite at node " + std::to_string(i)); return DFTATOM_E_ARG; }
     const int eb = (n_energies + 31) / 32;
     const long long n_warps_ll = (long long)n_channels * eb;
     if (n_warps_ll > (1LL << 30)) { set_error("dftatom_kb_log_derivatives: too many (channel, energy) lanes"); return DFTATOM_E_ARG; }
     const int n_warps = (int)n_warps_ll;
+    // a channel with a projector sweeps to max(i_c, i_s) + 1 and again to i_c
     std::vector<long long> cost(n_channels);
     for (int k = 0; k < n_channels; ++k) cost[k] = ch[k].proj < 0 ? ic[k] : (long long)std::max(ic[k], is[ch[k].proj]) + ic[k];
-    std::vector<int> chan_order(n_channels);
-    std::iota(chan_order.begin(), chan_order.end(), 0);
-    std::stable_sort(chan_order.begin(), chan_order.end(), [&](int a, int b) { return cost[a] > cost[b]; });
     const size_t nc = (size_t)n_channels, np = (size_t)std::max(n_proj, 1);
-    std::vector<int> h_int(4 * nc + np + n_warps);             // pot | l | ic | proj | is | warp_item
+    std::vector<int> h_int(4 * nc + np);                        // pot | l | ic | proj | is | warp_item
     for (size_t k = 0; k < nc; ++k) { h_int[k] = ch[k].pot; h_int[nc + k] = ch[k].l; h_int[2 * nc + k] = ic[k]; h_int[3 * nc + k] = ch[k].proj; }
     std::copy(is.begin(), is.end(), h_int.begin() + 4 * nc);
-    int* wi = h_int.data() + 4 * nc + np;
-    for (int q = 0, w = 0; q < n_channels; ++q)
-        for (int b = 0; b < eb; ++b) wi[w++] = chan_order[q] * eb + b;
+    const std::vector<int> wi = warp_order(cost, eb);
+    h_int.insert(h_int.end(), wi.begin(), wi.end());
     std::vector<double> h_dbl(E, E + n_energies);                // E | E_KB
     for (int k = 0; k < n_channels; ++k) h_dbl.push_back(ch[k].E_KB);
     const size_t nV = (size_t)n_pot * N, nP = (size_t)n_proj * N, n_out = nc * n_energies;
@@ -1872,7 +1840,8 @@ int dftatom_numerov_orbital(dftatom_ctx* c, const double* V, int levels, double 
     const GridDev g = *gp; const int N = g.N; cudaStream_t st = c->stream;
     std::vector<OrbitalDev> orbs(1); orbs[0] = OrbitalDev{ 0, 0, l, l, 1, 0, 0 };
     AtomDev* da; AtomState* ds; OrbitalDev* dorb; SearchState* dss; double* datab;
-    if ((rc = setup_single(c, g, V, 1, orbs, &da, &ds, &dorb, &dss, &datab))) return rc;
+    const int Z = 1;
+    if ((rc = setup_rows(c, g, V, 1, &Z, orbs, &da, &ds, &dorb, &dss, &datab))) return rc;
     SearchState s{}; s.E = E; s.stage = 3; s.converged = 1;
     DFT_CHECK(cudaMemcpyAsync(dss, &s, sizeof(s), cudaMemcpyHostToDevice, st));
     // single-atom ScfBuffers so that density_update's normalisation path is the one exercised

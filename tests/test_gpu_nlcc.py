@@ -2,7 +2,7 @@
 dftatom_tm_pseudize_core, Context.solve_pseudo_batch with a core / dftatom_solve_pseudo_batch_core): the partial core against the numpy
 reference of tests/nlcc_ref.py, the calls without a core against the calls of the parent entries (bit for bit), the reference
 configuration and parity of the core-corrected pseudo-atom, the transferability of Na and Cu with no core, the partial core and the full
-core, and the CLI flag --pseudo-core."""
+core, the CLI flag --pseudo-core, and the argument validation of the three entry points."""
 import ctypes as C
 import os
 import subprocess
@@ -12,8 +12,9 @@ import numpy as np
 import pytest
 
 import dftatom_b200 as D
+import logderiv_ref as LR
 import nlcc_ref as NR
-from dftatom_b200.api import _CConfig, _COccupation, _CPseudoAtom, _CResult, _CStep, _CTmChannel, _CTmResult
+from dftatom_b200.api import _CConfig, _CCoreOrbital, _COccupation, _CPccResult, _CPseudoAtom, _CResult, _CStep, _CTmChannel, _CTmResult
 
 pytestmark = pytest.mark.gpu
 
@@ -379,3 +380,133 @@ def test_cli_core_table_equals_the_python_calls(ctx):
     ps = ctx.solve_pseudo_batch(pp, [_ref_valence(pp), *tests])
     for q, row in enumerate(rows):
         assert float(row[3]) == ps[q].Etotal, (q, row)
+
+
+def test_invalid_arguments_are_rejected_before_any_launch(ctx):
+    """Every rule of the validation of dftatom_partial_core, the rho_pc rows of dftatom_tm_pseudize_core and pc_row / rho_pc of
+    dftatom_solve_pseudo_batch_core: the return code, the row, entry or atom (and node) the message names, and the outputs untouched."""
+    lib = D.load_library()
+    dp = C.POINTER(C.c_double)
+    levels, delta, max_r = 12, 0.002, 25.0
+    N, r, _, _ = LR.grid(levels, delta, max_r)
+    u = np.stack([r * r * np.exp(-r / 2), r * (1 - r / 2) * np.exp(-r / 2)])
+
+    def pc_call(u=u, n_orb=2, core=((0, 0, 2.0), (1, 1, 1.0)), n_core=None, r_pc=(0.0, 1.5), n_rows=None, null=()):
+        u = np.ascontiguousarray(u, dtype=np.float64)
+        cc = np.zeros(max(1, len(core)), dtype=np.dtype(_CCoreOrbital))
+        for k, e in enumerate(core):
+            cc[k] = e
+        rp = np.ascontiguousarray(r_pc, dtype=np.float64)
+        n_core = len(core) if n_core is None else n_core
+        n_rows = len(r_pc) if n_rows is None else n_rows
+        out = np.full(max(1, len(r_pc)), 7.0, dtype=np.dtype(_CPccResult))
+        rows = [np.full((max(1, len(r_pc)), N), 7.0) for _ in range(2)]
+        args = {"u": u.ctypes.data_as(dp), "core": cc.ctypes.data_as(C.POINTER(_CCoreOrbital)), "r_pc": rp.ctypes.data_as(dp),
+                "out": out.ctypes.data_as(C.POINTER(_CPccResult))}
+        for k in null:
+            args[k] = None
+        rc = lib.dftatom_partial_core(ctx._h, levels, delta, max_r, args["u"], n_orb, args["core"], n_core, args["r_pc"], n_rows, args["out"],
+                                      *[x.ctypes.data_as(dp) for x in rows])
+        untouched = bool(np.all(out["A"] == 7.0) and all(np.all(x == 7.0) for x in rows))
+        return rc, lib.dftatom_last_error().decode(), untouched
+
+    rc, msg, _ = pc_call()
+    assert rc == 0, msg
+    bad_u = u.copy(); bad_u[1, 9] = np.inf
+    cases = [
+        (dict(null=("u",)), "NULL"),
+        (dict(null=("r_pc",)), "NULL"),
+        (dict(null=("out",)), "NULL"),
+        (dict(null=("core",)), "NULL"),                                         # core = NULL with n_core > 0
+        (dict(n_orb=0), "n_orb"),
+        (dict(n_rows=0), "n_rows"),
+        (dict(n_core=-1), "n_core"),
+        (dict(r_pc=(0.0, np.nan)), "row 1: r_pc"),
+        (dict(r_pc=(-0.5, 1.5)), "row 0: r_pc"),
+        (dict(r_pc=(0.0, 0.5 * (r[2] + r[3]))), "row 1: r_pc"),                 # inside (0, r_3)
+        (dict(r_pc=(0.0, r[N - 3] * 1.0001)), "row 1: r_pc"),                   # above r_(N-3)
+        (dict(core=((0, 0, 2.0), (2, 1, 1.0))), "core entry 1: row"),
+        (dict(core=((-1, 0, 2.0), (1, 1, 1.0))), "core entry 0: row"),
+        (dict(core=((0, 0, 2.0), (1, 2, 1.0))), "core entry 1: orbital"),
+        (dict(core=((0, -1, 2.0), (1, 1, 1.0))), "core entry 0: orbital"),
+        (dict(core=((0, 0, -0.5), (1, 1, 1.0))), "core entry 0: occ"),
+        (dict(core=((0, 0, 2.0), (1, 1, 14.5))), "core entry 1: occ"),
+        (dict(core=((0, 0, np.nan), (1, 1, 1.0))), "core entry 0: occ"),
+        (dict(u=bad_u), "orbital row 1: u is not finite at node 9"),
+    ]
+    for kw, text in cases:
+        rc, msg, untouched = pc_call(**kw)
+        assert rc == -5, (kw, rc, msg)
+        assert text in msg, (kw, msg)
+        assert untouched, kw
+
+    # dftatom_tm_pseudize_core: a rho_pc row not finite or negative at a node >= 1
+    V = np.zeros((2, N))
+    V[:, 1:] = -1.0 / r[1:]
+    ch = np.zeros(1, dtype=np.dtype(_CTmChannel))
+    ch[0] = (0, 0, 1, 0, -0.125, 1.0, 2.0)
+
+    def tm_call(rho_pc):
+        rho_pc = np.ascontiguousarray(rho_pc, dtype=np.float64)
+        out = np.full(1, 7.0, dtype=np.dtype(_CTmResult))
+        rows = [np.full((1, N), 7.0) for _ in range(3)] + [np.full((2, N), 7.0)]
+        rc = lib.dftatom_tm_pseudize_core(ctx._h, levels, delta, max_r, V.ctypes.data_as(dp), 2, u.ctypes.data_as(dp), 2,
+                                          ch.ctypes.data_as(C.POINTER(_CTmChannel)), 1, out.ctypes.data_as(C.POINTER(_CTmResult)),
+                                          *[x.ctypes.data_as(dp) for x in rows], rho_pc.ctypes.data_as(dp))
+        untouched = bool(np.all(out["q"] == 7.0) and all(np.all(x == 7.0) for x in rows))
+        return rc, lib.dftatom_last_error().decode(), untouched
+
+    pc = np.zeros((2, N))
+    rc, msg, _ = tm_call(pc)
+    assert rc == 0, msg
+    for row, node, x in ((1, 9, np.nan), (0, 3, -1e-30), (1, N - 1, np.inf)):
+        bad = pc.copy(); bad[row, node] = x
+        rc, msg, untouched = tm_call(bad)
+        assert rc == -5 and untouched, (row, node, rc, msg)
+        assert f"rho_pc row {row}: " in msg and f"at node {node}" in msg, msg
+
+    # dftatom_solve_pseudo_batch_core: pc_row out of range, a rho_pc row not finite or negative
+    pp = pseudo(ctx, "Si", None)
+    pcr = pseudo(ctx, "Si", 0.0).rho_pc
+    n = 2
+    ca = (_CPseudoAtom * n)()
+    for a in range(n):
+        ca[a].row[:] = [-1] * 4
+        for c_, l in enumerate(pp.l.tolist()):
+            ca[a].row[l] = c_
+            ca[a].n_ref[l] = int(pp.n[c_])
+        ca[a].z_val = float(np.sum(pp.occ)); ca[a].mixing = 0.5; ca[a].method = 0
+    cc = (_CConfig * n)()
+    for a in range(n):
+        e = [(x[0], x[1], 0, x[2]) for x in D.parse_config("3s2 3p2 3d0")]
+        cc[a].n_orbitals = len(e)
+        for k, x in enumerate(e):
+            cc[a].orb[k] = _COccupation(*x)
+    VI = np.ascontiguousarray(pp.V_ion)
+
+    def ps_call(rho_pc, pc_row):
+        out = (_CResult * n)()
+        C.memset(out, 0x5A, C.sizeof(out))
+        PC = None if rho_pc is None else np.ascontiguousarray(rho_pc, dtype=np.float64)
+        PR = np.ascontiguousarray(pc_row, np.int32)
+        rc = lib.dftatom_solve_pseudo_batch_core(ctx._h, *GRID, VI.ctypes.data_as(dp), VI.shape[0], ca, cc, n, out, None, 0, None,
+                                                 None if PC is None else PC.ctypes.data_as(dp), 0 if PC is None else PC.shape[0],
+                                                 PR.ctypes.data_as(C.POINTER(C.c_int)))
+        return rc, lib.dftatom_last_error().decode(), all(b == 0x5A for b in bytes(out))
+
+    two = np.stack([pcr[0], pcr[0]])
+    assert ps_call(two, [0, 1])[0] == 0
+    nan_row = two.copy(); nan_row[1, 50] = np.nan
+    neg_row = two.copy(); neg_row[0, 4] = -1e-3
+    cases = [
+        ((two, [0, 2]), "atom 1: pc_row = 2"),
+        ((two, [-2, 1]), "atom 0: pc_row = -2"),
+        ((None, [0, -1]), "atom 0: pc_row = 0"),                                # no rho_pc: only -1 is in range
+        ((nan_row, [0, -1]), "rho_pc row 1"),                                   # every row is checked, used or not
+        ((neg_row, [-1, 1]), "rho_pc row 0"),
+    ]
+    for (rho_pc, pc_row), text in cases:
+        rc, msg, untouched = ps_call(rho_pc, pc_row)
+        assert rc == -2 and untouched, (pc_row, rc, msg)
+        assert text in msg, (pc_row, msg)
+    assert "at node 50" in ps_call(nan_row, [0, -1])[1] and "at node 4" in ps_call(neg_row, [-1, 1])[1]
